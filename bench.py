@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the CFL all-pairs compatibility-scoring hot path on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2], "Amazon dyadic co-purchase latents", SURVEY 8d C3):
 F=1024 GoogLeNet-pool5-like features, FCPCD encoder K=3 prototypes, d=64, a 1M-item catalog
@@ -40,6 +40,7 @@ PKG = os.path.join(ROOT, "compatibility-family-learning_b200")
 for _p in (ROOT, PKG):
     if _p not in sys.path:
         sys.path.insert(0, _p)
+sys.dont_write_bytecode = True     # the tree may be read-only: the benchmark writes nothing into it
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -289,6 +290,15 @@ def _ensure_library():
     return mod.build()
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes every tensor as out_dir/<name>.npy, floating point as float32 and integers (the global catalog indices)
+    as float64, which holds them exactly: the files of two builds can be compared array for array."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype.kind == "f" else np.float64))
+
+
 def run_ours(args):
     _ensure_library()
     from cfl import _native as nat
@@ -349,6 +359,7 @@ def run_ours(args):
         if len(inflight) >= INFLIGHT:
             inflight.pop(0)[2].synchronize()
         inflight.append(index.rank_async(xq_dev[i % nb], TOPK))
+        return inflight[-1][:2]
 
     out_ring = [(out_v, out_i), (torch.empty_like(out_v).pin_memory(), torch.empty_like(out_i).pin_memory())]
     pending = []
@@ -361,10 +372,13 @@ def run_ours(args):
         if len(pending) >= 2:
             pending.pop(0).synchronize()                          # the ring slot's previous result was delivered
         pending.append(index.rank_host(xq_host[i % nb], TOPK, ov, oi))
+        return ov, oi
 
     def timed(step_fn, steps, warmup, kernel_events=False):
+        # -> (ms, kernel ms per step, clocks, what the last timed step returned).  The warm-up holds a step's result
+        # across the next step as the timed loop does, so the allocator is in the same state when the timing starts.
         for i in range(warmup):
-            step_fn(i)
+            last = step_fn(i)
         barrier()
         ks, ke = [], []
         sampler = ClockSampler(local) if rank == 0 else None
@@ -377,7 +391,7 @@ def run_ours(args):
                 a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 nat.set_kernel_timer(a, b)
                 ks.append(a); ke.append(b)
-            step_fn(i)
+            last = step_fn(i)
         for ev_ in pending:
             ev_.synchronize()
         pending.clear()
@@ -394,10 +408,15 @@ def run_ours(args):
             torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
             ms = float(t.item())
         kms = [a.elapsed_time(b) for a, b in zip(ks, ke)] if kernel_events else []
-        return ms, kms, clocks
+        return ms, kms, clocks, last
 
-    ms_dev, kernel_ms, clocks = timed(step_device, args.steps, args.warmup, kernel_events=True)
-    ms_e2e, _, _ = timed(step_e2e, args.steps, args.warmup)
+    ms_dev, kernel_ms, clocks, out_dev = timed(step_device, args.steps, args.warmup, kernel_events=True)
+    ms_e2e, _, _, out_e2e = timed(step_e2e, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        # the last timed step's results of both entry points (the same query batch): device tensors from rank() and
+        # the pinned host buffers rank_host() filled
+        dump_outputs(args.dump_outputs, {"topk_dist": out_dev[0], "topk_index": out_dev[1],
+                                         "e2e_topk_dist": out_e2e[0], "e2e_topk_index": out_e2e[1]})
 
     # survivor statistics of one more (untimed) step and every rank's kernel time: stragglers / slow paths
     filt = index.rank_local_stats(xq_dev[0], TOPK)[2]
@@ -637,7 +656,14 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU arms (kernel experiments only)")
     ap.add_argument("--quick", action="store_true", help="headline line only: no C5 / small-Q side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the top-k distances and indices of the last timed step (device and host-buffer entry "
+                         "points, 2.5 MB in all) as DIR/<name>.npy; the inputs are seeded, identical from run to run")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

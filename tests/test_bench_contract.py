@@ -38,6 +38,42 @@ def test_device_arm_does_not_fall_back_to_the_cpu():
     assert r.returncode != 0 and "scores/s" not in r.stdout
 
 
+def test_bad_arguments_are_refused_before_any_work():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra],
+                           capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert r.returncode == 2 and r.stdout == "" and "error:" in r.stderr
+
+
+@pytest.mark.gpu
+def test_dumped_outputs_are_the_last_timed_step_and_repeat(tmp_path):
+    """--dump-outputs writes the top-k lists of the last timed step: 2 and 6 steps both end on query batch 1 of the
+    four the benchmark cycles through, so two runs must write the same arrays; the device entry point and the
+    host-buffer one must agree."""
+    import numpy as np
+
+    def run(steps):
+        out = tmp_path / f"s{steps}"
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--quick", "--no-cpu-baseline",
+                            "--steps", str(steps), "--warmup", "3", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == steps
+        return {f.stem: np.load(f) for f in out.iterdir()}
+
+    a, b = run(2), run(6)
+    assert sorted(a) == ["e2e_topk_dist", "e2e_topk_index", "topk_dist", "topk_index"]
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    for name, v in a.items():
+        assert v.shape == (1024, 100) and v.dtype == (np.float32 if name.endswith("dist") else np.float64)
+        np.testing.assert_array_equal(v, b[name], err_msg=name)
+    np.testing.assert_array_equal(a["topk_dist"], a["e2e_topk_dist"])
+    np.testing.assert_array_equal(a["topk_index"], a["e2e_topk_index"])
+    idx = a["topk_index"]
+    assert (idx == np.round(idx)).all() and idx.min() >= 0 and idx.max() < 1_000_000
+    assert (np.diff(a["topk_dist"], axis=1) >= 0).all()
+
+
 def test_smoke_tie_check_accepts_fp32_ties_and_rejects_real_differences():
     """The index-set check of __graft_entry__.smoke(): a swap inside an fp32 tie at the k-th distance passes
     (and leaves smoke()'s helpers callable), a swap with a clearly worse candidate fails."""
