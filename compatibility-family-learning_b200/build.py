@@ -20,7 +20,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIBDIR = os.path.join(HERE, "cfl", "_lib")
 LIB = os.path.join(LIBDIR, "libcfl_b200.so")
-SOURCES = ["api.cu", "pair.cu", "project.cu", "project_umma.cu", "project_bwd_umma.cu", "score.cu", "score_umma.cu", "score_lb.cu", "score_monomer.cu", "score_monomer_tc.cu", "rank_counts.cu", "rank_counts_tc.cu", "auc.cu"]
+SOURCES = ["api.cu", "pair.cu", "project.cu", "project_umma.cu", "project_bwd_umma.cu", "score.cu", "score_umma.cu", "score_lb.cu", "score_monomer.cu", "score_monomer_tc.cu", "rank_counts.cu", "rank_counts_tc.cu", "within.cu", "auc.cu"]
 EXTRA = os.environ.get("CFL_NVCC_EXTRA", "").split()
 NVCC_FLAGS = EXTRA + ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v", "-I", os.path.join(ROOT, "include"), "-I", CSRC]

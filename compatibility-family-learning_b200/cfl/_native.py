@@ -74,6 +74,11 @@ SIGNATURES = {
     "cfl_rank_counts_packed": (_int, [_int, _vp, _i64, _int, _int, _i64, _vp, _vp, _i64, _i64, _vp, _vp, _int,
                                       _vp, _vp, _sz, _vp]),
     "cfl_rank_counts_packed_stats": (_int, [_i64, _int, _int, _i64, _vp, _sz, _vp, _vp]),
+    "cfl_score_within_workspace_bytes": (_sz, [_int, _i64, _int, _int, _i64]),
+    "cfl_score_within": (_int, [_int, _vp, _i64, _int, _int, _i64, _vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp, _i64,
+                                _vp, _vp, _vp, _sz, _vp]),
+    "cfl_score_within_stats": (_int, [_vp, _sz, _vp, _vp]),
+    "cfl_within_merge": (_int, [_vp, _vp, _vp, _i64, _int, _i64, _vp, _vp, _vp, _vp]),
     "cfl_auc_workspace_bytes": (_sz, [_i64, _i64]),
     "cfl_auc": (_int, [_vp, _i64, _vp, _i64, _vp, _vp, _sz, _vp]),
     "cfl_adam_step": (_int, [_vp, _vp, _vp, _vp, _i64, _int, _f32, _f32, _f32, _f32, _f32, _vp]),
@@ -532,6 +537,92 @@ def dense_rank_counts(dense, pos_dist):
     _check(lib().cfl_dense_rank_counts(_ptr(dense), Q, N, ldn, _ptr(pos_dist), J, _ptr(out), _stream()),
            "cfl_dense_rank_counts")
     return out
+
+
+WITHIN_MAX_RESULTS = 1 << 28          # rows of one range query result: 3 GB of int64 index + fp32 distance
+WITHIN_STAT_NAMES = ("records", "worst_ratio", "beyond_half_band", "reemitted_queries", "count_mismatch_queries")
+
+
+def within_radius(radius, Q, device):
+    """A scalar or a [Q] radius -> contiguous float32 [Q] on ``device``."""
+    r = torch.as_tensor(radius, dtype=torch.float32, device=device)
+    if r.dim() == 0:
+        r = r.expand(Q)
+    if tuple(r.shape) != (Q,):
+        raise CflNativeError(f"radius must be a scalar or [{Q}], got {tuple(r.shape)}")
+    return r.contiguous()
+
+
+def within_counts(mode, query, catalog, radius, w=None, image=None, mu=None):
+    """Result size of every query of ``score_within``: #{c : dist(q, c) < radius[q]} -> int64 [Q] (device).  The
+    counting pass of ``rank_counts_packed`` (image given, pcd) or ``rank_counts`` with J = 1."""
+    if image is not None and catalog.shape[0] > 0:
+        c = rank_counts_packed(query, catalog, image, mu, radius[:, None])
+    else:
+        c = rank_counts(mode, query, catalog, radius[:, None], w=w)
+    return c[:, 0, 0]
+
+
+def score_within(mode, query, catalog, radius, w=None, image=None, mu=None, idx_base=0,
+                 max_results=WITHIN_MAX_RESULTS, want_stats=False, counts=None):
+    """Every catalog row closer than the radius: ``{c : dist(q, c) < radius[q]}`` (strict), exact, as CSR lists
+    ``(offsets [Q+1] int64, index [T] int64 = idx_base + row, dist [T] float32)`` ordered by (distance, index) within
+    each query.  The distances are the direct-form values of ``pair_dist_rows``, bit for bit; NaN selects nothing.
+
+    ``radius``: a scalar or [Q].  Operands as ``rank_counts``.  ``image`` (= ``catalog_pack(catalog, K, mu)``, pcd)
+    emits the rows from the tensor-core scoring epilogue; without it (monomer, shapes without a tcgen05 tiling) the
+    CUDA cores evaluate every pair in the direct form.  ``counts`` = ``within_counts`` of the same call when the caller
+    has them already.
+
+    The result size is data-dependent, so the call reads T = offsets[Q] back to the host once to size the outputs
+    (it waits for the counting pass).  T > ``max_results`` raises CflNativeError before the outputs are allocated.
+    want_stats: also a dict of the call's counters (WITHIN_STAT_NAMES; ``count_mismatch_queries`` must be 0)."""
+    q2, Q, K, d, ldq, w, E2, N, lde = _rank_operands(mode, query, catalog, w)
+    dev = E2.device
+    r = within_radius(radius, Q, dev)
+    mu = None if mu is None else _f32c(mu, "mu").contiguous()
+    if N == 0:
+        image = None
+    if counts is None:
+        counts = within_counts(mode, query, catalog, r, w=w, image=image, mu=mu)
+    offsets = torch.zeros(Q + 1, dtype=torch.int64, device=dev)
+    torch.cumsum(counts, 0, out=offsets[1:])
+    T = int(offsets[-1])
+    if T > max_results:
+        raise CflNativeError(f"score_within: the result has {T} rows, more than max_results = {max_results}")
+    out_idx = torch.empty(T, dtype=torch.int64, device=dev)
+    out_dist = torch.empty(T, dtype=torch.float32, device=dev)
+    tot = dict.fromkeys(WITHIN_STAT_NAMES, 0)
+    if T == 0:                                                 # nothing to emit (empty outputs have no storage)
+        return (offsets, out_idx, out_dist, tot) if want_stats else (offsets, out_idx, out_dist)
+    chunk = 65536                                              # one call holds at most 4096 scoring CTAs
+    for lo in range(0, Q, chunk):
+        hi = min(Q, lo + chunk)
+        ws = _ws.get(lib().cfl_score_within_workspace_bytes(MODES[mode], hi - lo, K, d, N), dev)
+        _check(lib().cfl_score_within(MODES[mode], _ptr(q2[lo:hi]), hi - lo, K, d, ldq,
+                                      None if w is None else _ptr(w[lo:hi]), _ptr(E2), _ptr(image), N, lde, _ptr(mu),
+                                      _ptr(r[lo:hi]), _ptr(offsets[lo:hi + 1]), int(idx_base), _ptr(out_idx),
+                                      _ptr(out_dist), _ptr(ws), ws.numel(), _stream()), "cfl_score_within")
+        if want_stats and hi > lo:
+            raw = (C.c_int64 * 5)()
+            _check(lib().cfl_score_within_stats(_ptr(ws), ws.numel(), raw, _stream()), "cfl_score_within_stats")
+            for i, n in enumerate(WITHIN_STAT_NAMES):
+                tot[n] = max(tot[n], raw[i] / 1048576.0) if n == "worst_ratio" else tot[n] + int(raw[i])
+    return (offsets, out_idx, out_dist, tot) if want_stats else (offsets, out_idx, out_dist)
+
+
+def within_merge(offsets, idx, dist, out_offsets):
+    """Sharded range-query result: rank r's CSR lists (global indices) in row r of ``idx`` / ``dist`` [R, ld] with
+    ``offsets`` [R, Q+1] -> the merged (index [T], dist [T]) under ``out_offsets`` [Q+1], ordered by (distance, index)."""
+    R, Q1 = offsets.shape
+    ld = idx.shape[1]
+    T = int(out_offsets[-1])
+    out_idx = torch.empty(T, dtype=torch.int64, device=idx.device)
+    out_dist = torch.empty(T, dtype=torch.float32, device=idx.device)
+    _check(lib().cfl_within_merge(_ptr(offsets.contiguous()), _ptr(idx.contiguous()), _ptr(_f32c(dist, "dist").contiguous()),
+                                  ld, R, Q1 - 1, _ptr(out_offsets.contiguous()), _ptr(out_idx), _ptr(out_dist), _stream()),
+           "cfl_within_merge")
+    return out_idx, out_dist
 
 
 def auc_counts(pos_scores, neg_scores):

@@ -14,6 +14,7 @@ from dataclasses import dataclass
 from types import SimpleNamespace
 from typing import Optional
 
+import numpy as np
 import torch
 
 from . import _native as nat
@@ -225,9 +226,71 @@ class CatalogIndex:
         return _auc_per_query("pcd", Pq, self.E, None, pos_idx, self.idx_base, self.n_total, self.group, self._world(),
                               packed=packed)
 
+    def within(self, xq: torch.Tensor, radius, max_results: int = nat.WITHIN_MAX_RESULTS):
+        """Every catalog row closer than ``radius`` (a scalar or one per query): ``{c : dist(q, c) < r_q}``, exact.
+        -> CSR lists (offsets [Q+1] int64, index [T] int64 global, dist [T] float32), each query's rows ordered by
+        (distance, index); the distances are the direct-form values of ``pair_dist_rows``.  The rows are emitted from
+        the tensor-core scoring epilogue (near-ties checked in the direct form), on the CUDA cores for shapes without
+        a tcgen05 tiling.  Sharded: every rank lists its shard, the lists are all-gathered and merged (the result does
+        not depend on the rank count).  One device->host read of the result size per call; more than ``max_results``
+        rows raise CflNativeError before anything is allocated for them."""
+        Pq = self.project_queries(xq)
+        return _within("pcd", Pq, self.E, None, radius, self.idx_base, self.group, self._world(), max_results,
+                       image=self.image, mu=self.mu)
+
+    def compatible(self, xq: torch.Tensor, max_results: int = nat.WITHIN_MAX_RESULTS):
+        """The rows the model calls compatible with each query: Thresholder score max(theta, 1e-6) - dist > 0
+        (blocks.py:21-22; the accuracy counts of cfl/utils.py:247,264), i.e. ``within`` at r = max(theta, 1e-6)."""
+        return self.within(xq, compatible_radius(self.theta), max_results=max_results)
+
     def scores(self, dist: torch.Tensor) -> torch.Tensor:
         """Thresholder (blocks.py:21-22): max(theta, 1e-6) - dist."""
         return max(self.theta, 1e-6) - dist
+
+
+def compatible_radius(theta: float) -> float:
+    """r with (score > 0  <=>  dist < r) for fp32 distances: max(float32(theta), float32(1e-6))."""
+    return float(max(np.float32(theta), np.float32(1e-6)))
+
+
+def _within(mode, query, catalog, gate, radius, idx_base, group, world, max_results, image=None, mu=None):
+    """Range query over this shard, then (sharded) the exchange: per-query counts first (all-gather, so the size guard
+    sees the whole result before anything is emitted), then every rank's lists padded to the longest one, one
+    all-gather each for indices and distances, and the merge kernel."""
+    Q = query.shape[0]
+    r = nat.within_radius(radius, Q, catalog.device)
+    if catalog.shape[0] == 0:
+        image = None
+    counts = nat.within_counts(mode, query, catalog, r, w=gate, image=image, mu=mu)
+    if world == 1:
+        return nat.score_within(mode, query, catalog, r, w=gate, image=image, mu=mu, idx_base=idx_base,
+                                max_results=max_results, counts=counts)
+    cnt = torch.empty(world * Q, dtype=torch.int64, device=counts.device)
+    torch.distributed.all_gather_into_tensor(cnt, counts.contiguous(), group=group)
+    cnt = cnt.view(world, Q)
+    per_rank = cnt.sum(1).cpu()
+    if int(per_rank.sum()) > max_results:
+        raise nat.CflNativeError(f"within: the result has {int(per_rank.sum())} rows, more than max_results = "
+                                 f"{max_results}")
+    off, idx, dist = nat.score_within(mode, query, catalog, r, w=gate, image=image, mu=mu, idx_base=idx_base,
+                                      max_results=max_results, counts=counts)
+    offs = torch.zeros(world, Q + 1, dtype=torch.int64, device=cnt.device)
+    offs[:, 1:] = torch.cumsum(cnt, 1)
+    out_off = torch.zeros(Q + 1, dtype=torch.int64, device=cnt.device)
+    out_off[1:] = torch.cumsum(cnt.sum(0), 0)
+    ld = int(per_rank.max())
+    if ld == 0:
+        return out_off, idx, dist
+    pi = torch.zeros(ld, dtype=torch.int64, device=idx.device)
+    pd = torch.zeros(ld, dtype=torch.float32, device=idx.device)
+    pi[:idx.shape[0]] = idx
+    pd[:dist.shape[0]] = dist
+    gi = torch.empty(world * ld, dtype=torch.int64, device=idx.device)
+    gd = torch.empty(world * ld, dtype=torch.float32, device=idx.device)
+    torch.distributed.all_gather_into_tensor(gi, pi, group=group)
+    torch.distributed.all_gather_into_tensor(gd, pd, group=group)
+    mi, md = nat.within_merge(offs, gi.view(world, ld), gd.view(world, ld), out_off)
+    return out_off, mi, md
 
 
 def auc_from_rank_counts(counts: torch.Tensor, pos_dist: torch.Tensor, n_total: int):
@@ -396,6 +459,15 @@ class MonomerCatalogIndex:
         a, gate = self.project_queries(xq)
         return _auc_per_query("monomer", a, self.P, gate, pos_idx, self.idx_base, self.n_total, self.group,
                               self._world())
+
+    def within(self, xq: torch.Tensor, radius, max_results: int = nat.WITHIN_MAX_RESULTS):
+        """As ``CatalogIndex.within`` with the monomer distance (direct form on the CUDA cores)."""
+        a, gate = self.project_queries(xq)
+        return _within("monomer", a, self.P, gate, radius, self.idx_base, self.group, self._world(), max_results)
+
+    def compatible(self, xq: torch.Tensor, max_results: int = nat.WITHIN_MAX_RESULTS):
+        """As ``CatalogIndex.compatible``: ``within`` at the Thresholder radius max(theta, 1e-6)."""
+        return self.within(xq, compatible_radius(self.theta), max_results=max_results)
 
     def scores(self, dist: torch.Tensor) -> torch.Tensor:
         return max(self.theta, 1e-6) - dist

@@ -34,6 +34,12 @@ struct RcArgs {
   int parts;
   int64_t tiles;
 };
+// emitting variant (cfl_score_within, J = 1): rows dist < thr[q] appended to out[offsets[q], offsets[q + 1])
+struct RcEmit {
+  const int64_t* offsets;
+  unsigned int* cursor;
+  int64_t* out;
+};
 
 // Four queries per pass through a catalog row: every shared-memory load of the row serves four distance
 // evaluations and the query operands arrive as one 128-bit broadcast load (the first version issued two
@@ -116,9 +122,10 @@ __device__ __forceinline__ void monomer_direct4(const float* __restrict__ er, co
 }
 
 // VW = floats per staging load (4 when the row length, the row stride and the base pointer allow 128-bit loads).
-template <int K, bool MONO, int VW>
-__global__ void __launch_bounds__(RC_THREADS)
-rank_count_kernel(RcArgs A) {
+// EMIT: instead of counting, the rows closer than the (single) threshold are appended to their query's segment -- one
+// ballot and one cursor atomic per (warp, query); with `only`, for the flagged queries alone.
+template <int K, bool MONO, int VW, bool EMIT>
+__device__ __forceinline__ void rank_count_body(const RcArgs& A, const RcEmit& X) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int d = A.d, J = A.J;
   const int ew = MONO ? K * d : d;            // floats per catalog row
@@ -134,10 +141,15 @@ rank_count_kernel(RcArgs A) {
   const int part = blockIdx.x;
   const int64_t q0 = (int64_t)blockIdx.y * RC_QT;
   const int nq = (int)((A.Q - q0 < RC_QT) ? (A.Q - q0) : RC_QT);
+  unsigned emit_mask = 0xffffffffu;
   if (A.only != nullptr) {                                   // restricted recount: leave unless a query here is flagged
     int flagged = 0;
     for (int ql = 0; ql < nq; ++ql) flagged |= A.only[q0 + ql];
     if (!flagged) return;
+    if constexpr (EMIT) {
+      emit_mask = 0u;
+      for (int ql = 0; ql < nq; ++ql) emit_mask |= (A.only[q0 + ql] != 0 ? 1u : 0u) << ql;
+    }
   }
   for (int i = tid; i < RC_QT * qw; i += RC_THREADS) {
     const int ql = i / qw, e = i % qw;
@@ -179,6 +191,21 @@ rank_count_kernel(RcArgs A) {
       for (int c = 0; c < 4; ++c) {
         const int ql = qh * 4 + c;
         if (ql < nq) {                                         // warp-uniform
+          if constexpr (EMIT) {
+            const bool mine = valid && dist[c] < thr[ql];
+            const unsigned lt = __ballot_sync(0xffffffffu, mine);
+            if (lt != 0u && ((emit_mask >> ql) & 1u)) {        // warp-uniform
+              const int64_t q = q0 + ql;
+              unsigned int basei = 0;
+              if (lane == 0) basei = atomicAdd(X.cursor + q, (unsigned int)__popc(lt));
+              basei = __shfl_sync(0xffffffffu, basei, 0);
+              if (mine) {
+                const int64_t at = (int64_t)basei + __popc(lt & ((1u << lane) - 1u));
+                const int64_t o = X.offsets[q];
+                if (at < X.offsets[q + 1] - o) X.out[o + at] = r0 + tid;   // beyond the count: reported at the finish
+              }
+            }
+          } else {
           for (int j = 0; j < J; ++j) {
             const float t = thr[ql * J + j];
             const unsigned lt = __ballot_sync(0xffffffffu, valid && dist[c] < t);
@@ -188,10 +215,12 @@ rank_count_kernel(RcArgs A) {
               mycnt[(ql * J + j) * 2 + 1] += __popc(eq);
             }
           }
+          }
         }
       }
     }
   }
+  if constexpr (EMIT) return;
   __syncthreads();
   for (int i = tid; i < nq * J * 2; i += RC_THREADS) {
     unsigned long long s = 0;
@@ -199,6 +228,18 @@ rank_count_kernel(RcArgs A) {
     if (A.only != nullptr && !A.only[q0 + i / (J * 2)]) continue;
     if (s) atomicAdd(&A.counts[q0 * J * 2 + i], s);
   }
+}
+
+template <int K, bool MONO, int VW>
+__global__ void __launch_bounds__(RC_THREADS)
+rank_count_kernel(RcArgs A) {
+  rank_count_body<K, MONO, VW, false>(A, RcEmit{});
+}
+
+template <int K, bool MONO, int VW>
+__global__ void __launch_bounds__(RC_THREADS)
+within_emit_kernel(RcArgs A, RcEmit X) {
+  rank_count_body<K, MONO, VW, true>(A, X);
 }
 
 // One thread per (query, positive): the same device functions on rows gathered from global memory.
@@ -270,7 +311,7 @@ static size_t rc_smem_bytes(int K, int d, int J, bool mono) {
 }
 
 template <int K, bool MONO>
-static int rc_launch(const RcArgs& a, bool gather, cudaStream_t cs) {
+static int rc_launch(const RcArgs& a, bool gather, const RcEmit* emit, cudaStream_t cs) {
   if (gather) {
     const int64_t n = a.Q * a.J;
     pair_dist_rows_kernel<K, MONO><<<(unsigned)((n + 127) / 128), 128, 0, cs>>>(a);
@@ -279,11 +320,17 @@ static int rc_launch(const RcArgs& a, bool gather, cudaStream_t cs) {
     const int ew = MONO ? K * a.d : a.d;
     const bool v4 = ew % 4 == 0 && a.lde % 4 == 0 && ((uintptr_t)a.E & 15u) == 0;
     auto kern = v4 ? rank_count_kernel<K, MONO, 4> : rank_count_kernel<K, MONO, 1>;
-    CFL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    auto ekern = v4 ? within_emit_kernel<K, MONO, 4> : within_emit_kernel<K, MONO, 1>;
     // one wave: as many catalog parts as keep every CTA resident at once (only resident warps hide the
     // shared-memory latency; a partial second wave idles most SMs)
     int resident = 0;
-    CFL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, RC_THREADS, smem));
+    if (emit) {
+      CFL_CUDA(cudaFuncSetAttribute(ekern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      CFL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, ekern, RC_THREADS, smem));
+    } else {
+      CFL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      CFL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, RC_THREADS, smem));
+    }
     if (resident < 1) resident = 1;
     int sms = sm_count();
     if (sms <= 0) sms = 148;
@@ -294,15 +341,17 @@ static int rc_launch(const RcArgs& a, bool gather, cudaStream_t cs) {
     RcArgs b = a;
     b.parts = (int)parts;
     dim3 grid((unsigned)parts, (unsigned)nqt);
-    kern<<<grid, RC_THREADS, smem, cs>>>(b);
+    if (emit) ekern<<<grid, RC_THREADS, smem, cs>>>(b, *emit);
+    else kern<<<grid, RC_THREADS, smem, cs>>>(b);
   }
   CFL_LAUNCH_CHECK();
   return CFL_OK;
 }
 
-static int rc_dispatch(const RcArgs& a, bool gather, cudaStream_t cs) {
+static int rc_dispatch(const RcArgs& a, bool gather, cudaStream_t cs, const RcEmit* emit = nullptr) {
   const bool mono = a.mode == CFL_MONOMER;
-#define CFL_RC_CASE(KK) case KK: return mono ? rc_launch<KK, true>(a, gather, cs) : rc_launch<KK, false>(a, gather, cs);
+#define CFL_RC_CASE(KK) \
+  case KK: return mono ? rc_launch<KK, true>(a, gather, emit, cs) : rc_launch<KK, false>(a, gather, emit, cs);
   switch (a.K) {
     CFL_RC_CASE(1) CFL_RC_CASE(2) CFL_RC_CASE(3) CFL_RC_CASE(4)
     CFL_RC_CASE(5) CFL_RC_CASE(6) CFL_RC_CASE(7) CFL_RC_CASE(8)
@@ -339,6 +388,18 @@ int rank_counts_only_launch(int mode, const float* Pq, int64_t Q, int K, int d, 
   a.tiles = (N + 127) / 128;
   a.parts = 1;
   return rc_dispatch(a, false, st);
+}
+
+int within_emit_launch(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* Wq, const float* E,
+                       int64_t N, int64_t lde, const float* radius, const int64_t* offsets, unsigned int* cursor,
+                       int64_t* out, const int* only, cudaStream_t st) {
+  RcArgs a = {};
+  a.mode = mode; a.K = K; a.d = d; a.J = 1; a.Q = Q; a.N = N; a.ldq = ldq; a.lde = lde;
+  a.Pq = Pq; a.Wq = Wq; a.E = E; a.thr = radius; a.only = only;
+  a.tiles = (N + 127) / 128;
+  a.parts = 1;
+  const RcEmit x = {offsets, cursor, out};
+  return rc_dispatch(a, false, st, &x);
 }
 
 }  // namespace cfl

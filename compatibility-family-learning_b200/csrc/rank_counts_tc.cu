@@ -64,6 +64,10 @@ struct RtArgs {
   unsigned int* rec_n;            // [CTAs] records written per slice
   int* only;                      // [Q]: 1 = records dropped, recount this query from scratch
   float rel1, rel2;
+  // emitting pass only
+  const int64_t* offsets;         // [Q + 1]: segment of query q = out[offsets[q], offsets[q + 1])
+  unsigned int* cursor;           // [Q]: rows appended so far
+  int64_t* out;                   // local catalog rows
 };
 
 struct RtLayout { uint32_t b_img, a_ring, qpar, qpl, thr, qm, skp, cs, rcn, bars, tmem_slot, total; };
@@ -99,9 +103,12 @@ __device__ __forceinline__ float sqrt_approx(float x) {
   return y;
 }
 
-template <int K>
-__global__ void __launch_bounds__(RT_THREADS, 1)     // 18 warps = 5 on one sub-partition: 5 x 32 x 96 registers is its whole file
-rank_count_umma_kernel(RtArgs A) {
+// The scoring skeleton and the classifying epilogue, shared by the counting kernel (EMIT = false: packed counters, J
+// thresholds) and the emitting kernel of cfl_score_within (EMIT = true, J = 1: a pair with D~ < t - m is appended to its
+// query's result segment at once, a pair inside the band goes to the record list exactly as for the counts).  Both
+// instantiations classify with the same arithmetic, so the emitted set and the count of the same radius agree pair for pair.
+template <int K, bool EMIT>
+__device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
   extern __shared__ __align__(1024) unsigned char smem[];
   constexpr int GQ = K <= 2 ? 16 : (K <= 4 ? 8 : 4);     // queries per epilogue group
   constexpr int NGW = K <= 2 ? 1 : (K <= 4 ? 2 : 3);     // query groups per warp: ceil((qt / GQ) / RT_WPQ), qt <= 64 (48 at K = 5)
@@ -359,7 +366,7 @@ rank_count_umma_kernel(RtArgs A) {
           for (int k = 0; k < K; ++k) { gA[k] = gk[k][2 * pi]; gB[k] = gk[k][2 * pi + 1]; }
           softmin_pair_var<K>(gA, gB, e2, qv, dist[2 * pi], dist[2 * pi + 1], var[2 * pi], var[2 * pi + 1]);
         }
-        uint32_t amb = 0u;
+        uint32_t amb = 0u, sure = 0u;
 #pragma unroll
         for (int i = 0; i < GQ; ++i) {
           const int ql = g * GQ + i;
@@ -374,15 +381,43 @@ rank_count_umma_kernel(RtArgs A) {
           const ulonglong2 tb = *(const ulonglong2*)(thr + ql * RT_JC + 4);
           const f2_t tp[RT_JC / 2] = {ta.x, ta.y, tb.x, tb.y};
           float near = INF;
-#pragma unroll
-          for (int jp = 0; jp < RT_JC / 2; ++jp) {
+          if constexpr (EMIT) {                               // one radius in slot 0; slot 1 is padding (-inf)
             float x, y;
-            upk2(add2(tp[jp], nd), x, y);                     // t_j - D~ for two thresholds
+            upk2(add2(tp[0], nd), x, y);
             near = fminf(fminf(fabsf(x), fabsf(y)), near);
-            count_pos(c[gi][i], x, 1u << (8 * jp));
-            count_pos(c[gi][i], y, 1u << (8 * jp + 4));
+            if (x > m) sure |= 1u << i;                       // closer than t - m: inside whatever the direct form says
+          } else {
+#pragma unroll
+            for (int jp = 0; jp < RT_JC / 2; ++jp) {
+              float x, y;
+              upk2(add2(tp[jp], nd), x, y);                   // t_j - D~ for two thresholds
+              near = fminf(fminf(fabsf(x), fabsf(y)), near);
+              count_pos(c[gi][i], x, 1u << (8 * jp));
+              count_pos(c[gi][i], y, 1u << (8 * jp + 4));
+            }
           }
           if (!(near > m)) amb |= 1u << i;                    // some threshold inside the band (or NaN)
+        }
+        if constexpr (EMIT) {
+          // sure pairs straight to the query's segment: one ballot and one cursor atomic per (warp, query)
+          if (__any_sync(0xffffffffu, sure != 0u)) {
+#pragma unroll
+            for (int i = 0; i < GQ; ++i) {
+              const bool mine = (sure >> i) & 1u;
+              const uint32_t mk = __ballot_sync(0xffffffffu, mine);
+              if (mk == 0u) continue;                         // warp-uniform
+              const int64_t q = q0 + g * GQ + i;
+              const int leader = __ffs(mk) - 1;
+              unsigned int basei = 0;
+              if (lane == leader) basei = atomicAdd(A.cursor + q, (unsigned int)__popc(mk));
+              basei = __shfl_sync(0xffffffffu, basei, leader);
+              if (mine) {
+                const int64_t at = (int64_t)basei + __popc(mk & lane_lt);
+                const int64_t o = A.offsets[q];
+                if (at < A.offsets[q + 1] - o) A.out[o + at] = row;     // beyond the count: reported by the finish kernel
+              }
+            }
+          }
         }
         if (__any_sync(0xffffffffu, amb != 0u)) {
 #pragma unroll
@@ -409,13 +444,17 @@ rank_count_umma_kernel(RtArgs A) {
       if (t == 15 && grp_skipped * 2 < grp_seen) bound_on = false;
       tc_fence_before();
       mbar_arrive(&tempty[buf]);
-      if (++since_flush == 15) { flush(); since_flush = 0; }
+      if constexpr (!EMIT) {
+        if (++since_flush == 15) { flush(); since_flush = 0; }
+      }
     }
-    flush();
+    if constexpr (!EMIT) flush();
     asm volatile("bar.sync 1, %0;" ::"n"(RT_EPI_THREADS) : "memory");
-    for (int i = tid; i < nq * RT_JC; i += RT_EPI_THREADS) {
-      const int ql = i / RT_JC, j = i % RT_JC;
-      if (j < jn && cs[i]) atomicAdd(&A.counts[((q0 + ql) * A.J + A.j0 + j) * 2], (unsigned long long)cs[i]);
+    if constexpr (!EMIT) {
+      for (int i = tid; i < nq * RT_JC; i += RT_EPI_THREADS) {
+        const int ql = i / RT_JC, j = i % RT_JC;
+        if (j < jn && cs[i]) atomicAdd(&A.counts[((q0 + ql) * A.J + A.j0 + j) * 2], (unsigned long long)cs[i]);
+      }
     }
     if (tid == 0) A.rec_n[cta] = *rcn < A.rec_slice ? *rcn : A.rec_slice;
   }
@@ -424,18 +463,34 @@ rank_count_umma_kernel(RtArgs A) {
   if (warp == RT_NEPI) tmem_dealloc(tmem_base, ncols);
 }
 
+template <int K>
+__global__ void __launch_bounds__(RT_THREADS, 1)     // 18 warps = 5 on one sub-partition: 5 x 32 x 96 registers is its whole file
+rank_count_umma_kernel(RtArgs A) {
+  rank_umma_body<K, false>(A);
+}
+
+// cfl_score_within's emitting pass (J = 1: A.thr = the radii)
+template <int K>
+__global__ void __launch_bounds__(RT_THREADS, 1)
+within_emit_umma_kernel(RtArgs A) {
+  rank_umma_body<K, true>(A);
+}
+
 // Exact verdicts of the ambiguous pairs: one thread per record, the direct-form device function of direct.cuh on the raw
 // rows (bit-identical to cfl_pair_dist_rows / cfl_rank_counts; the operands are staged in shared memory -- the slice's
 // query tile once per block, 32 catalog rows per warp and step with coalesced loads -- which changes no arithmetic).  stats: [0] records, [1] max |D~ - direct| / m in units
 // of 2^-20, [2] records whose deviation exceeded m / 2.
 constexpr int FX_THREADS = 128;
 constexpr int FX_BLOCKS = 4;                        // blocks per list slice
-template <int K>
-__global__ void __launch_bounds__(FX_THREADS)
-rank_fix_kernel(const uint4* __restrict__ recs_all, const unsigned int* __restrict__ rec_n, unsigned int slice,
-                const float* __restrict__ Pq, int64_t ldq, const float* __restrict__ E, int64_t lde, int64_t N, int64_t Q,
-                int d, int qt, int parts, const float* __restrict__ thr, int J, int j0, const int* __restrict__ only,
-                unsigned long long* __restrict__ counts, unsigned long long* __restrict__ stats) {
+// EMIT (cfl_score_within, J = 1): a record whose direct-form distance is below the radius is appended to its query's
+// segment instead of correcting a count.
+template <int K, bool EMIT>
+__device__ __forceinline__ void
+rank_fix_body(const uint4* __restrict__ recs_all, const unsigned int* __restrict__ rec_n, unsigned int slice,
+              const float* __restrict__ Pq, int64_t ldq, const float* __restrict__ E, int64_t lde, int64_t N, int64_t Q,
+              int d, int qt, int parts, const float* __restrict__ thr, int J, int j0, const int* __restrict__ only,
+              unsigned long long* __restrict__ counts, unsigned long long* __restrict__ stats,
+              const int64_t* __restrict__ offsets, unsigned int* __restrict__ cursor, int64_t* __restrict__ out) {
   extern __shared__ __align__(16) float fx_smem[];
   const unsigned int n = rec_n[blockIdx.y];                  // grid.y = the scoring kernel's CTAs, one list slice each
   if (n == 0 || (unsigned int)blockIdx.x * FX_THREADS >= n) return;
@@ -473,6 +528,13 @@ rank_fix_kernel(const uint4* __restrict__ recs_all, const unsigned int* __restri
     const float* qv = pq + (int)(q - q0) * ldp;
     const float dist = pcd_direct<K>([&](int j) { return ev[j]; }, [&](int k, int j) { return qv[k * d + j]; }, d);
     const float Dg = __uint_as_float(r.z), m = __uint_as_float(r.w);
+    if constexpr (EMIT) {
+      if (dist < thr[q]) {                                   // every record of a J = 1 pass lies inside its band
+        const int64_t at = atomicAdd(cursor + q, 1u);
+        const int64_t o = offsets[q];
+        if (at < offsets[q + 1] - o) out[o + at] = row;
+      }
+    } else {
     for (int j = 0; j < RT_JC && j0 + j < J; ++j) {
       const float t = thr[q * J + j0 + j];
       if (!(t == t)) continue;                               // NaN: no positive in this slot
@@ -482,6 +544,7 @@ rank_fix_kernel(const uint4* __restrict__ recs_all, const unsigned int* __restri
       const int lt = dist < t ? 1 : 0;
       if (lt != fast) atomicAdd(&counts[((q * J) + j0 + j) * 2], (unsigned long long)(long long)(lt - fast));
       if (dist == t) atomicAdd(&counts[((q * J) + j0 + j) * 2 + 1], 1ull);
+    }
     }
     const float dev = fabsf(Dg - dist);
     const float ratio = m > 0.0f ? dev / m : (dev > 0.0f ? 4096.0f : 0.0f);
@@ -494,6 +557,27 @@ rank_fix_kernel(const uint4* __restrict__ recs_all, const unsigned int* __restri
     if (over) atomicAdd(&stats[2], over);
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&stats[0], (unsigned long long)n);
   }
+}
+
+template <int K>
+__global__ void __launch_bounds__(FX_THREADS)
+rank_fix_kernel(const uint4* __restrict__ recs_all, const unsigned int* __restrict__ rec_n, unsigned int slice,
+                const float* __restrict__ Pq, int64_t ldq, const float* __restrict__ E, int64_t lde, int64_t N, int64_t Q,
+                int d, int qt, int parts, const float* __restrict__ thr, int J, int j0, const int* __restrict__ only,
+                unsigned long long* __restrict__ counts, unsigned long long* __restrict__ stats) {
+  rank_fix_body<K, false>(recs_all, rec_n, slice, Pq, ldq, E, lde, N, Q, d, qt, parts, thr, J, j0, only, counts, stats,
+                          nullptr, nullptr, nullptr);
+}
+
+template <int K>
+__global__ void __launch_bounds__(FX_THREADS)
+within_fix_kernel(const uint4* __restrict__ recs_all, const unsigned int* __restrict__ rec_n, unsigned int slice,
+                  const float* __restrict__ Pq, int64_t ldq, const float* __restrict__ E, int64_t lde, int64_t N,
+                  int64_t Q, int d, int qt, int parts, const float* __restrict__ radius, const int* __restrict__ only,
+                  unsigned long long* __restrict__ stats, const int64_t* __restrict__ offsets,
+                  unsigned int* __restrict__ cursor, int64_t* __restrict__ out) {
+  rank_fix_body<K, true>(recs_all, rec_n, slice, Pq, ldq, E, lde, N, Q, d, qt, parts, radius, 1, 0, only, nullptr, stats,
+                         offsets, cursor, out);
 }
 
 // queries whose records were dropped are recounted from scratch: clear what the fast path added
@@ -562,6 +646,102 @@ static int rank_tc_launch(const RtArgs& a, const float* Pq, int64_t ldq, const f
   return CFL_OK;
 }
 
+// Query prep shared by the counting and the emitting pass: centred prototypes, soft-min and plane-bound blocks, the
+// packed query image, the grid, the record list (cleared flags) and the band constants.
+static int rank_tc_prepare(const char* what, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const void* image,
+                           int64_t N, const float* mu, void* ws, const RtWs& w, RtArgs& a, cudaStream_t cs) {
+  const int qt = rank_tc_qt(K, d);
+  CFL_REQUIRE(qt > 0 && score_umma_supported(K, d), CFL_ERR_UNSUPPORTED, "%s: shape K=%d d=%d has no tcgen05 tiling",
+              what, K, d);
+  char* base = (char*)ws;
+  float* Pc = (float*)(base + w.pc);
+  float* qpar = (float*)(base + w.qpar);
+  float* qplane = qpar + (size_t)Q * qpar_stride(K);
+  int st = score_prep_queries_launch(Pq, Q, K, d, ldq, mu, Pc, qpar, qplane, cs);
+  if (st != CFL_OK) return st;
+  ScoreArgs sa = {};
+  sa.K = K; sa.d = d; sa.Q = Q; sa.Pc = Pc;
+  sa.plan.qt = qt; sa.plan.nqt = (int)((Q + qt - 1) / qt); sa.plan.dpad = (d + 7) / 8 * 8;
+  st = score_umma_pack_queries(sa, base + w.qimg, cs);
+  if (st != CFL_OK) return st;
+
+  a.K = K; a.d = d; a.Q = Q; a.N = N;
+  a.qt = qt; a.nqt = sa.plan.nqt; a.dpad = sa.plan.dpad;
+  a.tiles = (N + 127) / 128;
+  int sms = sm_count();
+  if (sms <= 0) sms = 148;
+  int64_t parts = sms / a.nqt;
+  if (parts < 1) parts = 1;
+  if (parts > a.tiles) parts = a.tiles;
+  a.parts = (int)parts;
+  a.qpar = qpar; a.qplane = qplane; a.qimg = base + w.qimg; a.cimg = image;
+  a.e2 = (const float*)((const char*)image + (size_t)a.tiles * (a.dpad / 8) * 8192);
+  CFL_REQUIRE((int64_t)a.parts * a.nqt <= 4096, CFL_ERR_UNSUPPORTED, "%s: Q=%lld needs more than 4096 CTAs", what,
+              (long long)Q);
+  a.recs = (uint4*)(base + w.recs); a.rec_slice = rank_tc_rec_cap(Q, N) / (unsigned int)(a.parts * a.nqt);
+  a.rec_n = (unsigned int*)(base + w.recn);
+  a.only = (int*)(base + w.only);
+  rank_tc_rel(&a.rel1, &a.rel2);
+  CFL_CUDA(cudaMemsetAsync(a.only, 0, (size_t)Q * sizeof(int), cs));
+  return CFL_OK;
+}
+
+__global__ void within_reset_flagged_kernel(const int* __restrict__ only, int64_t Q, unsigned int* cursor,
+                                            unsigned long long* stats) {
+  const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= Q || !only[q]) return;
+  cursor[q] = 0u;
+  atomicAdd(&stats[3], 1ull);
+}
+
+template <int K>
+static int within_tc_launch(const RtArgs& a, const float* Pq, int64_t ldq, const float* E, int64_t lde,
+                            unsigned long long* stats, cudaStream_t cs) {
+  const RtLayout L = rt_layout(K, a.qt, a.dpad);
+  const size_t smem = L.total + 1024;
+  CFL_SMEM_LIMIT(within_emit_umma_kernel<K>, smem);
+  within_emit_umma_kernel<K><<<dim3((unsigned)a.parts, (unsigned)a.nqt), RT_THREADS, smem, cs>>>(a);
+  CFL_LAUNCH_CHECK();
+  const size_t fx_smem = ((size_t)a.qt * (K * a.d + 1) + (size_t)FX_THREADS * (a.d + 1)) * sizeof(float);
+  CFL_SMEM_LIMIT(within_fix_kernel<K>, fx_smem);
+  within_fix_kernel<K><<<dim3(FX_BLOCKS, (unsigned)(a.parts * a.nqt)), FX_THREADS, fx_smem, cs>>>(
+      a.recs, a.rec_n, a.rec_slice, Pq, ldq, E, lde, a.N, a.Q, a.d, a.qt, a.parts, a.thr, a.only, stats, a.offsets,
+      a.cursor, a.out);
+  CFL_LAUNCH_CHECK();
+  return CFL_OK;
+}
+
+size_t within_tc_workspace_bytes(int64_t Q, int K, int d, int64_t N) { return rank_tc_ws(Q, K, d, N).total; }
+
+// Emitting pass of cfl_score_within on the tensor cores (pcd / siamese): sure rows straight from the scoring epilogue,
+// band rows after the direct-form check, queries whose records overflowed the list re-emitted from scratch on the
+// CUDA cores.  cursor[Q] must be zero; stats as CFL_WITHIN_NSTATS.
+int within_tc_emit(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* E, const void* image,
+                   int64_t N, int64_t lde, const float* mu, const float* radius, const int64_t* offsets,
+                   unsigned int* cursor, int64_t* out, void* ws, unsigned long long* stats, cudaStream_t cs) {
+  const RtWs w = rank_tc_ws(Q, K, d, N);
+  RtArgs a = {};
+  int st = rank_tc_prepare("score_within", Pq, Q, K, d, ldq, image, N, mu, ws, w, a, cs);
+  if (st != CFL_OK) return st;
+  a.J = 1; a.j0 = 0; a.thr = radius;
+  a.offsets = offsets; a.cursor = cursor; a.out = out;
+  CFL_CUDA(cudaMemsetAsync(a.rec_n, 0, 4096 * sizeof(unsigned int), cs));
+  switch (K) {
+    case 1: st = within_tc_launch<1>(a, Pq, ldq, E, lde, stats, cs); break;
+    case 2: st = within_tc_launch<2>(a, Pq, ldq, E, lde, stats, cs); break;
+    case 3: st = within_tc_launch<3>(a, Pq, ldq, E, lde, stats, cs); break;
+    case 4: st = within_tc_launch<4>(a, Pq, ldq, E, lde, stats, cs); break;
+    case 5: st = within_tc_launch<5>(a, Pq, ldq, E, lde, stats, cs); break;
+    case 6: st = within_tc_launch<6>(a, Pq, ldq, E, lde, stats, cs); break;
+    case 7: st = within_tc_launch<7>(a, Pq, ldq, E, lde, stats, cs); break;
+    default: st = within_tc_launch<8>(a, Pq, ldq, E, lde, stats, cs); break;
+  }
+  if (st != CFL_OK) return st;
+  within_reset_flagged_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, cs>>>(a.only, Q, cursor, stats);
+  CFL_LAUNCH_CHECK();
+  return within_emit_launch(mode, Pq, Q, K, d, ldq, nullptr, E, N, lde, radius, offsets, cursor, out, a.only, cs);
+}
+
 }  // namespace cfl
 
 using namespace cfl;
@@ -592,45 +772,17 @@ int cfl_rank_counts_packed(int mode, const float* Pq, int64_t Q, int K, int d, i
   CFL_CUDA(cudaMemsetAsync(counts, 0, (size_t)Q * J * 2 * sizeof(int64_t), cs));
   if (N == 0) return CFL_OK;
   CFL_REQUIRE(E && image, CFL_ERR_INVALID, "rank_counts_packed: NULL catalog / image");
-  const int qt = rank_tc_qt(K, d);
-  CFL_REQUIRE(qt > 0 && score_umma_supported(K, d), CFL_ERR_UNSUPPORTED,
+  CFL_REQUIRE(rank_tc_qt(K, d) > 0 && score_umma_supported(K, d), CFL_ERR_UNSUPPORTED,
               "rank_counts_packed: shape K=%d d=%d has no tcgen05 tiling", K, d);
   const RtWs w = rank_tc_ws(Q, K, d, N);
   CFL_REQUIRE(ws && ws_bytes >= w.total, CFL_ERR_WORKSPACE, "rank_counts_packed: workspace too small (%zu < %zu)",
               ws_bytes, w.total);
-  char* base = (char*)ws;
-  float* Pc = (float*)(base + w.pc);
-  float* qpar = (float*)(base + w.qpar);
-  float* qplane = qpar + (size_t)Q * qpar_stride(K);
-  st = score_prep_queries_launch(Pq, Q, K, d, ldq, mu, Pc, qpar, qplane, cs);
-  if (st != CFL_OK) return st;
-  ScoreArgs sa = {};
-  sa.K = K; sa.d = d; sa.Q = Q; sa.Pc = Pc;
-  sa.plan.qt = qt; sa.plan.nqt = (int)((Q + qt - 1) / qt); sa.plan.dpad = (d + 7) / 8 * 8;
-  st = score_umma_pack_queries(sa, base + w.qimg, cs);
-  if (st != CFL_OK) return st;
-
   RtArgs a = {};
-  a.K = K; a.d = d; a.J = J; a.Q = Q; a.N = N;
-  a.qt = qt; a.nqt = sa.plan.nqt; a.dpad = sa.plan.dpad;
-  a.tiles = (N + 127) / 128;
-  int sms = sm_count();
-  if (sms <= 0) sms = 148;
-  int64_t parts = sms / a.nqt;
-  if (parts < 1) parts = 1;
-  if (parts > a.tiles) parts = a.tiles;
-  a.parts = (int)parts;
-  a.qpar = qpar; a.qplane = qplane; a.qimg = base + w.qimg; a.cimg = image;
-  a.e2 = (const float*)((const char*)image + (size_t)a.tiles * (a.dpad / 8) * 8192);
+  st = rank_tc_prepare("rank_counts_packed", Pq, Q, K, d, ldq, image, N, mu, ws, w, a, cs);
+  if (st != CFL_OK) return st;
+  a.J = J;
   a.thr = pos_dist; a.counts = (unsigned long long*)counts;
-  CFL_REQUIRE((int64_t)a.parts * a.nqt <= 4096, CFL_ERR_UNSUPPORTED, "rank_counts_packed: Q=%lld needs more than 4096 CTAs",
-              (long long)Q);
-  a.recs = (uint4*)(base + w.recs); a.rec_slice = rank_tc_rec_cap(Q, N) / (unsigned int)(a.parts * a.nqt);
-  a.rec_n = (unsigned int*)(base + w.recn);
-  a.only = (int*)(base + w.only);
-  rank_tc_rel(&a.rel1, &a.rel2);
-  unsigned long long* stats = (unsigned long long*)(base + w.stats);
-  CFL_CUDA(cudaMemsetAsync(a.only, 0, (size_t)Q * sizeof(int), cs));
+  unsigned long long* stats = (unsigned long long*)((char*)ws + w.stats);
   CFL_CUDA(cudaMemsetAsync(stats, 0, CFL_RANK_NSTATS * sizeof(unsigned long long), cs));
   timer_record(0, cs);
   for (int j0 = 0; j0 < J; j0 += RT_JC) {

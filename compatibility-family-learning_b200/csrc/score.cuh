@@ -116,6 +116,15 @@ int score_prep_queries_launch(const float* Pq, int64_t Q, int K, int d, int64_t 
 int rank_counts_only_launch(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* E, int64_t N,
                             int64_t lde, const float* pos_dist, int J, unsigned long long* counts, const int* only,
                             cudaStream_t st);
+// cfl_score_within (within.cu): the CUDA-core emitting pass (rank_counts.cu; every query, or the ones flagged in only[Q])
+// and the tensor-core one (rank_counts_tc.cu) append local rows dist < radius[q] to out[offsets[q], offsets[q + 1])
+int within_emit_launch(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* Wq, const float* E,
+                       int64_t N, int64_t lde, const float* radius, const int64_t* offsets, unsigned int* cursor,
+                       int64_t* out, const int* only, cudaStream_t st);
+size_t within_tc_workspace_bytes(int64_t Q, int K, int d, int64_t N);
+int within_tc_emit(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* E, const void* image,
+                   int64_t N, int64_t lde, const float* mu, const float* radius, const int64_t* offsets,
+                   unsigned int* cursor, int64_t* out, void* ws, unsigned long long* stats, cudaStream_t st);
 
 #ifdef __CUDACC__
 __device__ __forceinline__ float fast_ex2(float x) {

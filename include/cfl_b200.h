@@ -274,6 +274,40 @@ int cfl_rank_counts_packed(int mode, const float* Pq, int64_t Q, int K, int d, i
 int cfl_rank_counts_packed_stats(int64_t Q, int K, int d, int64_t N, const void* ws, size_t ws_bytes, int64_t* out,
                                  void* stream);
 
+/* ---------------------------------------------------------------------------------------
+ * Catalog range queries (extension): every catalog row a query is compatible with.  The Thresholder
+ * (cfl/models/blocks.py:21-22) scores a pair max(theta, 1e-6) - dist and the accuracy counts of
+ * cfl/utils.py:247,264 call it compatible when that score is > 0, i.e. when dist < r with
+ * r = max(theta, 1e-6).  For a radius r[q] per query (fp32) the result of q is the set
+ *   { c < N : dist(q, c) < r[q] }   (strict; dist = the fp32 direct form of cfl_pair_dist_rows)
+ * as CSR lists: rows offsets[q] .. offsets[q + 1] of out_idx (idx_base + row, int64) and out_dist (the
+ * direct-form distance, bit-identical to cfl_pair_dist_rows), ordered by (distance, index).  NaN selects
+ * nothing, +inf every row.  Operands per mode as cfl_rank_counts.
+ * Two steps: the caller counts first -- counts[q] = cfl_rank_counts_packed / cfl_rank_counts with
+ * pos_dist = r (J = 1), whose verdicts are the same arithmetic -- and lays out offsets[Q + 1] (device,
+ * an exclusive scan of the counts; offsets[0] may be non-zero, out_idx / out_dist are indexed by them) and
+ * the outputs; cfl_score_within then fills the segments.
+ *   image != NULL (pcd / siamese, cfl_catalog_pack of E / mu): rows emitted from the tensor-core scoring
+ *   epilogue (3xTF32 Gram form, rounding band, direct-form check of the pairs inside it); image == NULL: the
+ *   CUDA-core direct form (monomer; pcd shapes without a tcgen05 tiling).  N < 2^32; one call takes up to
+ *   4096 scoring CTAs' worth of queries (split larger batches).  Segments beyond 16384 rows are sorted in
+ *   global memory by one CTA (correct, slower).
+ * cfl_score_within_stats (synchronises the stream): out[CFL_WITHIN_NSTATS] of the last call on `ws` = {band
+ * records, largest |Gram - direct| / band in units of 2^-20, records beyond half the band, queries re-emitted
+ * on the CUDA cores (record list overflow), queries whose emitted row count differed from their count (0)}.
+ * cfl_within_merge: the sharded result.  Rank r's list (global indices) of query q is rows offsets[r][q] ..
+ * offsets[r][q + 1] of idx[r], dist[r] (offsets [R, Q + 1], idx / dist [R, ld]); out_offsets[Q + 1] = the
+ * scan of the per-query sums.  The merged lists are ordered by (distance, index), independent of R. */
+#define CFL_WITHIN_NSTATS 5
+size_t cfl_score_within_workspace_bytes(int mode, int64_t Q, int K, int d, int64_t N);
+int cfl_score_within(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* Wq, const float* E,
+                     const void* image, int64_t N, int64_t lde, const float* mu, const float* radius,
+                     const int64_t* offsets, int64_t idx_base, int64_t* out_idx, float* out_dist, void* ws,
+                     size_t ws_bytes, void* stream);
+int cfl_score_within_stats(const void* ws, size_t ws_bytes, int64_t* out, void* stream);
+int cfl_within_merge(const int64_t* offsets, const int64_t* idx, const float* dist, int64_t ld, int R, int64_t Q,
+                     const int64_t* out_offsets, int64_t* out_idx, float* out_dist, void* stream);
+
 /* TF-1.x Adam (cfl/models/cfl.py:1083-1085): lr_t = lr*sqrt(1-b2^t)/(1-b1^t);
  * p -= lr_t*m/(sqrt(v)+eps).  grad_scale multiplies g first (1/world for DP averaging). */
 int cfl_adam_step(float* p, const float* g, float* m, float* v, int64_t n, int step,
