@@ -4,8 +4,8 @@
 // tensor-core route wrote and re-read a dense 4 GB matrix).  roc_auc_score of cfl/utils.py:267-268 over every
 // catalog row follows from these integers (cfl.ranking.auc_from_rank_counts).
 //
-// The kernel is score_umma_kernel's skeleton (score_umma.cu: packed catalog image through a TMA ring, 3xTF32
-// tcgen05.mma into double-buffered TMEM accumulators, soft-min epilogue of score.cuh) with a counting epilogue:
+// The kernel runs the Gram pipeline of gram_pipe.cuh (packed catalog image through a TMA ring, 3xTF32 tcgen05.mma into
+// double-buffered TMEM accumulators, the same as score_umma_kernel) with the soft-min of score.cuh and a counting epilogue:
 //   * every (row, query) distance D~ (Gram form, 3xTF32) gets a rounding band
 //       m = S * (REL1 + REL2 * sqrt(D~ * V)),   S = |e|^2 + max_k |p_k|^2,   V = spread of the prototypes under the
 //     soft-min weights (softmin_pair_var: the sensitivity of the distance to an error of the soft-min exponents, which
@@ -22,8 +22,7 @@
 // maximum of |D~ - direct| / m over all ambiguous records; rank_fix_kernel reports it in the call's statistics and
 // tests/test_rank_counts.py asserts the headroom).  A query whose records do not fit the list is recounted from
 // scratch by the CUDA-core kernel (rank_count_kernel, restricted by `only`).
-#include "score.cuh"
-#include "umma.cuh"
+#include "gram_pipe.cuh"
 #include <stdlib.h>
 #include "direct.cuh"
 
@@ -31,12 +30,6 @@ namespace cfl {
 
 using namespace umma;
 
-constexpr int RT_NEPI = 16;                         // epilogue warps: four per TMEM lane quarter
-constexpr int RT_THREADS = (RT_NEPI + 2) * 32;
-constexpr int RT_EPI_THREADS = RT_NEPI * 32;
-constexpr int RT_WPQ = RT_NEPI / 4;
-constexpr int RT_NSTAGE = 6;
-constexpr uint32_t RT_ASTAGE = 4u * 128u * 16u;     // one K-step of the catalog image: [hl][chunk][128 rows][16 B]
 constexpr int RT_JC = 8;                            // thresholds per launch (J > 8: several launches)
 constexpr int RT_QT_MAX = 64;
 constexpr float RT_REL1_DEFAULT = 1.0f / 262144.0f;     // 2^-18: Gram-form (3xTF32) + direct-form rounding, relative to S
@@ -70,22 +63,19 @@ struct RtArgs {
   int64_t* out;                   // local catalog rows
 };
 
-struct RtLayout { uint32_t b_img, a_ring, qpar, qpl, thr, qm, skp, cs, rcn, bars, tmem_slot, total; };
+// Shared memory of the counting / emitting kernels: the Gram pipeline's regions and, behind the query blocks, the
+// epilogue's thresholds, max_k |p_k|^2, skip-test constants per query, per-threshold counts and records written.
+struct RtLayout { GramLayout g; uint32_t thr, qm, skp, cs, rcn; };
 __host__ __device__ inline RtLayout rt_layout(int K, int qt, int dpad) {
   RtLayout L;
-  uint32_t off = 0;
-  L.b_img = off;   off += (uint32_t)dpad * 8u * (uint32_t)(K * qt);  off = (off + 1023u) & ~1023u;
-  L.a_ring = off;  off += RT_NSTAGE * 2u * RT_ASTAGE;
-  L.qpar = off;    off += (uint32_t)qt * (uint32_t)qpar_stride(K) * 4u;  off = (off + 15u) & ~15u;
-  L.qpl = off;     off += (uint32_t)qt * (uint32_t)qplane_stride(K) * 4u; off = (off + 15u) & ~15u;
+  L.g = gram_layout(K, qt, dpad, 0u);
+  uint32_t off = L.g.back;
   L.thr = off;     off += (uint32_t)qt * RT_JC * 4u;
   L.qm = off;      off += (uint32_t)qt * 4u;                           off = (off + 15u) & ~15u;
   L.skp = off;     off += (uint32_t)qt * 16u;                          // per query: (tmax, kappa0, kappa1, -)
   L.cs = off;      off += (uint32_t)qt * RT_JC * 4u;
   L.rcn = off;     off += 16u;
-  L.bars = off;    off += (2u * RT_NSTAGE + 5u) * 8u;
-  L.tmem_slot = off; off += 16u;
-  L.total = off;
+  gram_layout_end(L.g, off);
   return L;
 }
 
@@ -103,36 +93,24 @@ __device__ __forceinline__ float sqrt_approx(float x) {
   return y;
 }
 
-// The scoring skeleton and the classifying epilogue, shared by the counting kernel (EMIT = false: packed counters, J
+// The Gram pipeline and the classifying epilogue, shared by the counting kernel (EMIT = false: packed counters, J
 // thresholds) and the emitting kernel of cfl_score_within (EMIT = true, J = 1: a pair with D~ < t - m is appended to its
 // query's result segment at once, a pair inside the band goes to the record list exactly as for the counts).  Both
 // instantiations classify with the same arithmetic, so the emitted set and the count of the same radius agree pair for pair.
 template <int K, bool EMIT>
 __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
   extern __shared__ __align__(1024) unsigned char smem[];
-  constexpr int GQ = K <= 2 ? 16 : (K <= 4 ? 8 : 4);     // queries per epilogue group
-  constexpr int NGW = K <= 2 ? 1 : (K <= 4 ? 2 : 3);     // query groups per warp: ceil((qt / GQ) / RT_WPQ), qt <= 64 (48 at K = 5)
+  constexpr int GQ = gram_gq(K);
+  constexpr int NGW = K <= 2 ? 1 : (K <= 4 ? 2 : 3);     // query groups per warp: ceil((qt / GQ) / GP_WPQ), qt <= 64 (48 at K = 5)
   constexpr int QPS = qpar_stride(K);
   const int QT = A.qt;
-  const int NC = K * QT;
-  const int dpad = A.dpad;
-  const int nks = dpad / 8;
-  const RtLayout L = rt_layout(K, QT, dpad);
-  unsigned char* b_img = smem + L.b_img;
-  unsigned char* a_ring = smem + L.a_ring;
-  float* qpar = (float*)(smem + L.qpar);
+  const RtLayout L = rt_layout(K, QT, A.dpad);
+  const GramPipe P = gram_pipe(smem, L.g, K, QT, A.dpad);
   float* thr = (float*)(smem + L.thr);
   float* qm = (float*)(smem + L.qm);
-  float* qpl = (float*)(smem + L.qpl);
   float4* skp = (float4*)(smem + L.skp);
   unsigned int* cs = (unsigned int*)(smem + L.cs);
   unsigned int* rcn = (unsigned int*)(smem + L.rcn);
-  uint64_t* full = (uint64_t*)(smem + L.bars);
-  uint64_t* empty = full + RT_NSTAGE;
-  uint64_t* tfull = empty + RT_NSTAGE;
-  uint64_t* tempty = tfull + 2;
-  uint64_t* bfull = tempty + 2;
-  uint32_t* tmem_slot = (uint32_t*)(smem + L.tmem_slot);
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int part = blockIdx.x, qtile = blockIdx.y;
@@ -141,31 +119,11 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
   const int64_t t0 = A.tiles * part / A.parts;
   const int64_t t1 = A.tiles * (part + 1) / A.parts;
   const int ntiles = (int)(t1 - t0);
-  const int kss = (nks % 2 == 0) ? 2 : 1;                    // K-steps per ring stage
   const int jn = (A.J - A.j0 < RT_JC) ? (A.J - A.j0) : RT_JC;
 
-  uint32_t ncols = 32;
-  while ((int)ncols < 2 * NC) ncols <<= 1;
-  if (warp == RT_NEPI) {
-    if (lane == 0) {
-      for (int s = 0; s < RT_NSTAGE; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-      mbar_init(&tfull[0], 1); mbar_init(&tfull[1], 1);
-      mbar_init(&tempty[0], RT_EPI_THREADS); mbar_init(&tempty[1], RT_EPI_THREADS);
-      mbar_init(bfull, 1);
-      fence_barrier_init();
-    }
-    __syncwarp();
-    tmem_alloc(tmem_slot, ncols);
-  }
-  // per-query soft-min blocks, interleaved by query pair with the first K entries negated (softmin_pair)
-  for (int i = tid; i < QT * QPS; i += RT_THREADS) {
-    const int ql = i / QPS, j = i % QPS;
-    float v = (ql < nq) ? A.qpar[(q0 + ql) * QPS + j] : 0.0f;
-    if (j < K) v = -v;
-    qpar[((ql >> 1) * QPS + j) * 2 + (ql & 1)] = v;
-  }
+  gram_setup<K>(P, A.qpar, A.qplane, q0, nq, QT);
   // thresholds: NaN (no positive in the slot), padding slots and padding queries become -inf = "count nothing"
-  for (int i = tid; i < QT * RT_JC; i += RT_THREADS) {
+  for (int i = tid; i < QT * RT_JC; i += GP_THREADS) {
     const int ql = i / RT_JC, j = i % RT_JC;
     float t = __int_as_float(0xff800000);
     if (ql < nq && j < jn) {
@@ -175,24 +133,17 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
     thr[i] = t;
     cs[i] = 0u;
   }
-  for (int ql = tid; ql < QT; ql += RT_THREADS) {
+  for (int ql = tid; ql < QT; ql += GP_THREADS) {
     float pm = 0.0f;
     if (ql < nq)
       for (int k = 0; k < K; ++k) pm = fmaxf(pm, A.qpar[(q0 + ql) * QPS + k]);      // log2(e) |p_k|^2
     qm[ql] = pm * CFL_LN2;                                    // max_k |p_k|^2
   }
-  {
-    constexpr int PBS0 = qplane_stride(K);                     // pair interleave, as the soft-min blocks
-    for (int i = tid; i < QT * PBS0; i += RT_THREADS) {
-      const int ql = i / PBS0, j = i % PBS0;
-      qpl[((ql >> 1) * PBS0 + j) * 2 + (ql & 1)] = (ql < nq) ? A.qplane[(q0 + ql) * PBS0 + j] : 0.0f;
-    }
-  }
   // Skip test of a whole query group (epilogue): with LB <= D~ the affine-hull lower bound and Vq >= V,
   //   D~ - m(D~) >= LB - S (rel1 + rel2 sqrt(LB Vq)) >= LB (1 - S k1) - S k0   (AM-GM with c = sqrt(Vq / tmax)),
   // k0 = rel1 + rel2 Vq / (2c), k1 = rel2 c / 2: when that exceeds the query's largest threshold the pair is farther than
   // every threshold and outside every band -- nothing to count, nothing to record.
-  for (int ql = tid; ql < QT; ql += RT_THREADS) {
+  for (int ql = tid; ql < QT; ql += GP_THREADS) {
     float tmax = __int_as_float(0xff800000);
     float k0 = A.rel1, k1 = 0.0f;
     if (ql < nq) {
@@ -214,56 +165,12 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
   if (tid == 0) *rcn = 0u;
   const unsigned int cta = blockIdx.y * gridDim.x + blockIdx.x;
   uint4* myrecs = A.recs + (size_t)cta * A.rec_slice;
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t tmem_base = gram_start(P);
 
-  if (warp == RT_NEPI) {
-    // ================================ MMA issuer (one lane) =================================
-    if (elect_one()) {
-      mbar_wait(bfull, 0);
-      const Step3Desc sd = make_step3((uint32_t)NC, make_idesc_tf32(128, (uint32_t)NC));
-      const uint32_t a_base = smem_u32(a_ring), b_base = smem_u32(b_img);
-      const uint32_t b_step = 4u * (uint32_t)NC * 16u;
-      int stage = 0; uint32_t phase = 0;
-      for (int t = 0; t < ntiles; ++t) {
-        const int buf = t & 1;
-        mbar_wait(&tempty[buf], ((uint32_t)(t >> 1) & 1u) ^ 1u);
-        tc_fence_after();
-        const uint32_t d_tmem = tmem_base + (uint32_t)(buf * NC);
-        for (int ks = 0; ks < nks; ks += kss) {
-          mbar_wait(&full[stage], phase);
-          tc_fence_after();
-          for (int j = 0; j < kss; ++j)
-            mma_step3(sd, d_tmem, a_base + (stage * 2 + j) * RT_ASTAGE, b_base + (ks + j) * b_step, ks + j == 0);
-          mma_commit(&empty[stage]);
-          if (++stage == RT_NSTAGE) { stage = 0; phase ^= 1u; }
-        }
-        mma_commit(&tfull[buf]);
-      }
-    }
-  } else if (warp == RT_NEPI + 1) {
-    // ================================ TMA producer (one lane) ===============================
-    if (elect_one()) {
-      const uint32_t bbytes = (uint32_t)dpad * 8u * (uint32_t)NC;
-      const unsigned char* qsrc = (const unsigned char*)A.qimg + (size_t)qtile * bbytes;
-      mbar_arrive_expect_tx(bfull, bbytes);
-      for (uint32_t o = 0; o < bbytes; o += 32768u) {
-        uint32_t n = bbytes - o < 32768u ? bbytes - o : 32768u;
-        bulk_g2s(b_img + o, qsrc + o, n, bfull);
-      }
-      int stage = 0; uint32_t phase = 0;
-      for (int t = 0; t < ntiles; ++t) {
-        const unsigned char* src = (const unsigned char*)A.cimg + (size_t)(t0 + t) * nks * RT_ASTAGE;
-        for (int ks = 0; ks < nks; ks += kss) {
-          mbar_wait(&empty[stage], phase ^ 1u);
-          mbar_arrive_expect_tx(&full[stage], (uint32_t)kss * RT_ASTAGE);
-          bulk_g2s(a_ring + stage * 2 * RT_ASTAGE, src + (size_t)ks * RT_ASTAGE, (uint32_t)kss * RT_ASTAGE, &full[stage]);
-          if (++stage == RT_NSTAGE) { stage = 0; phase ^= 1u; }
-        }
-      }
-    }
+  if (warp == GP_NEPI) {
+    gram_mma(P, tmem_base, ntiles);
+  } else if (warp == GP_NEPI + 1) {
+    gram_tma(P, A.qimg, qtile, A.cimg, t0, 1, ntiles);
   } else {
     // ======================================= epilogue ========================================
     const int lq = warp & 3, sub = warp >> 2;
@@ -280,7 +187,7 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
     auto flush = [&]() {
 #pragma unroll
       for (int gi = 0; gi < NGW; ++gi) {
-        const int g = sub + gi * RT_WPQ;
+        const int g = sub + gi * GP_WPQ;
         if (g * GQ < nq) {                                    // warp-uniform
 #pragma unroll
           for (int i = 0; i < GQ; ++i) {
@@ -308,25 +215,16 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
     bool bound_on = true;
     int grp_seen = 0, grp_skipped = 0;
     for (int t = 0; t < ntiles; ++t) {
-      const int buf = t & 1;
       const int64_t row = (t0 + t) * 128 + lrow;
       const bool valid = row < A.N;
       const float e2 = __ldg(A.e2 + row);                    // padded to whole tiles
-      mbar_wait(&tfull[buf], (uint32_t)(t >> 1) & 1u);
-      tc_fence_after();
-      const uint32_t taddr = tmem_base + ((uint32_t)(lq * 32) << 16) + (uint32_t)(buf * NC);
+      const uint32_t taddr = gram_acquire(P, tmem_base, t, lq);
 #pragma unroll
       for (int gi = 0; gi < NGW; ++gi) {
-        const int g = sub + gi * RT_WPQ;
+        const int g = sub + gi * GP_WPQ;
         if (g * GQ >= nq) continue;                           // warp-uniform
         float gk[K][GQ];
-#pragma unroll
-        for (int k = 0; k < K; ++k) {
-          if constexpr (GQ == 16)     tmem_ld16(taddr + (uint32_t)(k * QT + g * GQ), gk[k]);
-          else if constexpr (GQ == 8) tmem_ld8(taddr + (uint32_t)(k * QT + g * GQ), gk[k]);
-          else                        tmem_ld4(taddr + (uint32_t)(k * QT + g * GQ), gk[k]);
-        }
-        tmem_ld_wait();
+        gram_load_group<K, GQ>(taddr, QT, g, gk);
         if (bound_on) {
           constexpr int PBS = qplane_stride(K);
           const float e2s = e2 * (1.0f - CFL_PLANE_REL);
@@ -335,9 +233,7 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
 #pragma unroll
           for (int pi = 0; pi < GQ / 2; ++pi) {
             f2_t pv[PBS];
-            const ulonglong2* src = (const ulonglong2*)(qpl + (g * (GQ / 2) + pi) * PBS * 2);
-#pragma unroll
-            for (int j = 0; j < PBS; j += 2) { const ulonglong2 u = src[j >> 1]; pv[j] = u.x; pv[j + 1] = u.y; }
+            load_pair_block<PBS>(P.qpl + (g * (GQ / 2) + pi) * PBS * 2, pv);
             float gA[K], gB[K], lbA, lbB;
 #pragma unroll
             for (int k = 0; k < K; ++k) { gA[k] = gk[k][2 * pi]; gB[k] = gk[k][2 * pi + 1]; }
@@ -353,14 +249,12 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
           ++grp_seen;
           if (!__any_sync(0xffffffffu, need && valid)) { ++grp_skipped; continue; }
         }
-        const float* qg = qpar + g * GQ * QPS;
+        const float* qg = P.qpar + g * GQ * QPS;
         float dist[GQ], var[GQ];
 #pragma unroll
         for (int pi = 0; pi < GQ / 2; ++pi) {
           f2_t qv[QPS];
-          const ulonglong2* src = (const ulonglong2*)(qg + pi * QPS * 2);
-#pragma unroll
-          for (int j = 0; j < QPS; j += 2) { const ulonglong2 u = src[j >> 1]; qv[j] = u.x; qv[j + 1] = u.y; }
+          load_pair_block<QPS>(qg + pi * QPS * 2, qv);
           float gA[K], gB[K];
 #pragma unroll
           for (int k = 0; k < K; ++k) { gA[k] = gk[k][2 * pi]; gB[k] = gk[k][2 * pi + 1]; }
@@ -442,36 +336,33 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
         }
       }
       if (t == 15 && grp_skipped * 2 < grp_seen) bound_on = false;
-      tc_fence_before();
-      mbar_arrive(&tempty[buf]);
+      gram_release(P, t);
       if constexpr (!EMIT) {
         if (++since_flush == 15) { flush(); since_flush = 0; }
       }
     }
     if constexpr (!EMIT) flush();
-    asm volatile("bar.sync 1, %0;" ::"n"(RT_EPI_THREADS) : "memory");
+    asm volatile("bar.sync 1, %0;" ::"n"(GP_EPI_THREADS) : "memory");
     if constexpr (!EMIT) {
-      for (int i = tid; i < nq * RT_JC; i += RT_EPI_THREADS) {
+      for (int i = tid; i < nq * RT_JC; i += GP_EPI_THREADS) {
         const int ql = i / RT_JC, j = i % RT_JC;
         if (j < jn && cs[i]) atomicAdd(&A.counts[((q0 + ql) * A.J + A.j0 + j) * 2], (unsigned long long)cs[i]);
       }
     }
     if (tid == 0) A.rec_n[cta] = *rcn < A.rec_slice ? *rcn : A.rec_slice;
   }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == RT_NEPI) tmem_dealloc(tmem_base, ncols);
+  gram_finish(P, tmem_base);
 }
 
 template <int K>
-__global__ void __launch_bounds__(RT_THREADS, 1)     // 18 warps = 5 on one sub-partition: 5 x 32 x 96 registers is its whole file
+__global__ void __launch_bounds__(GP_THREADS, 1)     // 18 warps = 5 on one sub-partition: 5 x 32 x 96 registers is its whole file
 rank_count_umma_kernel(RtArgs A) {
   rank_umma_body<K, false>(A);
 }
 
 // cfl_score_within's emitting pass (J = 1: A.thr = the radii)
 template <int K>
-__global__ void __launch_bounds__(RT_THREADS, 1)
+__global__ void __launch_bounds__(GP_THREADS, 1)
 within_emit_umma_kernel(RtArgs A) {
   rank_umma_body<K, true>(A);
 }
@@ -620,7 +511,7 @@ static RtWs rank_tc_ws(int64_t Q, int K, int d, int64_t N) {
   size_t off = 0;
   w.pc = off;    off = align_up(off + (size_t)Q * K * d * 4, 256);
   w.qpar = off;  off = align_up(off + (size_t)Q * (qpar_stride(K) + qplane_stride(K)) * 4, 256);
-  w.qimg = off;  off = align_up(off + (size_t)nqt * dpad * 8 * (size_t)(K * qt), 1024);
+  w.qimg = off;  off = align_up(off + (size_t)nqt * qimg_tile_bytes(dpad, K * qt), 1024);
   w.recs = off;  off = align_up(off + (size_t)rank_tc_rec_cap(Q, N) * sizeof(uint4), 256);
   w.recn = off;  off = align_up(off + 4096 * sizeof(unsigned int), 256);
   w.only = off;  off = align_up(off + (size_t)Q * sizeof(int), 256);
@@ -632,11 +523,10 @@ static RtWs rank_tc_ws(int64_t Q, int K, int d, int64_t N) {
 template <int K>
 static int rank_tc_launch(const RtArgs& a, const float* Pq, int64_t ldq, const float* E, int64_t lde,
                           unsigned long long* stats, cudaStream_t cs) {
-  const RtLayout L = rt_layout(K, a.qt, a.dpad);
-  const size_t smem = L.total + 1024;
+  const size_t smem = rt_layout(K, a.qt, a.dpad).g.total + 1024;
   CFL_SMEM_LIMIT(rank_count_umma_kernel<K>, smem);
   dim3 grid((unsigned)a.parts, (unsigned)a.nqt);
-  rank_count_umma_kernel<K><<<grid, RT_THREADS, smem, cs>>>(a);
+  rank_count_umma_kernel<K><<<grid, GP_THREADS, smem, cs>>>(a);
   CFL_LAUNCH_CHECK();
   const size_t fx_smem = ((size_t)a.qt * (K * a.d + 1) + (size_t)FX_THREADS * (a.d + 1)) * sizeof(float);
   CFL_SMEM_LIMIT(rank_fix_kernel<K>, fx_smem);
@@ -675,7 +565,7 @@ static int rank_tc_prepare(const char* what, const float* Pq, int64_t Q, int K, 
   if (parts > a.tiles) parts = a.tiles;
   a.parts = (int)parts;
   a.qpar = qpar; a.qplane = qplane; a.qimg = base + w.qimg; a.cimg = image;
-  a.e2 = (const float*)((const char*)image + (size_t)a.tiles * (a.dpad / 8) * 8192);
+  a.e2 = (const float*)((const char*)image + catalog_e2_offset(N, d));
   CFL_REQUIRE((int64_t)a.parts * a.nqt <= 4096, CFL_ERR_UNSUPPORTED, "%s: Q=%lld needs more than 4096 CTAs", what,
               (long long)Q);
   a.recs = (uint4*)(base + w.recs); a.rec_slice = rank_tc_rec_cap(Q, N) / (unsigned int)(a.parts * a.nqt);
@@ -697,10 +587,9 @@ __global__ void within_reset_flagged_kernel(const int* __restrict__ only, int64_
 template <int K>
 static int within_tc_launch(const RtArgs& a, const float* Pq, int64_t ldq, const float* E, int64_t lde,
                             unsigned long long* stats, cudaStream_t cs) {
-  const RtLayout L = rt_layout(K, a.qt, a.dpad);
-  const size_t smem = L.total + 1024;
+  const size_t smem = rt_layout(K, a.qt, a.dpad).g.total + 1024;
   CFL_SMEM_LIMIT(within_emit_umma_kernel<K>, smem);
-  within_emit_umma_kernel<K><<<dim3((unsigned)a.parts, (unsigned)a.nqt), RT_THREADS, smem, cs>>>(a);
+  within_emit_umma_kernel<K><<<dim3((unsigned)a.parts, (unsigned)a.nqt), GP_THREADS, smem, cs>>>(a);
   CFL_LAUNCH_CHECK();
   const size_t fx_smem = ((size_t)a.qt * (K * a.d + 1) + (size_t)FX_THREADS * (a.d + 1)) * sizeof(float);
   CFL_SMEM_LIMIT(within_fix_kernel<K>, fx_smem);

@@ -827,7 +827,7 @@ static CerLayout cer_layout(int K, int d, int qt, int dpad) {
   L.pc = off;     off = align_up(off + (size_t)qt * K * d * sizeof(float), 256);
   L.qpar = off;   off = align_up(off + (size_t)qt * qpar_stride(K) * sizeof(float), 256);
   L.qplane = off; off = align_up(off + (size_t)qt * qplane_stride(K) * sizeof(float), 1024);
-  L.qimg = off;   off = align_up(off + (size_t)dpad * 8 * (size_t)(K * qt), 1024);
+  L.qimg = off;   off = align_up(off + qimg_tile_bytes(dpad, K * qt), 1024);
   L.total = off;
   return L;
 }
@@ -910,7 +910,7 @@ static size_t score_ws_layout(int64_t Q, int K, int d, int64_t N, const ScorePla
   const int kparts = p.parts > lb.parts ? p.parts : lb.parts;          // key buffers serve both tilings
   *o_pc = off;   off = align_up(off + (size_t)Q * K * d * 4, 256);
   *o_qpar = off; off = align_up(off + (size_t)Q * (qpar_stride(K) + qplane_stride(K)) * 4, 256);
-  *o_qimg = off; off = align_up(off + (p.impl ? score_umma_qimg_bytes(p, K) : 0), 1024);
+  *o_qimg = off; off = align_up(off + (p.impl ? (size_t)p.nqt * qimg_tile_bytes(p.dpad, K * p.qt) : 0), 1024);
   if (o_lbimg) *o_lbimg = off;
   off = align_up(off + (p.impl ? score_lb_qimg_bytes(lb, K, d) : 0), 1024);
   *o_keys = off; off = align_up(off + (size_t)kparts * Q * TOPK_STRIDE * sizeof(tkey_t), 256);
@@ -977,7 +977,7 @@ static int score_topk_impl(int mode, const float* Pq, int64_t Q, int K, int d, i
   a.keys = (tkey_t*)(base + o_keys); a.counts = (int*)(base + o_cnt); a.dist_out = dist_out;
   a.cimg = nullptr; a.e2 = nullptr;
   a.phase = 0; a.tile_stride = 1; a.thr_init = nullptr;
-  a.dbg = nullptr; a.redo_tile = nullptr; a.spill = nullptr; a.spill_cnt = nullptr;
+  a.redo_tile = nullptr; a.spill = nullptr; a.spill_cnt = nullptr;
   a.cimg16 = nullptr; a.qimg16 = nullptr; a.cflag16 = nullptr; a.qflag16 = nullptr; a.lbrow = nullptr; a.lbq = nullptr;
   bool lb_pass = false;
   const float* redo_only = nullptr;
@@ -1000,7 +1000,7 @@ static int score_topk_impl(int mode, const float* Pq, int64_t Q, int K, int d, i
         image = base + o_cimg;
       }
       a.cimg = image;
-      a.e2 = (const float*)((const char*)image + (size_t)plan.tiles * (plan.dpad / 8) * 8192);
+      a.e2 = (const float*)((const char*)image + catalog_e2_offset(N, d));
       a.cimg16 = (const char*)image + catalog_f16_offset(N, d);
       a.cflag16 = (const int*)((const char*)a.cimg16 + catalog_f16_bytes(N, d));
       a.lbrow = (const float2*)((const char*)image + catalog_lbrow_offset(N, d));

@@ -61,10 +61,10 @@ struct ScoreArgs {
   const int* qflag16;
   const float2* lbrow;
   const float* lbq;
-  int dbg_mode;          // experiments (CFL_SCORE_DBG_MODE bits): 1 = epilogue does nothing, 2 = no TMA / no full-barrier
-                         // waits, 4 = lower-bound epilogue only reads TMEM, 8 = TMEM reads + bound, no pushes, 16 = MMA issue does
-                         // not wait for the epilogue (honoured only under CFL_EXPERIMENTS=1)
-  unsigned long long* dbg; // optional counters {groups seen, skipped, selective, full} (CFL_SCORE_DEBUG)
+  int dbg_mode;          // timing experiments of the lower-bound pass (CFL_SCORE_DBG_MODE bits, score_lb_kernel built with
+                         // -DCFL_LB_EXPERIMENTS): 1 = epilogue does nothing, 2 = no TMA / no full-barrier waits, 4 = epilogue
+                         // only reads TMEM, 8 = TMEM reads + bound, no pushes, 16 = MMA issue does not wait for the epilogue
+                         // (honoured only under CFL_EXPERIMENTS=1)
   ScorePlan plan;
   LbPlan lb;
 };
@@ -93,9 +93,13 @@ __host__ __device__ constexpr int qplane_stride(int K) {
 }
 constexpr float CFL_PLANE_REL = 2.0e-4f;     // relative safety margin of the bound (fp32 / 3xTF32 rounding)
 
+// Bytes of one query tile's tcgen05 B-operand image (score_umma.cu): [kstep][hl][chunk][nc = K*qt rows][16 B].
+__host__ __device__ constexpr uint32_t qimg_tile_bytes(int dpad, int nc) { return (uint32_t)dpad * 8u * (uint32_t)nc; }
+
 ScorePlan make_score_plan(int64_t Q, int K, int d, int64_t N, int k, bool umma_ok);
 bool score_umma_supported(int K, int d);
 size_t catalog_image_bytes(int64_t N, int d);
+size_t catalog_e2_offset(int64_t N, int d);      // byte offset of |e - mu|^2 per row (float, padded to whole tiles)
 size_t catalog_f16_offset(int64_t N, int d);     // byte offset of the fp16 plane inside the catalog image
 size_t catalog_f16_bytes(int64_t N, int d);      // plane only; the flag word follows it
 size_t catalog_lbrow_offset(int64_t N, int d);   // byte offset of lbrow[tiles*128] (float2) inside the catalog image
@@ -103,7 +107,6 @@ LbPlan make_lb_plan(int64_t Q, int K, int d, int64_t tiles);
 size_t score_lb_qimg_bytes(const LbPlan& p, int K, int d);   // lower-bound image + flag word + lbq
 int catalog_pack_launch(const float* E, int64_t N, int d, int64_t lde, const float* mu, void* image,
                         cudaStream_t st);
-size_t score_umma_qimg_bytes(const ScorePlan& p, int K);
 int score_umma_pack_queries(const ScoreArgs& a, void* qimg, cudaStream_t st);
 int score_lb_prep_queries(const ScoreArgs& a, cudaStream_t st);   // lower-bound image + lbq of the query batch
 int score_umma_launch(const ScoreArgs& a, cudaStream_t st);

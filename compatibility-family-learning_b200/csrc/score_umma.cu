@@ -1,43 +1,26 @@
-// Fused all-pairs scoring kernel for sm_100a: Gram-form GEMM on tcgen05 tensor cores (3xTF32,
-// fp32 accumulators in TMEM), soft-min epilogue and running per-query top-k behind the MMA; the
-// Q x N score matrix never reaches HBM.
+// Fused all-pairs scoring kernel for sm_100a: the Gram pipeline of gram_pipe.cuh (3xTF32 tcgen05.mma into double-
+// buffered TMEM accumulators) with a soft-min epilogue and running per-query top-k behind the MMA; the Q x N score matrix
+// never reaches HBM.
 //
-//   D[c, k*QT + q] = e_c . p_{q,k}        M = 128 catalog rows (TMEM lanes), N = K*QT columns,
-//                                         MMA-K = the embedding dimension d (8 per K-step)
-//
-// Both operands are consumed as pre-split (hi, lo) tf32 images in the canonical K-major
-// SWIZZLE_NONE layout (umma.cuh):
-//   * the CATALOG image is built once per catalog by cfl_catalog_pack (centred on mu, split,
-//     one 8 KB block per (tile, K-step), plus |e|^2 per row) -- the catalog is static across
-//     query batches, so no per-query work is spent on it;
-//   * the QUERY image of the CTA's query tile (<= 96 KB) is packed per call and stays resident
-//     in shared memory for the whole kernel.
-// CTA (part, qtile) streams its contiguous range of 128-row catalog tiles.  Warp-specialised:
-//   warp  NEPI    one lane issues tcgen05.mma (3 per K-step) and tcgen05.commit
-//   warp  NEPI+1  one lane drives the TMA engine: cp.async.bulk of the query image, then one
-//                 8 KB catalog block per ring stage (mbarrier expect_tx / complete_tx)
-//   warps 0..NEPI-1  epilogue: tcgen05.ld of the K Gram values of 8 (16) queries for the thread's
-//                 catalog row, soft-min distance (score.cuh), threshold test, warp-aggregated push
-//                 into the per-query buffers (topk.cuh).  Accumulators are double-buffered in
-//                 TMEM so the epilogue of tile t overlaps the MMAs of tile t+1.
+// Both operands are consumed as pre-split (hi, lo) tf32 images in the canonical K-major SWIZZLE_NONE layout (umma.cuh),
+// both laid out by this file:
+//   * the CATALOG image is built once per catalog by cfl_catalog_pack (centred on mu, split, one 8 KB block per (tile,
+//     K-step), plus |e|^2 per row and the lower-bound pass's planes) -- the catalog is static across query batches, so
+//     no per-query work is spent on it;
+//   * the QUERY image of the CTA's query tile (<= 96 KB) is packed per call and stays resident in shared memory for the
+//     whole kernel.
+// Epilogue (16 warps): the K Gram values of a group of 4, 8 or 16 queries for the thread's catalog row, the affine-hull
+// lower bound and the soft-min distance (score.cuh), threshold test, warp-aggregated push into the per-query buffers
+// (topk.cuh), cooperative compaction of over-full buffers.
 // Work per score: 2*K*d flops (x3 MMAs); catalog bytes per row per query tile: 8*dpad + 4.
 #include <cuda_fp16.h>
-#include "score.cuh"
-#include "umma.cuh"
+#include "gram_pipe.cuh"
 
 namespace cfl {
 
 using namespace umma;
 
-#ifndef CFL_SU_NEPI
-#define CFL_SU_NEPI 16
-#endif
-constexpr int SU_NEPI = CFL_SU_NEPI;                // epilogue warps (a multiple of 4: TMEM lane quarters)
-constexpr int SU_THREADS = (SU_NEPI + 2) * 32;
-constexpr int SU_EPI_THREADS = SU_NEPI * 32;
-constexpr int SU_NSTAGE = 6;                        // ring stages of up to 2 K-steps (16 KB) each
-constexpr uint32_t SU_ASTAGE = 4u * 128u * 16u;     // [hl][chunk][128 rows][16 B] = 8 KB
-constexpr size_t SU_B_BUDGET = 96 * 1024;
+constexpr size_t SU_B_BUDGET = 96 * 1024;             // query image per CTA
 
 int score_umma_qt(int K, int d) {
   if (K < 1 || K > CFL_MAX_K || d < 1 || d > 128) return 0;
@@ -47,7 +30,7 @@ int score_umma_qt(int K, int d) {
   for (int qt : cand) {
     int nc = K * qt;
     if (nc > 256 || nc % 16 != 0 || qt % gq != 0) continue;
-    if ((size_t)dpad * nc * 8 > SU_B_BUDGET) continue;
+    if (qimg_tile_bytes(dpad, nc) > SU_B_BUDGET) continue;
     return qt;
   }
   return 0;
@@ -58,22 +41,19 @@ bool score_umma_supported(int K, int d) {
   return score_umma_qt(K, d) != 0;
 }
 
-size_t score_umma_qimg_bytes(const ScorePlan& p, int K) {      // tf32 hi/lo query image
-  return (size_t)p.nqt * p.dpad * 8 * (size_t)(K * p.qt);
-}
-
 // ---- catalog image ----------------------------------------------------------------------------
 // [tile][kstep][hl][chunk][row 0..127][4 floats]  (8 KB per (tile,kstep)), then e2[tiles*128].
 // ... then the fp16 plane of the lower-bound pass: [tile][kstep16][chunk 0|1][row 0..127][8 halfs] (4 KB per
 // (tile, 16 columns)), then one flag word (non-zero: a centred value left the fp16 range, plane unusable).
+size_t catalog_e2_offset(int64_t N, int d) {
+  return (size_t)((N + 127) / 128) * ((d + 7) / 8) * GP_ASTAGE;
+}
 size_t catalog_f16_offset(int64_t N, int d) {
-  const int64_t tiles = (N + 127) / 128;
-  const int nks = (d + 7) / 8;
-  return (size_t)tiles * nks * SU_ASTAGE + (size_t)tiles * 128 * sizeof(float);
+  return catalog_e2_offset(N, d) + (size_t)((N + 127) / 128) * 128 * sizeof(float);
 }
 size_t catalog_f16_bytes(int64_t N, int d) {
   const int64_t tiles = (N + 127) / 128;
-  return (size_t)tiles * ((d + 15) / 16) * (SU_ASTAGE / 2);
+  return (size_t)tiles * ((d + 15) / 16) * (GP_ASTAGE / 2);
 }
 // ... then lbrow[tiles*128] float2 = (|e - mu|^2, |e - mu|) per row, (+inf, 0) for the padding rows of the last tile:
 // what the lower-bound pass needs per row (its margin has a term in |e|), one 8-byte load per row and tile.
@@ -107,7 +87,7 @@ pack_catalog_kernel(const float* __restrict__ E, int64_t N, int d, int64_t lde,
     float4 h0, l0, h1, l1;
     split_tf32x4(make_float4(v[0], v[1], v[2], v[3]), h0, l0);
     split_tf32x4(make_float4(v[4], v[5], v[6], v[7]), h1, l1);
-    unsigned char* st = img + ((size_t)tile * nks + ks) * SU_ASTAGE;
+    unsigned char* st = img + ((size_t)tile * nks + ks) * GP_ASTAGE;
     *(float4*)(st + ((0 * 2 + 0) * 128 + r) * 16) = h0;
     *(float4*)(st + ((0 * 2 + 1) * 128 + r) * 16) = h1;
     *(float4*)(st + ((1 * 2 + 0) * 128 + r) * 16) = l0;
@@ -116,11 +96,11 @@ pack_catalog_kernel(const float* __restrict__ E, int64_t N, int d, int64_t lde,
     __align__(16) __half h[8];
 #pragma unroll
     for (int jj = 0; jj < 8; ++jj) { h[jj] = __float2half_rn(v[jj]); vmax = fmaxf(vmax, fabsf(v[jj])); }
-    unsigned char* st16 = img16 + ((size_t)tile * nks16 + (ks >> 1)) * (SU_ASTAGE / 2);
+    unsigned char* st16 = img16 + ((size_t)tile * nks16 + (ks >> 1)) * (GP_ASTAGE / 2);
     *(uint4*)(st16 + ((ks & 1) * 128 + r) * 16) = *(const uint4*)h;
   }
   if (nks & 1) {                                             // odd number of 8-column steps: zero the last half K-step
-    unsigned char* st16 = img16 + ((size_t)tile * nks16 + (nks >> 1)) * (SU_ASTAGE / 2);
+    unsigned char* st16 = img16 + ((size_t)tile * nks16 + (nks >> 1)) * (GP_ASTAGE / 2);
     *(uint4*)(st16 + (1 * 128 + r) * 16) = make_uint4(0u, 0u, 0u, 0u);
   }
   e2g[row] = e2;
@@ -131,9 +111,8 @@ pack_catalog_kernel(const float* __restrict__ E, int64_t N, int d, int64_t lde,
 int catalog_pack_launch(const float* E, int64_t N, int d, int64_t lde, const float* mu, void* image,
                         cudaStream_t st) {
   const int64_t tiles = (N + 127) / 128;
-  const int nks = (d + 7) / 8;
   unsigned char* img = (unsigned char*)image;
-  float* e2g = (float*)(img + (size_t)tiles * nks * SU_ASTAGE);
+  float* e2g = (float*)(img + catalog_e2_offset(N, d));
   unsigned char* img16 = img + catalog_f16_offset(N, d);
   int* flag16 = (int*)(img16 + catalog_f16_bytes(N, d));
   CFL_CUDA(cudaMemsetAsync(flag16, 0, 16, st));
@@ -143,23 +122,17 @@ int catalog_pack_launch(const float* E, int64_t N, int d, int64_t lde, const flo
   return CFL_OK;
 }
 
-struct SuLayout {
-  uint32_t b_img, a_ring, scratch, qpar, qpl, thr, cnt, need, bars, tmem_slot, total;
-};
+// Shared memory of the exact kernel: the Gram pipeline's regions with the compaction scratch in front of the query blocks
+// and, behind them, running thresholds, key counts and compaction requests.
+struct SuLayout { GramLayout g; uint32_t thr, cnt, need; };
 __host__ __device__ inline SuLayout su_layout(int K, int qt, int dpad) {
   SuLayout L;
-  uint32_t off = 0;
-  L.b_img = off;   off += (uint32_t)dpad * 8u * (uint32_t)(K * qt);   off = (off + 1023u) & ~1023u;
-  L.a_ring = off;  off += SU_NSTAGE * 2u * SU_ASTAGE;
-  L.scratch = off; off += TOPK_STRIDE * 8u;
-  L.qpar = off;    off += (uint32_t)qt * (uint32_t)qpar_stride(K) * 4u;  off = (off + 15u) & ~15u;
-  L.qpl = off;     off += (uint32_t)qt * (uint32_t)qplane_stride(K) * 4u; off = (off + 15u) & ~15u;
+  L.g = gram_layout(K, qt, dpad, TOPK_STRIDE * 8u);
+  uint32_t off = L.g.back;
   L.thr = off;     off += (uint32_t)qt * 4u;
   L.cnt = off;     off += (uint32_t)qt * 4u;
-  L.need = off;    off += 16u;                                        off = (off + 15u) & ~15u;
-  L.bars = off;    off += (2u * SU_NSTAGE + 5u) * 8u;
-  L.tmem_slot = off; off += 16u;
-  L.total = off;
+  L.need = off;    off += 16u;
+  gram_layout_end(L.g, off);
   return L;
 }
 
@@ -169,7 +142,7 @@ __global__ void pack_queries_kernel(const float* __restrict__ Pc, int64_t Q, int
   const int nc = K * qt;
   const int nks = dpad / 8;
   const int qtile = blockIdx.x;
-  float* base = img + (size_t)qtile * dpad * 2 * nc;        // floats: dpad*8*nc bytes / 4
+  float* base = (float*)((char*)img + (size_t)qtile * qimg_tile_bytes(dpad, nc));
   for (int e = threadIdx.x; e < nks * 2 * nc; e += blockDim.x) {
     int n = e % nc;
     int c = (e / nc) % 2;
@@ -201,34 +174,22 @@ int score_umma_pack_queries(const ScoreArgs& a, void* qimg, cudaStream_t st) {
 }
 
 __device__ __forceinline__ void epi_bar_sync() {
-  asm volatile("bar.sync 1, %0;" ::"n"(SU_EPI_THREADS) : "memory");
+  asm volatile("bar.sync 1, %0;" ::"n"(GP_EPI_THREADS) : "memory");
 }
 
 // ---- the kernel ---------------------------------------------------------------------------
 template <int K>
-__global__ void __launch_bounds__(SU_THREADS, 1)
+__global__ void __launch_bounds__(GP_THREADS, 1)
 score_umma_kernel(ScoreArgs A) {
   extern __shared__ __align__(1024) unsigned char smem[];
-  constexpr int GQ = K <= 2 ? 16 : (K <= 4 ? 8 : 4);     // queries per epilogue group (register budget)
+  constexpr int GQ = gram_gq(K);
   const int QT = A.plan.qt;
-  const int NC = K * QT;
-  const int dpad = A.plan.dpad;
-  const int nks = dpad / 8;
-  const SuLayout L = su_layout(K, QT, dpad);
-  unsigned char* b_img = smem + L.b_img;
-  unsigned char* a_ring = smem + L.a_ring;
-  tkey_t* scratch = (tkey_t*)(smem + L.scratch);
-  float* qpar = (float*)(smem + L.qpar);
-  float* qpl = (float*)(smem + L.qpl);
+  const SuLayout L = su_layout(K, QT, A.plan.dpad);
+  const GramPipe P = gram_pipe(smem, L.g, K, QT, A.plan.dpad);
+  tkey_t* scratch = (tkey_t*)(smem + L.g.front);
   float* thr = (float*)(smem + L.thr);
   int* cnt = (int*)(smem + L.cnt);
   int* need = (int*)(smem + L.need);
-  uint64_t* full = (uint64_t*)(smem + L.bars);
-  uint64_t* empty = full + SU_NSTAGE;
-  uint64_t* tfull = empty + SU_NSTAGE;
-  uint64_t* tempty = tfull + 2;
-  uint64_t* bfull = tempty + 2;
-  uint32_t* tmem_slot = (uint32_t*)(smem + L.tmem_slot);
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int part = blockIdx.x, qtile = blockIdx.y;
@@ -241,42 +202,13 @@ score_umma_kernel(ScoreArgs A) {
   const int ts = A.tile_stride;                              // phase 1 visits every ts-th tile
   const int ntiles = (int)((t1 - t0 + ts - 1) / ts);
   const bool filter = A.phase == 2;
-  const int qps = qpar_stride(K);
-  const int kss = (nks % 2 == 0) ? 2 : 1;                    // K-steps per ring stage
 
   // ---- one-time setup ----
-  uint32_t ncols = 32;
-  while ((int)ncols < 2 * NC) ncols <<= 1;
-  if (warp == SU_NEPI) {
-    if (lane == 0) {
-      for (int s = 0; s < SU_NSTAGE; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-      mbar_init(&tfull[0], 1); mbar_init(&tfull[1], 1);
-      mbar_init(&tempty[0], SU_EPI_THREADS); mbar_init(&tempty[1], SU_EPI_THREADS);
-      mbar_init(bfull, 1);
-      fence_barrier_init();
-    }
-    __syncwarp();
-    tmem_alloc(tmem_slot, ncols);
-  }
-  // per-query blocks are stored interleaved by query PAIR: qpar[(pair*qps + j)*2 + (q&1)], with the
-  // first K entries negated, ready for the packed (FP32x2) epilogue
-  for (int i = tid; i < QT * qps; i += SU_THREADS) {
-    const int ql = i / qps, j = i % qps;
-    float v = (ql < nq) ? A.qpar[(q0 + ql) * qps + j] : 0.0f;
-    if (j < K) v = -v;
-    qpar[((ql >> 1) * qps + j) * 2 + (ql & 1)] = v;
-  }
-  {
-    const int pbs = qplane_stride(K);                        // same pair interleave for the plane blocks
-    for (int i = tid; i < QT * pbs; i += SU_THREADS) {
-      const int ql = i / pbs, j = i % pbs;
-      qpl[((ql >> 1) * pbs + j) * 2 + (ql & 1)] = (ql < nq) ? A.qplane[(q0 + ql) * pbs + j] : 0.0f;
-    }
-  }
+  gram_setup<K>(P, A.qpar, A.qplane, q0, nq, QT);
   // padding queries of the last tile get thr = -inf: they can never be pushed
   // phase 2: fixed thresholds from the sample pass, bumped one ulp so that the strict compare
   // below implements dist <= tau (every candidate tied with the bound must be kept)
-  for (int i = tid; i < QT; i += SU_THREADS) {
+  for (int i = tid; i < QT; i += GP_THREADS) {
     float th = __int_as_float(i < nq ? 0x7f800000 : 0xff800000);
     if (filter && i < nq && A.thr_init != nullptr) {
       const float tau = A.thr_init[q0 + i];
@@ -286,61 +218,15 @@ score_umma_kernel(ScoreArgs A) {
     cnt[i] = 0;
   }
   if (tid < 4) need[tid] = 0;
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t tmem_base = gram_start(P);
 
-  if (warp == SU_NEPI) {
-    // ================================ MMA issuer (one lane) =================================
-    if (elect_one()) {
-      mbar_wait(bfull, 0);
-      const Step3Desc sd = make_step3((uint32_t)NC, make_idesc_tf32(128, (uint32_t)NC));
-      const uint32_t a_base = smem_u32(a_ring), b_base = smem_u32(b_img);
-      const uint32_t b_step = 4u * (uint32_t)NC * 16u;
-      int stage = 0; uint32_t phase = 0;
-      for (int t = 0; t < ntiles; ++t) {
-        const int buf = t & 1;
-        mbar_wait(&tempty[buf], ((uint32_t)(t >> 1) & 1u) ^ 1u);
-        tc_fence_after();
-        const uint32_t d_tmem = tmem_base + (uint32_t)(buf * NC);
-        for (int ks = 0; ks < nks; ks += kss) {
-          if (!(A.dbg_mode & 2)) mbar_wait(&full[stage], phase);
-          tc_fence_after();
-          for (int j = 0; j < kss; ++j)
-            mma_step3(sd, d_tmem, a_base + (stage * 2 + j) * SU_ASTAGE, b_base + (ks + j) * b_step, ks + j == 0);
-          mma_commit(&empty[stage]);
-          if (++stage == SU_NSTAGE) { stage = 0; phase ^= 1u; }
-        }
-        mma_commit(&tfull[buf]);
-      }
-    }
-  } else if (warp == SU_NEPI + 1) {
-    // ================================ TMA producer (one lane) ===============================
-    if (elect_one()) {
-      const uint32_t bbytes = (uint32_t)dpad * 8u * (uint32_t)NC;
-      const unsigned char* qsrc = (const unsigned char*)A.qimg + (size_t)qtile * bbytes;
-      mbar_arrive_expect_tx(bfull, bbytes);
-      for (uint32_t o = 0; o < bbytes; o += 32768u) {
-        uint32_t n = bbytes - o < 32768u ? bbytes - o : 32768u;
-        bulk_g2s(b_img + o, qsrc + o, n, bfull);
-      }
-      int stage = 0; uint32_t phase = 0;
-      for (int t = 0; t < ((A.dbg_mode & 2) ? 0 : ntiles); ++t) {
-        const unsigned char* src = (const unsigned char*)A.cimg + (size_t)(t0 + (int64_t)t * ts) * nks * SU_ASTAGE;
-        for (int ks = 0; ks < nks; ks += kss) {
-          mbar_wait(&empty[stage], phase ^ 1u);
-          mbar_arrive_expect_tx(&full[stage], (uint32_t)kss * SU_ASTAGE);
-          bulk_g2s(a_ring + stage * 2 * SU_ASTAGE, src + (size_t)ks * SU_ASTAGE, (uint32_t)kss * SU_ASTAGE, &full[stage]);
-          if (++stage == SU_NSTAGE) { stage = 0; phase ^= 1u; }
-        }
-      }
-    }
+  if (warp == GP_NEPI) {
+    gram_mma(P, tmem_base, ntiles);
+  } else if (warp == GP_NEPI + 1) {
+    gram_tma(P, A.qimg, qtile, A.cimg, t0, ts, ntiles);
   } else {
     // ======================================= epilogue ========================================
     constexpr int QPS = qpar_stride(K);
-    constexpr int CQ = K + qpar_tri(K);
-    constexpr int WPQ = SU_NEPI / 4;                         // warps per TMEM lane quarter
     const int lq = warp & 3, sub = warp >> 2;
     const int lrow = lq * 32 + lane;
     const uint32_t lane_lt = (1u << lane) - 1u;
@@ -355,18 +241,13 @@ score_umma_kernel(ScoreArgs A) {
     constexpr int PBS = qplane_stride(K);
     bool bound_on = (K > 1) && !dense;
     int grp_seen = 0, grp_skipped = 0;
-    unsigned dbg_seen = 0, dbg_skip = 0, dbg_sel = 0, dbg_full = 0;
     for (int t = 0; t < ntiles; ++t) {
-      const int buf = t & 1;
       const int64_t row = (t0 + (int64_t)t * ts) * 128 + lrow;
       const bool valid = row < A.N;
       const float e2 = __ldg(A.e2 + row);                    // padded to whole tiles
-      mbar_wait(&tfull[buf], (uint32_t)(t >> 1) & 1u);
-      tc_fence_after();
-      const uint32_t taddr = tmem_base + ((uint32_t)(lq * 32) << 16) + (uint32_t)(buf * NC);
+      const uint32_t taddr = gram_acquire(P, tmem_base, t, lq);
       const int nslot = filter ? 2 + ((t >> 2) & 1) : (t & 1);
       const int trig = filter ? TOPK_STRIDE / 2 : TOPK_TRIGGER;
-      if (A.dbg_mode & 1) { tc_fence_before(); mbar_arrive(&tempty[buf]); continue; }
       // push the passing lanes of query ql (warp-uniform call) into its key buffer
       auto push = [&](int ql, bool pass, float dv) {
         const uint32_t m = __ballot_sync(0xffffffffu, pass);
@@ -380,16 +261,10 @@ score_umma_kernel(ScoreArgs A) {
         basei = __shfl_sync(0xffffffffu, basei, leader);
         if (pass) kbase[(int64_t)ql * TOPK_STRIDE + basei + __popc(m & lane_lt)] = pack_key(dv, (uint32_t)row);
       };
-      for (int g = sub; g * GQ < nq; g += WPQ) {
+      for (int g = sub; g * GQ < nq; g += GP_WPQ) {
         float gk[K][GQ];
-#pragma unroll
-        for (int k = 0; k < K; ++k) {
-          if constexpr (GQ == 16)     tmem_ld16(taddr + (uint32_t)(k * QT + g * GQ), gk[k]);
-          else if constexpr (GQ == 8) tmem_ld8(taddr + (uint32_t)(k * QT + g * GQ), gk[k]);
-          else                        tmem_ld4(taddr + (uint32_t)(k * QT + g * GQ), gk[k]);
-        }
-        tmem_ld_wait();
-        const float* qg = qpar + g * GQ * QPS;                 // GQ/2 pair blocks of 2*QPS floats
+        gram_load_group<K, GQ>(taddr, QT, g, gk);
+        const float* qg = P.qpar + g * GQ * QPS;               // GQ/2 pair blocks of 2*QPS floats
         float tg[GQ];
 #pragma unroll
         for (int i = 0; i < GQ; i += 4) {
@@ -405,24 +280,21 @@ score_umma_kernel(ScoreArgs A) {
 #pragma unroll
             for (int pi = 0; pi < GQ / 2; ++pi) {
               f2_t pv[PBS];
-              const ulonglong2* src = (const ulonglong2*)(qpl + (g * (GQ / 2) + pi) * PBS * 2);
-#pragma unroll
-              for (int j = 0; j < PBS; j += 2) { const ulonglong2 u = src[j >> 1]; pv[j] = u.x; pv[j + 1] = u.y; }
+              load_pair_block<PBS>(P.qpl + (g * (GQ / 2) + pi) * PBS * 2, pv);
               float gA[K], gB[K];
 #pragma unroll
               for (int k = 0; k < K; ++k) { gA[k] = gk[k][2 * pi]; gB[k] = gk[k][2 * pi + 1]; }
               plane_bound_pair<K>(gA, gB, e2sp, pv, lb[2 * pi], lb[2 * pi + 1]);
               nd |= (lb[2 * pi] < tg[2 * pi]) | (lb[2 * pi + 1] < tg[2 * pi + 1]);
             }
-            ++grp_seen; ++dbg_seen;
-            if (!__any_sync(0xffffffffu, nd && valid)) { ++grp_skipped; ++dbg_skip; continue; }
+            ++grp_seen;
+            if (!__any_sync(0xffffffffu, nd && valid)) { ++grp_skipped; continue; }
             uint32_t nb = 0;
 #pragma unroll
             for (int i = 0; i < GQ; ++i) nb |= (lb[i] < tg[i]) ? (1u << i) : 0u;
             if (!valid) nb = 0;
             const uint32_t anyn = __reduce_or_sync(0xffffffffu, nb);
             if (__popc(anyn) <= GQ / 4) {                      // a few queries: soft-min only for those
-              ++dbg_sel;
 #pragma unroll
               for (int i = 0; i < GQ; ++i) {
                 if (anyn & (1u << i)) {                        // warp-uniform
@@ -437,14 +309,11 @@ score_umma_kernel(ScoreArgs A) {
             }
           }
         }
-        ++dbg_full;
         float dist[GQ];
 #pragma unroll
         for (int pi = 0; pi < GQ / 2; ++pi) {
           f2_t qv[QPS];
-          const ulonglong2* src = (const ulonglong2*)(qg + pi * QPS * 2);
-#pragma unroll
-          for (int j = 0; j < QPS; j += 2) { const ulonglong2 u = src[j >> 1]; qv[j] = u.x; qv[j + 1] = u.y; }
+          load_pair_block<QPS>(qg + pi * QPS * 2, qv);
           float gA[K], gB[K];
 #pragma unroll
           for (int k = 0; k < K; ++k) { gA[k] = gk[k][2 * pi]; gB[k] = gk[k][2 * pi + 1]; }
@@ -473,8 +342,7 @@ score_umma_kernel(ScoreArgs A) {
         if (!filter && t == 15) { grp_seen = 0; grp_skipped = 0; }
         if (t == (filter ? 15 : 31) && grp_skipped * 2 < grp_seen) bound_on = false;
       }
-      tc_fence_before();
-      mbar_arrive(&tempty[buf]);
+      gram_release(P, t);
       // ---- compaction point: all epilogue warps sort one over-full buffer together ----
       // adaptive phases: checked every tile (a tile adds <= 128 keys per query, buffers hold 512);
       // filter phase: every 4th tile (<= 512 new keys, buffers hold 1024) and it almost never fires.
@@ -490,9 +358,9 @@ score_umma_kernel(ScoreArgs A) {
             for (uint32_t m = over; m; m &= m - 1) {          // identical in every warp
               const int ql = qb + __ffs(m) - 1;
               if (filter) {
-                coop_compact_big<SU_EPI_THREADS>(kbase + (int64_t)ql * TOPK_STRIDE, cnt[ql], A.plan.kk, scratch, tid, &cnt[ql], &thr[ql]);
+                coop_compact_big<GP_EPI_THREADS>(kbase + (int64_t)ql * TOPK_STRIDE, cnt[ql], A.plan.kk, scratch, tid, &cnt[ql], &thr[ql]);
               } else {
-                coop_compact<SU_EPI_THREADS>(kbase + (int64_t)ql * TOPK_STRIDE, cnt[ql], A.plan.kk, scratch, tid, &cnt[ql], &thr[ql]);
+                coop_compact<GP_EPI_THREADS>(kbase + (int64_t)ql * TOPK_STRIDE, cnt[ql], A.plan.kk, scratch, tid, &cnt[ql], &thr[ql]);
               }
             }
           }
@@ -501,37 +369,29 @@ score_umma_kernel(ScoreArgs A) {
         }
       }
     }
-    if (A.dbg != nullptr && lane == 0) {
-      atomicAdd(&A.dbg[0], (unsigned long long)dbg_seen); atomicAdd(&A.dbg[1], (unsigned long long)dbg_skip);
-      atomicAdd(&A.dbg[2], (unsigned long long)dbg_sel);  atomicAdd(&A.dbg[3], (unsigned long long)dbg_full);
-    }
     if (!filter) {
       for (int ql = 0; ql < nq; ++ql) {
-        coop_compact<SU_EPI_THREADS>(kbase + (int64_t)ql * TOPK_STRIDE, cnt[ql], A.plan.kk, scratch, tid, &cnt[ql], nullptr);
+        coop_compact<GP_EPI_THREADS>(kbase + (int64_t)ql * TOPK_STRIDE, cnt[ql], A.plan.kk, scratch, tid, &cnt[ql], nullptr);
         if (tid == 0) A.counts[(int64_t)part * A.Q + q0 + ql] = cnt[ql];
       }
     } else {
       epi_bar_sync();                                         // all pushes done; lists stay unsorted
-      for (int ql = tid; ql < nq; ql += SU_EPI_THREADS) {
+      for (int ql = tid; ql < nq; ql += GP_EPI_THREADS) {
         // a redo launch restarts only the queries it was asked to redo (thr_init > -inf)
         if (redo && !(A.thr_init[q0 + ql] > __int_as_float(0xff800000))) continue;
         A.counts[(int64_t)part * A.Q + q0 + ql] = cnt[ql];
       }
     }
   }
-  // ---- teardown ----
-  tc_fence_before();
-  __syncthreads();
-  if (warp == SU_NEPI) tmem_dealloc(tmem_base, ncols);
+  gram_finish(P, tmem_base);
 }
 
 template <int K>
 static int launch_umma(const ScoreArgs& a, cudaStream_t st) {
-  SuLayout L = su_layout(K, a.plan.qt, a.plan.dpad);
-  size_t smem = L.total + 1024;      // slack for the alignment of the dynamic segment
+  size_t smem = su_layout(K, a.plan.qt, a.plan.dpad).g.total + 1024;      // slack for the alignment of the dynamic segment
   CFL_SMEM_LIMIT(score_umma_kernel<K>, smem);
   dim3 grid(a.plan.parts, a.plan.nqt);
-  score_umma_kernel<K><<<grid, SU_THREADS, smem, st>>>(a);
+  score_umma_kernel<K><<<grid, GP_THREADS, smem, st>>>(a);
   CFL_LAUNCH_CHECK();
   return CFL_OK;
 }
