@@ -140,6 +140,29 @@ def _rows(t, name):
     return t, (t.stride(0) if t.shape[0] > 1 else t.shape[1])
 
 
+def _out(t, shape, name, dense=False):
+    """A caller's output buffer -> (buffer the kernel writes, caller's tensor or None).
+
+    The kernel writes the first of the pair.  When the caller's tensor cannot be written in place (not row-major with
+    unit inner stride, or not dense where ``dense``), the first is a dense copy of it (so accumulating kernels see its
+    values) and the second is the tensor that ``_copy_back`` refreshes after the call.  A wrong dtype, device or shape
+    raises: the buffer would otherwise be left stale or written out of bounds."""
+    t = _f32c(t, name)
+    shape = tuple(int(s) for s in shape)
+    if tuple(t.shape) != shape:
+        raise CflNativeError(f"{name} must have shape {shape}, got {tuple(t.shape)}")
+    if dense:
+        ok = t.is_contiguous()
+    else:
+        ok = t.dim() == 2 and (t.numel() == 0 or (t.stride(1) == 1 and (t.shape[0] <= 1 or t.stride(0) >= t.shape[1])))
+    return (t, None) if ok else (t.contiguous(), t)
+
+
+def _copy_back(buf, caller):
+    if caller is not None:
+        caller.copy_(buf.view(caller.shape))
+
+
 class _WorkspaceCache:
     """One growing byte buffer per (device, stream) -- the C ABI never allocates."""
 
@@ -208,13 +231,20 @@ def project_bwd(x, V, g, bias, weight_norm, in_scale, act, y, z, dy, dV=None, dg
         dg = torch.empty(N, dtype=torch.float32, device=dev)
     if dbias is None and want_dbias:
         dbias = torch.empty(N, dtype=torch.float32, device=dev)
+    # the kernels write dense [F, N] / [N] float32 buffers (and read them back when accumulating)
+    dV_k, dV_c = _out(dV, (F, N), "dV", dense=True)
+    dg_k, dg_c = (None, None) if dg is None else _out(dg, (N,), "dg", dense=True)
+    db_k, db_c = (None, None) if dbias is None else _out(dbias, (N,), "dbias", dense=True)
     nws = lib().cfl_project_bwd_workspace_bytes(B, F, N)
     ws = _ws.get(nws, dev)
     _check(lib().cfl_project_bwd(_ptr(x), B, F, ldx, _ptr(V), N, ldV, _ptr(g), _ptr(bias),
                                  1 if weight_norm else 0, float(in_scale), ACTS[act], _ptr(y), ldy,
-                                 _ptr(z), _ptr(dy), lddy, _ptr(dV), _ptr(dg), _ptr(dbias),
+                                 _ptr(z), _ptr(dy), lddy, _ptr(dV_k), _ptr(dg_k), _ptr(db_k),
                                  1 if accumulate else 0, float(reg_c), _ptr(ws), ws.numel(), _stream()),
            "cfl_project_bwd")
+    _copy_back(dV_k, dV_c)
+    _copy_back(dg_k, dg_c)
+    _copy_back(db_k, db_c)
     return dV, dg, dbias
 
 
@@ -260,8 +290,17 @@ def pair_loss_bwd(mode, a, P, w=None, theta=None, label=1, margin=0.0, c_ce=0.0,
         da = torch.empty(B, d, dtype=torch.float32, device=dev)
     if dP is None:
         dP = torch.empty(B, K * d, dtype=torch.float32, device=dev)
-    da2, ldda = _rows(da, "da")
-    dP2, lddP = _rows(dP.reshape(B, K * d), "dP")
+    # caller buffers the kernel cannot write in place (e.g. transposed) receive the result by copy-back
+    da2, da_c = _out(da, (B, d), "da")
+    dP = _f32c(dP, "dP")
+    if tuple(dP.shape) not in ((B, K, d), (B, K * d)):
+        raise CflNativeError(f"dP must have shape {(B, K, d)} or {(B, K * d)}, got {tuple(dP.shape)}")
+    try:
+        dP2, dP_c = _out(dP.view(B, K * d), (B, K * d), "dP")
+    except RuntimeError:                                     # no [B, K*d] view of the caller's buffer
+        dP2, dP_c = dP.reshape(B, K * d).contiguous(), dP
+    ldda = da2.stride(0) if B > 1 else d
+    lddP = dP2.stride(0) if B > 1 else K * d
     dw = torch.empty(B, K, dtype=torch.float32, device=dev) if mode == "monomer" else None
     dth = torch.empty(1, dtype=torch.float64, device=dev) if want_dtheta else None
     w = None if w is None else _f32c(w, "w").contiguous()
@@ -272,6 +311,8 @@ def pair_loss_bwd(mode, a, P, w=None, theta=None, label=1, margin=0.0, c_ce=0.0,
                                    float(c_margin), _ptr(ddist), _ptr(da2), ldda, _ptr(dP2), lddP,
                                    _ptr(dw), _ptr(dth), _ptr(ws), ws.numel(), _stream()),
            "cfl_pair_loss_bwd")
+    _copy_back(da2, da_c)
+    _copy_back(dP2, dP_c)
     return da, dP.reshape(B, K, d) if dP.dim() == 2 else dP, dw, dth
 
 

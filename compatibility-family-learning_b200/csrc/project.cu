@@ -6,8 +6,10 @@
 //           (project_umma.cu) whenever the shape fits its tiling (F % 8 == 0, 16-byte aligned
 //           rows, N <= 256); the fp32 CUDA-core tile kernel below covers the remaining shapes
 //           (tiny / odd F) and is the reference point for the tensor-core kernel's parity test.
-// Backward: dV = x^T dpre with the weight-norm column terms (SURVEY App. A.5), fp32 CUDA cores,
-//           batch split into slabs and reduced in a fixed order (deterministic).
+// Backward: dV = x^T dpre with the weight-norm column terms (SURVEY App. A.5).  The GEMM runs on tcgen05
+//           tensor cores as 3xTF32 (project_bwd_umma.cu) for B >= 256 and N <= 256; the fp32 CUDA-core
+//           kernel below covers the rest.  Both split the batch into slabs reduced in a fixed order
+//           (deterministic).
 #include "common.cuh"
 
 namespace cfl {

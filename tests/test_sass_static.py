@@ -73,3 +73,19 @@ def test_bench_step_kernels_do_not_spill(census):
     spill_free += [f"cfl::project_bwd_umma_tma_kernel<{S}, {wn}>" for S in (1, 2, 4) for wn in ("false", "true")]
     for k in spill_free:
         assert census[k]["STL"] == 0 and census[k]["LDL"] == 0, f"{k}: local-memory traffic (STL {census[k]['STL']}, LDL {census[k]['LDL']})"
+
+
+def test_every_projection_and_pair_kernel_has_a_path_test(census):
+    """Every projection / paired-loss kernel in the library is reached by a case of tests/test_kernel_paths_gpu.py (its
+    KERNEL_TABLE) or allowed there with a reason: a dispatch path added without a parity case fails here, without a GPU."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("kernel_paths", os.path.join(ROOT, "tests", "test_kernel_paths_gpu.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    family = re.compile(r"cfl::(project_\w+|pair_\w+|colnorm_kernel|colstats_\w+)(<.*>)?$")
+    ours = sorted(k for k in census if family.match(k))
+    assert len(ours) >= 60, f"census found only {ours}"
+    missing = [k for k in ours if k not in mod.KERNEL_TABLE and not any(p.fullmatch(k) for p in mod.KERNEL_ALLOW)]
+    assert not missing, f"kernels without a path case in test_kernel_paths_gpu.py: {missing}"
+    stale = [k for k in mod.KERNEL_TABLE if k not in census]
+    assert not stale, f"KERNEL_TABLE names kernels the library does not have: {stale}"
