@@ -5,6 +5,7 @@
 #include <stdio.h>
 #include <stdarg.h>
 #include <math.h>
+#include <type_traits>
 #include "cfl_b200.h"
 
 namespace cfl {
@@ -48,6 +49,25 @@ void timer_record(int which, cudaStream_t st);  // api.cu: 0 = start, 1 = stop (
   } while (0)
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
+
+// The one dispatch of a runtime K onto the kernels' compile-time K: f(std::integral_constant<int, K>{}) for K in
+// [1, CFL_MAX_K], CFL_ERR_UNSUPPORTED otherwise.  f returns a CFL status.
+template <class F>
+int with_k(int K, F&& f) {
+  static_assert(CFL_MAX_K == 8, "with_k lists K = 1..8");
+  switch (K) {
+    case 1: return f(std::integral_constant<int, 1>{});
+    case 2: return f(std::integral_constant<int, 2>{});
+    case 3: return f(std::integral_constant<int, 3>{});
+    case 4: return f(std::integral_constant<int, 4>{});
+    case 5: return f(std::integral_constant<int, 5>{});
+    case 6: return f(std::integral_constant<int, 6>{});
+    case 7: return f(std::integral_constant<int, 7>{});
+    case 8: return f(std::integral_constant<int, 8>{});
+  }
+  set_error("K=%d outside [1,%d]", K, CFL_MAX_K);
+  return CFL_ERR_UNSUPPORTED;
+}
 
 // Bump allocator over the caller's workspace.
 struct Workspace {

@@ -565,7 +565,7 @@ static int rank_tc_prepare(const char* what, const float* Pq, int64_t Q, int K, 
   if (parts > a.tiles) parts = a.tiles;
   a.parts = (int)parts;
   a.qpar = qpar; a.qplane = qplane; a.qimg = base + w.qimg; a.cimg = image;
-  a.e2 = (const float*)((const char*)image + catalog_e2_offset(N, d));
+  a.e2 = catalog_view(image, N, d).e2;
   CFL_REQUIRE((int64_t)a.parts * a.nqt <= 4096, CFL_ERR_UNSUPPORTED, "%s: Q=%lld needs more than 4096 CTAs", what,
               (long long)Q);
   a.recs = (uint4*)(base + w.recs); a.rec_slice = rank_tc_rec_cap(Q, N) / (unsigned int)(a.parts * a.nqt);
@@ -615,16 +615,7 @@ int within_tc_emit(int mode, const float* Pq, int64_t Q, int K, int d, int64_t l
   a.J = 1; a.j0 = 0; a.thr = radius;
   a.offsets = offsets; a.cursor = cursor; a.out = out;
   CFL_CUDA(cudaMemsetAsync(a.rec_n, 0, 4096 * sizeof(unsigned int), cs));
-  switch (K) {
-    case 1: st = within_tc_launch<1>(a, Pq, ldq, E, lde, stats, cs); break;
-    case 2: st = within_tc_launch<2>(a, Pq, ldq, E, lde, stats, cs); break;
-    case 3: st = within_tc_launch<3>(a, Pq, ldq, E, lde, stats, cs); break;
-    case 4: st = within_tc_launch<4>(a, Pq, ldq, E, lde, stats, cs); break;
-    case 5: st = within_tc_launch<5>(a, Pq, ldq, E, lde, stats, cs); break;
-    case 6: st = within_tc_launch<6>(a, Pq, ldq, E, lde, stats, cs); break;
-    case 7: st = within_tc_launch<7>(a, Pq, ldq, E, lde, stats, cs); break;
-    default: st = within_tc_launch<8>(a, Pq, ldq, E, lde, stats, cs); break;
-  }
+  st = with_k(K, [&](auto KC) { return within_tc_launch<KC>(a, Pq, ldq, E, lde, stats, cs); });
   if (st != CFL_OK) return st;
   within_reset_flagged_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, cs>>>(a.only, Q, cursor, stats);
   CFL_LAUNCH_CHECK();
@@ -677,16 +668,7 @@ int cfl_rank_counts_packed(int mode, const float* Pq, int64_t Q, int K, int d, i
   for (int j0 = 0; j0 < J; j0 += RT_JC) {
     a.j0 = j0;
     CFL_CUDA(cudaMemsetAsync(a.rec_n, 0, 4096 * sizeof(unsigned int), cs));
-    switch (K) {
-      case 1: st = rank_tc_launch<1>(a, Pq, ldq, E, lde, stats, cs); break;
-      case 2: st = rank_tc_launch<2>(a, Pq, ldq, E, lde, stats, cs); break;
-      case 3: st = rank_tc_launch<3>(a, Pq, ldq, E, lde, stats, cs); break;
-      case 4: st = rank_tc_launch<4>(a, Pq, ldq, E, lde, stats, cs); break;
-      case 5: st = rank_tc_launch<5>(a, Pq, ldq, E, lde, stats, cs); break;
-      case 6: st = rank_tc_launch<6>(a, Pq, ldq, E, lde, stats, cs); break;
-      case 7: st = rank_tc_launch<7>(a, Pq, ldq, E, lde, stats, cs); break;
-      default: st = rank_tc_launch<8>(a, Pq, ldq, E, lde, stats, cs); break;
-    }
+    st = with_k(K, [&](auto KC) { return rank_tc_launch<KC>(a, Pq, ldq, E, lde, stats, cs); });
     if (st != CFL_OK) return st;
   }
   timer_record(1, cs);

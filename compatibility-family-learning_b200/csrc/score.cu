@@ -5,6 +5,7 @@
 // both kernels share the soft-min epilogue (score.cuh) and the top-k machinery (topk.cuh).
 #include <stdlib.h>
 #include "score.cuh"
+#include "direct.cuh"
 #include "umma.cuh"
 
 namespace cfl {
@@ -244,17 +245,17 @@ static int launch_simt(const ScoreArgs& a, cudaStream_t st) {
 }
 
 // ---- merge of the catalog parts + direct-form rescoring + final sort ---------------------
-// Exact distance of the kk survivors in direct-difference form (cfl/models/base.py:129-138
-// arithmetic) on the raw rows, then (value, index) order, best k written out.
-__global__ void __launch_bounds__(MRG_THREADS)
-merge_rescore_kernel(int mode, const tkey_t* __restrict__ keys, const int* __restrict__ counts,
-                     int parts, int64_t Q, int kk, int k, const float* __restrict__ Pq,
-                     int64_t ldq, int K, int d, const float* __restrict__ E, int64_t lde,
+// Exact distance of the kk survivors in direct-difference form (pcd_direct, direct.cuh: the arithmetic of
+// cfl/models/base.py:129-138) on the raw rows, then (value, index) order, best k written out.
+template <int K>
+__global__ void __launch_bounds__(MRG_THREADS, 8)            // 32 registers: eight blocks per SM
+merge_rescore_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ counts, int parts, int64_t Q, int kk, int k,
+                     const float* __restrict__ Pq, int64_t ldq, int d, const float* __restrict__ E, int64_t lde,
                      int64_t idx_base, float* __restrict__ top_val, int64_t* __restrict__ top_idx,
-                     const float* __restrict__ only_redo = nullptr,
+                     const float* __restrict__ only_redo,
                      // compact exact redo: blocks [Q, Q + cq) merge the compact tile's slots (own buffers, query map)
-                     int cq = 0, const tkey_t* __restrict__ ckeys = nullptr, const int* __restrict__ ccounts = nullptr,
-                     int cparts = 0, const float* __restrict__ cthr = nullptr, const int* __restrict__ cmap = nullptr) {
+                     int cq, const tkey_t* __restrict__ ckeys, const int* __restrict__ ccounts, int cparts,
+                     const float* __restrict__ cthr, const int* __restrict__ cmap) {
   __shared__ tkey_t s[TOPK_CAP];
   __shared__ int s_fill;
   __shared__ tkey_t s_thr;
@@ -274,29 +275,7 @@ merge_rescore_kernel(int mode, const tkey_t* __restrict__ keys, const int* __res
   if (t < fill) {
     const uint32_t idx = (uint32_t)(s[t] & 0xffffffffu);
     const float* e = E + (int64_t)idx * lde;
-    float dk[CFL_MAX_K];
-    float mn = 3.0e38f;
-    for (int kq = 0; kq < K; ++kq) {
-      float acc = 0.0f;
-      for (int j = 0; j < d; ++j) { float df = e[j] - pq[kq * d + j]; acc = fmaf(df, df, acc); }
-      dk[kq] = acc;
-      mn = fminf(mn, acc);
-    }
-    float dist;
-    if (K == 1) {
-      dist = dk[0];
-    } else {
-      float sum = 0.0f;
-      for (int kq = 0; kq < K; ++kq) { dk[kq] = expf(mn - dk[kq]); sum += dk[kq]; }
-      float inv = 1.0f / sum;
-      dist = 0.0f;
-      for (int j = 0; j < d; ++j) {
-        float m = 0.0f;
-        for (int kq = 0; kq < K; ++kq) m = fmaf(dk[kq] * inv, pq[kq * d + j], m);
-        float r = e[j] - m;
-        dist = fmaf(r, r, dist);
-      }
-    }
+    const float dist = pcd_direct<K, 1>([&](int j) { return e[j]; }, [&](int kq, int j) { return pq[kq * d + j]; }, d);
     s[t] = pack_key(dist, idx);
   }
   __syncthreads();
@@ -315,50 +294,23 @@ merge_rescore_kernel(int mode, const tkey_t* __restrict__ keys, const int* __res
 }
 
 // ---- merge after the lower-bound filter pass: EVERY surviving row is scored exactly -------------
-// The keys of score_lb_kernel carry a lower bound, not the distance, so nothing may be discarded
-// before its exact value is known: each thread evaluates the direct-difference form (the arithmetic
-// of cfl/models/base.py:129-138) of one (query, row), then the keys stream through the same
-// 512-slot selection as block_merge_topkk.  Output as merge_rescore_kernel.
-__device__ __forceinline__ float exact_softmin_dist(const float* __restrict__ e, const float* __restrict__ pq,
-                                                    int K, int d, int ldp) {
-  float dk[CFL_MAX_K];
-  float mn = 3.0e38f;
-  for (int kq = 0; kq < K; ++kq) {
-    float acc = 0.0f;
-    for (int j = 0; j < d; ++j) { float df = e[j] - pq[kq * ldp + j]; acc = fmaf(df, df, acc); }
-    dk[kq] = acc;
-    mn = fminf(mn, acc);
-  }
-  if (K == 1) return dk[0];
-  float sum = 0.0f;
-  for (int kq = 0; kq < K; ++kq) { dk[kq] = expf(mn - dk[kq]); sum += dk[kq]; }
-  const float inv = 1.0f / sum;
-  float dist = 0.0f;
-  for (int j = 0; j < d; ++j) {
-    float m = 0.0f;
-    for (int kq = 0; kq < K; ++kq) m = fmaf(dk[kq] * inv, pq[kq * ldp + j], m);
-    const float r = e[j] - m;
-    dist = fmaf(r, r, dist);
-  }
-  return dist;
-}
-
-// Stage 1 (all survivors): each warp stages 32 candidate rows through shared memory with coalesced
+// The keys of score_lb_kernel carry a lower bound, not the distance, so nothing may be discarded before its exact value
+// is known.  Stage 1 (all survivors): each warp stages 32 candidate rows through shared memory with coalesced
 // reads, 32 dimensions at a time; every thread then owns one row and accumulates d_k = |e - p_k|^2,
 // from which dist = sum_k s_k d_k - sum_{k<l} s_k s_l |p_k - p_l|^2 (the same quantity as the direct
 // form, SURVEY App. A.3, good to a few ulp) picks the kk best.  Stage 2 rescores those kk in the
-// direct-difference form and sorts by (value, index), exactly as merge_rescore_kernel does.
+// direct-difference form (pcd_direct) and sorts by (value, index), exactly as merge_rescore_kernel does.
 constexpr int RSC_CH = 16;                 // dimensions per staging chunk (small: 8 CTAs per SM = one wave)
 constexpr int RSC_LD = RSC_CH + 4;         // row stride in floats: 16 B aligned, conflict-free LDS.128
 
 template <int K>
-__global__ void __launch_bounds__(MRG_THREADS)
+__global__ void __launch_bounds__(MRG_THREADS, 4)            // 64 registers: four blocks per SM
 rescore_merge_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ counts, int parts, int64_t Q,
                      int kk, int k, const float* __restrict__ Pq, int64_t ldq, int d,
                      const float* __restrict__ E, int64_t lde, int64_t idx_base,
                      float* __restrict__ top_val, int64_t* __restrict__ top_idx,
                      const float* __restrict__ tau, const float* __restrict__ tau_opt, int qt,
-                     float* __restrict__ thr_redo, int* __restrict__ redo_tile, unsigned long long* __restrict__ dbg,
+                     float* __restrict__ thr_redo, int* __restrict__ redo_tile, unsigned long long* __restrict__ stats,
                      const tkey_t* __restrict__ spill, const int* __restrict__ spill_cnt,
                      const float* __restrict__ only_redo, const float* __restrict__ prev_redo,
                      float* __restrict__ second_round) {
@@ -370,7 +322,10 @@ rescore_merge_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ co
     if (threadIdx.x == 0) {
       const float pr = prev_redo[blockIdx.x];
       thr_redo[blockIdx.x] = pr;
-      if (pr > __int_as_float(0xff800000)) { redo_tile[blockIdx.x / qt] = 1; if (dbg) atomicAdd(&dbg[5], 1ull); }
+      if (pr > __int_as_float(0xff800000)) {
+        redo_tile[blockIdx.x / qt] = 1;
+        if (stats) atomicAdd(&stats[STAT_EXACT_REDO_QUERIES], 1ull);
+      }
     }
     return;
   }
@@ -502,13 +457,13 @@ rescore_merge_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ co
     // buffers, raised range flags or queries the probe took out (tau_opt = -inf)
     if (second_round)
       second_round[q] = (redo && !s_over && tau_opt[q] > __int_as_float(0xff800000)) ? tau[q] : __int_as_float(0xff800000);
-    if (dbg && only_redo != nullptr && redo) atomicAdd(&dbg[5], 1ull);
-    if (dbg && only_redo == nullptr) {                       // statistics of the call (cfl_score_topk_stats)
-      atomicAdd(&dbg[0], (unsigned long long)total);
-      if (spill_cnt[q] > 0) atomicAdd(&dbg[1], 1ull);
-      if (!(tau_opt[q] > __int_as_float(0xff800000))) atomicAdd(&dbg[2], 1ull);
-      if (redo) atomicAdd(&dbg[3], 1ull);
-      if (q == 0) dbg[4] = 1ull;
+    if (stats && only_redo != nullptr && redo) atomicAdd(&stats[STAT_EXACT_REDO_QUERIES], 1ull);
+    if (stats && only_redo == nullptr) {                     // statistics of the call (cfl_score_topk_stats)
+      atomicAdd(&stats[STAT_SURVIVORS], (unsigned long long)total);
+      if (spill_cnt[q] > 0) atomicAdd(&stats[STAT_SPILL_QUERIES], 1ull);
+      if (!(tau_opt[q] > __int_as_float(0xff800000))) atomicAdd(&stats[STAT_PROBE_DROPPED_QUERIES], 1ull);
+      if (redo) atomicAdd(&stats[STAT_REDO_QUERIES], 1ull);
+      if (q == 0) stats[STAT_LOWER_BOUND_PASS] = 1ull;
     }
   }
   __syncthreads();
@@ -539,10 +494,12 @@ rescore_merge_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ co
             }
           }
           __syncwarp();
-          if (mine) dist = exact_softmin_dist(rows + lane * ld2, s_pq, K, d, dp);
+          const float* er = rows + lane * ld2;
+          if (mine) dist = pcd_direct<K>([&](int j) { return er[j]; }, [&](int kq, int j) { return s_pq[kq * dp + j]; }, d);
         }
       } else if (mine) {                                     // very wide rows: straight from global memory
-        dist = exact_softmin_dist(E + (int64_t)idx * lde, s_pq, K, d, dp);
+        const float* er = E + (int64_t)idx * lde;
+        dist = pcd_direct<K>([&](int j) { return er[j]; }, [&](int kq, int j) { return s_pq[kq * dp + j]; }, d);
       }
       __syncthreads();
       if (mine) s[kidx] = pack_key(dist, idx);
@@ -567,26 +524,9 @@ rescore_merge_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ co
 // ---- thresholds from the sample pass ------------------------------------------------------
 // tau[q] = kk-th smallest distance among the sampled candidates of ALL parts.  Any subset's kk-th
 // best is an upper bound of the catalog's kk-th best, so every member of the final top-kk
-// satisfies dist <= tau[q].
-__global__ void __launch_bounds__(MRG_THREADS)
-sample_threshold_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ counts, int parts,
-                        int64_t Q, int kk, float* __restrict__ tau, float* __restrict__ tau_opt = nullptr,
-                        int r_opt = 0) {
-  __shared__ tkey_t s[TOPK_CAP];
-  __shared__ int s_fill;
-  __shared__ tkey_t s_thr;
-  const int64_t q = blockIdx.x;
-  const int fill = block_merge_topkk(keys, counts, parts, Q, q, kk, s, &s_fill, &s_thr);
-  if (threadIdx.x == 0) {
-    const float safe = (fill >= kk) ? ord2f((uint32_t)(s[kk - 1] >> 32)) : __int_as_float(0x7f800000);
-    tau[q] = safe;
-    // optimistic bound: the r_opt-th best of the 1/S sample.  About r_opt*S candidates of the whole
-    // range lie under it -- several times kk, but not guaranteed: verify_counts_kernel checks.
-    if (tau_opt) tau_opt[q] = (r_opt >= 1 && r_opt < kk && fill >= kk) ? ord2f((uint32_t)(s[r_opt - 1] >> 32)) : safe;
-  }
-}
-
-// Same thresholds by radix selection instead of sorting: only the VALUES of the kk-th and r_opt-th
+// satisfies dist <= tau[q].  The optimistic bound tau_opt[q] is the r_opt-th best of the 1/S sample: about r_opt*S
+// candidates of the whole range lie under it -- several times kk, but not guaranteed (the verification checks).
+// Radix selection: only the VALUES of the kk-th and r_opt-th
 // smallest distances are needed, so four 8-bit passes over the 32-bit ordered distances (staged in
 // shared memory when they fit) replace the ~20 cooperative sorts of block_merge_topkk.
 constexpr int SEL_THREADS = 1024;              // few blocks (one per query) when Q is small: they must be wide
@@ -693,16 +633,12 @@ select_threshold_kernel(const tkey_t* __restrict__ keys, const int* __restrict__
 // off or loose) is taken out of the lower-bound pass (tau_opt = -inf: nothing is pushed, verification
 // fails, the exact kernel redoes it) -- and a query tile with no live query costs nothing there.
 __global__ void probe_classify_kernel(const int* __restrict__ counts, int parts, int64_t Q, float scale,
-                                      float limit, float* __restrict__ tau_opt, unsigned long long* __restrict__ dbg,
-                                      const int* __restrict__ spill_cnt) {
+                                      float limit, float* __restrict__ tau_opt, const int* __restrict__ spill_cnt) {
   const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (q >= Q) return;
   long long tot = spill_cnt ? spill_cnt[q] : 0;
   for (int p = 0; p < parts; ++p) tot += counts[(int64_t)p * Q + q];
-  if ((float)tot * scale > limit) {
-    tau_opt[q] = __int_as_float(0xff800000);
-    (void)dbg;
-  }
+  if ((float)tot * scale > limit) tau_opt[q] = __int_as_float(0xff800000);
 }
 
 // After the filter pass under the optimistic thresholds: a query whose parts hold fewer than kk keys
@@ -711,7 +647,7 @@ __global__ void probe_classify_kernel(const int* __restrict__ counts, int parts,
 __global__ void verify_counts_kernel(const int* __restrict__ counts, int parts, int64_t Q, int kk, int qt,
                                      const float* __restrict__ tau, const float* __restrict__ tau_opt,
                                      float* __restrict__ thr_redo, int* __restrict__ redo_tile,
-                                     unsigned long long* __restrict__ dbg) {
+                                     unsigned long long* __restrict__ stats) {
   const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (q >= Q) return;
   long long tot = 0;
@@ -724,9 +660,9 @@ __global__ void verify_counts_kernel(const int* __restrict__ counts, int parts, 
   const bool redo = over || (tot < kk && tau_opt[q] < tau[q]);
   thr_redo[q] = redo ? tau[q] : __int_as_float(0xff800000);
   if (redo) redo_tile[q / qt] = 1;
-  if (dbg) {
-    atomicAdd(&dbg[0], (unsigned long long)tot);
-    if (redo) atomicAdd(&dbg[3], 1ull);
+  if (stats) {
+    atomicAdd(&stats[STAT_SURVIVORS], (unsigned long long)tot);
+    if (redo) atomicAdd(&stats[STAT_REDO_QUERIES], 1ull);
   }
 }
 
@@ -831,7 +767,6 @@ static CerLayout cer_layout(int K, int d, int qt, int dpad) {
   L.total = off;
   return L;
 }
-static size_t cer_bytes(int K, int d, int qt, int dpad) { return cer_layout(K, d, qt, dpad).total; }
 
 // One block.  Takes the first `cap` flagged queries (thr[q] > -inf) in query order: idx_c / thr_c / gathered prototype
 // and parameter rows; un-flags them in thr, rebuilds the per-tile flags for what is left, flag_c = "something taken".
@@ -902,44 +837,306 @@ redo_compact_kernel(float* __restrict__ thr, int64_t Q, int cap, int K, int d, i
   }
 }
 
-static size_t score_ws_layout(int64_t Q, int K, int d, int64_t N, const ScorePlan& p, bool own_image,
-                              size_t* o_pc, size_t* o_qpar, size_t* o_qimg, size_t* o_keys, size_t* o_cnt,
-                              size_t* o_cimg, size_t* o_lbimg = nullptr) {
-  size_t off = 0;
+// Workspace of one cfl_score_topk[_packed] call under plan p: the byte offset of every region.  Only the tensor-core
+// plan has the lower-bound pass's spill lists, the statistics and the compact-redo area.
+struct ScoreWs {
+  size_t pc, qpar, qplane;            // centred prototypes [Q,K,d]; soft-min and plane-bound blocks per query
+  size_t qimg, lbimg;                 // query images of the exact kernel and of the lower-bound pass
+  size_t keys, counts;                // key buffers [parts,Q,TOPK_STRIDE] and counts [parts,Q] of the larger tiling
+  size_t cimg;                        // catalog image, packed here by cfl_score_topk (empty for the _packed entry)
+  size_t tau, tau_opt;                // per query: safe and optimistic thresholds
+  size_t thr_redo, redo_tile;         // per query: threshold of the exact redo (-inf = none); per query tile: 1 = redo
+  size_t thr_redo2, redo_tile2;       // the same after the second lower-bound round
+  size_t lb2;                         // per query: threshold of the second lower-bound round, -inf = none
+  size_t spill, spill_cnt;            // lower-bound pass: [Q,LB_SPILL] keys that did not fit their buffer, count [Q]
+  size_t stats;                       // CFL_SCORE_NSTATS counters (ScoreStat)
+  size_t cer;                         // compact exact redo: cer_layout at the next 1024-byte aligned ADDRESS from here
+  CerLayout cl;
+  size_t total;
+};
+
+static ScoreWs score_ws(int64_t Q, int K, int d, int64_t N, const ScorePlan& p, bool own_image) {
+  ScoreWs w = {};
   const LbPlan lb = p.impl ? make_lb_plan(Q, K, d, p.tiles) : LbPlan{0, 0, 0, 0, 0};
   const int kparts = p.parts > lb.parts ? p.parts : lb.parts;          // key buffers serve both tilings
-  *o_pc = off;   off = align_up(off + (size_t)Q * K * d * 4, 256);
-  *o_qpar = off; off = align_up(off + (size_t)Q * (qpar_stride(K) + qplane_stride(K)) * 4, 256);
-  *o_qimg = off; off = align_up(off + (p.impl ? (size_t)p.nqt * qimg_tile_bytes(p.dpad, K * p.qt) : 0), 1024);
-  if (o_lbimg) *o_lbimg = off;
-  off = align_up(off + (p.impl ? score_lb_qimg_bytes(lb, K, d) : 0), 1024);
-  *o_keys = off; off = align_up(off + (size_t)kparts * Q * TOPK_STRIDE * sizeof(tkey_t), 256);
-  *o_cnt = off;  off = align_up(off + (size_t)kparts * Q * sizeof(int), 1024);
-  *o_cimg = off; off = align_up(off + ((p.impl && own_image) ? catalog_image_bytes(N, d) : 0), 1024);
-  // tau[Q], tau_opt[Q], thr_redo[Q], redo flags per query tile, then the second round's thr_redo2[Q] and tile flags:
-  // live right after (see `tau` below)
-  off = align_up(off + (size_t)(5 * Q + 2 * p.nqt + 12) * sizeof(float), 256);
-  // lower-bound pass: per-query spill list for keys that do not fit their (part, query) buffer + counters
-  if (p.impl) off = align_up(off + (size_t)Q * LB_SPILL * sizeof(tkey_t) + (size_t)Q * sizeof(int), 256);
-  // statistics of the call (cfl_score_topk_stats): CFL_SCORE_NSTATS 64-bit counters
-  if (p.impl) off = align_up(off + CFL_SCORE_NSTATS * sizeof(unsigned long long), 256);
-  // compact exact redo (one query tile of gathered queries): index map, thresholds, flag, prototypes, parameter blocks, image
-  if (p.impl) off = align_up(off + cer_bytes(K, d, p.qt, p.dpad), 1024);
-  return off + 1024;
+  size_t off = 0;
+  w.pc = off;         off = align_up(off + (size_t)Q * K * d * 4, 256);
+  w.qpar = off;       w.qplane = off + (size_t)Q * qpar_stride(K) * 4;
+  off = align_up(off + (size_t)Q * (qpar_stride(K) + qplane_stride(K)) * 4, 256);
+  w.qimg = off;       off = align_up(off + (p.impl ? (size_t)p.nqt * qimg_tile_bytes(p.dpad, K * p.qt) : 0), 1024);
+  w.lbimg = off;      off = align_up(off + (p.impl ? score_lb_qimg_bytes(lb, K, d) : 0), 1024);
+  w.keys = off;       off = align_up(off + (size_t)kparts * Q * TOPK_STRIDE * sizeof(tkey_t), 256);
+  w.counts = off;     off = align_up(off + (size_t)kparts * Q * sizeof(int), 1024);
+  w.cimg = off;       off = align_up(off + ((p.impl && own_image) ? catalog_image_bytes(N, d) : 0), 1024);
+  w.tau = off;        off += (size_t)Q * sizeof(float);
+  w.tau_opt = off;    off += (size_t)Q * sizeof(float);
+  w.thr_redo = off;   off += (size_t)Q * sizeof(float);
+  w.redo_tile = off;  off += (size_t)(p.nqt + 4) * sizeof(int);
+  w.thr_redo2 = off;  off += (size_t)Q * sizeof(float);
+  w.redo_tile2 = off; off += (size_t)(p.nqt + 4) * sizeof(int);
+  w.lb2 = off;        off = align_up(off + (size_t)(Q + 4) * sizeof(float), 256);
+  if (p.impl) {
+    w.spill = off;    w.spill_cnt = off + (size_t)Q * LB_SPILL * sizeof(tkey_t);
+    off = align_up(w.spill_cnt + (size_t)Q * sizeof(int), 256);
+    w.stats = off;    off = align_up(off + CFL_SCORE_NSTATS * sizeof(unsigned long long), 256);
+    w.cl = cer_layout(K, d, p.qt, p.dpad);
+    w.cer = off;      off = align_up(off + w.cl.total, 1024);
+  }
+  w.total = off + 1024;
+  return w;
 }
 
 static size_t score_ws_bytes(int64_t Q, int K, int d, int64_t N, int k, bool own_image) {
   if (Q <= 0 || N <= 0) return 4096;
   // the plan (hence the size) differs between the two kernels: take the larger
-  size_t a, b, c, e, f, g;
-  ScorePlan p0 = make_score_plan(Q, K, d, N, k, false);
-  size_t s0 = score_ws_layout(Q, K, d, N, p0, own_image, &a, &b, &c, &e, &f, &g);
-  size_t s1 = 0;
+  size_t s = score_ws(Q, K, d, N, make_score_plan(Q, K, d, N, k, false), own_image).total;
   if (score_umma_qt(K, d) > 0) {
-    ScorePlan p1 = make_score_plan(Q, K, d, N, k, true);
-    s1 = score_ws_layout(Q, K, d, N, p1, own_image, &a, &b, &c, &e, &f, &g);
+    const size_t s1 = score_ws(Q, K, d, N, make_score_plan(Q, K, d, N, k, true), own_image).total;
+    if (s1 > s) s = s1;
   }
-  return (s0 > s1 ? s0 : s1) + 1024;
+  return s + 1024;
+}
+
+// One cfl_score_topk call as its stages see it: the caller's arguments, plan, knobs, workspace, and the argument block
+// of the tensor-core kernels, which the stages update as the call proceeds.
+struct ScoreCall {
+  const float* Pq; int64_t ldq; int k; int64_t idx_base; float* top_val; int64_t* top_idx;
+  ScorePlan plan; ScoreKnobs kn; ScoreWs ws; char* base; cudaStream_t cs;
+  ScoreArgs a;
+  template <class T> T* at(size_t off) const { return (T*)(base + off); }
+};
+
+// What the final merge_rescore_kernel launch reads besides the call's key buffers.
+struct MergeInput {
+  int parts;                          // catalog parts of the key buffers
+  const float* only = nullptr;        // after a lower-bound pass: only the queries with only[q] > -inf are merged
+  // compact exact redo (cparts = 0: none): key buffers, counts, parts, per-slot thresholds, slot -> query map
+  const tkey_t* ckeys = nullptr; const int* ccounts = nullptr; int cparts = 0;
+  const float* cthr = nullptr; const int* cmap = nullptr;
+};
+
+// Stage: centred prototypes and parameter blocks; on the tensor-core plan also the catalog image (packed into the
+// workspace unless the caller packed it), its views and the query images.
+static int prep_and_pack(ScoreCall& c, const void* image) {
+  ScoreArgs& a = c.a;
+  prep_queries_kernel<<<(unsigned)((a.Q + 3) / 4), 128, 0, c.cs>>>(c.Pq, a.Q, a.K, a.d, c.ldq, a.mu, (float*)a.Pc,
+                                                                   (float*)a.qpar, (float*)a.qplane);
+  CFL_LAUNCH_CHECK();
+  if (c.plan.impl != 1) return CFL_OK;
+  if (!image) {
+    void* own = c.base + c.ws.cimg;
+    const int st = catalog_pack_launch(a.E, a.N, a.d, a.lde, a.mu, own, c.cs);
+    if (st != CFL_OK) return st;
+    image = own;
+  }
+  const CatalogView cv = catalog_view(image, a.N, a.d);
+  a.cimg = image; a.e2 = cv.e2; a.cimg16 = cv.f16; a.cflag16 = cv.flag16; a.lbrow = cv.lbrow;
+  const LbQimgView qv = score_lb_qimg_view(c.base + c.ws.lbimg, a.lb, a.K, a.d);
+  a.qimg16 = qv.img; a.qflag16 = qv.flag; a.lbq = qv.lbq;
+  return score_umma_pack_queries(a, c.base + c.ws.qimg, c.cs);
+}
+
+// Stage: the thresholds.  Long catalog ranges are scored in two passes: a sparse sample pass (every S-th tile) whose
+// merged kk-th best distance bounds the final threshold (tau), then the full pass that only filters against a fixed
+// bound (no barriers, no compaction).
+static int sample_thresholds(ScoreCall& c) {
+  ScoreArgs& a = c.a;
+  const ScorePlan& plan = c.plan;
+  const int64_t Q = a.Q;
+  const int sstride = c.kn.sample_stride;
+  float* tau = c.at<float>(c.ws.tau);
+  // Threshold selection: one block per query.  Many queries -> narrow blocks with 32 KB of staged keys each (a whole
+  // wave of them is resident; a query with more keys selects from global memory); few queries -> wide blocks that
+  // stage up to 148 parts x kk keys.
+  const int sel_threads = Q >= 2 * (int64_t)sm_count() ? 256 : SEL_THREADS;
+  const int sel_cap = Q >= 2 * (int64_t)sm_count() ? 8192 : SEL_SMEM_KEYS;
+  auto sel_keys = [&](int64_t bound) { return (int)(bound < sel_cap ? (bound < 1024 ? 1024 : bound) : sel_cap); };
+  CFL_SMEM_LIMIT(select_threshold_kernel, ((size_t)plan.parts + 1 + SEL_SMEM_KEYS) * sizeof(uint32_t));
+  // Sample = every sstride-th tile of each part.  When a few collect-everything tiles per
+  // part already give a bound tau_a under which the sample yields <= ~384 keys per buffer,
+  // the sample itself is scored in filter mode (no barriers); otherwise it runs adaptively.
+  const int64_t tpp = plan.tiles / plan.parts;
+  const int64_t tiles_b = (tpp + sstride - 1) / sstride;
+  int64_t tiles_a = ((int64_t)plan.kk * tiles_b + 384 * (int64_t)plan.parts - 1) / (384 * (int64_t)plan.parts);
+  if (tiles_a < 1) tiles_a = 1;
+  // The cascade needs a pass-B sample several times larger than pass A's: tau_a (kk-th best of pass A) leaves
+  // about kk * |B| / |A| rows of pass B under it, and pass B must find at least kk of them to define the
+  // thresholds (with |B| ~ |A| -- short part ranges, e.g. a few queries on 148 parts -- a seventh of the queries
+  // ended up without thresholds and fell through to the exact redo pass).  Pass A visits up to tiles_a + 1 tiles.
+  const bool cascade = tiles_a <= 7 && tiles_a * 128 * plan.parts >= 2 * plan.kk && tiles_b >= 4 * (tiles_a + 1) &&
+                       !c.kn.no_cascade;
+  int st;
+  if (cascade) {
+    a.phase = 2; a.thr_init = nullptr;                 // +inf thresholds: keep every sampled row
+    a.tile_stride = (int)((tpp + tiles_a - 1) / tiles_a);
+    if (a.tile_stride < 1) a.tile_stride = 1;
+    // guard: ceil(range / stride) <= 7 tiles even for the longest part range
+    while ((tpp + 1 + a.tile_stride - 1) / a.tile_stride > 7) ++a.tile_stride;
+    st = score_umma_launch(a, c.cs);
+    if (st != CFL_OK) return st;
+    const int nk = sel_keys((int64_t)plan.parts * 7 * 128);   // pass A: at most 7 tiles of 128 rows per part
+    select_threshold_kernel<<<(unsigned)Q, sel_threads, ((size_t)plan.parts + 1 + nk) * sizeof(uint32_t), c.cs>>>(
+        a.keys, a.counts, plan.parts, Q, plan.kk, tau, nullptr, 0, nk);
+    CFL_LAUNCH_CHECK();
+    a.phase = 2; a.tile_stride = sstride; a.thr_init = tau;
+    st = score_umma_launch(a, c.cs);
+  } else {
+    a.phase = 1; a.tile_stride = sstride; a.thr_init = nullptr;
+    st = score_umma_launch(a, c.cs);
+  }
+  if (st != CFL_OK) return st;
+  // The full pass filters under an OPTIMISTIC threshold (r_opt-th best of the sample: about 4*kk rows of the whole
+  // range pass instead of sstride*kk), which lets the bounds reject almost every (row, query).  Each query is then
+  // verified, and the rare query that fails is redone under the safe bound.
+  CFL_CUDA(cudaMemsetAsync(c.at<unsigned long long>(c.ws.stats), 0, CFL_SCORE_NSTATS * sizeof(unsigned long long), c.cs));
+  int r_opt = (int)((c.kn.opt_mult * (int64_t)plan.kk + sstride - 1) / sstride);
+  if (c.kn.no_optimistic) r_opt = 0;
+  const int nk = sel_keys((int64_t)plan.parts * TOPK_STRIDE);
+  select_threshold_kernel<<<(unsigned)Q, sel_threads, ((size_t)plan.parts + 1 + nk) * sizeof(uint32_t), c.cs>>>(
+      a.keys, a.counts, plan.parts, Q, plan.kk, tau, c.at<float>(c.ws.tau_opt), r_opt, nk);
+  CFL_LAUNCH_CHECK();
+  CFL_CUDA(cudaMemsetAsync(c.at<int>(c.ws.redo_tile), 0, (size_t)plan.nqt * sizeof(int), c.cs));
+  return CFL_OK;
+}
+
+// One round of rescore_merge_kernel over the lower-bound pass's survivors: the threshold they were filtered under and
+// where the verdicts go.
+struct RescoreRound {
+  const float* tau_opt;               // threshold of the filter pass (the safe tau in the second round)
+  float* thr_redo;                    // per query: threshold of the exact redo, -inf = verified and written
+  int* redo_tile;                     // per query tile: 1 = some query must be redone
+  const float* only;                  // second round: the queries it rescores (> -inf); NULL in the first
+  const float* prev;                  // second round: the first round's thr_redo, kept by every other query
+  float* second;                      // first round: the thresholds of the second round (lb2)
+};
+static int rescore_round(const ScoreCall& c, const RescoreRound& r) {
+  const ScoreArgs& a = c.a;
+  const int dp = (a.d + RSC_CH - 1) / RSC_CH * RSC_CH;
+  const size_t smem = ((size_t)a.K * dp + (size_t)(MRG_THREADS / 32) * 32 * RSC_LD + a.lb.parts + 2 + 4) * sizeof(float);
+  return with_k(a.K, [&](auto K) {
+    CFL_SMEM_LIMIT(rescore_merge_kernel<K>, smem);
+    rescore_merge_kernel<K><<<(unsigned)a.Q, MRG_THREADS, smem, c.cs>>>(
+        a.keys, a.counts, a.lb.parts, a.Q, c.plan.kk, c.k, c.Pq, c.ldq, a.d, a.E, a.lde, c.idx_base, c.top_val,
+        c.top_idx, c.at<float>(c.ws.tau), r.tau_opt, c.plan.qt, r.thr_redo, r.redo_tile,
+        c.at<unsigned long long>(c.ws.stats), a.spill, a.spill_cnt, r.only, r.prev, r.second);
+    CFL_LAUNCH_CHECK();
+    return CFL_OK;
+  });
+}
+
+// Stage: the single-product lower-bound filter (K <= 4), its survivors rescored exactly by rescore_merge_kernel, which
+// also verifies the optimistic threshold.  Verdicts in thr_redo2 / redo_tile2.
+static int lower_bound_rounds(ScoreCall& c) {
+  ScoreArgs& a = c.a;
+  const int64_t Q = a.Q;
+  float* tau_opt = c.at<float>(c.ws.tau_opt);
+  float* lb2 = c.at<float>(c.ws.lb2);
+  int st = score_lb_prep_queries(a, c.cs);
+  if (st != CFL_OK) return st;
+  if (!c.kn.no_probe) {
+    const int64_t tpp_lb = c.plan.tiles / a.lb.parts;    // the lower-bound pass has its own catalog parts
+    int probe_stride = (int)((tpp_lb + 3) / 4);          // about 4 tiles per part
+    if (probe_stride < 1) probe_stride = 1;
+    const int64_t probe_tiles = (tpp_lb + probe_stride - 1) / probe_stride;
+    a.phase = 3; a.tile_stride = probe_stride;
+    CFL_CUDA(cudaMemsetAsync(a.spill_cnt, 0, (size_t)Q * sizeof(int), c.cs));
+    st = score_lb_launch(a, c.cs);
+    if (st != CFL_OK) return st;
+    // only the pathological regimes (most rows survive) are taken out: 4x the total key capacity
+    const float limit = 4.0f * ((float)a.lb.parts * (float)TOPK_STRIDE + (float)LB_SPILL);
+    probe_classify_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, c.cs>>>(
+        a.counts, a.lb.parts, Q, (float)tpp_lb / (float)probe_tiles, limit, tau_opt, a.spill_cnt);
+    CFL_LAUNCH_CHECK();
+    a.phase = 2; a.tile_stride = 1;
+    timer_record(0, c.cs);
+  }
+  CFL_CUDA(cudaMemsetAsync(a.spill_cnt, 0, (size_t)Q * sizeof(int), c.cs));
+  a.phase = 3; st = score_lb_launch(a, c.cs); a.phase = 2;
+  timer_record(1, c.cs);
+  if (st != CFL_OK) return st;
+  float* thr_redo = c.at<float>(c.ws.thr_redo);
+  st = rescore_round(c, {tau_opt, thr_redo, c.at<int>(c.ws.redo_tile), nullptr, nullptr, lb2});
+  if (st != CFL_OK) return st;
+  // Second chance for the queries whose optimistic threshold was not confirmed (fewer than kk survivors under
+  // it): the lower-bound pass again, under the SAFE threshold and only for them -- query tiles without such a
+  // query leave at once -- then the exact rescoring of THEIR survivors.  Bounded by one more filter pass; the
+  // exact 3xTF32 redo (a few CTAs per query tile walk the whole catalog) remains for overflowing buffers,
+  // raised range flags and the queries the probe took out.
+  int* redo_tile2 = c.at<int>(c.ws.redo_tile2);
+  CFL_CUDA(cudaMemsetAsync(redo_tile2, 0, (size_t)c.plan.nqt * sizeof(int), c.cs));
+  CFL_CUDA(cudaMemsetAsync(a.spill_cnt, 0, (size_t)Q * sizeof(int), c.cs));
+  a.thr_init = lb2;
+  a.phase = 3; st = score_lb_launch(a, c.cs); a.phase = 2;
+  if (st != CFL_OK) return st;
+  return rescore_round(c, {c.at<float>(c.ws.tau), c.at<float>(c.ws.thr_redo2), redo_tile2, lb2, thr_redo, nullptr});
+}
+
+// Stage: the exact 3xTF32 filter (K > 4 or CFL_SCORE_NO_LB) under the optimistic threshold; verify_counts_kernel
+// flags the queries with fewer than kk keys.  Verdicts in thr_redo / redo_tile.
+static int exact_filter(ScoreCall& c) {
+  const int st = score_umma_launch(c.a, c.cs);
+  timer_record(1, c.cs);
+  if (st != CFL_OK) return st;
+  const int64_t Q = c.a.Q;
+  verify_counts_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, c.cs>>>(
+      c.a.counts, c.plan.parts, Q, c.plan.kk, c.plan.qt, c.at<float>(c.ws.tau), c.at<float>(c.ws.tau_opt),
+      c.at<float>(c.ws.thr_redo), c.at<int>(c.ws.redo_tile), c.at<unsigned long long>(c.ws.stats));
+  CFL_LAUNCH_CHECK();
+  return CFL_OK;
+}
+
+// Stage: the exact kernel redoes the flagged queries (thr_redo > -inf) under the safe threshold.
+static int exact_redo(ScoreCall& c, bool lb_pass, float* thr_redo, int* redo_tile, MergeInput& m) {
+  ScoreArgs& a = c.a;
+  const ScorePlan& plan = c.plan;
+  int st;
+  if (lb_pass && plan.nqt > 1) {
+    // compact exact redo: up to one query tile of flagged queries, every SM on a slice of the catalog.  Its key
+    // buffers live in the spill lists (free once the rescoring rounds are done): [parts][qt][TOPK_STRIDE] + counts.
+    int sms_c = sm_count();
+    if (sms_c <= 0) sms_c = 148;
+    int64_t pc_parts = ((int64_t)a.Q * LB_SPILL) / ((int64_t)plan.qt * (TOPK_STRIDE + 1));
+    if (pc_parts > sms_c) pc_parts = sms_c;
+    if (pc_parts > plan.tiles) pc_parts = plan.tiles;
+    if (pc_parts >= 1) {
+      const CerLayout& CL = c.ws.cl;
+      char* cer = (char*)align_up((size_t)(uintptr_t)(c.base + c.ws.cer), 1024);
+      int* cmap = (int*)(cer + CL.idx);
+      float* cthr = (float*)(cer + CL.thr);
+      int* flag_c = (int*)(cer + CL.flag);
+      tkey_t* ckeys = a.spill;
+      int* ccounts = (int*)(a.spill + (size_t)pc_parts * plan.qt * TOPK_STRIDE);
+      redo_compact_kernel<<<1, 256, 0, c.cs>>>(thr_redo, a.Q, plan.qt, a.K, a.d, plan.qt, plan.nqt, a.Pc, a.qpar,
+                                               a.qplane, cmap, cthr, flag_c, (float*)(cer + CL.pc),
+                                               (float*)(cer + CL.qpar), (float*)(cer + CL.qplane), redo_tile, plan.dpad,
+                                               (float*)(cer + CL.qimg));
+      CFL_LAUNCH_CHECK();
+      m.ckeys = ckeys; m.ccounts = ccounts; m.cparts = (int)pc_parts; m.cthr = cthr; m.cmap = cmap;
+      ScoreArgs b = a;
+      b.Q = plan.qt; b.Pc = (const float*)(cer + CL.pc); b.qpar = (const float*)(cer + CL.qpar);
+      b.qplane = (const float*)(cer + CL.qplane); b.qimg = cer + CL.qimg;
+      b.keys = ckeys; b.counts = ccounts;
+      b.thr_init = cthr; b.redo_tile = flag_c; b.phase = 2; b.tile_stride = 1; b.dist_out = nullptr;
+      b.plan.nqt = 1; b.plan.parts = m.cparts;
+      st = score_umma_launch(b, c.cs);
+      if (st != CFL_OK) return st;
+    }
+  }
+  a.thr_init = thr_redo; a.redo_tile = redo_tile;
+  if (lb_pass && a.lb.parts > plan.parts) {
+    // After a lower-bound pass only the redone queries use the exact kernel's key buffers, and the buffers exist
+    // for the lower-bound tiling's (more numerous) catalog parts: cut the catalog that finely, so that the few
+    // query tiles with something to redo are spread over more SMs (the others leave at once).
+    ScoreArgs r = a;
+    r.plan.parts = a.lb.parts;
+    st = score_umma_launch(r, c.cs);
+    m.parts = a.lb.parts;
+  } else {
+    st = score_umma_launch(a, c.cs);
+  }
+  a.redo_tile = nullptr;
+  m.only = lb_pass ? thr_redo : nullptr;
+  return st;
 }
 
 // Shared body of cfl_score_topk (image == NULL: packed into the workspace on every call) and
@@ -963,276 +1160,65 @@ static int score_topk_impl(int mode, const float* Pq, int64_t Q, int K, int d, i
   CFL_REQUIRE(N == 0 || E, CFL_ERR_INVALID, "score_topk: NULL catalog");
   bool umma_ok = N > 0 && score_umma_supported(K, d);
   CFL_REQUIRE(!image || umma_ok, CFL_ERR_UNSUPPORTED, "score_topk_packed: shape K=%d d=%d has no tcgen05 tiling", K, d);
-  ScorePlan plan = make_score_plan(Q, K, d, N > 0 ? N : 1, k, umma_ok);
-  size_t o_pc, o_qpar, o_qimg, o_keys, o_cnt, o_cimg, o_lbimg;
-  size_t need = score_ws_layout(Q, K, d, N, plan, image == nullptr, &o_pc, &o_qpar, &o_qimg, &o_keys, &o_cnt, &o_cimg,
-                                &o_lbimg);
-  CFL_REQUIRE(ws && ws_bytes >= need, CFL_ERR_WORKSPACE, "score_topk: workspace too small (%zu < %zu)",
-              ws_bytes, need);
-  char* base = (char*)ws;
-  ScoreArgs a;
+  ScoreCall c;
+  c.Pq = Pq; c.ldq = ldq; c.k = k; c.idx_base = idx_base; c.top_val = top_val; c.top_idx = top_idx;
+  c.plan = make_score_plan(Q, K, d, N > 0 ? N : 1, k, umma_ok);
+  c.kn = read_knobs();
+  c.ws = score_ws(Q, K, d, N, c.plan, image == nullptr);
+  c.base = (char*)ws;
+  c.cs = cs;
+  CFL_REQUIRE(ws && ws_bytes >= c.ws.total, CFL_ERR_WORKSPACE, "score_topk: workspace too small (%zu < %zu)",
+              ws_bytes, c.ws.total);
+  const ScorePlan& plan = c.plan;
+  ScoreArgs& a = c.a;
+  a = ScoreArgs{};
   a.mode = mode; a.K = K; a.d = d; a.Q = Q; a.N = N; a.lde = lde; a.E = E; a.mu = mu;
-  a.Pc = (float*)(base + o_pc); a.qpar = (float*)(base + o_qpar); a.qimg = base + o_qimg;
-  a.qplane = a.qpar + (size_t)Q * qpar_stride(K);
-  a.keys = (tkey_t*)(base + o_keys); a.counts = (int*)(base + o_cnt); a.dist_out = dist_out;
-  a.cimg = nullptr; a.e2 = nullptr;
-  a.phase = 0; a.tile_stride = 1; a.thr_init = nullptr;
-  a.redo_tile = nullptr; a.spill = nullptr; a.spill_cnt = nullptr;
-  a.cimg16 = nullptr; a.qimg16 = nullptr; a.cflag16 = nullptr; a.qflag16 = nullptr; a.lbrow = nullptr; a.lbq = nullptr;
-  bool lb_pass = false;
-  const float* redo_only = nullptr;
-  int redo_parts = 0;                                        // parts of the exact redo launch when it differs from the plan's
-  int* cer_idx = nullptr; float* cer_thr = nullptr; tkey_t* cer_keys = nullptr; int* cer_counts = nullptr; int cer_parts = 0;
-  const ScoreKnobs kn = read_knobs();
-  a.dbg_mode = kn.dbg_mode;
+  a.Pc = c.at<float>(c.ws.pc); a.qpar = c.at<float>(c.ws.qpar); a.qplane = c.at<float>(c.ws.qplane);
+  a.qimg = c.at<char>(c.ws.qimg);
+  a.keys = c.at<tkey_t>(c.ws.keys); a.counts = c.at<int>(c.ws.counts); a.dist_out = dist_out;
+  a.tile_stride = 1;
+  a.dbg_mode = c.kn.dbg_mode;
   a.plan = plan;
   a.lb = plan.impl ? make_lb_plan(Q, K, d, plan.tiles) : LbPlan{0, 0, 0, 0, 0};
+  MergeInput m;
+  m.parts = plan.parts;
   if (N == 0) {
     CFL_CUDA(cudaMemsetAsync(a.counts, 0, (size_t)plan.parts * Q * sizeof(int), cs));
   } else {
-    prep_queries_kernel<<<(unsigned)((Q + 3) / 4), 128, 0, cs>>>(Pq, Q, K, d, ldq, mu,
-                                                                (float*)a.Pc, (float*)a.qpar, (float*)a.qplane);
-    CFL_LAUNCH_CHECK();
-    if (plan.impl == 1) {
-      if (!image) {
-        st = catalog_pack_launch(E, N, d, lde, mu, base + o_cimg, cs);
-        if (st != CFL_OK) return st;
-        image = base + o_cimg;
-      }
-      a.cimg = image;
-      a.e2 = (const float*)((const char*)image + catalog_e2_offset(N, d));
-      a.cimg16 = (const char*)image + catalog_f16_offset(N, d);
-      a.cflag16 = (const int*)((const char*)a.cimg16 + catalog_f16_bytes(N, d));
-      a.lbrow = (const float2*)((const char*)image + catalog_lbrow_offset(N, d));
-      a.qimg16 = base + o_lbimg;
-      a.qflag16 = (const int*)((const char*)a.qimg16 + (size_t)a.lb.nqt * a.lb.sub * a.lb.qt * ((d + 15) / 16) * 2 * K * 16);
-      a.lbq = (const float*)((const char*)a.qflag16 + 16);
-      st = score_umma_pack_queries(a, base + o_qimg, cs);
-      if (st != CFL_OK) return st;
-      // Long catalog ranges are scored in two passes: a sparse sample pass (every S-th tile,
-      // running thresholds) whose merged kk-th best distance bounds the final threshold, then the
-      // full pass that only filters against that fixed bound (no barriers, no compaction).
-      const int sstride = kn.sample_stride;
-      const bool two_pass = score_two_pass(kn, plan, dist_out != nullptr);
-      float* tau = (float*)(base + align_up(o_cimg + ((image == (const void*)(base + o_cimg)) ? catalog_image_bytes(N, d) : 0), 1024));
-      if (!two_pass) timer_record(0, cs);
-      // Threshold selection: one block per query.  Many queries -> narrow blocks with 32 KB of staged keys each (a whole
-      // wave of them is resident; a query with more keys selects from global memory); few queries -> wide blocks that
-      // stage up to 148 parts x kk keys.
-      const int sel_threads = Q >= 2 * (int64_t)sm_count() ? 256 : SEL_THREADS;
-      const int sel_cap = Q >= 2 * (int64_t)sm_count() ? 8192 : SEL_SMEM_KEYS;
-      auto sel_keys = [&](int64_t bound) { return (int)(bound < sel_cap ? (bound < 1024 ? 1024 : bound) : sel_cap); };
-      if (two_pass) {
-        CFL_SMEM_LIMIT(select_threshold_kernel, ((size_t)plan.parts + 1 + SEL_SMEM_KEYS) * sizeof(uint32_t));
-        // Sample = every sstride-th tile of each part.  When a few collect-everything tiles per
-        // part already give a bound tau_a under which the sample yields <= ~384 keys per buffer,
-        // the sample itself is scored in filter mode (no barriers); otherwise it runs adaptively.
-        const int64_t tpp = plan.tiles / plan.parts;
-        const int64_t tiles_b = (tpp + sstride - 1) / sstride;
-        int64_t tiles_a = ((int64_t)plan.kk * tiles_b + 384 * (int64_t)plan.parts - 1) / (384 * (int64_t)plan.parts);
-        if (tiles_a < 1) tiles_a = 1;
-        // The cascade needs a pass-B sample several times larger than pass A's: tau_a (kk-th best of pass A) leaves
-        // about kk * |B| / |A| rows of pass B under it, and pass B must find at least kk of them to define the
-        // thresholds (with |B| ~ |A| -- short part ranges, e.g. a few queries on 148 parts -- a seventh of the queries
-        // ended up without thresholds and fell through to the exact redo pass).  Pass A visits up to tiles_a + 1 tiles.
-        const bool cascade = tiles_a <= 7 && tiles_a * 128 * plan.parts >= 2 * plan.kk && tiles_b >= 4 * (tiles_a + 1) &&
-                             !kn.no_cascade;
-        if (cascade) {
-          a.phase = 2; a.thr_init = nullptr;                 // +inf thresholds: keep every sampled row
-          a.tile_stride = (int)((tpp + tiles_a - 1) / tiles_a);
-          if (a.tile_stride < 1) a.tile_stride = 1;
-          // guard: ceil(range / stride) <= 7 tiles even for the longest part range
-          while ((tpp + 1 + a.tile_stride - 1) / a.tile_stride > 7) ++a.tile_stride;
-          st = score_umma_launch(a, cs);
-          if (st != CFL_OK) return st;
-          {
-            const int nk = sel_keys((int64_t)plan.parts * 7 * 128);   // pass A: at most 7 tiles of 128 rows per part
-            select_threshold_kernel<<<(unsigned)Q, sel_threads, ((size_t)plan.parts + 1 + nk) * sizeof(uint32_t), cs>>>(
-                a.keys, a.counts, plan.parts, Q, plan.kk, tau, nullptr, 0, nk);
-          }
-          CFL_LAUNCH_CHECK();
-          a.phase = 2; a.tile_stride = sstride; a.thr_init = tau;
-          st = score_umma_launch(a, cs);
-        } else {
-          a.phase = 1; a.tile_stride = sstride; a.thr_init = nullptr;
-          st = score_umma_launch(a, cs);
-        }
-        if (st != CFL_OK) return st;
-        // Final pass: filter under an OPTIMISTIC threshold (r_opt-th best of the sample: about 4*kk
-        // rows of the whole range pass instead of sstride*kk), which lets the affine-hull bound
-        // reject almost every (row, query) before the soft-min.  The key counts then prove, per
-        // query, that at least kk rows passed; the rare query that fails is redone under the safe
-        // bound by a second launch whose CTAs exit at once when their query tile has nothing to redo.
-        float* tau_opt = tau + Q;
-        float* thr_redo = tau + 2 * Q;
-        int* redo_tile = (int*)(tau + 3 * Q);
-        a.spill = (tkey_t*)((char*)tau + align_up((size_t)(5 * Q + 2 * plan.nqt + 12) * sizeof(float), 256));
-        a.spill_cnt = (int*)(a.spill + (size_t)Q * LB_SPILL);
-        unsigned long long* stats = (unsigned long long*)((char*)a.spill + align_up((size_t)Q * LB_SPILL * sizeof(tkey_t) + (size_t)Q * sizeof(int), 256));
-        CFL_CUDA(cudaMemsetAsync(stats, 0, CFL_SCORE_NSTATS * sizeof(unsigned long long), cs));
-        int r_opt = (int)((kn.opt_mult * (int64_t)plan.kk + sstride - 1) / sstride);
-        if (kn.no_optimistic) r_opt = 0;
-        {
-          const int nk = sel_keys((int64_t)plan.parts * TOPK_STRIDE);
-          select_threshold_kernel<<<(unsigned)Q, sel_threads, ((size_t)plan.parts + 1 + nk) * sizeof(uint32_t), cs>>>(
-              a.keys, a.counts, plan.parts, Q, plan.kk, tau, tau_opt, r_opt, nk);
-        }
-        CFL_LAUNCH_CHECK();
-        CFL_CUDA(cudaMemsetAsync(redo_tile, 0, (size_t)plan.nqt * sizeof(int), cs));
-        a.phase = 2; a.tile_stride = 1; a.thr_init = tau_opt;
-        timer_record(0, cs);                 // bench.py times the dominant launch: the full filter pass
-        // single-product lower-bound filter (survivors rescored exactly by rescore_merge_kernel), or the exact 3xTF32
-        // filter when disabled / for K > 4
-        lb_pass = score_lb_pass(kn, K);
-        if (lb_pass) {
-          st = score_lb_prep_queries(a, cs);
-          if (st != CFL_OK) return st;
-        }
-        if (lb_pass && !kn.no_probe) {
-          const int64_t tpp_lb = plan.tiles / a.lb.parts;    // the lower-bound pass has its own catalog parts
-          int probe_stride = (int)((tpp_lb + 3) / 4);        // about 4 tiles per part
-          if (probe_stride < 1) probe_stride = 1;
-          const int64_t probe_tiles = (tpp_lb + probe_stride - 1) / probe_stride;
-          a.phase = 3; a.tile_stride = probe_stride;
-          CFL_CUDA(cudaMemsetAsync(a.spill_cnt, 0, (size_t)Q * sizeof(int), cs));
-          st = score_lb_launch(a, cs);
-          if (st != CFL_OK) return st;
-          // only the pathological regimes (most rows survive) are taken out: 4x the total key capacity
-          const float limit = 4.0f * ((float)a.lb.parts * (float)TOPK_STRIDE + (float)LB_SPILL);
-          probe_classify_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, cs>>>(
-              a.counts, a.lb.parts, Q, (float)tpp_lb / (float)probe_tiles, limit, tau_opt, nullptr, a.spill_cnt);
-          CFL_LAUNCH_CHECK();
-          a.phase = 2; a.tile_stride = 1;
-          timer_record(0, cs);
-        }
-        if (lb_pass) {
-          CFL_CUDA(cudaMemsetAsync(a.spill_cnt, 0, (size_t)Q * sizeof(int), cs));
-          a.phase = 3; st = score_lb_launch(a, cs); a.phase = 2;
-        }
-        else st = score_umma_launch(a, cs);
-        timer_record(1, cs);
-        if (st != CFL_OK) return st;
-        if (lb_pass) {
-          // exact rescoring of every survivor + verification; flagged queries are redone below
-          const int dp = (d + RSC_CH - 1) / RSC_CH * RSC_CH;
-          const size_t rs_smem = ((size_t)K * dp + (size_t)(MRG_THREADS / 32) * 32 * RSC_LD + a.lb.parts + 2 + 4) * sizeof(float);
-#define CFL_RSC_CASE(KK)                                                                                        \
-  case KK:                                                                                                      \
-    CFL_SMEM_LIMIT(rescore_merge_kernel<KK>, rs_smem);                                                           \
-    rescore_merge_kernel<KK><<<(unsigned)Q, MRG_THREADS, rs_smem, cs>>>(                                        \
-        a.keys, a.counts, a.lb.parts, Q, plan.kk, k, Pq, ldq, d, E, lde, idx_base, top_val, top_idx, tau,       \
-        rs_tau_opt, plan.qt, rs_thr_out, rs_tile_out, stats, a.spill, a.spill_cnt, rs_only, rs_prev, rs_second); \
-    break;
-#define CFL_RSC_LAUNCH()                                                                                        \
-  switch (K) {                                                                                                  \
-    CFL_RSC_CASE(1) CFL_RSC_CASE(2) CFL_RSC_CASE(3) CFL_RSC_CASE(4)                                             \
-    CFL_RSC_CASE(5) CFL_RSC_CASE(6) CFL_RSC_CASE(7) CFL_RSC_CASE(8)                                             \
-  }
-          const float* rs_tau_opt = tau_opt;
-          float* rs_thr_out = thr_redo;
-          int* rs_tile_out = redo_tile;
-          const float* rs_only = nullptr;
-          const float* rs_prev = nullptr;
-          float* lb2 = tau + 4 * Q + 2 * plan.nqt + 8;         // per query: threshold of the second round, -inf = none
-          float* rs_second = lb2;
-          CFL_RSC_LAUNCH()
-          CFL_LAUNCH_CHECK();
-          // Second chance for the queries whose optimistic threshold was not confirmed (fewer than kk survivors under
-          // it): the lower-bound pass again, under the SAFE threshold and only for them -- query tiles without such a
-          // query leave at once -- then the exact rescoring of THEIR survivors.  Bounded by one more filter pass; the
-          // exact 3xTF32 redo below (a few CTAs per query tile walk the whole catalog) remains for overflowing buffers,
-          // raised range flags and the queries the probe took out.
-          float* thr_redo2 = tau + 3 * Q + plan.nqt + 4;
-          int* redo_tile2 = (int*)(thr_redo2 + Q);
-          CFL_CUDA(cudaMemsetAsync(redo_tile2, 0, (size_t)plan.nqt * sizeof(int), cs));
-          CFL_CUDA(cudaMemsetAsync(a.spill_cnt, 0, (size_t)Q * sizeof(int), cs));
-          a.thr_init = lb2;
-          a.phase = 3; st = score_lb_launch(a, cs); a.phase = 2;
-          if (st != CFL_OK) return st;
-          rs_tau_opt = tau; rs_thr_out = thr_redo2; rs_tile_out = redo_tile2; rs_only = lb2; rs_prev = thr_redo; rs_second = nullptr;
-          CFL_RSC_LAUNCH()
-          thr_redo = thr_redo2; redo_tile = redo_tile2;
-#undef CFL_RSC_LAUNCH
-#undef CFL_RSC_CASE
-        } else {
-          verify_counts_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, cs>>>(a.counts, plan.parts, Q, plan.kk, plan.qt,
-                                                                           tau, tau_opt, thr_redo, redo_tile, stats);
-        }
-        CFL_LAUNCH_CHECK();
-        if (lb_pass && plan.nqt > 1) {
-          // compact exact redo: up to one query tile of flagged queries, every SM on a slice of the catalog.  Its key
-          // buffers live in the spill lists (free once the rescoring rounds are done): [parts][qt][TOPK_STRIDE] + counts.
-          int sms_c = sm_count();
-          if (sms_c <= 0) sms_c = 148;
-          int64_t pc_parts = ((int64_t)Q * LB_SPILL) / ((int64_t)plan.qt * (TOPK_STRIDE + 1));
-          if (pc_parts > sms_c) pc_parts = sms_c;
-          if (pc_parts > plan.tiles) pc_parts = plan.tiles;
-          if (pc_parts >= 1) {
-            const CerLayout CL = cer_layout(K, d, plan.qt, plan.dpad);
-            char* cer = (char*)stats + align_up(CFL_SCORE_NSTATS * sizeof(unsigned long long), 256);
-            cer = (char*)align_up((size_t)(uintptr_t)cer, 1024);
-            cer_idx = (int*)(cer + CL.idx);
-            cer_thr = (float*)(cer + CL.thr);
-            int* flag_c = (int*)(cer + CL.flag);
-            cer_keys = a.spill;
-            cer_counts = (int*)(a.spill + (size_t)pc_parts * plan.qt * TOPK_STRIDE);
-            cer_parts = (int)pc_parts;
-            redo_compact_kernel<<<1, 256, 0, cs>>>(thr_redo, Q, plan.qt, K, d, plan.qt, plan.nqt, a.Pc, a.qpar, a.qplane, cer_idx,
-                                                  cer_thr, flag_c, (float*)(cer + CL.pc), (float*)(cer + CL.qpar),
-                                                  (float*)(cer + CL.qplane), redo_tile, plan.dpad, (float*)(cer + CL.qimg));
-            CFL_LAUNCH_CHECK();
-            ScoreArgs b = a;
-            b.Q = plan.qt; b.Pc = (const float*)(cer + CL.pc); b.qpar = (const float*)(cer + CL.qpar);
-            b.qplane = (const float*)(cer + CL.qplane); b.qimg = cer + CL.qimg;
-            b.keys = cer_keys; b.counts = cer_counts;
-            b.thr_init = cer_thr; b.redo_tile = flag_c; b.phase = 2; b.tile_stride = 1; b.dist_out = nullptr;
-            b.plan.nqt = 1; b.plan.parts = cer_parts;
-            st = score_umma_launch(b, cs);
-            if (st != CFL_OK) return st;
-          }
-        }
-        a.thr_init = thr_redo; a.redo_tile = redo_tile;
-        if (lb_pass && a.lb.parts > plan.parts) {
-          // After a lower-bound pass only the redone queries use the exact kernel's key buffers, and the buffers exist
-          // for the lower-bound tiling's (more numerous) catalog parts: cut the catalog that finely, so that the few
-          // query tiles with something to redo are spread over more SMs (the others leave at once).
-          ScoreArgs r = a;
-          r.plan.parts = a.lb.parts;
-          st = score_umma_launch(r, cs);
-          redo_parts = a.lb.parts;
-        } else {
-          st = score_umma_launch(a, cs);
-        }
-        a.redo_tile = nullptr;
-        redo_only = lb_pass ? thr_redo : nullptr;
-      } else {
-        a.phase = 0; a.tile_stride = 1; a.thr_init = nullptr;
-        st = score_umma_launch(a, cs);
-      }
-      if (!two_pass) timer_record(1, cs);
-      if (st != CFL_OK) return st;
-    } else {
+    st = prep_and_pack(c, image);
+    if (st != CFL_OK) return st;
+    if (plan.impl != 1) {
       timer_record(0, cs);
-      switch (K) {
-        case 1: st = launch_simt<1>(a, cs); break;
-        case 2: st = launch_simt<2>(a, cs); break;
-        case 3: st = launch_simt<3>(a, cs); break;
-        case 4: st = launch_simt<4>(a, cs); break;
-        case 5: st = launch_simt<5>(a, cs); break;
-        case 6: st = launch_simt<6>(a, cs); break;
-        case 7: st = launch_simt<7>(a, cs); break;
-        default: st = launch_simt<8>(a, cs); break;
-      }
+      st = with_k(K, [&](auto KC) { return launch_simt<KC>(a, cs); });
       timer_record(1, cs);
+    } else if (!score_two_pass(c.kn, plan, dist_out != nullptr)) {
+      timer_record(0, cs);
+      a.phase = 0; a.tile_stride = 1; a.thr_init = nullptr;
+      st = score_umma_launch(a, cs);
+      timer_record(1, cs);
+    } else {
+      st = sample_thresholds(c);
       if (st != CFL_OK) return st;
+      a.spill = c.at<tkey_t>(c.ws.spill); a.spill_cnt = c.at<int>(c.ws.spill_cnt);
+      a.phase = 2; a.tile_stride = 1; a.thr_init = c.at<float>(c.ws.tau_opt);
+      timer_record(0, cs);                 // bench.py times the dominant launch: the full filter pass
+      const bool lb_pass = score_lb_pass(c.kn, K);
+      st = lb_pass ? lower_bound_rounds(c) : exact_filter(c);
+      if (st != CFL_OK) return st;
+      float* thr_redo = c.at<float>(lb_pass ? c.ws.thr_redo2 : c.ws.thr_redo);
+      int* redo_tile = c.at<int>(lb_pass ? c.ws.redo_tile2 : c.ws.redo_tile);
+      st = exact_redo(c, lb_pass, thr_redo, redo_tile, m);
     }
+    if (st != CFL_OK) return st;
   }
   // after a lower-bound pass the verified queries are already written; only the redone ones remain
-  merge_rescore_kernel<<<(unsigned)(Q + (cer_parts ? plan.qt : 0)), MRG_THREADS, 0, cs>>>(
-      mode, a.keys, a.counts, redo_parts ? redo_parts : plan.parts, Q, plan.kk, k, Pq, ldq, K, d, E, lde, idx_base, top_val, top_idx,
-      redo_only, plan.qt, cer_keys, cer_counts, cer_parts, cer_thr, cer_idx);
-  CFL_LAUNCH_CHECK();
-  return CFL_OK;
+  return with_k(K, [&](auto KC) {
+    merge_rescore_kernel<KC><<<(unsigned)(Q + (m.cparts ? plan.qt : 0)), MRG_THREADS, 0, cs>>>(
+        a.keys, a.counts, m.parts, Q, plan.kk, k, Pq, ldq, d, E, lde, idx_base, top_val, top_idx, m.only, plan.qt,
+        m.ckeys, m.ccounts, m.cparts, m.cthr, m.cmap);
+    CFL_LAUNCH_CHECK();
+    return CFL_OK;
+  });
 }
 
 extern "C" {
@@ -1291,12 +1277,11 @@ int cfl_score_topk_stats(int64_t Q, int K, int d, int64_t N, int k, int packed, 
     if (thr_out) CFL_CUDA(cudaMemsetAsync(thr_out, 0, (size_t)3 * Q * sizeof(float), cs));
     return CFL_OK;
   }
-  size_t o_pc, o_qpar, o_qimg, o_keys, o_cnt, o_cimg;
-  const size_t need = score_ws_layout(Q, K, d, N, plan, packed == 0, &o_pc, &o_qpar, &o_qimg, &o_keys, &o_cnt, &o_cimg);
-  CFL_REQUIRE(ws_bytes >= need, CFL_ERR_WORKSPACE, "score_topk_stats: workspace too small (%zu < %zu)", ws_bytes, need);
-  const char* tau = (const char*)ws + align_up(o_cimg + (packed == 0 ? catalog_image_bytes(N, d) : 0), 1024);
-  const char* spill = tau + align_up((size_t)(5 * Q + 2 * plan.nqt + 12) * sizeof(float), 256);
-  const char* stats = spill + align_up((size_t)Q * LB_SPILL * sizeof(tkey_t) + (size_t)Q * sizeof(int), 256);
+  const ScoreWs w = score_ws(Q, K, d, N, plan, packed == 0);
+  CFL_REQUIRE(ws_bytes >= w.total, CFL_ERR_WORKSPACE, "score_topk_stats: workspace too small (%zu < %zu)", ws_bytes,
+              w.total);
+  const char* stats = (const char*)ws + w.stats;
+  const char* tau = (const char*)ws + w.tau;                  // tau, tau_opt and thr_redo are consecutive
   CFL_CUDA(cudaMemcpyAsync(stats_out, stats, CFL_SCORE_NSTATS * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, cs));
   if (thr_out) CFL_CUDA(cudaMemcpyAsync(thr_out, tau, (size_t)3 * Q * sizeof(float), cudaMemcpyDeviceToDevice, cs));
   return CFL_OK;

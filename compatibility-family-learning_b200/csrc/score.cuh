@@ -96,15 +96,29 @@ constexpr float CFL_PLANE_REL = 2.0e-4f;     // relative safety margin of the bo
 // Bytes of one query tile's tcgen05 B-operand image (score_umma.cu): [kstep][hl][chunk][nc = K*qt rows][16 B].
 __host__ __device__ constexpr uint32_t qimg_tile_bytes(int dpad, int nc) { return (uint32_t)dpad * 8u * (uint32_t)nc; }
 
+// Slots of the statistics counters of one cfl_score_topk call (cfl_score_topk_stats, cfl_b200.h; the order of
+// SCORE_STAT_NAMES in cfl/_native.py).
+enum ScoreStat {
+  STAT_SURVIVORS = 0,              // keys that survived the full filter pass, summed over queries
+  STAT_SPILL_QUERIES,              // queries that used their spill list
+  STAT_PROBE_DROPPED_QUERIES,      // queries the probe took out of the lower-bound pass
+  STAT_REDO_QUERIES,               // queries that failed the first verification
+  STAT_LOWER_BOUND_PASS,           // 1 when the lower-bound pass ran
+  STAT_EXACT_REDO_QUERIES,         // queries redone by the exact kernel under the safe threshold
+};
+
 ScorePlan make_score_plan(int64_t Q, int K, int d, int64_t N, int k, bool umma_ok);
 bool score_umma_supported(int K, int d);
+// Catalog image of cfl_catalog_pack (layout in score_umma.cu): behind the tf32 planes, |e - mu|^2 per row, the fp16
+// plane of the lower-bound pass, its range flag and lbrow = (|e - mu|^2, |e - mu|) per row.
+struct CatalogView { float* e2; unsigned char* f16; int* flag16; float2* lbrow; };
 size_t catalog_image_bytes(int64_t N, int d);
-size_t catalog_e2_offset(int64_t N, int d);      // byte offset of |e - mu|^2 per row (float, padded to whole tiles)
-size_t catalog_f16_offset(int64_t N, int d);     // byte offset of the fp16 plane inside the catalog image
-size_t catalog_f16_bytes(int64_t N, int d);      // plane only; the flag word follows it
-size_t catalog_lbrow_offset(int64_t N, int d);   // byte offset of lbrow[tiles*128] (float2) inside the catalog image
+CatalogView catalog_view(const void* image, int64_t N, int d);
 LbPlan make_lb_plan(int64_t Q, int K, int d, int64_t tiles);
-size_t score_lb_qimg_bytes(const LbPlan& p, int K, int d);   // lower-bound image + flag word + lbq
+// Query image of the lower-bound pass (score_lb.cu): the fp16 image, its flag word, lbq[2 per query slot].
+struct LbQimgView { unsigned char* img; int* flag; float* lbq; };
+size_t score_lb_qimg_bytes(const LbPlan& p, int K, int d);
+LbQimgView score_lb_qimg_view(void* base, const LbPlan& p, int K, int d);
 int catalog_pack_launch(const float* E, int64_t N, int d, int64_t lde, const float* mu, void* image,
                         cudaStream_t st);
 int score_umma_pack_queries(const ScoreArgs& a, void* qimg, cudaStream_t st);

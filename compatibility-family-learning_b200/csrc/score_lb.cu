@@ -103,10 +103,18 @@ LbPlan make_lb_plan(int64_t Q, int K, int d, int64_t tiles) {
   return best;
 }
 
+static size_t lb_qimg_image_bytes(const LbPlan& p, int K, int d) {
+  return (size_t)p.nqt * p.sub * p.qt * ((d + 15) / 16) * 2 * K * 16;
+}
 size_t score_lb_qimg_bytes(const LbPlan& p, int K, int d) {      // images + flag word + lbq[2 per query slot]
-  const int nks16 = (d + 15) / 16;
-  const size_t slots = (size_t)p.nqt * p.sub * p.qt;
-  return slots * nks16 * 2 * K * 16 + 16 + slots * 2 * sizeof(float);
+  return lb_qimg_image_bytes(p, K, d) + 16 + (size_t)p.nqt * p.sub * p.qt * 2 * sizeof(float);
+}
+LbQimgView score_lb_qimg_view(void* base, const LbPlan& p, int K, int d) {
+  LbQimgView v;
+  v.img = (unsigned char*)base;
+  v.flag = (int*)(v.img + lb_qimg_image_bytes(p, K, d));
+  v.lbq = (float*)((char*)v.flag + 16);
+  return v;
 }
 
 // fp16 lower-bound image: [qtile][kstep16][chunk][row n][8 halfs] with n = g*(GQ*K) + k*GQ + i for the query
@@ -619,18 +627,7 @@ lb_selftest_kernel(const float* __restrict__ Af, const float* __restrict__ Bf, f
 }
 
 int score_lb_launch(const ScoreArgs& a, cudaStream_t st) {
-  switch (a.K) {
-    case 1: return launch_lb<1>(a, st);
-    case 2: return launch_lb<2>(a, st);
-    case 3: return launch_lb<3>(a, st);
-    case 4: return launch_lb<4>(a, st);
-    case 5: return launch_lb<5>(a, st);
-    case 6: return launch_lb<6>(a, st);
-    case 7: return launch_lb<7>(a, st);
-    case 8: return launch_lb<8>(a, st);
-  }
-  set_error("score_lb: K=%d unsupported", a.K);
-  return CFL_ERR_UNSUPPORTED;
+  return with_k(a.K, [&](auto K) { return launch_lb<K>(a, st); });
 }
 
 }  // namespace cfl

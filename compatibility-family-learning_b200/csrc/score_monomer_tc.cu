@@ -41,6 +41,14 @@ size_t mono_image_bytes(int64_t N, int K, int d) {
   const int64_t tiles = (N + 127) / 128;
   return (size_t)tiles * (mono_dp(K, d) / 16) * 4096 + 16 + (size_t)tiles * 128 * sizeof(float2);
 }
+struct MonoImage { unsigned char* plane; int* flag; float2* lbrow; };
+static MonoImage mono_image(const void* image, int64_t N, int K, int d) {
+  MonoImage v;
+  v.plane = (unsigned char*)const_cast<void*>(image);
+  v.flag = (int*)(v.plane + (size_t)((N + 127) / 128) * (mono_dp(K, d) / 16) * 4096);
+  v.lbrow = (float2*)((char*)v.flag + 16);
+  return v;
+}
 
 __global__ void __launch_bounds__(128)
 mono_pack_kernel(const float* __restrict__ P, int64_t N, int K, int d, int64_t ldp, const float* __restrict__ mu,
@@ -229,10 +237,10 @@ mono_rescore_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ cou
     thr_redo[q] = redo ? 1.0f : __int_as_float(0xff800000);
     if (redo) redo_tile[q / MONO_QT] = 1;
     if (stats) {
-      atomicAdd(&stats[0], (unsigned long long)total);
-      if (spill_cnt[q] > 0) atomicAdd(&stats[1], 1ull);
-      if (redo) atomicAdd(&stats[3], 1ull);
-      if (q == 0) stats[4] = 1ull;
+      atomicAdd(&stats[STAT_SURVIVORS], (unsigned long long)total);
+      if (spill_cnt[q] > 0) atomicAdd(&stats[STAT_SPILL_QUERIES], 1ull);
+      if (redo) atomicAdd(&stats[STAT_REDO_QUERIES], 1ull);
+      if (q == 0) stats[STAT_LOWER_BOUND_PASS] = 1ull;
     }
   }
   __syncthreads();
@@ -249,7 +257,7 @@ mono_rescore_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ cou
 }
 
 struct MonoTcLayout {
-  size_t keys_m, cnt_m, sval, sidx, tau, lbimg, keys_lb, cnt_lb, spill, spill_cnt, stats, total;
+  size_t keys_m, cnt_m, sval, sidx, tau, tau_opt, thr_redo, redo_tile, lbimg, keys_lb, cnt_lb, spill, spill_cnt, stats, total;
 };
 static MonoTcLayout mono_tc_layout(int64_t Q, int K, int d, int64_t N, int k, const LbPlan& lb) {
   MonoTcLayout L;
@@ -259,7 +267,11 @@ static MonoTcLayout mono_tc_layout(int64_t Q, int K, int d, int64_t N, int k, co
   L.cnt_m = off;     off = align_up(off + (size_t)parts_m * Q * sizeof(int), 256);
   L.sval = off;      off = align_up(off + (size_t)Q * k * sizeof(float), 256);
   L.sidx = off;      off = align_up(off + (size_t)Q * k * sizeof(int64_t), 256);
-  L.tau = off;       off = align_up(off + (size_t)(3 * Q + (Q + MONO_QT - 1) / MONO_QT + 4) * sizeof(float), 256);
+  // tau[Q], tau_opt[Q], thr_redo[Q], then the redo flag per query tile of the CUDA-core kernel
+  L.tau = off;       off += (size_t)Q * sizeof(float);
+  L.tau_opt = off;   off += (size_t)Q * sizeof(float);
+  L.thr_redo = off;  off += (size_t)Q * sizeof(float);
+  L.redo_tile = off; off = align_up(off + (size_t)((Q + MONO_QT - 1) / MONO_QT + 4) * sizeof(int), 256);
   L.lbimg = off;     off = align_up(off + score_lb_qimg_bytes(lb, 1, mono_dp(K, d)), 1024);
   L.keys_lb = off;   off = align_up(off + (size_t)lb.parts * Q * TOPK_STRIDE * sizeof(tkey_t), 256);
   L.cnt_lb = off;    off = align_up(off + (size_t)lb.parts * Q * sizeof(int), 256);
@@ -289,13 +301,10 @@ int cfl_monomer_pack(const float* Pc, int64_t N, int K, int d, int64_t ldp, cons
   CFL_REQUIRE(cfl_monomer_pack_bytes(N, K, d) > 0, CFL_ERR_UNSUPPORTED, "monomer_pack: K(d+1) = %d exceeds 128", K * (d + 1));
   CFL_REQUIRE(image_bytes >= mono_image_bytes(N, K, d), CFL_ERR_WORKSPACE, "monomer_pack: image buffer too small");
   CFL_REQUIRE(((uintptr_t)image & 1023u) == 0, CFL_ERR_INVALID, "monomer_pack: image must be 1024-byte aligned");
-  const int64_t tiles = (N + 127) / 128;
-  unsigned char* img = (unsigned char*)image;
-  const size_t plane = (size_t)tiles * (mono_dp(K, d) / 16) * 4096;
-  int* flag = (int*)(img + plane);
+  const MonoImage v = mono_image(image, N, K, d);
   cudaStream_t cs = (cudaStream_t)stream;
-  CFL_CUDA(cudaMemsetAsync(flag, 0, 16, cs));
-  mono_pack_kernel<<<(unsigned)tiles, 128, 0, cs>>>(Pc, N, K, d, ldp, mu, img, flag, (float2*)(img + plane + 16));
+  CFL_CUDA(cudaMemsetAsync(v.flag, 0, 16, cs));
+  mono_pack_kernel<<<(unsigned)((N + 127) / 128), 128, 0, cs>>>(Pc, N, K, d, ldp, mu, v.plane, v.flag, v.lbrow);
   CFL_LAUNCH_CHECK();
   return CFL_OK;
 }
@@ -332,9 +341,9 @@ int cfl_score_topk_monomer_packed(const float* Aq, int64_t lda, const float* Wq,
   float* sval = (float*)(base + L.sval);
   int64_t* sidx = (int64_t*)(base + L.sidx);
   float* tau = (float*)(base + L.tau);
-  float* tau_opt = tau + Q;
-  float* thr_redo = tau + 2 * Q;
-  int* redo_tile = (int*)(tau + 3 * Q);
+  float* tau_opt = (float*)(base + L.tau_opt);
+  float* thr_redo = (float*)(base + L.thr_redo);
+  int* redo_tile = (int*)(base + L.redo_tile);
   const int nredo = (int)((Q + MONO_QT - 1) / MONO_QT);
   unsigned long long* stats = (unsigned long long*)(base + L.stats);
   CFL_CUDA(cudaMemsetAsync(stats, 0, CFL_SCORE_NSTATS * sizeof(unsigned long long), cs));
@@ -361,21 +370,18 @@ int cfl_score_topk_monomer_packed(const float* Aq, int64_t lda, const float* Wq,
   a.mode = CFL_MONOMER; a.K = 1; a.d = dp; a.Q = Q; a.N = N;
   a.plan.impl = 1; a.plan.tiles = tiles; a.plan.dpad = dp; a.plan.kk = k;
   a.lb = lb;
-  const unsigned char* img = (const unsigned char*)image;
-  const size_t plane = (size_t)tiles * (dp / 16) * 4096;
-  a.cimg16 = img; a.cflag16 = (const int*)(img + plane); a.lbrow = (const float2*)(img + plane + 16);
-  a.qimg16 = base + L.lbimg;
-  a.qflag16 = (const int*)((const char*)a.qimg16 + (size_t)lb.nqt * lb.sub * lb.qt * (dp / 16) * 2 * 16);
-  a.lbq = (const float*)((const char*)a.qflag16 + 16);
+  const MonoImage mi = mono_image(image, N, K, d);
+  a.cimg16 = mi.plane; a.cflag16 = mi.flag; a.lbrow = mi.lbrow;
+  const LbQimgView qv = score_lb_qimg_view(base + L.lbimg, lb, 1, dp);
+  a.qimg16 = qv.img; a.qflag16 = qv.flag; a.lbq = qv.lbq;
   a.keys = (tkey_t*)(base + L.keys_lb); a.counts = (int*)(base + L.cnt_lb);
   a.spill = (tkey_t*)(base + L.spill); a.spill_cnt = spill_cnt;
   a.thr_init = thr_redo;                                       // filter thresholds (overwritten by the rescoring kernel later)
   a.phase = 3; a.tile_stride = 1;
-  CFL_CUDA(cudaMemsetAsync(const_cast<int*>(a.qflag16), 0, 16, cs));
+  CFL_CUDA(cudaMemsetAsync(qv.flag, 0, 16, cs));
   const int64_t slots = (int64_t)lb.nqt * lb.sub * lb.qt;
   mono_prep_lb_kernel<<<(unsigned)((slots + 3) / 4), 128, 0, cs>>>(Aq, lda, Wq, Q, K, d, mu, lb.qt, lb.nqt * lb.sub, dp,
-                                                                  (unsigned char*)const_cast<void*>(a.qimg16),
-                                                                  const_cast<int*>(a.qflag16), const_cast<float*>(a.lbq));
+                                                                  qv.img, qv.flag, qv.lbq);
   CFL_LAUNCH_CHECK();
   timer_record(0, cs);
   st = score_lb_launch(a, cs);
@@ -384,18 +390,14 @@ int cfl_score_topk_monomer_packed(const float* Aq, int64_t lda, const float* Wq,
 
   // 3. exact rescoring + verification
   const size_t rs_smem = ((size_t)d + K + lb.parts + 2 + 4) * sizeof(float);
-#define CFL_MRS_CASE(KK)                                                                                             \
-  case KK:                                                                                                           \
-    mono_rescore_kernel<KK><<<(unsigned)Q, MRG_THREADS, rs_smem, cs>>>(                                              \
-        a.keys, a.counts, lb.parts, Q, k, Aq, lda, Wq, d, Pc, ldp, idx_base, top_val, top_idx, tau, tau_opt, thr_redo,   \
-        redo_tile, a.spill, a.spill_cnt, stats);                                                                      \
-    break;
-  switch (K) {
-    CFL_MRS_CASE(1) CFL_MRS_CASE(2) CFL_MRS_CASE(3) CFL_MRS_CASE(4)
-    CFL_MRS_CASE(5) CFL_MRS_CASE(6) CFL_MRS_CASE(7) CFL_MRS_CASE(8)
-  }
-#undef CFL_MRS_CASE
-  CFL_LAUNCH_CHECK();
+  st = with_k(K, [&](auto KC) {
+    mono_rescore_kernel<KC><<<(unsigned)Q, MRG_THREADS, rs_smem, cs>>>(
+        a.keys, a.counts, lb.parts, Q, k, Aq, lda, Wq, d, Pc, ldp, idx_base, top_val, top_idx, tau, tau_opt, thr_redo,
+        redo_tile, a.spill, a.spill_cnt, stats);
+    CFL_LAUNCH_CHECK();
+    return CFL_OK;
+  });
+  if (st != CFL_OK) return st;
 
   // 4. redo: exact CUDA-core pass for the query tiles that hold a flagged query, merged for the flagged queries only
   st = mono_exact_launch(Aq, lda, Wq, Q, K, d, Pc, N, ldp, k, 1, redo_tile, keys_m, cnt_m, &parts_m, cs);

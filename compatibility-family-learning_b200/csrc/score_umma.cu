@@ -45,24 +45,33 @@ bool score_umma_supported(int K, int d) {
 // [tile][kstep][hl][chunk][row 0..127][4 floats]  (8 KB per (tile,kstep)), then e2[tiles*128].
 // ... then the fp16 plane of the lower-bound pass: [tile][kstep16][chunk 0|1][row 0..127][8 halfs] (4 KB per
 // (tile, 16 columns)), then one flag word (non-zero: a centred value left the fp16 range, plane unusable).
-size_t catalog_e2_offset(int64_t N, int d) {
+static size_t catalog_e2_offset(int64_t N, int d) {
   return (size_t)((N + 127) / 128) * ((d + 7) / 8) * GP_ASTAGE;
 }
-size_t catalog_f16_offset(int64_t N, int d) {
+static size_t catalog_f16_offset(int64_t N, int d) {
   return catalog_e2_offset(N, d) + (size_t)((N + 127) / 128) * 128 * sizeof(float);
 }
-size_t catalog_f16_bytes(int64_t N, int d) {
+static size_t catalog_f16_bytes(int64_t N, int d) {
   const int64_t tiles = (N + 127) / 128;
   return (size_t)tiles * ((d + 15) / 16) * (GP_ASTAGE / 2);
 }
 // ... then lbrow[tiles*128] float2 = (|e - mu|^2, |e - mu|) per row, (+inf, 0) for the padding rows of the last tile:
 // what the lower-bound pass needs per row (its margin has a term in |e|), one 8-byte load per row and tile.
-size_t catalog_lbrow_offset(int64_t N, int d) {
+static size_t catalog_lbrow_offset(int64_t N, int d) {
   return catalog_f16_offset(N, d) + catalog_f16_bytes(N, d) + 16;
 }
 size_t catalog_image_bytes(int64_t N, int d) {
   const int64_t tiles = (N + 127) / 128;
   return catalog_lbrow_offset(N, d) + (size_t)tiles * 128 * sizeof(float2);
+}
+CatalogView catalog_view(const void* image, int64_t N, int d) {
+  unsigned char* img = (unsigned char*)const_cast<void*>(image);
+  CatalogView v;
+  v.e2 = (float*)(img + catalog_e2_offset(N, d));
+  v.f16 = img + catalog_f16_offset(N, d);
+  v.flag16 = (int*)(v.f16 + catalog_f16_bytes(N, d));
+  v.lbrow = (float2*)(img + catalog_lbrow_offset(N, d));
+  return v;
 }
 
 __global__ void __launch_bounds__(128)
@@ -111,13 +120,10 @@ pack_catalog_kernel(const float* __restrict__ E, int64_t N, int d, int64_t lde,
 int catalog_pack_launch(const float* E, int64_t N, int d, int64_t lde, const float* mu, void* image,
                         cudaStream_t st) {
   const int64_t tiles = (N + 127) / 128;
-  unsigned char* img = (unsigned char*)image;
-  float* e2g = (float*)(img + catalog_e2_offset(N, d));
-  unsigned char* img16 = img + catalog_f16_offset(N, d);
-  int* flag16 = (int*)(img16 + catalog_f16_bytes(N, d));
-  CFL_CUDA(cudaMemsetAsync(flag16, 0, 16, st));
-  float2* lbrow = (float2*)(img + catalog_lbrow_offset(N, d));
-  pack_catalog_kernel<<<(unsigned)tiles, 128, 0, st>>>(E, N, d, lde, mu, img, e2g, img16, flag16, lbrow);
+  const CatalogView v = catalog_view(image, N, d);
+  CFL_CUDA(cudaMemsetAsync(v.flag16, 0, 16, st));
+  pack_catalog_kernel<<<(unsigned)tiles, 128, 0, st>>>(E, N, d, lde, mu, (unsigned char*)image, v.e2, v.f16, v.flag16,
+                                                       v.lbrow);
   CFL_LAUNCH_CHECK();
   return CFL_OK;
 }
@@ -397,18 +403,7 @@ static int launch_umma(const ScoreArgs& a, cudaStream_t st) {
 }
 
 int score_umma_launch(const ScoreArgs& a, cudaStream_t st) {
-  switch (a.K) {
-    case 1: return launch_umma<1>(a, st);
-    case 2: return launch_umma<2>(a, st);
-    case 3: return launch_umma<3>(a, st);
-    case 4: return launch_umma<4>(a, st);
-    case 5: return launch_umma<5>(a, st);
-    case 6: return launch_umma<6>(a, st);
-    case 7: return launch_umma<7>(a, st);
-    case 8: return launch_umma<8>(a, st);
-  }
-  set_error("score_umma: K=%d unsupported", a.K);
-  return CFL_ERR_UNSUPPORTED;
+  return with_k(a.K, [&](auto K) { return launch_umma<K>(a, st); });
 }
 
 }  // namespace cfl
