@@ -53,6 +53,11 @@ SIGNATURES = {
     "cfl_score_topk_packed": (_int, [_int, _vp, _i64, _int, _int, _i64, _vp, _vp, _i64, _i64, _vp, _int, _i64,
                                      _vp, _vp, _vp, _vp, _sz, _vp]),
     "cfl_score_topk_stats": (_int, [_i64, _int, _int, _i64, _int, _int, _vp, _sz, _vp, _vp, _vp]),
+    "cfl_source_catalog_pack_bytes": (_sz, [_i64, _int, _int]),
+    "cfl_source_catalog_pack": (_int, [_vp, _i64, _int, _int, _i64, _vp, _vp, _sz, _vp]),
+    "cfl_score_topk_source_workspace_bytes": (_sz, [_i64, _int, _int, _i64, _int]),
+    "cfl_score_topk_source": (_int, [_vp, _i64, _i64, _int, _int, _vp, _vp, _i64, _i64, _vp, _int, _i64,
+                                     _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "cfl_score_topk_monomer_workspace_bytes": (_sz, [_i64, _int, _int, _i64, _int]),
     "cfl_score_topk_monomer": (_int, [_vp, _i64, _vp, _i64, _int, _int, _vp, _i64, _i64, _int, _i64,
                                       _vp, _vp, _vp, _vp, _sz, _vp]),
@@ -386,6 +391,62 @@ def score_topk(Pq, E, k, mu=None, mode="pcd", idx_base=0, want_dense=False, imag
 SCORE_NSTATS = 8
 SCORE_STAT_NAMES = ("survivors", "spill_queries", "probe_dropped_queries", "redo_queries", "lower_bound_pass",
                     "exact_redo_queries")
+
+
+def source_catalog_pack(P, mu=None):
+    """Tensor-core image of a SOURCE catalog P [N,K,d] (the K prototypes of every source item), centred on mu, for
+    score_topk_source; built once per shard.  None for an empty catalog."""
+    P = _f32c(P, "P")
+    if P.dim() != 3:
+        raise CflNativeError("source_catalog_pack: P must be [N,K,d]")
+    N, K, d = P.shape
+    if N == 0:
+        return None
+    nbytes = lib().cfl_source_catalog_pack_bytes(N, K, d)
+    if nbytes == 0:
+        raise CflNativeError(f"source_catalog_pack: K={K} d={d} outside K <= {MAX_K}, d <= 128")
+    P2, ldp = _rows(P.reshape(N, K * d), "P")
+    img = torch.empty(nbytes + 1024, dtype=torch.uint8, device=P.device)
+    off = (-img.data_ptr()) % 1024
+    img = img[off:off + nbytes]
+    mu = None if mu is None else _f32c(mu, "mu").contiguous()
+    _check(lib().cfl_source_catalog_pack(_ptr(P2), N, K, d, ldp, _ptr(mu), _ptr(img), nbytes, _stream()),
+           "cfl_source_catalog_pack")
+    return img
+
+
+def score_topk_source(Eq, P, image, k, mu=None, idx_base=0, want_dense=False, want_stats=False):
+    """The other direction of pcd: top-k SOURCE items (catalog P [N,K,d], image = source_catalog_pack(P, mu)) of every
+    TARGET query Eq [Q,d], dist(q,c) = pcd(v = Eq[q], P = P[c]) (base.py:125-139); exact (rescored) values, ties ->
+    lower index.  ``want_dense`` appends the un-rescored Gram values [Q,N], ``want_stats`` the int64 counters
+    (SCORE_STAT_NAMES) of this call."""
+    Eq, ldq = _rows(Eq, "Eq")
+    P = _f32c(P, "P")
+    if P.dim() != 3:
+        raise CflNativeError("score_topk_source: P must be [N,K,d]")
+    N, K, d = P.shape
+    Q = Eq.shape[0]
+    if Eq.shape[1] != d:
+        raise CflNativeError(f"score_topk_source: Eq is {tuple(Eq.shape)} but P is {tuple(P.shape)}")
+    if N > 0 and image is None:
+        raise CflNativeError("score_topk_source: a non-empty catalog needs its image (source_catalog_pack)")
+    P2, ldp = _rows(P.reshape(N, K * d), "P")
+    dev = P.device
+    top_val = torch.empty(Q, k, dtype=torch.float32, device=dev)
+    top_idx = torch.empty(Q, k, dtype=torch.int64, device=dev)
+    dense = torch.empty(Q, N, dtype=torch.float32, device=dev) if want_dense else None
+    stats = torch.zeros(SCORE_NSTATS, dtype=torch.int64, device=dev) if want_stats else None
+    mu = None if mu is None else _f32c(mu, "mu").contiguous()
+    ws = _ws.get(lib().cfl_score_topk_source_workspace_bytes(Q, K, d, N, k), dev)
+    _check(lib().cfl_score_topk_source(_ptr(Eq), ldq, Q, K, d, _ptr(image), _ptr(P2), N, ldp, _ptr(mu), int(k),
+                                       int(idx_base), _ptr(top_val), _ptr(top_idx), _ptr(dense), _ptr(stats),
+                                       _ptr(ws), ws.numel(), _stream()), "cfl_score_topk_source")
+    out = (top_val, top_idx)
+    if want_dense:
+        out += (dense,)
+    if want_stats:
+        out += (stats,)
+    return out
 
 
 def score_topk_monomer(a, w, P, k, idx_base=0, want_dense=False):

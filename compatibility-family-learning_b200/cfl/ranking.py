@@ -471,3 +471,82 @@ class MonomerCatalogIndex:
 
     def scores(self, dist: torch.Tensor) -> torch.Tensor:
         return max(self.theta, 1e-6) - dist
+
+
+class SourceCatalogIndex:
+    """The other direction of pcd: rank the SOURCE items of a catalog for TARGET queries.
+
+    pcd is not symmetric (DistBase.build_dist, cfl/models/base.py:125-139): dist = |v - sum_k s_k p_k|^2 takes v = e0 of
+    the target item and p_k = the K prototypes of the source item.  ``CatalogIndex`` answers "which targets go with
+    this source"; this index answers "which sources is this target compatible with" -- e.g. which existing items
+    should now recommend a newly added item.  One shard holds the sources' prototypes ``[N, K, d]`` resident on the GPU
+    with their tensor-core image (``source_catalog_pack``), centred on the mean of all prototypes of all shards;
+    sharding, the all-gather + merge and the tie rule are those of ``CatalogIndex``.
+
+    ``weights``: the catalog side goes through the prototype head ``Vp/gp/bp`` (``from_features``), the queries through
+    the embedding head ``V0/g0/b0`` (``project_queries``).  For a directed model (e.g. Polyvore ``top_to_other``, where
+    ``DistEncoderSrc`` encodes the source side and ``DistEncoderDst`` the target side) build ``EncoderWeights`` with
+    ``Vp, gp, bp`` from the Src encoder's prototype head and ``V0, g0, b0`` from the Dst encoder's embedding head."""
+
+    def __init__(self, weights: EncoderWeights, prototypes: torch.Tensor, idx_base: int = 0,
+                 n_total: Optional[int] = None, theta: float = 1e-6, group=None):
+        if not prototypes.is_cuda:
+            raise nat.CflNativeError("SourceCatalogIndex needs CUDA prototypes (there is no CPU path)")
+        self.w = weights
+        self.P = prototypes.view(prototypes.shape[0], weights.K, weights.d)
+        self.idx_base = int(idx_base)
+        self.n_total = int(n_total if n_total is not None else prototypes.shape[0])
+        self.theta = float(theta)
+        self.group = group
+        self.mu = self._global_mean()
+        self.image = nat.source_catalog_pack(self.P, self.mu)
+
+    def _global_mean(self):
+        """Mean of every prototype of every shard, so that all ranks centre on the same vector."""
+        s = self.P.double().sum(dim=(0, 1))
+        n = torch.tensor([float(self.P.shape[0] * self.P.shape[1])], dtype=torch.float64, device=self.P.device)
+        if self._world() > 1:
+            torch.distributed.all_reduce(s, group=self.group)
+            torch.distributed.all_reduce(n, group=self.group)
+        return (s / n.clamp(min=1)).float()
+
+    @classmethod
+    def from_features(cls, weights: EncoderWeights, features: torch.Tensor, idx_base: int = 0,
+                      n_total: Optional[int] = None, chunk: int = 1 << 16, **kw):
+        """Projects this rank's source rows through the prototype head (no communication)."""
+        dev = weights.Vp.device
+        n = features.shape[0]
+        P = torch.empty(n, weights.K * weights.d, dtype=torch.float32, device=dev)
+        for lo in range(0, n, chunk):
+            xb = features[lo:lo + chunk]
+            if not xb.is_cuda:
+                xb = xb.to(dev, non_blocking=True)
+            y, _, _ = nat.project_fwd(xb, weights.Vp, weights.gp, weights.bp, weights.weight_norm,
+                                      weights.in_scale, weights.act)
+            P[lo:lo + chunk] = y
+        return cls(weights, P, idx_base=idx_base, n_total=n_total, **kw)
+
+    def _world(self):
+        if torch.distributed.is_available() and torch.distributed.is_initialized():
+            return torch.distributed.get_world_size(self.group)
+        return 1
+
+    def project_queries(self, xq: torch.Tensor) -> torch.Tensor:
+        """Query side = e0 of the target item (base.py:47-57)."""
+        if not xq.is_cuda:
+            xq = xq.to(self.P.device, non_blocking=True)
+        e, _, _ = nat.project_fwd(xq, self.w.V0, self.w.g0, self.w.b0, self.w.weight_norm, self.w.in_scale, self.w.act)
+        return e
+
+    def rank_local(self, Eq: torch.Tensor, k: int):
+        return nat.score_topk_source(Eq, self.P, self.image, k, mu=self.mu, idx_base=self.idx_base)
+
+    def rank(self, xq: torch.Tensor, k: int = 100):
+        """-> (dist [Q,k] ascending, index [Q,k] int64 global source rows).  score = theta+ - dist."""
+        tv, ti = self.rank_local(self.project_queries(xq), k)
+        world = self._world()
+        return (tv, ti) if world == 1 else _gather_merge(tv, ti, self.group, world)
+
+    def scores(self, dist: torch.Tensor) -> torch.Tensor:
+        """Thresholder (blocks.py:21-22): max(theta, 1e-6) - dist."""
+        return max(self.theta, 1e-6) - dist

@@ -4,6 +4,11 @@
 //   D[c, k*QT + q] = e_c . p_{q,k}        M = 128 catalog rows (TMEM lanes), N = NC = K*QT columns,
 //                                         MMA-K = the embedding dimension (8 per K-step), 3xTF32 (umma.cuh)
 //
+// The source-catalog kernel score_src_umma_kernel (score_umma.cu) runs the same pipeline in the other direction: the
+// catalog rows carry K prototype planes and the query tile one vector per query, D[c, k*QT + q] = p_{c,k} . e_q.  Its
+// tiles have PLANES = K A planes, each multiplied by the same QT-column B image into its own QT columns (gram_mma /
+// gram_tma template argument; 1 for the other kernels).
+//
 // A CTA (part, qtile) keeps its query tile's tf32 hi/lo image resident in shared memory and streams a range of 128-row
 // tiles of the packed catalog image (score_umma.cu).  18 warps:
 //   warp  GP_NEPI      one lane issues tcgen05.mma (3 per K-step) and tcgen05.commit       (gram_mma)
@@ -33,15 +38,18 @@ __host__ __device__ constexpr int gram_gq(int K) { return K <= 2 ? 16 : (K <= 4 
 // mbarriers and the TMEM address slot, placed by gram_layout_end once the caller knows where its back region ends.
 // The front region sits at a fixed distance from the 1024-aligned end of the query image, so the epilogue addresses a
 // buffer there with an immediate offset instead of one more live register.
+// SRC (the source-catalog kernel): a query image of QT vectors, and qpar holds one float per query, |e_q - mu|^2; no
+// plane-bound block.
 struct GramLayout { uint32_t b_img, a_ring, front, qpar, qpl, back, bars, tmem_slot, total; };
+template <bool SRC = false>
 __host__ __device__ inline GramLayout gram_layout(int K, int qt, int dpad, uint32_t front_bytes) {
   GramLayout L;
   uint32_t off = 0;
-  L.b_img = off;   off += qimg_tile_bytes(dpad, K * qt);                      off = (off + 1023u) & ~1023u;
+  L.b_img = off;   off += qimg_tile_bytes(dpad, SRC ? qt : K * qt);           off = (off + 1023u) & ~1023u;
   L.a_ring = off;  off += GP_NSTAGE * 2u * GP_ASTAGE;
   L.front = off;   off += front_bytes;
-  L.qpar = off;    off += (uint32_t)qt * (uint32_t)qpar_stride(K) * 4u;      off = (off + 15u) & ~15u;
-  L.qpl = off;     off += (uint32_t)qt * (uint32_t)qplane_stride(K) * 4u;    off = (off + 15u) & ~15u;
+  L.qpar = off;    off += (uint32_t)qt * (uint32_t)(SRC ? 1 : qpar_stride(K)) * 4u;      off = (off + 15u) & ~15u;
+  L.qpl = off;     off += (uint32_t)qt * (uint32_t)(SRC ? 0 : qplane_stride(K)) * 4u;    off = (off + 15u) & ~15u;
   L.back = off;
   return L;
 }
@@ -88,13 +96,8 @@ __device__ __forceinline__ GramPipe gram_pipe(unsigned char* smem, const GramLay
   return P;
 }
 
-// First half of the one-time setup: barriers and TMEM columns (MMA warp), and the per-query blocks of queries
-// [q0, q0 + nq) stored interleaved by query PAIR, qpar[(pair*QPS + j)*2 + (q&1)], with the soft-min block's first K
-// entries negated: ready for softmin_pair / plane_bound_pair.  The padding queries of the tile get zeros.  The caller
-// stages its own epilogue state, then calls gram_start.
-template <int K>
-__device__ __forceinline__ void gram_setup(const GramPipe& P, const float* __restrict__ qpar,
-                                           const float* __restrict__ qplane, int64_t q0, int nq, int QT) {
+// First half of the one-time setup: barriers and TMEM columns (MMA warp).
+__device__ __forceinline__ void gram_init(const GramPipe& P) {
   const int tid = threadIdx.x, warp = tid >> 5;
   if (warp == GP_NEPI) {
     if ((tid & 31) == 0) {
@@ -107,6 +110,17 @@ __device__ __forceinline__ void gram_setup(const GramPipe& P, const float* __res
     __syncwarp();
     umma::tmem_alloc(P.tmem_slot, P.ncols);
   }
+}
+
+// gram_init, and the per-query blocks of queries [q0, q0 + nq) stored interleaved by query PAIR,
+// qpar[(pair*QPS + j)*2 + (q&1)], with the soft-min block's first K entries negated: ready for softmin_pair /
+// plane_bound_pair.  The padding queries of the tile get zeros.  The caller stages its own epilogue state, then calls
+// gram_start.
+template <int K>
+__device__ __forceinline__ void gram_setup(const GramPipe& P, const float* __restrict__ qpar,
+                                           const float* __restrict__ qplane, int64_t q0, int nq, int QT) {
+  const int tid = threadIdx.x;
+  gram_init(P);
   constexpr int QPS = qpar_stride(K);
   for (int i = tid; i < QT * QPS; i += GP_THREADS) {
     const int ql = i / QPS, j = i % QPS;
@@ -129,25 +143,31 @@ __device__ __forceinline__ uint32_t gram_start(const GramPipe& P) {
   return *P.tmem_slot;
 }
 
-// MMA warp: one lane issues the K-steps of ntiles catalog tiles, tile t into accumulator buffer t & 1.
+// MMA warp: one lane issues the A-steps of ntiles catalog tiles, tile t into accumulator buffer t & 1.  A tile is
+// PLANES * nks A-steps; step s multiplies A block s by B K-step s % nks into the columns [(s / nks) * N, +N) of the
+// buffer, N = NC / PLANES, starting a fresh sum when s % nks == 0.
+template <int PLANES = 1>
 __device__ __forceinline__ void gram_mma(const GramPipe& P, uint32_t tmem_base, int ntiles) {
   using namespace umma;
   if (!elect_one()) return;
   mbar_wait(P.bfull, 0);
-  const Step3Desc sd = make_step3((uint32_t)P.NC, make_idesc_tf32(128, (uint32_t)P.NC));
+  const uint32_t N = (uint32_t)(P.NC / PLANES);
+  const Step3Desc sd = make_step3(N, make_idesc_tf32(128, N));
   const uint32_t a_base = smem_u32(P.a_ring), b_base = smem_u32(P.b_img);
-  const uint32_t b_step = 4u * (uint32_t)P.NC * 16u;
+  const uint32_t b_step = 4u * N * 16u;
   int stage = 0; uint32_t phase = 0;
   for (int t = 0; t < ntiles; ++t) {
     const int buf = t & 1;
     mbar_wait(&P.tempty[buf], ((uint32_t)(t >> 1) & 1u) ^ 1u);
     tc_fence_after();
     const uint32_t d_tmem = tmem_base + (uint32_t)(buf * P.NC);
-    for (int ks = 0; ks < P.nks; ks += P.kss) {
+    for (int s = 0; s < PLANES * P.nks; s += P.kss) {
       mbar_wait(&P.full[stage], phase);
       tc_fence_after();
+      const int ks = PLANES == 1 ? s : s % P.nks;             // kss divides nks: a stage never straddles two planes
+      const uint32_t d_col = PLANES == 1 ? d_tmem : d_tmem + (uint32_t)(s / P.nks) * N;
       for (int j = 0; j < P.kss; ++j)
-        mma_step3(sd, d_tmem, a_base + (stage * 2 + j) * GP_ASTAGE, b_base + (ks + j) * b_step, ks + j == 0);
+        mma_step3(sd, d_col, a_base + (stage * 2 + j) * GP_ASTAGE, b_base + (ks + j) * b_step, ks + j == 0);
       mma_commit(&P.empty[stage]);
       if (++stage == GP_NSTAGE) { stage = 0; phase ^= 1u; }
     }
@@ -155,13 +175,14 @@ __device__ __forceinline__ void gram_mma(const GramPipe& P, uint32_t tmem_base, 
   }
 }
 
-// TMA warp: one lane loads query tile qtile's image, then streams the catalog tiles t0, t0 + ts, ... (ntiles of them)
-// through the ring.
+// TMA warp: one lane loads query tile qtile's image, then streams the catalog tiles t0, t0 + ts, ... (ntiles of them,
+// PLANES * nks A blocks each) through the ring.
+template <int PLANES = 1>
 __device__ __forceinline__ void gram_tma(const GramPipe& P, const void* qimg, int qtile, const void* cimg, int64_t t0,
                                          int ts, int ntiles) {
   using namespace umma;
   if (!elect_one()) return;
-  const uint32_t bbytes = qimg_tile_bytes(8 * P.nks, P.NC);
+  const uint32_t bbytes = qimg_tile_bytes(8 * P.nks, P.NC / PLANES);
   const unsigned char* qsrc = (const unsigned char*)qimg + (size_t)qtile * bbytes;
   mbar_arrive_expect_tx(P.bfull, bbytes);
   for (uint32_t o = 0; o < bbytes; o += 32768u) {
@@ -170,8 +191,8 @@ __device__ __forceinline__ void gram_tma(const GramPipe& P, const void* qimg, in
   }
   int stage = 0; uint32_t phase = 0;
   for (int t = 0; t < ntiles; ++t) {
-    const unsigned char* src = (const unsigned char*)cimg + (size_t)(t0 + (int64_t)t * ts) * P.nks * GP_ASTAGE;
-    for (int ks = 0; ks < P.nks; ks += P.kss) {
+    const unsigned char* src = (const unsigned char*)cimg + (size_t)(t0 + (int64_t)t * ts) * PLANES * P.nks * GP_ASTAGE;
+    for (int ks = 0; ks < PLANES * P.nks; ks += P.kss) {
       mbar_wait(&P.empty[stage], phase ^ 1u);
       mbar_arrive_expect_tx(&P.full[stage], (uint32_t)P.kss * GP_ASTAGE);
       bulk_g2s(P.a_ring + stage * 2 * GP_ASTAGE, src + (size_t)ks * GP_ASTAGE, (uint32_t)P.kss * GP_ASTAGE, &P.full[stage]);

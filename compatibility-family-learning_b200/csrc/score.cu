@@ -22,9 +22,13 @@ static int choose_kk(int k) {
 }
 
 ScorePlan make_score_plan(int64_t Q, int K, int d, int64_t N, int k, bool umma_ok) {
+  return make_score_plan_qt(Q, umma_ok ? score_umma_qt(K, d) : SIMT_QT, d, N, k, umma_ok);
+}
+
+ScorePlan make_score_plan_qt(int64_t Q, int qt, int d, int64_t N, int k, bool umma_ok) {
   ScorePlan p;
   p.impl = umma_ok ? 1 : 0;
-  p.qt = umma_ok ? score_umma_qt(K, d) : SIMT_QT;
+  p.qt = qt;
   p.nqt = (int)((Q + p.qt - 1) / p.qt);
   p.tiles = (N + 127) / 128;
   int sms = sm_count();
@@ -149,6 +153,23 @@ int score_prep_queries_launch(const float* Pq, int64_t Q, int K, int d, int64_t 
   prep_queries_kernel<<<(unsigned)((Q + 3) / 4), 128, 0, st>>>(Pq, Q, K, d, ldq, mu, Pc, qpar, qplane);
   CFL_LAUNCH_CHECK();
   return CFL_OK;
+}
+
+// ---- query prep of the source-catalog call: centred target embeddings [Q,d] and |e_q - mu|^2 ------------------------
+__global__ void prep_source_queries_kernel(const float* __restrict__ Eq, int64_t Q, int d, int64_t ldq,
+                                           const float* __restrict__ mu, float* __restrict__ Ec,
+                                           float* __restrict__ e2q) {
+  const int64_t q = (int64_t)blockIdx.x * (blockDim.x / 32) + threadIdx.x / 32;
+  const int lane = threadIdx.x & 31;
+  if (q >= Q) return;
+  float acc = 0.0f;
+  for (int j = lane; j < d; j += 32) {
+    const float v = Eq[q * ldq + j] - (mu ? mu[j] : 0.0f);
+    Ec[q * d + j] = v;
+    acc = fmaf(v, v, acc);
+  }
+  acc = warp_sum(acc);
+  if (lane == 0) e2q[q] = acc;
 }
 
 // ---- CUDA-core scoring kernel ---------------------------------------------------------------
@@ -282,6 +303,41 @@ merge_rescore_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ co
   if (t == 0) s_fill = fill;
   __syncthreads();
   mrg_compact(s, &s_fill, &s_thr, kk, t);           // re-sort by the exact values
+  for (int i = t; i < k; i += MRG_THREADS) {
+    if (i < fill) {
+      top_val[q * k + i] = ord2f((uint32_t)(s[i] >> 32));
+      top_idx[q * k + i] = idx_base + (int64_t)(uint32_t)(s[i] & 0xffffffffu);
+    } else {
+      top_val[q * k + i] = __int_as_float(0x7f800000);
+      top_idx[q * k + i] = -1;
+    }
+  }
+}
+
+// The merge of cfl_score_topk_source (no lower-bound pass, no compact redo): the query row Eq[q] is the embedding e and
+// catalog row Pc[idx] holds the K prototypes p of the direct form.
+template <int K>
+__global__ void __launch_bounds__(MRG_THREADS, 8)
+merge_rescore_src_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ counts, int parts, int64_t Q, int kk,
+                         int k, const float* __restrict__ Eq, int64_t ldq, int d, const float* __restrict__ Pc, int64_t ldp,
+                         int64_t idx_base, float* __restrict__ top_val, int64_t* __restrict__ top_idx) {
+  __shared__ tkey_t s[TOPK_CAP];
+  __shared__ int s_fill;
+  __shared__ tkey_t s_thr;
+  const int t = threadIdx.x;
+  const int64_t q = blockIdx.x;
+  const int fill = block_merge_topkk(keys, counts, parts, Q, q, kk, s, &s_fill, &s_thr);
+  const float* e = Eq + q * ldq;
+  if (t < fill) {
+    const uint32_t idx = (uint32_t)(s[t] & 0xffffffffu);
+    const float* p = Pc + (int64_t)idx * ldp;
+    const float dist = pcd_direct<K, 1>([&](int j) { return e[j]; }, [&](int kq, int j) { return p[kq * d + j]; }, d);
+    s[t] = pack_key(dist, idx);
+  }
+  __syncthreads();
+  if (t == 0) s_fill = fill;
+  __syncthreads();
+  mrg_compact(s, &s_fill, &s_thr, kk, t);
   for (int i = t; i < k; i += MRG_THREADS) {
     if (i < fill) {
       top_val[q * k + i] = ord2f((uint32_t)(s[i] >> 32));
@@ -855,16 +911,20 @@ struct ScoreWs {
   size_t total;
 };
 
-static ScoreWs score_ws(int64_t Q, int K, int d, int64_t N, const ScorePlan& p, bool own_image) {
+// src (cfl_score_topk_source): one vector per query (pc = [Q,d], qpar = |e_q - mu|^2, a query image of qt vectors per
+// tile), no lower-bound pass (no lbimg, spill lists or compact-redo area) and never an own catalog image.
+static ScoreWs score_ws(int64_t Q, int K, int d, int64_t N, const ScorePlan& p, bool own_image, bool src = false) {
   ScoreWs w = {};
-  const LbPlan lb = p.impl ? make_lb_plan(Q, K, d, p.tiles) : LbPlan{0, 0, 0, 0, 0};
+  const bool lbp = p.impl && !src;
+  const LbPlan lb = lbp ? make_lb_plan(Q, K, d, p.tiles) : LbPlan{0, 0, 0, 0, 0};
   const int kparts = p.parts > lb.parts ? p.parts : lb.parts;          // key buffers serve both tilings
+  const int Kq = src ? 1 : K;                                          // vectors per query
   size_t off = 0;
-  w.pc = off;         off = align_up(off + (size_t)Q * K * d * 4, 256);
-  w.qpar = off;       w.qplane = off + (size_t)Q * qpar_stride(K) * 4;
-  off = align_up(off + (size_t)Q * (qpar_stride(K) + qplane_stride(K)) * 4, 256);
-  w.qimg = off;       off = align_up(off + (p.impl ? (size_t)p.nqt * qimg_tile_bytes(p.dpad, K * p.qt) : 0), 1024);
-  w.lbimg = off;      off = align_up(off + (p.impl ? score_lb_qimg_bytes(lb, K, d) : 0), 1024);
+  w.pc = off;         off = align_up(off + (size_t)Q * Kq * d * 4, 256);
+  w.qpar = off;       w.qplane = off + (size_t)Q * (src ? 1 : qpar_stride(K)) * 4;
+  off = align_up(off + (size_t)Q * (src ? 1 : qpar_stride(K) + qplane_stride(K)) * 4, 256);
+  w.qimg = off;       off = align_up(off + (p.impl ? (size_t)p.nqt * qimg_tile_bytes(p.dpad, Kq * p.qt) : 0), 1024);
+  w.lbimg = off;      off = align_up(off + (lbp ? score_lb_qimg_bytes(lb, K, d) : 0), 1024);
   w.keys = off;       off = align_up(off + (size_t)kparts * Q * TOPK_STRIDE * sizeof(tkey_t), 256);
   w.counts = off;     off = align_up(off + (size_t)kparts * Q * sizeof(int), 1024);
   w.cimg = off;       off = align_up(off + ((p.impl && own_image) ? catalog_image_bytes(N, d) : 0), 1024);
@@ -876,11 +936,15 @@ static ScoreWs score_ws(int64_t Q, int K, int d, int64_t N, const ScorePlan& p, 
   w.redo_tile2 = off; off += (size_t)(p.nqt + 4) * sizeof(int);
   w.lb2 = off;        off = align_up(off + (size_t)(Q + 4) * sizeof(float), 256);
   if (p.impl) {
-    w.spill = off;    w.spill_cnt = off + (size_t)Q * LB_SPILL * sizeof(tkey_t);
-    off = align_up(w.spill_cnt + (size_t)Q * sizeof(int), 256);
+    if (!src) {
+      w.spill = off;  w.spill_cnt = off + (size_t)Q * LB_SPILL * sizeof(tkey_t);
+      off = align_up(w.spill_cnt + (size_t)Q * sizeof(int), 256);
+    }
     w.stats = off;    off = align_up(off + CFL_SCORE_NSTATS * sizeof(unsigned long long), 256);
-    w.cl = cer_layout(K, d, p.qt, p.dpad);
-    w.cer = off;      off = align_up(off + w.cl.total, 1024);
+    if (!src) {
+      w.cl = cer_layout(K, d, p.qt, p.dpad);
+      w.cer = off;    off = align_up(off + w.cl.total, 1024);
+    }
   }
   w.total = off + 1024;
   return w;
@@ -1221,7 +1285,123 @@ static int score_topk_impl(int mode, const float* Pq, int64_t Q, int K, int d, i
   });
 }
 
+// The source-catalog call: the exact filter cascade of score_topk_impl on score_src_umma_kernel (sample thresholds,
+// exact filter under the optimistic threshold, in-place exact redo, merge with direct-form rescoring).  There is no
+// lower-bound pass and no CUDA-core kernel: every K <= 8, d <= 128 has a tensor-core tiling (score_src_qt).
+static ScorePlan source_plan(int64_t Q, int K, int d, int64_t N, int k) {
+  return make_score_plan_qt(Q, score_src_qt(K, d), d, N > 0 ? N : 1, k, true);
+}
+
+static int score_topk_source_impl(const float* Eq, int64_t ldq, int64_t Q, int K, int d, const void* image,
+                                  const float* Pc, int64_t N, int64_t ldp, const float* mu, int k, int64_t idx_base,
+                                  float* top_val, int64_t* top_idx, float* dist_out, unsigned long long* stats_out,
+                                  void* ws, size_t ws_bytes, cudaStream_t cs) {
+  int st = device_check();
+  if (st != CFL_OK) return st;
+  CFL_REQUIRE(K >= 1 && K <= CFL_MAX_K, CFL_ERR_UNSUPPORTED, "score_topk_source: K=%d outside [1,%d]", K, CFL_MAX_K);
+  CFL_REQUIRE(d >= 1 && d <= 128, CFL_ERR_UNSUPPORTED, "score_topk_source: d=%d outside [1,128]", d);
+  CFL_REQUIRE(k >= 1 && k <= CFL_MAX_TOPK, CFL_ERR_UNSUPPORTED, "score_topk_source: k=%d outside [1,%d]", k, CFL_MAX_TOPK);
+  CFL_REQUIRE(Q >= 0 && N >= 0 && N < ((int64_t)1 << 32), CFL_ERR_INVALID, "score_topk_source: bad Q/N");
+  CFL_REQUIRE(ldq >= d && ldp >= (int64_t)K * d, CFL_ERR_INVALID, "score_topk_source: leading dimension too small");
+  if (stats_out) CFL_CUDA(cudaMemsetAsync(stats_out, 0, CFL_SCORE_NSTATS * sizeof(unsigned long long), cs));
+  if (Q == 0) return CFL_OK;
+  CFL_REQUIRE(Eq && top_val && top_idx, CFL_ERR_INVALID, "score_topk_source: NULL argument");
+  CFL_REQUIRE(N == 0 || (Pc && image), CFL_ERR_INVALID, "score_topk_source: NULL catalog or image");
+  CFL_REQUIRE(((uintptr_t)image & 1023u) == 0, CFL_ERR_INVALID, "score_topk_source: image must be 1024-byte aligned");
+  ScoreCall c;
+  c.Pq = Eq; c.ldq = ldq; c.k = k; c.idx_base = idx_base; c.top_val = top_val; c.top_idx = top_idx;
+  c.plan = source_plan(Q, K, d, N, k);
+  c.kn = read_knobs();
+  c.ws = score_ws(Q, K, d, N, c.plan, false, true);
+  c.base = (char*)ws;
+  c.cs = cs;
+  CFL_REQUIRE(ws && ws_bytes >= c.ws.total, CFL_ERR_WORKSPACE, "score_topk_source: workspace too small (%zu < %zu)",
+              ws_bytes, c.ws.total);
+  const ScorePlan& plan = c.plan;
+  ScoreArgs& a = c.a;
+  a = ScoreArgs{};
+  a.src = true;
+  a.mode = CFL_PCD; a.K = K; a.d = d; a.Q = Q; a.N = N; a.lde = ldp; a.E = Pc; a.mu = mu;
+  a.Pc = c.at<float>(c.ws.pc); a.qpar = c.at<float>(c.ws.qpar);
+  a.qimg = c.at<char>(c.ws.qimg);
+  a.keys = c.at<tkey_t>(c.ws.keys); a.counts = c.at<int>(c.ws.counts); a.dist_out = dist_out;
+  a.tile_stride = 1;
+  a.plan = plan;
+  MergeInput m;
+  m.parts = plan.parts;
+  bool two_pass = false;
+  if (N == 0) {
+    CFL_CUDA(cudaMemsetAsync(a.counts, 0, (size_t)plan.parts * Q * sizeof(int), cs));
+  } else {
+    prep_source_queries_kernel<<<(unsigned)((Q + 3) / 4), 128, 0, cs>>>(Eq, Q, d, ldq, mu, (float*)a.Pc, (float*)a.qpar);
+    CFL_LAUNCH_CHECK();
+    const SourceCatalogView v = source_catalog_view(image, N, K, d);
+    a.cimg = v.blocks; a.e2 = v.rowpar;
+    st = score_umma_pack_queries(a, c.base + c.ws.qimg, cs);
+    if (st != CFL_OK) return st;
+    if (!score_two_pass(c.kn, plan, dist_out != nullptr)) {
+      timer_record(0, cs);
+      a.phase = 0; a.tile_stride = 1; a.thr_init = nullptr;
+      st = score_umma_launch(a, cs);
+      timer_record(1, cs);
+    } else {
+      two_pass = true;
+      st = sample_thresholds(c);
+      if (st != CFL_OK) return st;
+      a.phase = 2; a.tile_stride = 1; a.thr_init = c.at<float>(c.ws.tau_opt);
+      timer_record(0, cs);
+      st = exact_filter(c);
+      if (st != CFL_OK) return st;
+      st = exact_redo(c, false, c.at<float>(c.ws.thr_redo), c.at<int>(c.ws.redo_tile), m);
+    }
+    if (st != CFL_OK) return st;
+  }
+  st = with_k(K, [&](auto KC) {
+    merge_rescore_src_kernel<KC><<<(unsigned)Q, MRG_THREADS, 0, cs>>>(a.keys, a.counts, m.parts, Q, plan.kk, k, Eq, ldq, d,
+                                                                       Pc, ldp, idx_base, top_val, top_idx);
+    CFL_LAUNCH_CHECK();
+    return CFL_OK;
+  });
+  if (st != CFL_OK) return st;
+  if (stats_out && two_pass)
+    CFL_CUDA(cudaMemcpyAsync(stats_out, c.at<unsigned long long>(c.ws.stats), CFL_SCORE_NSTATS * sizeof(unsigned long long),
+                             cudaMemcpyDeviceToDevice, cs));
+  return CFL_OK;
+}
+
 extern "C" {
+
+size_t cfl_source_catalog_pack_bytes(int64_t N, int K, int d) {
+  if (N <= 0 || score_src_qt(K, d) == 0) return 0;
+  return source_catalog_image_bytes(N, K, d);
+}
+
+int cfl_source_catalog_pack(const float* Pc, int64_t N, int K, int d, int64_t ldp, const float* mu, void* image,
+                            size_t image_bytes, void* stream) {
+  int st = device_check();
+  if (st != CFL_OK) return st;
+  CFL_REQUIRE(score_src_qt(K, d) != 0, CFL_ERR_UNSUPPORTED, "source_catalog_pack: K=%d d=%d outside K <= %d, d <= 128", K,
+              d, CFL_MAX_K);
+  CFL_REQUIRE(Pc && image && N > 0 && N < ((int64_t)1 << 32) && ldp >= (int64_t)K * d, CFL_ERR_INVALID,
+              "source_catalog_pack: bad arguments");
+  CFL_REQUIRE(image_bytes >= source_catalog_image_bytes(N, K, d), CFL_ERR_WORKSPACE,
+              "source_catalog_pack: image buffer too small");
+  CFL_REQUIRE(((uintptr_t)image & 1023u) == 0, CFL_ERR_INVALID, "source_catalog_pack: image must be 1024-byte aligned");
+  return source_catalog_pack_launch(Pc, N, K, d, ldp, mu, image, (cudaStream_t)stream);
+}
+
+size_t cfl_score_topk_source_workspace_bytes(int64_t Q, int K, int d, int64_t N, int k) {
+  if (Q <= 0 || score_src_qt(K, d) == 0) return 4096;
+  return score_ws(Q, K, d, N, source_plan(Q, K, d, N, k), false, true).total + 1024;
+}
+
+int cfl_score_topk_source(const float* Eq, int64_t ldq, int64_t Q, int K, int d, const void* image, const float* Pc,
+                          int64_t N, int64_t ldp, const float* mu, int k, int64_t idx_base, float* top_val,
+                          int64_t* top_idx, float* dist_out, unsigned long long* stats_out, void* ws, size_t ws_bytes,
+                          void* stream) {
+  return score_topk_source_impl(Eq, ldq, Q, K, d, image, Pc, N, ldp, mu, k, idx_base, top_val, top_idx, dist_out,
+                                stats_out, ws, ws_bytes, (cudaStream_t)stream);
+}
 
 size_t cfl_score_topk_workspace_bytes(int64_t Q, int K, int d, int64_t N, int k) {
   return score_ws_bytes(Q, K, d, N, k, true);

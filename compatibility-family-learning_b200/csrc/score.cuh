@@ -67,6 +67,10 @@ struct ScoreArgs {
                          // (honoured only under CFL_EXPERIMENTS=1)
   ScorePlan plan;
   LbPlan lb;
+  // Source-catalog call (cfl_score_topk_source): the catalog rows carry K prototypes (cimg = cfl_source_catalog_pack's
+  // image, e2 = its per-row soft-min blocks), the queries one vector each (Pc = the centred vectors [Q,d], qpar =
+  // |e_q - mu|^2 per query, qimg of QT vectors per tile); E = the raw prototypes [N, lde], Pq (merge) = the raw queries.
+  bool src;
 };
 
 // Per-query parameter block (floats), padded to a multiple of 4 so it loads as float4:
@@ -108,6 +112,7 @@ enum ScoreStat {
 };
 
 ScorePlan make_score_plan(int64_t Q, int K, int d, int64_t N, int k, bool umma_ok);
+ScorePlan make_score_plan_qt(int64_t Q, int qt, int d, int64_t N, int k, bool umma_ok);
 bool score_umma_supported(int K, int d);
 // Catalog image of cfl_catalog_pack (layout in score_umma.cu): behind the tf32 planes, |e - mu|^2 per row, the fp16
 // plane of the lower-bound pass, its range flag and lbrow = (|e - mu|^2, |e - mu|) per row.
@@ -126,6 +131,15 @@ int score_lb_prep_queries(const ScoreArgs& a, cudaStream_t st);   // lower-bound
 int score_umma_launch(const ScoreArgs& a, cudaStream_t st);
 int score_lb_launch(const ScoreArgs& a, cudaStream_t st);
 int score_umma_qt(int K, int d);
+// Source-catalog image of cfl_source_catalog_pack (layout in score_umma.cu): K*nks tf32 blocks per 128-row tile, then
+// per tile the soft-min blocks of its rows, [tile][j][row], j < source_rowpar_len(K).
+__host__ __device__ constexpr int source_rowpar_len(int K) { return K + qpar_tri(K); }
+struct SourceCatalogView { unsigned char* blocks; float* rowpar; };
+size_t source_catalog_image_bytes(int64_t N, int K, int d);
+SourceCatalogView source_catalog_view(const void* image, int64_t N, int K, int d);
+int source_catalog_pack_launch(const float* P, int64_t N, int K, int d, int64_t ldp, const float* mu, void* image,
+                               cudaStream_t st);
+int score_src_qt(int K, int d);
 // query prep shared with the rank-count path (rank_counts_tc.cu): centred prototypes, soft-min and plane-bound blocks
 int score_prep_queries_launch(const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* mu, float* Pc,
                               float* qpar, float* qplane, cudaStream_t st);
@@ -234,11 +248,12 @@ __device__ __forceinline__ f2_t mul2(f2_t a, f2_t b) {
   return r;
 }
 
+// e2p = (|e|^2 of pair member A, of member B): one catalog row (both the same) for score_umma_kernel, two queries for
+// score_src_umma_kernel, whose qp2 is then its row's block broadcast to both members.
 template <int K>
-__device__ __forceinline__ void softmin_pair(const float (&gA)[K], const float (&gB)[K], float e2,
-                                             const f2_t* __restrict__ qp2, float& dA, float& dB) {
+__device__ __forceinline__ void softmin_pair2(const float (&gA)[K], const float (&gB)[K], f2_t e2p,
+                                              const f2_t* __restrict__ qp2, float& dA, float& dB) {
   const f2_t C2 = pk2(2.0f * CFL_LOG2E, 2.0f * CFL_LOG2E);
-  const f2_t e2p = pk2(e2, e2);
   f2_t g[K], a[K];
 #pragma unroll
   for (int k = 0; k < K; ++k) { g[k] = pk2(gA[k], gB[k]); a[k] = fma2(C2, g[k], qp2[k]); }
@@ -277,6 +292,11 @@ __device__ __forceinline__ void softmin_pair(const float (&gA)[K], const float (
   // dist = e2 - 2 inv (t1 - inv t2)
   const f2_t v = fma2(ninv, t2, t1);
   upk2(fma2(add2(ninv, ninv), v, e2p), dA, dB);
+}
+template <int K>
+__device__ __forceinline__ void softmin_pair(const float (&gA)[K], const float (&gB)[K], float e2,
+                                             const f2_t* __restrict__ qp2, float& dA, float& dB) {
+  softmin_pair2<K>(gA, gB, pk2(e2, e2), qp2, dA, dB);
 }
 
 // softmin_pair that also returns V = sum_k s_k |p_k|^2 - |sum_k s_k p_k|^2, the spread of the prototypes under the

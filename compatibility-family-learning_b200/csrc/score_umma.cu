@@ -13,6 +13,12 @@
 // lower bound and the soft-min distance (score.cuh), threshold test, warp-aggregated push into the per-query buffers
 // (topk.cuh), cooperative compaction of over-full buffers.
 // Work per score: 2*K*d flops (x3 MMAs); catalog bytes per row per query tile: 8*dpad + 4.
+//
+// score_src_umma_kernel is the same kernel for the other direction of the asymmetric pcd distance (cfl_score_topk_source):
+// the catalog rows are SOURCE items with K prototypes each (cfl_source_catalog_pack: K planes of tf32 blocks per tile and
+// each row's soft-min block), the queries are TARGET embeddings (one vector each).  The Gram values land in TMEM where the
+// forward kernel puts them; the soft-min constants belong to the row and |e_q|^2 to the query.  It has no plane bound: the
+// affine hull is per row.  Catalog bytes per row per query tile: K*8*dpad + 4*(K + K(K+1)/2).
 #include <cuda_fp16.h>
 #include "gram_pipe.cuh"
 
@@ -128,12 +134,106 @@ int catalog_pack_launch(const float* E, int64_t N, int d, int64_t lde, const flo
   return CFL_OK;
 }
 
+// ---- source-catalog image ----------------------------------------------------------------------
+// [tile][k][kstep][hl][chunk][row 0..127][4 floats]  (8 KB per (tile, k, kstep): prototype k of the tile's rows, centred on
+// mu, in the block format of the catalog image), then rowpar[tile][j][row 0..127], j < K + K(K+1)/2: log2(e)*|p_k|^2 and
+// the upper triangle of p_k.p_l with the diagonal pre-halved (the first entries of the qpar format, score.cuh), zeros for
+// the padding rows of the last tile.  The epilogue reads its row's block once per tile, coalesced.
+static size_t source_rowpar_offset(int64_t N, int K, int d) {
+  return (size_t)((N + 127) / 128) * K * ((d + 7) / 8) * GP_ASTAGE;
+}
+size_t source_catalog_image_bytes(int64_t N, int K, int d) {
+  return source_rowpar_offset(N, K, d) + (size_t)((N + 127) / 128) * 128 * source_rowpar_len(K) * sizeof(float);
+}
+SourceCatalogView source_catalog_view(const void* image, int64_t N, int K, int d) {
+  unsigned char* img = (unsigned char*)const_cast<void*>(image);
+  return SourceCatalogView{img, (float*)(img + source_rowpar_offset(N, K, d))};
+}
+
+template <int K>
+__global__ void __launch_bounds__(128)
+pack_source_catalog_kernel(const float* __restrict__ P, int64_t N, int d, int64_t ldp, const float* __restrict__ mu,
+                           unsigned char* __restrict__ img, float* __restrict__ rowpar) {
+  const int64_t tile = blockIdx.x;
+  const int r = threadIdx.x;
+  const int64_t row = tile * 128 + r;
+  const bool valid = row < N;
+  const float* src = P + (valid ? row : 0) * ldp;
+  const int nks = (d + 7) / 8;
+  constexpr int T = qpar_tri(K);
+  float tri[T];
+#pragma unroll
+  for (int o = 0; o < T; ++o) tri[o] = 0.0f;
+  for (int ks = 0; ks < nks; ++ks) {
+    float v[K][8];
+#pragma unroll
+    for (int k = 0; k < K; ++k)
+#pragma unroll
+      for (int jj = 0; jj < 8; ++jj) {
+        const int j = ks * 8 + jj;
+        v[k][jj] = (valid && j < d) ? src[k * d + j] - (mu ? mu[j] : 0.0f) : 0.0f;
+      }
+    int o = 0;
+#pragma unroll
+    for (int k = 0; k < K; ++k)
+#pragma unroll
+      for (int l = k; l < K; ++l, ++o)
+#pragma unroll
+        for (int jj = 0; jj < 8; ++jj) tri[o] = fmaf(v[k][jj], v[l][jj], tri[o]);
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+      float4 h0, l0, h1, l1;
+      split_tf32x4(make_float4(v[k][0], v[k][1], v[k][2], v[k][3]), h0, l0);
+      split_tf32x4(make_float4(v[k][4], v[k][5], v[k][6], v[k][7]), h1, l1);
+      unsigned char* st = img + (((size_t)tile * K + k) * nks + ks) * GP_ASTAGE;
+      *(float4*)(st + ((0 * 2 + 0) * 128 + r) * 16) = h0;
+      *(float4*)(st + ((0 * 2 + 1) * 128 + r) * 16) = h1;
+      *(float4*)(st + ((1 * 2 + 0) * 128 + r) * 16) = l0;
+      *(float4*)(st + ((1 * 2 + 1) * 128 + r) * 16) = l1;
+    }
+  }
+  float* rp = rowpar + (size_t)tile * 128 * source_rowpar_len(K) + r;
+  int o = 0;
+#pragma unroll
+  for (int k = 0; k < K; ++k)
+#pragma unroll
+    for (int l = k; l < K; ++l, ++o) {
+      if (l == k) rp[k * 128] = CFL_LOG2E * tri[o];
+      rp[(K + o) * 128] = (l == k) ? 0.5f * tri[o] : tri[o];
+    }
+}
+
+int source_catalog_pack_launch(const float* P, int64_t N, int K, int d, int64_t ldp, const float* mu, void* image,
+                               cudaStream_t st) {
+  const SourceCatalogView v = source_catalog_view(image, N, K, d);
+  return with_k(K, [&](auto KC) {
+    pack_source_catalog_kernel<KC><<<(unsigned)((N + 127) / 128), 128, 0, st>>>(P, N, d, ldp, mu, v.blocks, v.rowpar);
+    CFL_LAUNCH_CHECK();
+    return CFL_OK;
+  });
+}
+
+// Query tile of the source-catalog kernel: QT vectors, a valid MMA N (a multiple of 16) with K*QT <= 256 TMEM columns
+// per accumulator buffer; QT = 16 always qualifies, so every K <= 8 and d <= 128 has a tiling.
+int score_src_qt(int K, int d) {
+  if (K < 1 || K > CFL_MAX_K || d < 1 || d > 128) return 0;
+  const int dpad = (d + 7) / 8 * 8;
+  const int cand[] = {128, 64, 48, 32, 16};
+  for (int qt : cand) {
+    if (K * qt > 256 || qt % gram_gq(K) != 0) continue;
+    if (qimg_tile_bytes(dpad, qt) > SU_B_BUDGET) continue;
+    return qt;
+  }
+  return 0;
+}
+
 // Shared memory of the exact kernel: the Gram pipeline's regions with the compaction scratch in front of the query blocks
 // and, behind them, running thresholds, key counts and compaction requests.
 struct SuLayout { GramLayout g; uint32_t thr, cnt, need; };
+template <bool SRC = false>
 __host__ __device__ inline SuLayout su_layout(int K, int qt, int dpad) {
   SuLayout L;
-  L.g = gram_layout(K, qt, dpad, TOPK_STRIDE * 8u);
+  L.g = gram_layout<SRC>(K, qt, dpad, TOPK_STRIDE * 8u);
   uint32_t off = L.g.back;
   L.thr = off;     off += (uint32_t)qt * 4u;
   L.cnt = off;     off += (uint32_t)qt * 4u;
@@ -174,7 +274,7 @@ __global__ void pack_queries_kernel(const float* __restrict__ Pc, int64_t Q, int
 }
 
 int score_umma_pack_queries(const ScoreArgs& a, void* qimg, cudaStream_t st) {
-  pack_queries_kernel<<<a.plan.nqt, 256, 0, st>>>(a.Pc, a.Q, a.K, a.d, a.plan.qt, a.plan.dpad, (float*)qimg);
+  pack_queries_kernel<<<a.plan.nqt, 256, 0, st>>>(a.Pc, a.Q, a.src ? 1 : a.K, a.d, a.plan.qt, a.plan.dpad, (float*)qimg);
   CFL_LAUNCH_CHECK();
   return CFL_OK;
 }
@@ -183,14 +283,15 @@ __device__ __forceinline__ void epi_bar_sync() {
   asm volatile("bar.sync 1, %0;" ::"n"(GP_EPI_THREADS) : "memory");
 }
 
-// ---- the kernel ---------------------------------------------------------------------------
-template <int K>
-__global__ void __launch_bounds__(GP_THREADS, 1)
-score_umma_kernel(ScoreArgs A) {
+// ---- the kernels ---------------------------------------------------------------------------
+// SRC = false: score_umma_kernel (catalog of embeddings, queries of K prototypes); SRC = true: score_src_umma_kernel
+// (catalog of K prototypes per row, queries of one vector).
+template <int K, bool SRC>
+__device__ __forceinline__ void score_umma_body(const ScoreArgs& A) {
   extern __shared__ __align__(1024) unsigned char smem[];
   constexpr int GQ = gram_gq(K);
   const int QT = A.plan.qt;
-  const SuLayout L = su_layout(K, QT, A.plan.dpad);
+  const SuLayout L = su_layout<SRC>(K, QT, A.plan.dpad);
   const GramPipe P = gram_pipe(smem, L.g, K, QT, A.plan.dpad);
   tkey_t* scratch = (tkey_t*)(smem + L.g.front);
   float* thr = (float*)(smem + L.thr);
@@ -210,7 +311,12 @@ score_umma_kernel(ScoreArgs A) {
   const bool filter = A.phase == 2;
 
   // ---- one-time setup ----
-  gram_setup<K>(P, A.qpar, A.qplane, q0, nq, QT);
+  if constexpr (SRC) {
+    gram_init(P);
+    for (int i = tid; i < QT; i += GP_THREADS) P.qpar[i] = (i < nq) ? A.qpar[q0 + i] : 0.0f;     // |e_q - mu|^2
+  } else {
+    gram_setup<K>(P, A.qpar, A.qplane, q0, nq, QT);
+  }
   // padding queries of the last tile get thr = -inf: they can never be pushed
   // phase 2: fixed thresholds from the sample pass, bumped one ulp so that the strict compare
   // below implements dist <= tau (every candidate tied with the bound must be kept)
@@ -227,9 +333,9 @@ score_umma_kernel(ScoreArgs A) {
   const uint32_t tmem_base = gram_start(P);
 
   if (warp == GP_NEPI) {
-    gram_mma(P, tmem_base, ntiles);
+    gram_mma<SRC ? K : 1>(P, tmem_base, ntiles);
   } else if (warp == GP_NEPI + 1) {
-    gram_tma(P, A.qimg, qtile, A.cimg, t0, ts, ntiles);
+    gram_tma<SRC ? K : 1>(P, A.qimg, qtile, A.cimg, t0, ts, ntiles);
   } else {
     // ======================================= epilogue ========================================
     constexpr int QPS = qpar_stride(K);
@@ -245,12 +351,25 @@ score_umma_kernel(ScoreArgs A) {
     // (prototypes far apart relative to the spread of the distances) each warp measures its hit rate
     // and switches the test off.
     constexpr int PBS = qplane_stride(K);
-    bool bound_on = (K > 1) && !dense;
+    bool bound_on = !SRC && (K > 1) && !dense;
+    constexpr int NRP = source_rowpar_len(K);
     int grp_seen = 0, grp_skipped = 0;
     for (int t = 0; t < ntiles; ++t) {
-      const int64_t row = (t0 + (int64_t)t * ts) * 128 + lrow;
+      const int64_t tile = t0 + (int64_t)t * ts;
+      const int64_t row = tile * 128 + lrow;
       const bool valid = row < A.N;
-      const float e2 = __ldg(A.e2 + row);                    // padded to whole tiles
+      float e2 = 0.0f;
+      f2_t rq[SRC ? NRP : 1];                                // SRC: the row's soft-min block, broadcast to a query pair
+      if constexpr (SRC) {
+        const float* rp = A.e2 + tile * 128 * NRP + lrow;
+#pragma unroll
+        for (int j = 0; j < NRP; ++j) {
+          const float v = __ldg(rp + j * 128);
+          rq[j] = (j < K) ? pk2(-v, -v) : pk2(v, v);
+        }
+      } else {
+        e2 = __ldg(A.e2 + row);                              // padded to whole tiles
+      }
       const uint32_t taddr = gram_acquire(P, tmem_base, t, lq);
       const int nslot = filter ? 2 + ((t >> 2) & 1) : (t & 1);
       const int trig = filter ? TOPK_STRIDE / 2 : TOPK_TRIGGER;
@@ -277,7 +396,7 @@ score_umma_kernel(ScoreArgs A) {
           const float4 t4 = *(const float4*)(thr + g * GQ + i);
           tg[i] = t4.x; tg[i + 1] = t4.y; tg[i + 2] = t4.z; tg[i + 3] = t4.w;
         }
-        if constexpr (K > 1) {
+        if constexpr (K > 1 && !SRC) {
           if (bound_on) {
             const float e2s = e2 * (1.0f - CFL_PLANE_REL);
             const f2_t e2sp = pk2(e2s, e2s);
@@ -318,12 +437,17 @@ score_umma_kernel(ScoreArgs A) {
         float dist[GQ];
 #pragma unroll
         for (int pi = 0; pi < GQ / 2; ++pi) {
-          f2_t qv[QPS];
-          load_pair_block<QPS>(qg + pi * QPS * 2, qv);
           float gA[K], gB[K];
 #pragma unroll
           for (int k = 0; k < K; ++k) { gA[k] = gk[k][2 * pi]; gB[k] = gk[k][2 * pi + 1]; }
-          softmin_pair<K>(gA, gB, e2, qv, dist[2 * pi], dist[2 * pi + 1]);
+          if constexpr (SRC) {
+            const f2_t e2q = *(const f2_t*)(P.qpar + g * GQ + 2 * pi);
+            softmin_pair2<K>(gA, gB, e2q, rq, dist[2 * pi], dist[2 * pi + 1]);
+          } else {
+            f2_t qv[QPS];
+            load_pair_block<QPS>(qg + pi * QPS * 2, qv);
+            softmin_pair<K>(gA, gB, e2, qv, dist[2 * pi], dist[2 * pi + 1]);
+          }
         }
         uint32_t bits = 0;
 #pragma unroll
@@ -393,17 +517,34 @@ score_umma_kernel(ScoreArgs A) {
 }
 
 template <int K>
+__global__ void __launch_bounds__(GP_THREADS, 1)
+score_umma_kernel(ScoreArgs A) {
+  score_umma_body<K, false>(A);
+}
+
+template <int K>
+__global__ void __launch_bounds__(GP_THREADS, 1)
+score_src_umma_kernel(ScoreArgs A) {
+  score_umma_body<K, true>(A);
+}
+
+template <int K, bool SRC>
 static int launch_umma(const ScoreArgs& a, cudaStream_t st) {
-  size_t smem = su_layout(K, a.plan.qt, a.plan.dpad).g.total + 1024;      // slack for the alignment of the dynamic segment
-  CFL_SMEM_LIMIT(score_umma_kernel<K>, smem);
+  size_t smem = su_layout<SRC>(K, a.plan.qt, a.plan.dpad).g.total + 1024;   // slack for the alignment of the dynamic segment
   dim3 grid(a.plan.parts, a.plan.nqt);
-  score_umma_kernel<K><<<grid, GP_THREADS, smem, st>>>(a);
+  if constexpr (SRC) {
+    CFL_SMEM_LIMIT(score_src_umma_kernel<K>, smem);
+    score_src_umma_kernel<K><<<grid, GP_THREADS, smem, st>>>(a);
+  } else {
+    CFL_SMEM_LIMIT(score_umma_kernel<K>, smem);
+    score_umma_kernel<K><<<grid, GP_THREADS, smem, st>>>(a);
+  }
   CFL_LAUNCH_CHECK();
   return CFL_OK;
 }
 
 int score_umma_launch(const ScoreArgs& a, cudaStream_t st) {
-  return with_k(a.K, [&](auto K) { return launch_umma<K>(a, st); });
+  return with_k(a.K, [&](auto K) { return a.src ? launch_umma<K, true>(a, st) : launch_umma<K, false>(a, st); });
 }
 
 }  // namespace cfl

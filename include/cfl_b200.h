@@ -152,6 +152,32 @@ int cfl_score_topk_packed(int mode, const float* Pq, int64_t Q, int K, int d, in
                           float* top_val, int64_t* top_idx, float* dist_out,
                           void* ws, size_t ws_bytes, void* stream);
 
+/* The other direction of the pcd distance: rank the SOURCE items of a catalog for TARGET queries.  pcd is not
+ * symmetric: dist = |v - sum_k s_k p_k|^2 takes v = e0 of the TARGET item and p_k = the K prototypes of the SOURCE
+ * item (DistBase.build_dist, cfl/models/base.py:125-139).  cfl_score_topk answers "which targets go with this source";
+ * cfl_score_topk_source answers "which sources is this target compatible with":
+ *   Eq[Q,d] (leading dimension ldq) = e0 of the target (query) items,
+ *   Pc[N,K,d] = the K prototypes of the source (catalog) items, prototype k of row c at columns [k*d,(k+1)*d) of a row
+ *   of length ldp; mu[d] optional centring vector (e.g. the mean of all prototypes), the one the image was built with;
+ *   dist(q,c) = pcd(v = Eq[q], P = Pc[c]).
+ * cfl_source_catalog_pack builds the catalog's tensor-core image once (cfl_source_catalog_pack_bytes; 0 when N <= 0 or
+ * K, d are out of range; `image` 1024-byte aligned): K planes of centred tf32 hi/lo blocks per 128-row tile and every
+ * row's soft-min constants.  cfl_score_topk_source: 3xTF32 Gram form with the soft-min epilogue and running top-k
+ * (the exact filter cascade of cfl_score_topk: sampled thresholds, filter, verification, exact redo), winners rescored in
+ * direct-difference form.  Outputs and tie rule as cfl_score_topk: top_val[Q,k] ascending exact distances, top_idx[Q,k]
+ * = idx_base + row, ties -> lower index, -1 / +inf when N < k; dist_out[Q,N] (optional) = un-rescored Gram values;
+ * stats_out (optional, device) = CFL_SCORE_NSTATS counters of this call as cfl_score_topk_stats (slot [4], the
+ * lower-bound pass, is always 0; all zero for catalogs short enough for the single adaptive pass).  K <= 8, d <= 128,
+ * k <= 128.  No reference call site (SURVEY App. A.6). */
+size_t cfl_source_catalog_pack_bytes(int64_t N, int K, int d);
+int cfl_source_catalog_pack(const float* Pc, int64_t N, int K, int d, int64_t ldp, const float* mu,
+                            void* image, size_t image_bytes, void* stream);
+size_t cfl_score_topk_source_workspace_bytes(int64_t Q, int K, int d, int64_t N, int k);
+int cfl_score_topk_source(const float* Eq, int64_t ldq, int64_t Q, int K, int d, const void* image,
+                          const float* Pc, int64_t N, int64_t ldp, const float* mu, int k, int64_t idx_base,
+                          float* top_val, int64_t* top_idx, float* dist_out, unsigned long long* stats_out,
+                          void* ws, size_t ws_bytes, void* stream);
+
 /* Statistics of the LAST cfl_score_topk / cfl_score_topk_packed call that used workspace `ws` with this shape
  * (packed = 1 for the _packed entry point): CFL_SCORE_NSTATS unsigned 64-bit counters copied to device memory
  * `stats_out` on `stream`: [0] keys that survived the full filter pass, summed over queries (each is rescored
