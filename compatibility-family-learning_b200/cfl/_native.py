@@ -66,6 +66,11 @@ SIGNATURES = {
     "cfl_score_topk_monomer_packed_workspace_bytes": (_sz, [_i64, _int, _int, _i64, _int]),
     "cfl_score_topk_monomer_packed": (_int, [_vp, _i64, _vp, _i64, _int, _int, _vp, _vp, _i64, _i64, _vp, _int, _i64,
                                              _vp, _vp, _vp, _vp, _sz, _vp]),
+    "cfl_monomer_source_pack_bytes": (_sz, [_i64, _int, _int]),
+    "cfl_monomer_source_pack": (_int, [_vp, _i64, _vp, _i64, _int, _int, _vp, _vp, _sz, _vp]),
+    "cfl_score_topk_monomer_source_workspace_bytes": (_sz, [_i64, _int, _int, _i64, _int]),
+    "cfl_score_topk_monomer_source": (_int, [_vp, _i64, _i64, _int, _int, _vp, _vp, _i64, _vp, _i64, _vp, _int, _i64,
+                                             _vp, _vp, _vp, _vp, _sz, _vp]),
     "cfl_topk_merge": (_int, [_vp, _vp, _int, _i64, _int, _vp, _vp, _vp]),
     "cfl_topk_record_bytes": (_sz, [_i64, _int]),
     "cfl_topk_pack_records": (_int, [_vp, _vp, _i64, _int, _vp, _vp]),
@@ -511,6 +516,61 @@ def score_topk_monomer_packed(a, w, P, image, k, mu=None, idx_base=0, want_stats
     _check(lib().cfl_score_topk_monomer_packed(_ptr(a), lda, _ptr(w), Q, K, d, _ptr(image), _ptr(P2), N, ldp, _ptr(mu),
                                                int(k), int(idx_base), _ptr(top_val), _ptr(top_idx), _ptr(stats), _ptr(ws),
                                                ws.numel(), _stream()), "cfl_score_topk_monomer_packed")
+    return (top_val, top_idx, stats) if want_stats else (top_val, top_idx)
+
+
+def _monomer_source_catalog(A, W, what):
+    A, lda = _rows(A, "A")
+    W = _f32c(W, "W").contiguous()
+    if W.dim() != 2 or W.shape[0] != A.shape[0]:
+        raise CflNativeError(f"{what}: A {tuple(A.shape)} and W {tuple(W.shape)} must be [N,d] and [N,K]")
+    return A, lda, W
+
+
+def monomer_source_pack(A, W, mu=None):
+    """Tensor-core image of a monomer SOURCE catalog: A [N,d] = the sources' act(e0), W [N,K] = their gate softmax,
+    centred on mu; for score_topk_monomer_source, built once per shard.  None when K(d+1) > 128 (CUDA-core route only)
+    or for an empty catalog."""
+    A, lda, W = _monomer_source_catalog(A, W, "monomer_source_pack")
+    (N, d), K = A.shape, W.shape[1]
+    nbytes = lib().cfl_monomer_source_pack_bytes(N, K, d)
+    if nbytes == 0:
+        return None
+    img = torch.empty(nbytes + 1024, dtype=torch.uint8, device=A.device)
+    off = (-img.data_ptr()) % 1024
+    img = img[off:off + nbytes]
+    mu = None if mu is None else _f32c(mu, "mu").contiguous()
+    _check(lib().cfl_monomer_source_pack(_ptr(A), lda, _ptr(W), N, K, d, _ptr(mu), _ptr(img), nbytes, _stream()),
+           "cfl_monomer_source_pack")
+    return img
+
+
+def score_topk_monomer_source(Pq, A, W, image, k, mu=None, idx_base=0, want_stats=False):
+    """The other direction of the monomer distance: top-k SOURCE items (catalog A [N,d], W [N,K], image =
+    monomer_source_pack(A, W, mu), or None for the CUDA-core route) of every TARGET query Pq [Q,K,d] (its K
+    prototypes), dist(q,c) = sum_k W[c,k] |A[c] - Pq[q,k]|^2 (base.py:109-117); exact values, ties -> lower index.
+    ``want_stats`` appends the int64 counters (SCORE_STAT_NAMES) of this call."""
+    Pq = _f32c(Pq, "Pq")
+    if Pq.dim() != 3:
+        raise CflNativeError("score_topk_monomer_source: Pq must be [Q,K,d]")
+    Q, K, d = Pq.shape
+    A, lda, W = _monomer_source_catalog(A, W, "score_topk_monomer_source")
+    N = A.shape[0]
+    if A.shape[1] != d or W.shape[1] != K:
+        raise CflNativeError(f"score_topk_monomer_source: A {tuple(A.shape)}, W {tuple(W.shape)} do not match "
+                             f"Pq {tuple(Pq.shape)}")
+    if A.device != Pq.device or W.device != Pq.device:
+        raise CflNativeError("score_topk_monomer_source: Pq, A and W must be on the same device")
+    P2, ldq = _rows(Pq.reshape(Q, K * d), "Pq")
+    dev = Pq.device
+    top_val = torch.empty(Q, k, dtype=torch.float32, device=dev)
+    top_idx = torch.empty(Q, k, dtype=torch.int64, device=dev)
+    stats = torch.zeros(SCORE_NSTATS, dtype=torch.int64, device=dev) if want_stats else None
+    mu = None if mu is None else _f32c(mu, "mu").contiguous()
+    ws = _ws.get(lib().cfl_score_topk_monomer_source_workspace_bytes(Q, K, d, N, k), dev)
+    _check(lib().cfl_score_topk_monomer_source(_ptr(P2), ldq, Q, K, d, _ptr(image), _ptr(A), lda, _ptr(W), N, _ptr(mu),
+                                               int(k), int(idx_base), _ptr(top_val), _ptr(top_idx), _ptr(stats),
+                                               _ptr(ws), ws.numel(), _stream()), "cfl_score_topk_monomer_source")
     return (top_val, top_idx, stats) if want_stats else (top_val, top_idx)
 
 

@@ -378,6 +378,14 @@ def _gather_merge(tv, ti, group, world):
     return nat.topk_merge_records(out, world, Q, k)
 
 
+def _monomer_source_side(w: EncoderWeights, x: torch.Tensor):
+    """The monomer SOURCE side of items x (base.py:94-105): a = act(e0) from the embedding head ``V0/g0/b0`` and the
+    gate softmax of ``pre @ Vg`` (weight norm with ``gg``, no bias), pre = the embedding head's pre-activation."""
+    a, pre, _ = nat.project_fwd(x, w.V0, w.g0, w.b0, w.weight_norm, w.in_scale, w.act, want_pre=True)
+    logits, _, _ = nat.project_fwd(pre, w.Vg, w.gg, None, True, 1.0, None)
+    return a, torch.softmax(logits, dim=-1)
+
+
 class MonomerCatalogIndex:
     """Monomer ranking (``--dist-type monomer``): the pair scorer's monomer branch
     (DistBase.build_dist, cfl/models/base.py:109-117) on the query x catalog cross product.
@@ -437,10 +445,7 @@ class MonomerCatalogIndex:
         """-> (a [Q,d], w [Q,K]): embedding and gate softmax of the source items (base.py:94-105)."""
         if not xq.is_cuda:
             xq = xq.to(self.P.device, non_blocking=True)
-        w = self.w
-        a, pre, _ = nat.project_fwd(xq, w.V0, w.g0, w.b0, w.weight_norm, w.in_scale, w.act, want_pre=True)
-        logits, _, _ = nat.project_fwd(pre, w.Vg, w.gg, None, True, 1.0, None)
-        return a, torch.softmax(logits, dim=-1)
+        return _monomer_source_side(self.w, xq)
 
     def rank_local(self, a: torch.Tensor, gate: torch.Tensor, k: int):
         if self.image is not None:
@@ -540,6 +545,90 @@ class SourceCatalogIndex:
 
     def rank_local(self, Eq: torch.Tensor, k: int):
         return nat.score_topk_source(Eq, self.P, self.image, k, mu=self.mu, idx_base=self.idx_base)
+
+    def rank(self, xq: torch.Tensor, k: int = 100):
+        """-> (dist [Q,k] ascending, index [Q,k] int64 global source rows).  score = theta+ - dist."""
+        tv, ti = self.rank_local(self.project_queries(xq), k)
+        world = self._world()
+        return (tv, ti) if world == 1 else _gather_merge(tv, ti, self.group, world)
+
+    def scores(self, dist: torch.Tensor) -> torch.Tensor:
+        """Thresholder (blocks.py:21-22): max(theta, 1e-6) - dist."""
+        return max(self.theta, 1e-6) - dist
+
+
+class MonomerSourceCatalogIndex:
+    """The other direction of the monomer distance: rank the SOURCE items of a catalog for TARGET queries.
+
+    The monomer distance is directed (DistBase.build_dist, cfl/models/base.py:109-117): dist = sum_k w_k |a - P'_k|^2
+    takes a and the gate w of the source item (base.py:94-105) and the K prototypes P' of the target item.
+    ``MonomerCatalogIndex`` answers "which targets go with this source"; this index answers "which sources is this
+    target compatible with" -- e.g. which existing items should now recommend a newly added item.  One shard holds the
+    sources' ``a`` [N, d] and gate ``w`` [N, K] resident on the GPU with their tensor-core image
+    (``monomer_source_pack``; None when K(d+1) > 128, where the CUDA-core kernel serves the shape), centred on the
+    mean of ``a`` over all shards; sharding, the all-gather + merge and the tie rule are those of ``CatalogIndex``.
+
+    ``weights``: the catalog side goes through the embedding head ``V0/g0/b0`` and the gate ``Vg/gg``
+    (``from_features``), the queries through the prototype head ``Vp/gp/bp`` (``project_queries``).  For a directed
+    model (e.g. Polyvore ``top_to_other``, where ``DistEncoderSrc`` encodes the source side and ``DistEncoderDst`` the
+    target side) build ``EncoderWeights`` with ``V0, g0, b0`` and ``Vg, gg`` from the Src encoder's embedding and gate
+    heads and ``Vp, gp, bp`` from the Dst encoder's prototype head."""
+
+    def __init__(self, weights: EncoderWeights, a: torch.Tensor, gate: torch.Tensor, idx_base: int = 0,
+                 n_total: Optional[int] = None, theta: float = 1e-6, group=None):
+        if not a.is_cuda or not gate.is_cuda:
+            raise nat.CflNativeError("MonomerSourceCatalogIndex needs CUDA embeddings and gates (there is no CPU path)")
+        self.w = weights
+        self.a = a.view(a.shape[0], weights.d)
+        self.gate = gate.view(gate.shape[0], weights.K)
+        self.idx_base = int(idx_base)
+        self.n_total = int(n_total if n_total is not None else a.shape[0])
+        self.theta = float(theta)
+        self.group = group
+        self.mu = self._global_mean()
+        self.image = nat.monomer_source_pack(self.a, self.gate, self.mu) if self.a.shape[0] else None
+
+    def _global_mean(self):
+        """Mean of the sources' a over every shard, so that all ranks centre on the same vector."""
+        s = self.a.double().sum(dim=0)
+        n = torch.tensor([float(self.a.shape[0])], dtype=torch.float64, device=self.a.device)
+        if self._world() > 1:
+            torch.distributed.all_reduce(s, group=self.group)
+            torch.distributed.all_reduce(n, group=self.group)
+        return (s / n.clamp(min=1)).float()
+
+    @classmethod
+    def from_features(cls, weights: EncoderWeights, features: torch.Tensor, idx_base: int = 0,
+                      n_total: Optional[int] = None, chunk: int = 1 << 16, **kw):
+        """Projects this rank's source rows through the embedding head and the gate (no communication)."""
+        if weights.Vg is None:
+            raise nat.CflNativeError("MonomerSourceCatalogIndex needs the gate head (EncoderWeights.Vg)")
+        dev = weights.V0.device
+        n = features.shape[0]
+        a = torch.empty(n, weights.d, dtype=torch.float32, device=dev)
+        gate = torch.empty(n, weights.K, dtype=torch.float32, device=dev)
+        for lo in range(0, n, chunk):
+            xb = features[lo:lo + chunk]
+            if not xb.is_cuda:
+                xb = xb.to(dev, non_blocking=True)
+            a[lo:lo + chunk], gate[lo:lo + chunk] = _monomer_source_side(weights, xb)
+        return cls(weights, a, gate, idx_base=idx_base, n_total=n_total, **kw)
+
+    def _world(self):
+        if torch.distributed.is_available() and torch.distributed.is_initialized():
+            return torch.distributed.get_world_size(self.group)
+        return 1
+
+    def project_queries(self, xq: torch.Tensor) -> torch.Tensor:
+        """-> [Q, K, d]: the K prototypes of the target items (base.py:47-57)."""
+        if not xq.is_cuda:
+            xq = xq.to(self.a.device, non_blocking=True)
+        w = self.w
+        P, _, _ = nat.project_fwd(xq, w.Vp, w.gp, w.bp, w.weight_norm, w.in_scale, w.act)
+        return P.view(P.shape[0], w.K, w.d)
+
+    def rank_local(self, Pq: torch.Tensor, k: int):
+        return nat.score_topk_monomer_source(Pq, self.a, self.gate, self.image, k, mu=self.mu, idx_base=self.idx_base)
 
     def rank(self, xq: torch.Tensor, k: int = 100):
         """-> (dist [Q,k] ascending, index [Q,k] int64 global source rows).  score = theta+ - dist."""

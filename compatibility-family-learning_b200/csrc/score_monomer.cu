@@ -152,6 +152,127 @@ score_monomer_kernel(MonoArgs A) {
   }
 }
 
+// The other direction (cfl_score_topk_monomer_source): the catalog rows are SOURCE items (a_c, w_c), the queries TARGET
+// items (K prototypes each), dist(q, c) = sum_k w_ck |a_c - P'_qk|^2.  One thread owns one source row of a 128-row tile
+// and 16 queries; the tile's a and w are staged once per tile, the queries' K prototypes sit in shared memory as query
+// PAIRS, negated, so the inner loop is packed FP32x2 as above.  Operation order of monomer_direct (direct.cuh): over k,
+// over j, a_j + (-p_kj), fmaf; then fmaf(w_k, dk, acc) -- the values are final.
+struct MonoSrcArgs {
+  int K, d;
+  int64_t Q, N, ldq, lda;
+  const float* P;    // [Q, ldq]  query prototypes, prototype k of query q at columns [k*d, (k+1)*d)
+  const float* A;    // [N, lda]  catalog embeddings a_c
+  const float* W;    // [N, K]    catalog gate weights (softmax), dense
+  tkey_t* keys;      // [parts, Q, MONO_KSTRIDE]
+  int* counts;       // [parts, Q]
+  int parts, kk;
+  int64_t tiles;
+  int tile_stride;
+  const int* redo_tile;
+};
+
+constexpr int MONO_SRC_CTAS_PER_SM = 4;   // 125 registers x 128 threads, no spills (at 8 CTAs per SM ptxas spills)
+
+__global__ void __launch_bounds__(MONO_THREADS, MONO_SRC_CTAS_PER_SM)
+score_monomer_src_kernel(MonoSrcArgs A) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int K = A.K, d = A.d, kd = K * d;
+  const int ldt = d | 1;                                              // odd stride: conflict-free row reads
+  tkey_t* scratch = (tkey_t*)smem_raw;                                // [4][512] compaction scratch
+  f2_t* np2 = (f2_t*)(scratch + (MONO_THREADS / 32) * TOPK_CAP);      // [K*d][QT/2]: -P'_(k,j) of queries (2p, 2p+1)
+  float* thr = (float*)(np2 + (size_t)kd * (MONO_QT / 2));            // [QT]
+  int* cnt = (int*)(thr + MONO_QT);                                   // [QT]
+  float* wt = (float*)(cnt + MONO_QT);                                // [K][128] gate weights of the tile's rows
+  float* at = wt + K * MONO_THREADS;                                  // [128][ldt] embeddings of the tile's rows
+
+  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  const int part = blockIdx.x;
+  if (A.redo_tile != nullptr && A.redo_tile[blockIdx.y] == 0) return;
+  const int64_t q0 = (int64_t)blockIdx.y * MONO_QT;
+  const int nq = (int)((A.Q - q0 < MONO_QT) ? (A.Q - q0) : MONO_QT);
+  for (int i = tid; i < MONO_QT * kd; i += MONO_THREADS) {
+    const int ql = i / kd, kj = i % kd;
+    ((float*)np2)[kj * MONO_QT + ql] = ql < nq ? -A.P[(q0 + ql) * A.ldq + kj] : 0.0f;
+  }
+  if (tid < MONO_QT) { thr[tid] = __int_as_float(0x7f800000); cnt[tid] = 0; }
+  const int64_t t0 = A.tiles * part / A.parts;
+  const int64_t t1 = A.tiles * (part + 1) / A.parts;
+  tkey_t* kbase = A.keys + ((int64_t)part * A.Q + q0) * MONO_KSTRIDE;
+  const int sr0 = tid / d, sj0 = tid % d, sdr = MONO_THREADS / d, sdj = MONO_THREADS % d;
+
+  for (int64_t tile = (t0 + A.tile_stride - 1) / A.tile_stride * A.tile_stride; tile < t1; tile += A.tile_stride) {
+    const int64_t r0 = tile * 128;
+    __syncthreads();                                     // queries loaded / previous tile consumed
+    for (int i = tid, r = sr0, j = sj0; i < 128 * d; i += MONO_THREADS) {
+      const int64_t row = r0 + r;
+      at[r * ldt + j] = row < A.N ? A.A[row * A.lda + j] : 0.0f;
+      r += sdr; j += sdj;
+      if (j >= d) { j -= d; ++r; }
+    }
+    for (int i = tid; i < 128 * K; i += MONO_THREADS) {
+      const int r = i / K, k = i % K;
+      const int64_t row = r0 + r;
+      wt[k * MONO_THREADS + r] = row < A.N ? A.W[row * K + k] : 0.0f;
+    }
+    __syncthreads();
+    const float* ar = at + tid * ldt;
+    f2_t acc[MONO_QT / 2];
+#pragma unroll
+    for (int p = 0; p < MONO_QT / 2; ++p) acc[p] = pk2(0.0f, 0.0f);
+    for (int k = 0; k < K; ++k) {
+      f2_t dk[MONO_QT / 2];
+#pragma unroll
+      for (int p = 0; p < MONO_QT / 2; ++p) dk[p] = pk2(0.0f, 0.0f);
+      const ulonglong2* pk = (const ulonglong2*)(np2 + (size_t)k * d * (MONO_QT / 2));
+      for (int j = 0; j < d; ++j) {
+        const float a = ar[j];
+        const f2_t a2 = pk2(a, a);
+        const ulonglong2* pj = pk + j * (MONO_QT / 4);
+#pragma unroll
+        for (int p = 0; p < MONO_QT / 4; ++p) {
+          const ulonglong2 np = pj[p];
+          const f2_t d0 = add2(a2, np.x), d1 = add2(a2, np.y);
+          dk[2 * p] = fma2(d0, d0, dk[2 * p]);
+          dk[2 * p + 1] = fma2(d1, d1, dk[2 * p + 1]);
+        }
+      }
+      const float w = wt[k * MONO_THREADS + tid];
+      const f2_t w2 = pk2(w, w);
+#pragma unroll
+      for (int p = 0; p < MONO_QT / 2; ++p) acc[p] = fma2(w2, dk[p], acc[p]);
+    }
+    const int64_t row = r0 + tid;
+    if (row < A.N) {
+#pragma unroll
+      for (int p = 0; p < MONO_QT / 2; ++p) {
+        float dv[2];
+        upk2(acc[p], dv[0], dv[1]);
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          const int ql = 2 * p + h;
+          if (ql < nq && dv[h] < thr[ql]) {
+            const int slot = atomicAdd(&cnt[ql], 1);
+            kbase[(int64_t)ql * MONO_KSTRIDE + slot] = pack_key(dv[h], (uint32_t)row);
+          }
+        }
+      }
+    }
+    __syncthreads();
+    for (int ql = wid; ql < nq; ql += MONO_THREADS / 32) {
+      const int n = cnt[ql];
+      if (n > TOPK_TRIGGER) {
+        const int nk = warp_compact(kbase + (int64_t)ql * MONO_KSTRIDE, n, A.kk, scratch + wid * TOPK_CAP, lane, &thr[ql]);
+        if (lane == 0) cnt[ql] = nk;
+      }
+    }
+  }
+  __syncthreads();
+  for (int ql = wid; ql < nq; ql += MONO_THREADS / 32) {
+    const int nk = warp_compact(kbase + (int64_t)ql * MONO_KSTRIDE, cnt[ql], A.kk, scratch + wid * TOPK_CAP, lane, nullptr);
+    if (lane == 0) A.counts[(int64_t)part * A.Q + q0 + ql] = nk;
+  }
+}
+
 // Merge of the catalog parts; the keys already carry exact distances.
 __global__ void __launch_bounds__(MRG_THREADS)
 merge_plain_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ counts, int parts, int64_t Q, int kk,
@@ -181,20 +302,25 @@ static size_t mono_smem_bytes(int K, int d) {
          MONO_QT * 8 + (size_t)128 * (d + 1) * 4;
 }
 
+static size_t mono_src_smem_bytes(int K, int d) {
+  return (size_t)(MONO_THREADS / 32) * TOPK_CAP * sizeof(tkey_t) + (size_t)K * d * MONO_QT * 4 + MONO_QT * 8 +
+         (size_t)K * MONO_THREADS * 4 + (size_t)MONO_THREADS * (d | 1) * 4;
+}
+
 struct MonoPlan { int nqt, parts; int64_t tiles; };
 
 // One wave: the grid is sized to the CTAs that are RESIDENT at once (64 registers x 128 threads -> 8 per SM;
 // 228 KB of shared memory per SM, 1 KB reserved per CTA), because only resident warps hide the staging latency
 // and a second, partial wave would idle most SMs (measured: 4 CTAs per SM left 76 % of the warp slots empty,
-// 8 per SM ran 1.1 waves).
-static MonoPlan mono_plan(int64_t Q, int64_t N, int K, int d) {
+// 8 per SM ran 1.1 waves).  smem = dynamic shared memory of one CTA of the kernel being planned.
+static MonoPlan mono_plan_smem(int64_t Q, int64_t N, size_t smem, int64_t max_resident) {
   MonoPlan p;
   p.nqt = (int)((Q + MONO_QT - 1) / MONO_QT);
   p.tiles = (N + 127) / 128;
   int sms = sm_count();
   if (sms <= 0) sms = 148;
-  int64_t resident = (228 * 1024) / (int64_t)(mono_smem_bytes(K, d) + 1024);
-  if (resident > 8) resident = 8;                      // 64 registers x 128 threads
+  int64_t resident = (228 * 1024) / (int64_t)(smem + 1024);
+  if (resident > max_resident) resident = max_resident;  // register-limited CTAs per SM
   if (resident < 1) resident = 1;
   const char* e = getenv("CFL_MONO_CTAS_PER_SM");
   if (e && atoi(e) > 0) resident = atoi(e);
@@ -203,6 +329,12 @@ static MonoPlan mono_plan(int64_t Q, int64_t N, int K, int d) {
   if (parts < 1) parts = 1;
   p.parts = (int)parts;
   return p;
+}
+static MonoPlan mono_plan(int64_t Q, int64_t N, int K, int d) {
+  return mono_plan_smem(Q, N, mono_smem_bytes(K, d), 8);                 // 64 registers x 128 threads
+}
+static MonoPlan mono_src_plan(int64_t Q, int64_t N, int K, int d) {
+  return mono_plan_smem(Q, N, mono_src_smem_bytes(K, d), MONO_SRC_CTAS_PER_SM);
 }
 
 // Launch of the CUDA-core kernel for the tensor-core path (score_monomer_tc.cu): threshold sample (tile_stride > 1)
@@ -236,6 +368,29 @@ int mono_exact_launch(const float* Aq, int64_t lda, const float* Wq, int64_t Q, 
   return CFL_OK;
 }
 int mono_exact_parts(int64_t Q, int64_t N, int K, int d) { return mono_plan(Q, N, K, d).parts; }
+
+// The same for the source direction (score_monomer_src_kernel): every S-th tile, the flagged query tiles, or (tile_stride
+// 1, redo_tile NULL) the whole catalog.
+int mono_src_exact_launch(const float* Pq, int64_t ldq, int64_t Q, int K, int d, const float* Ac, int64_t lda,
+                          const float* Wc, int64_t N, int kk, int tile_stride, const int* redo_tile, tkey_t* keys,
+                          int* counts, int* parts_out, cudaStream_t cs) {
+  MonoPlan plan = mono_src_plan(Q, N > 0 ? N : 1, K, d);
+  *parts_out = plan.parts;
+  if (N == 0) {
+    CFL_CUDA(cudaMemsetAsync(counts, 0, (size_t)plan.parts * Q * sizeof(int), cs));
+    return CFL_OK;
+  }
+  MonoSrcArgs a;
+  a.K = K; a.d = d; a.Q = Q; a.N = N; a.ldq = ldq; a.lda = lda; a.P = Pq; a.A = Ac; a.W = Wc;
+  a.keys = keys; a.counts = counts;
+  a.parts = plan.parts; a.kk = kk; a.tiles = plan.tiles; a.tile_stride = tile_stride; a.redo_tile = redo_tile;
+  const size_t smem = mono_src_smem_bytes(K, d);
+  CFL_CUDA(cudaFuncSetAttribute(score_monomer_src_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  score_monomer_src_kernel<<<dim3(plan.parts, plan.nqt), MONO_THREADS, smem, cs>>>(a);
+  CFL_LAUNCH_CHECK();
+  return CFL_OK;
+}
+int mono_src_exact_parts(int64_t Q, int64_t N, int K, int d) { return mono_src_plan(Q, N > 0 ? N : 1, K, d).parts; }
 int mono_merge_launch(const tkey_t* keys, const int* counts, int parts, int64_t Q, int k, int64_t idx_base, float* top_val,
                       int64_t* top_idx, const float* only_redo, cudaStream_t cs) {
   merge_plain_kernel<<<(unsigned)Q, MRG_THREADS, 0, cs>>>(keys, counts, parts, Q, k, k, idx_base, top_val, top_idx, only_redo);

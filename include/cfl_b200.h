@@ -223,6 +223,31 @@ int cfl_score_topk_monomer_packed(const float* Aq, int64_t lda, const float* Wq,
                                   int64_t idx_base, float* top_val, int64_t* top_idx,
                                   unsigned long long* stats_out, void* ws, size_t ws_bytes, void* stream);
 
+/* The other direction of the monomer distance: rank the SOURCE items of a catalog for TARGET queries.  The monomer
+ * distance is directed: a and the gate w come from the source item, the K prototypes from the target item
+ * (cfl/models/base.py:94-117).  cfl_score_topk_monomer answers "which targets go with this source";
+ * cfl_score_topk_monomer_source answers "which sources is this target compatible with":
+ *   Pq[Q,K*d] (leading dimension ldq) = the K prototypes of the target (query) items,
+ *   Ac[N,d] (leading dimension lda) = act(e0) of the source (catalog) items, Wc[N,K] = their gate softmax (dense);
+ *   dist(q,c) = sum_k Wc[c,k] * |Ac[c] - Pq[q,k]|^2.
+ * cfl_monomer_source_pack builds the catalog's fp16 image once (the layout of cfl_monomer_pack with the rows'
+ * v_c = [2 w_ck (a_c - mu)]_k || [-w_ck]_k; 1024-byte aligned; cfl_monomer_source_pack_bytes = 0 when K(d+1) > 128).
+ * cfl_score_topk_monomer_source runs the stages of cfl_score_topk_monomer_packed with the roles swapped (sampled
+ * thresholds on the CUDA cores, the transposed single-product fp16 Gram filter, exact rescoring, verification, exact
+ * redo); with image == NULL (required when K(d+1) > 128) it runs the exact CUDA-core kernel over every tile.  Both
+ * routes return identical bits.  Outputs as cfl_score_topk_monomer: top_val[Q,k] ascending exact distances,
+ * top_idx[Q,k] = idx_base + row, ties -> lower index, -1 / +inf when N < k.  stats_out: optional CFL_SCORE_NSTATS
+ * counters (device) as cfl_score_topk_stats (all zero on the CUDA-core route).  K <= 8, d <= 128, k <= 128;
+ * N = 0 is allowed.  Ac / Wc / mu must be the arrays the image was built from. */
+size_t cfl_monomer_source_pack_bytes(int64_t N, int K, int d);
+int cfl_monomer_source_pack(const float* Ac, int64_t lda, const float* Wc, int64_t N, int K, int d, const float* mu,
+                            void* image, size_t image_bytes, void* stream);
+size_t cfl_score_topk_monomer_source_workspace_bytes(int64_t Q, int K, int d, int64_t N, int k);
+int cfl_score_topk_monomer_source(const float* Pq, int64_t ldq, int64_t Q, int K, int d, const void* image,
+                                  const float* Ac, int64_t lda, const float* Wc, int64_t N, const float* mu, int k,
+                                  int64_t idx_base, float* top_val, int64_t* top_idx,
+                                  unsigned long long* stats_out, void* ws, size_t ws_bytes, void* stream);
+
 /* Merge R sorted lists per query (the per-rank results after ncclAllGather) into one:
  * vals[R,Q,k], idx[R,Q,k] -> top_val[Q,k], top_idx[Q,k]; order (value, index). */
 int cfl_topk_merge(const float* vals, const int64_t* idx, int R, int64_t Q, int k,
