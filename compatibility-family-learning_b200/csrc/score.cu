@@ -351,16 +351,72 @@ merge_rescore_src_kernel(const tkey_t* __restrict__ keys, const int* __restrict_
 
 // ---- merge after the lower-bound filter pass: EVERY surviving row is scored exactly -------------
 // The keys of score_lb_kernel carry a lower bound, not the distance, so nothing may be discarded before its exact value
-// is known.  Stage 1 (all survivors): each warp stages 32 candidate rows through shared memory with coalesced
-// reads, 32 dimensions at a time; every thread then owns one row and accumulates d_k = |e - p_k|^2,
-// from which dist = sum_k s_k d_k - sum_{k<l} s_k s_l |p_k - p_l|^2 (the same quantity as the direct
-// form, SURVEY App. A.3, good to a few ulp) picks the kk best.  Stage 2 rescores those kk in the
-// direct-difference form (pcd_direct) and sorts by (value, index), exactly as merge_rescore_kernel does.
-constexpr int RSC_CH = 16;                 // dimensions per staging chunk (small: 8 CTAs per SM = one wave)
-constexpr int RSC_LD = RSC_CH + 4;         // row stride in floats: 16 B aligned, conflict-free LDS.128
+// is known.  Stage 1 (all survivors): each warp takes 32 survivors per round and gathers their rows RSC_CH dimensions
+// at a time (16-byte loads, eight rows' segments per instruction) into its own slice of shared memory; every thread then
+// owns one row and accumulates d_k = |e - p_k|^2, from which dist = sum_k s_k d_k - sum_{k<l} s_k s_l |p_k - p_l|^2 (the
+// same quantity as the direct form, SURVEY App. A.3, good to a few ulp) picks the kk best.  The gather is software
+// pipelined: the loads of the next chunk -- the next round's first chunk during the last one -- are issued before the
+// current chunk is computed, so they stay in flight through the arithmetic, the selection and its barriers.  Stage 2
+// stages the kk best rows with all threads and rescores them in the direct-difference form (pcd_direct), then sorts by
+// (value, index), exactly as merge_rescore_kernel does.
+constexpr int RSC_CH = 32;                 // dimensions per gathered chunk: 8 float4 per thread for the warp's 32 rows
+constexpr int RSC_LD = RSC_CH + 4;         // row stride in floats: 16 B aligned, conflict-free LDS.128 / STS.128
+constexpr int RSC_CAP = 2 * TOPK_CAP;      // candidate keys under the admission bound
+
+// Row of the survivor f (0 when f >= total): the list p with s_pref[p] <= f < s_pref[p + 1], by binary search.
+// Lists 0..parts-1 are the part buffers, list `parts` is the query's spill list.
+__device__ __forceinline__ uint32_t rsc_row(int f, int total, const int* s_pref, int parts, const tkey_t* __restrict__ keys,
+                                            const tkey_t* __restrict__ spill, int64_t Q, int64_t q) {
+  if (f >= total) return 0u;
+  int lo = 0, hi = parts;
+  while (lo < hi) {
+    const int m = (lo + hi) >> 1;
+    if (s_pref[m + 1] <= f) lo = m + 1; else hi = m;
+  }
+  const tkey_t* src = (lo < parts) ? keys + ((int64_t)lo * Q + q) * TOPK_STRIDE : spill + q * (int64_t)LB_SPILL;
+  return (uint32_t)(src[f - s_pref[lo]] & 0xffffffffu);
+}
+
+// Loads dimensions [c0, c0 + RSC_CH) of the warp's 32 rows (row r of the warp = the row of lane r): instruction i reads
+// float4 (lane & 7) of row 4i + (lane >> 3).  Without 16-byte aligned rows (vec = false) the same elements come in
+// 4-byte loads.  Dimensions >= d read as 0.
+__device__ __forceinline__ void rsc_load(float4 (&v)[RSC_CH / 4], const float* __restrict__ E, int64_t lde, int d, bool vec,
+                                         uint32_t idx, int c0, int lane) {
+  const int j = c0 + 4 * (lane & 7);
+#pragma unroll
+  for (int i = 0; i < RSC_CH / 4; ++i) {
+    const uint32_t r = __shfl_sync(0xffffffffu, idx, 4 * i + (lane >> 3));
+    const float* e = E + (int64_t)r * lde + j;
+    if (vec) {
+      v[i] = (j < d) ? __ldg((const float4*)e) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    } else {
+      v[i] = make_float4(j < d ? __ldg(e) : 0.0f, j + 1 < d ? __ldg(e + 1) : 0.0f, j + 2 < d ? __ldg(e + 2) : 0.0f,
+                         j + 3 < d ? __ldg(e + 3) : 0.0f);
+    }
+  }
+}
+
+// The kk best of the candidate buffer, sorted ascending; the sort covers the smallest of TOPK_CAP, RSC_CAP keys that
+// holds the fill.  Same result and admission bound as mrg_compact.
+__device__ __forceinline__ void rsc_compact(tkey_t* s, int* s_fill, tkey_t* s_thr, int kk, int t) {
+  const int fill = *s_fill;
+  if (fill <= TOPK_CAP) {
+    mrg_compact(s, s_fill, s_thr, kk, t);
+    return;
+  }
+  for (int i = fill + t; i < RSC_CAP; i += MRG_THREADS) s[i] = CFL_KEY_INF;
+  __syncthreads();
+  coop_sort_generic<MRG_THREADS, RSC_CAP>(s, t);   // ends with a block barrier
+  if (t == 0) {
+    const int nf = fill < kk ? fill : kk;
+    *s_fill = nf;
+    if (nf >= kk) *s_thr = s[kk - 1];
+  }
+  __syncthreads();
+}
 
 template <int K>
-__global__ void __launch_bounds__(MRG_THREADS, 4)            // 64 registers: four blocks per SM
+__global__ void __launch_bounds__(MRG_THREADS, 2)            // <= 128 registers: two blocks per SM (at three, K >= 2 spills)
 rescore_merge_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ counts, int parts, int64_t Q,
                      int kk, int k, const float* __restrict__ Pq, int64_t ldq, int d,
                      const float* __restrict__ E, int64_t lde, int64_t idx_base,
@@ -387,9 +443,9 @@ rescore_merge_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ co
   }
   const int dp = (d + RSC_CH - 1) / RSC_CH * RSC_CH;        // d padded to whole chunks
   float* s_pq = s_dyn;                                       // [K][dp], zero padded
-  float* s_rows = s_pq + K * dp;                             // [warps][32][RSC_LD]
+  float* s_rows = s_pq + K * dp;                             // stage 1: [warps][32][RSC_LD]; stage 2: [rows][dp + 1]
   int* s_pref = (int*)(s_rows + (MRG_THREADS / 32) * 32 * RSC_LD);   // [parts + 2]
-  __shared__ tkey_t s[TOPK_CAP];
+  __shared__ tkey_t s[RSC_CAP];
   __shared__ int s_fill;
   __shared__ tkey_t s_thr;
   __shared__ float s_D[K * K];
@@ -426,47 +482,45 @@ rescore_merge_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ co
     for (int j = 0; j < d; ++j) { const float df = s_pq[a * dp + j] - s_pq[b * dp + j]; acc = fmaf(df, df, acc); }
     s_D[i] = acc;
   }
-  __syncthreads();
   const int total = s_pref[parts + 1];
+  const bool vec = (d % 4 == 0) && (lde % 4 == 0) && ((reinterpret_cast<uintptr_t>(E) & 15u) == 0);
   float* my_rows = s_rows + wid * 32 * RSC_LD;
-  for (int base = 0; base < total; base += MRG_THREADS) {
-    const int f = base + t;
-    uint32_t idx = 0;
-    const bool have = f < total;
-    if (have) {
-      int p = 0;
-      while (s_pref[p + 1] <= f) ++p;
-      const tkey_t* src = (p < parts) ? keys + ((int64_t)p * Q + q) * TOPK_STRIDE : spill + q * (int64_t)LB_SPILL;
-      idx = (uint32_t)(src[f - s_pref[p]] & 0xffffffffu);
-    }
+  // round r: thread t scores survivor f = 256 r + t; idx / nidx are the rows of this round and the next
+  int f = t;
+  uint32_t idx = rsc_row(f, total, s_pref, parts, keys, spill, Q, q);
+  uint32_t nidx = rsc_row(f + MRG_THREADS, total, s_pref, parts, keys, spill, Q, q);
+  float4 v[RSC_CH / 4];
+  if (f - lane < total) rsc_load(v, E, lde, d, vec, idx, 0, lane);
+  __syncthreads();                                           // s_D
+  for (int base = 0; base < total; base += MRG_THREADS, f += MRG_THREADS) {
     float dk[K];
 #pragma unroll
     for (int kq = 0; kq < K; ++kq) dk[kq] = 0.0f;
-    for (int c0 = 0; c0 < dp; c0 += RSC_CH) {
-      __syncwarp();
-      // coalesced: a load covers 16 dimensions (64 B) of TWO rows; 16 independent loads per thread
-      const int j = c0 + (lane & 15), half = lane >> 4;
-      float v[16];
+    if (f - lane < total) {                                  // the warp has survivors this round (warp-uniform)
+      for (int c0 = 0; c0 < dp; c0 += RSC_CH) {
+        __syncwarp();
 #pragma unroll
-      for (int r = 0; r < 16; ++r) {
-        const uint32_t ridx = __shfl_sync(0xffffffffu, idx, 2 * r + half);
-        v[r] = (j < d) ? __ldg(E + (int64_t)ridx * lde + j) : 0.0f;
-      }
+        for (int i = 0; i < RSC_CH / 4; ++i)
+          *(float4*)(my_rows + (4 * i + (lane >> 3)) * RSC_LD + 4 * (lane & 7)) = v[i];
+        __syncwarp();
+        if (c0 + RSC_CH < dp) rsc_load(v, E, lde, d, vec, idx, c0 + RSC_CH, lane);
+        else if (f - lane + MRG_THREADS < total) rsc_load(v, E, lde, d, vec, nidx, 0, lane);
+        const float4* er = (const float4*)(my_rows + lane * RSC_LD);
 #pragma unroll
-      for (int r = 0; r < 16; ++r) my_rows[(2 * r + half) * RSC_LD + (lane & 15)] = v[r];
-      __syncwarp();
-      const float4* er = (const float4*)(my_rows + lane * RSC_LD);
+        for (int j4 = 0; j4 < RSC_CH / 4; ++j4) {
+          const float4 e4 = er[j4];
 #pragma unroll
-      for (int j4 = 0; j4 < RSC_CH / 4; ++j4) {
-        const float4 e4 = er[j4];
-#pragma unroll
-        for (int kq = 0; kq < K; ++kq) {
-          const float4 p4 = *(const float4*)(s_pq + kq * dp + c0 + j4 * 4);
-          const float a0 = e4.x - p4.x, a1 = e4.y - p4.y, a2 = e4.z - p4.z, a3 = e4.w - p4.w;
-          dk[kq] = fmaf(a3, a3, fmaf(a2, a2, fmaf(a1, a1, fmaf(a0, a0, dk[kq]))));
+          for (int kq = 0; kq < K; ++kq) {
+            const float4 p4 = *(const float4*)(s_pq + kq * dp + c0 + j4 * 4);
+            const float a0 = e4.x - p4.x, a1 = e4.y - p4.y, a2 = e4.z - p4.z, a3 = e4.w - p4.w;
+            dk[kq] = fmaf(a3, a3, fmaf(a2, a2, fmaf(a1, a1, fmaf(a0, a0, dk[kq]))));
+          }
         }
       }
     }
+    const uint32_t row = idx;
+    idx = nidx;
+    nidx = rsc_row(f + 2 * MRG_THREADS, total, s_pref, parts, keys, spill, Q, q);
     float dist = dk[0];
     if (K > 1) {
       float mn = dk[0];
@@ -488,14 +542,14 @@ rescore_merge_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ co
     // selection protocol of block_merge_topkk: uniform branch on the fill level read between barriers
     const int f0 = s_fill;
     __syncthreads();
-    if (f0 + MRG_THREADS > TOPK_CAP) mrg_compact(s, &s_fill, &s_thr, kk, t);
-    if (have) {
-      const tkey_t key = pack_key(dist, idx);
+    if (f0 + MRG_THREADS > RSC_CAP) rsc_compact(s, &s_fill, &s_thr, kk, t);
+    if (f < total) {
+      const tkey_t key = pack_key(dist, row);
       if (key < s_thr) s[atomicAdd(&s_fill, 1)] = key;
     }
     __syncthreads();
   }
-  mrg_compact(s, &s_fill, &s_thr, kk, t);
+  rsc_compact(s, &s_fill, &s_thr, kk, t);
   const int fill = s_fill;
   // Verification.  The filter kept every row whose LOWER BOUND is under the threshold, so a key count
   // proves nothing; the exact values do: if kk survivors have dist <= tau_opt, no row outside the
@@ -526,40 +580,54 @@ rescore_merge_kernel(const tkey_t* __restrict__ keys, const int* __restrict__ co
   if (s_redo) return;
   {                                                          // stage 2: direct form for the kk survivors,
     const int ld2 = dp + 1;                                  // rows staged in full (stride dp+1: conflict-free)
-    int wcap = ((MRG_THREADS / 32) * 32 * RSC_LD) / (32 * ld2);
-    if (wcap > MRG_THREADS / 32) wcap = MRG_THREADS / 32;
-    for (int w0 = 0; w0 * 32 < fill; w0 += (wcap > 0 ? wcap : 1)) {
-      const int kidx = (w0 + wid) * 32 + lane;
-      const bool mine = wid < wcap && kidx < fill;
-      float dist = 0.0f;
-      uint32_t idx = mine ? (uint32_t)(s[kidx] & 0xffffffffu) : 0u;
-      if (wcap > 0) {
-        if (wid < wcap && (w0 + wid) * 32 < fill) {
-          float* rows = s_rows + wid * 32 * ld2;
-          for (int c0 = 0; c0 < dp; c0 += 32) {
-            const int j = c0 + lane;
-            for (int r0 = 0; r0 < 32; r0 += 16) {
-              float v[16];
+    const int nst = ((MRG_THREADS / 32) * 32 * RSC_LD) / ld2;  // rows the staging area holds at once
+    if (nst > 0) {
+      for (int r0 = 0; r0 < fill; r0 += nst) {
+        const int nr = (fill - r0 < nst) ? fill - r0 : nst;
+        // every thread loads: element i of the nr x (dp / 4) float4 grid, eight loads in flight before the stores
+        const int n4 = dp / 4, ne = nr * n4;
+        for (int i0 = 0; i0 < ne; i0 += 8 * MRG_THREADS) {
+          float4 w4[8];
 #pragma unroll
-              for (int r = 0; r < 16; ++r) {
-                const uint32_t ridx = __shfl_sync(0xffffffffu, idx, r0 + r);
-                v[r] = (j < d) ? __ldg(E + (int64_t)ridx * lde + j) : 0.0f;
-              }
-#pragma unroll
-              for (int r = 0; r < 16; ++r) if (j < dp) rows[(r0 + r) * ld2 + j] = v[r];
+          for (int u = 0; u < 8; ++u) {
+            const int i = i0 + u * MRG_THREADS + t;
+            const int rr = i / n4, j = 4 * (i - rr * n4);
+            w4[u] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+            if (i < ne && j < d) {
+              const float* e = E + (int64_t)(uint32_t)(s[r0 + rr] & 0xffffffffu) * lde + j;
+              if (vec) w4[u] = __ldg((const float4*)e);
+              else w4[u] = make_float4(__ldg(e), j + 1 < d ? __ldg(e + 1) : 0.0f, j + 2 < d ? __ldg(e + 2) : 0.0f,
+                                       j + 3 < d ? __ldg(e + 3) : 0.0f);
             }
           }
-          __syncwarp();
-          const float* er = rows + lane * ld2;
-          if (mine) dist = pcd_direct<K>([&](int j) { return er[j]; }, [&](int kq, int j) { return s_pq[kq * dp + j]; }, d);
+#pragma unroll
+          for (int u = 0; u < 8; ++u) {
+            const int i = i0 + u * MRG_THREADS + t;
+            const int rr = i / n4, j = 4 * (i - rr * n4);
+            if (i < ne) {
+              float* o = s_rows + rr * ld2 + j;
+              o[0] = w4[u].x; o[1] = w4[u].y; o[2] = w4[u].z; o[3] = w4[u].w;
+            }
+          }
         }
-      } else if (mine) {                                     // very wide rows: straight from global memory
-        const float* er = E + (int64_t)idx * lde;
-        dist = pcd_direct<K>([&](int j) { return er[j]; }, [&](int kq, int j) { return s_pq[kq * dp + j]; }, d);
+        __syncthreads();
+        float dist = 0.0f;
+        uint32_t ridx = 0u;
+        if (t < nr) {
+          ridx = (uint32_t)(s[r0 + t] & 0xffffffffu);
+          const float* er = s_rows + t * ld2;
+          dist = pcd_direct<K>([&](int j) { return er[j]; }, [&](int kq, int j) { return s_pq[kq * dp + j]; }, d);
+        }
+        __syncthreads();                                     // staged rows and keys read
+        if (t < nr) s[r0 + t] = pack_key(dist, ridx);
       }
-      __syncthreads();
-      if (mine) s[kidx] = pack_key(dist, idx);
-      __syncthreads();
+    } else {                                                 // very wide rows: straight from global memory
+      for (int kidx = t; kidx < fill; kidx += MRG_THREADS) {
+        const uint32_t ridx = (uint32_t)(s[kidx] & 0xffffffffu);
+        const float* er = E + (int64_t)ridx * lde;
+        const float dist = pcd_direct<K>([&](int j) { return er[j]; }, [&](int kq, int j) { return s_pq[kq * dp + j]; }, d);
+        s[kidx] = pack_key(dist, ridx);
+      }
     }
   }
   __syncthreads();
