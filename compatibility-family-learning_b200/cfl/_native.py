@@ -14,7 +14,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "_lib", "libcfl_b200.so")
 
-MODES = {"pcd": 0, "monomer": 1, "siamese": 2}
+MODES = {"pcd": 0, "monomer": 1, "siamese": 2, "pcd_source": 3, "monomer_source": 4}
 ACTS = {None: 0, "linear": 0, "tanh": 1, "sigmoid": 2, "relu": 3, "lrelu": 4}
 MAX_K, MAX_D, MAX_TOPK = 8, 256, 128
 
@@ -81,6 +81,7 @@ SIGNATURES = {
     "cfl_rank_counts": (_int, [_int, _vp, _i64, _int, _int, _i64, _vp, _vp, _i64, _i64, _vp, _int, _vp, _vp]),
     "cfl_dense_rank_counts": (_int, [_vp, _i64, _i64, _i64, _vp, _int, _vp, _vp]),
     "cfl_rank_counts_packed_workspace_bytes": (_sz, [_i64, _int, _int, _i64]),
+    "cfl_rank_counts_packed_source_workspace_bytes": (_sz, [_i64, _int, _int, _i64]),
     "cfl_rank_counts_packed": (_int, [_int, _vp, _i64, _int, _int, _i64, _vp, _vp, _i64, _i64, _vp, _vp, _int,
                                       _vp, _vp, _sz, _vp]),
     "cfl_rank_counts_packed_stats": (_int, [_i64, _int, _int, _i64, _vp, _sz, _vp, _vp]),
@@ -608,7 +609,34 @@ def topk_merge_records(recs, R, Q, k):
 
 
 def _rank_operands(mode, query, catalog, w):
-    """(Pq2, Q, K, d, ldq, w, E2, N, lde) for cfl_pair_dist_rows / cfl_rank_counts."""
+    """(Pq2, Q, K, d, ldq, w, E2, N, lde) for cfl_pair_dist_rows / cfl_rank_counts.
+
+    pcd / siamese: query [Q,K,d] (or [Q,d]) prototypes, catalog [N,d] embeddings; monomer: query [Q,d] = a, w [Q,K]
+    its gate, catalog [N,K,d] prototypes.  The source modes swap the roles: pcd_source: query [Q,d] = the targets'
+    e0, catalog [N,K,d] = the sources' prototypes; monomer_source: query [Q,K,d] = the targets' prototypes, catalog
+    [N,d] = the sources' a, w [N,K] = the sources' gate."""
+    if mode == "pcd_source":
+        if catalog.dim() != 3 or w is not None:
+            raise CflNativeError("rank counts (pcd_source): catalog must be [N,K,d] source prototypes, no gate")
+        N, K, d = catalog.shape
+        q2, ldq = _rows(query, "query")
+        E2, lde = _rows(_f32c(catalog, "catalog").reshape(N, K * d), "catalog")
+        if q2.shape[1] != d:
+            raise CflNativeError(f"rank counts (pcd_source): query has d={q2.shape[1]} but the catalog is "
+                                 f"{tuple(catalog.shape)}")
+        return q2, q2.shape[0], K, d, ldq, None, E2, N, lde
+    if mode == "monomer_source":
+        query = _f32c(query, "query")
+        if query.dim() != 3 or w is None:
+            raise CflNativeError("rank counts (monomer_source): query must be [Q,K,d] target prototypes and w the "
+                                 "sources' [N,K] gate")
+        Q, K, d = query.shape
+        q2, ldq = _rows(query.reshape(Q, K * d), "query")
+        E2, lde = _rows(catalog, "catalog")
+        w = _f32c(w, "w").contiguous()
+        if E2.shape[1] != d or tuple(w.shape) != (E2.shape[0], K):
+            raise CflNativeError("rank counts (monomer_source): catalog/gate shapes do not match the queries")
+        return q2, Q, K, d, ldq, w, E2, E2.shape[0], lde
     if mode == "monomer":
         if catalog.dim() != 3 or w is None:
             raise CflNativeError("rank counts (monomer): catalog must be [N,K,d] prototypes and w the [Q,K] gate")
@@ -656,24 +684,30 @@ def rank_counts(mode, query, catalog, pos_dist, w=None):
     return out
 
 
-def rank_counts_packed(query, catalog, image, mu, pos_dist, want_stats=False):
+def rank_counts_packed(query, catalog, image, mu, pos_dist, want_stats=False, mode=None):
     """``rank_counts("pcd", ...)`` on the tensor cores: the counts are taken inside the fused scoring kernel's epilogue
     over the packed catalog ``image`` (``catalog_pack`` of the same catalog / ``mu``), near-ties re-evaluated in the
     direct form -> the same int64 [Q,J,2] as ``rank_counts``.  want_stats: also a dict of the call's statistics.
-    Query batches beyond 65536 go through the C entry point in chunks (one call holds at most 4096 scoring CTAs)."""
-    q2, Q, K, d, ldq, _, E2, N, lde = _rank_operands("pcd", query, catalog, None)
+    Query batches beyond 65536 go through the C entry point in chunks (one call holds at most 4096 scoring CTAs).
+    ``mode``: None = pcd (siamese at K = 1) as ``rank_counts("pcd", ...)``; "pcd_source" = ``rank_counts("pcd_source",
+    ...)`` with ``image = source_catalog_pack(catalog, mu)``."""
+    src = mode == "pcd_source"
+    if mode not in (None, "pcd_source"):
+        raise CflNativeError(f"rank_counts_packed: mode {mode!r} has no tensor-core count (None or 'pcd_source')")
+    q2, Q, K, d, ldq, _, E2, N, lde = _rank_operands("pcd_source" if src else "pcd", query, catalog, None)
     pos_dist = _f32c(pos_dist, "pos_dist").contiguous()
     if pos_dist.dim() != 2 or pos_dist.shape[0] != Q:
         raise CflNativeError("rank_counts_packed: pos_dist must be [Q,J]")
     J = pos_dist.shape[1]
     out = torch.empty(Q, J, 2, dtype=torch.int64, device=E2.device)
-    mode = MODES["siamese"] if K == 1 else MODES["pcd"]
+    mode = MODES["pcd_source"] if src else MODES["siamese"] if K == 1 else MODES["pcd"]
+    ws_bytes = lib().cfl_rank_counts_packed_source_workspace_bytes if src else lib().cfl_rank_counts_packed_workspace_bytes
     mu = None if mu is None else _f32c(mu, "mu").contiguous()
     chunk = 65536
     tot = dict(records=0, worst_ratio=0.0, beyond_half_band=0, recounted_queries=0)
     for lo in range(0, max(Q, 1), chunk):
         hi = min(Q, lo + chunk)
-        need = lib().cfl_rank_counts_packed_workspace_bytes(hi - lo, K, d, N)
+        need = ws_bytes(hi - lo, K, d, N)
         ws = _ws.get(need, E2.device)
         _check(lib().cfl_rank_counts_packed(mode, _ptr(q2[lo:hi]), hi - lo, K, d, ldq, _ptr(E2), _ptr(image), N, lde,
                                             _ptr(mu), _ptr(pos_dist[lo:hi]), J, _ptr(out[lo:hi]), _ptr(ws), ws.numel(),
@@ -717,9 +751,10 @@ def within_radius(radius, Q, device):
 
 def within_counts(mode, query, catalog, radius, w=None, image=None, mu=None):
     """Result size of every query of ``score_within``: #{c : dist(q, c) < radius[q]} -> int64 [Q] (device).  The
-    counting pass of ``rank_counts_packed`` (image given, pcd) or ``rank_counts`` with J = 1."""
+    counting pass of ``rank_counts_packed`` (image given: pcd, pcd_source) or ``rank_counts`` with J = 1."""
     if image is not None and catalog.shape[0] > 0:
-        c = rank_counts_packed(query, catalog, image, mu, radius[:, None])
+        c = rank_counts_packed(query, catalog, image, mu, radius[:, None],
+                               mode="pcd_source" if mode == "pcd_source" else None)
     else:
         c = rank_counts(mode, query, catalog, radius[:, None], w=w)
     return c[:, 0, 0]
@@ -731,9 +766,9 @@ def score_within(mode, query, catalog, radius, w=None, image=None, mu=None, idx_
     ``(offsets [Q+1] int64, index [T] int64 = idx_base + row, dist [T] float32)`` ordered by (distance, index) within
     each query.  The distances are the direct-form values of ``pair_dist_rows``, bit for bit; NaN selects nothing.
 
-    ``radius``: a scalar or [Q].  Operands as ``rank_counts``.  ``image`` (= ``catalog_pack(catalog, K, mu)``, pcd)
-    emits the rows from the tensor-core scoring epilogue; without it (monomer, shapes without a tcgen05 tiling) the
-    CUDA cores evaluate every pair in the direct form.  ``counts`` = ``within_counts`` of the same call when the caller
+    ``radius``: a scalar or [Q].  Operands as ``rank_counts``.  ``image`` (= ``catalog_pack(catalog, K, mu)``, pcd;
+    ``source_catalog_pack(catalog, mu)``, pcd_source) emits the rows from the tensor-core scoring epilogue; without it
+    (monomer, monomer_source, shapes without a tcgen05 tiling) the CUDA cores evaluate every pair in the direct form.  ``counts`` = ``within_counts`` of the same call when the caller
     has them already.
 
     The result size is data-dependent, so the call reads T = offsets[Q] back to the host once to size the outputs
@@ -762,7 +797,8 @@ def score_within(mode, query, catalog, radius, w=None, image=None, mu=None, idx_
         hi = min(Q, lo + chunk)
         ws = _ws.get(lib().cfl_score_within_workspace_bytes(MODES[mode], hi - lo, K, d, N), dev)
         _check(lib().cfl_score_within(MODES[mode], _ptr(q2[lo:hi]), hi - lo, K, d, ldq,
-                                      None if w is None else _ptr(w[lo:hi]), _ptr(E2), _ptr(image), N, lde, _ptr(mu),
+                                      None if w is None else _ptr(w if mode == "monomer_source" else w[lo:hi]),
+                                      _ptr(E2), _ptr(image), N, lde, _ptr(mu),
                                       _ptr(r[lo:hi]), _ptr(offsets[lo:hi + 1]), int(idx_base), _ptr(out_idx),
                                       _ptr(out_dist), _ptr(ws), ws.numel(), _stream()), "cfl_score_within")
         if want_stats and hi > lo:

@@ -319,7 +319,7 @@ def auc_from_rank_counts(counts: torch.Tensor, pos_dist: torch.Tensor, n_total: 
 
 def _auc_per_query(mode, query, catalog, gate, pos_idx, idx_base, n_total, group, world, packed=None):
     """Positives' distances where they live, summed over shards; exact counts per shard, summed (SURVEY 8e).
-    packed = (catalog image, mu): count on the tensor cores (pcd)."""
+    packed = (catalog image, mu): count on the tensor cores (pcd, pcd_source)."""
     n_local = catalog.shape[0]
     pos_idx = pos_idx.to(catalog.device)
     local = pos_idx - idx_base
@@ -332,7 +332,8 @@ def _auc_per_query(mode, query, catalog, gate, pos_idx, idx_base, n_total, group
         torch.distributed.all_reduce(val, group=group)               # one owner per positive: the sum is its value
         pos_dist = torch.where(have > 0, val, torch.full_like(val, float("nan")))
     if packed is not None and n_local > 0:
-        counts = nat.rank_counts_packed(query, catalog, packed[0], packed[1], pos_dist)
+        counts = nat.rank_counts_packed(query, catalog, packed[0], packed[1], pos_dist,
+                                        mode="pcd_source" if mode == "pcd_source" else None)
     else:
         counts = nat.rank_counts(mode, query, catalog, pos_dist, w=gate)
     if world > 1:
@@ -552,6 +553,29 @@ class SourceCatalogIndex:
         world = self._world()
         return (tv, ti) if world == 1 else _gather_merge(tv, ti, self.group, world)
 
+    def auc_per_query(self, xq: torch.Tensor, pos_idx: torch.Tensor, method: str = "fused"):
+        """All-candidate AUC of every target query over the SOURCE rows: ``pos_idx`` [Q,J] int64 = GLOBAL source rows
+        of the query's labelled positives (unique per query; -1 pads), every other source row is a negative.  As
+        ``CatalogIndex.auc_per_query``: ``method="fused"`` counts inside the tensor-core scoring epilogue over the
+        source image, ``method="direct"`` evaluates every pair on the CUDA cores; the integers are the same."""
+        if method not in ("direct", "fused"):
+            raise ValueError("auc_per_query: method must be 'direct' or 'fused'")
+        packed = (self.image, self.mu) if method == "fused" else None
+        return _auc_per_query("pcd_source", self.project_queries(xq), self.P, None, pos_idx, self.idx_base,
+                              self.n_total, self.group, self._world(), packed=packed)
+
+    def within(self, xq: torch.Tensor, radius, max_results: int = nat.WITHIN_MAX_RESULTS):
+        """Every source row closer than ``radius`` (a scalar or one per query) to each target query, exact: CSR lists
+        as ``CatalogIndex.within``, distances bit-identical to those ``rank`` reports.  Emitted from the tensor-core
+        scoring epilogue over the source image; sharding and the size guard as ``CatalogIndex.within``."""
+        return _within("pcd_source", self.project_queries(xq), self.P, None, radius, self.idx_base, self.group,
+                       self._world(), max_results, image=self.image, mu=self.mu)
+
+    def compatible(self, xq: torch.Tensor, max_results: int = nat.WITHIN_MAX_RESULTS):
+        """The sources whose Thresholder calls each target compatible (score max(theta, 1e-6) - dist > 0): e.g. every
+        existing item that should now recommend a newly added one.  ``within`` at r = max(theta, 1e-6)."""
+        return self.within(xq, compatible_radius(self.theta), max_results=max_results)
+
     def scores(self, dist: torch.Tensor) -> torch.Tensor:
         """Thresholder (blocks.py:21-22): max(theta, 1e-6) - dist."""
         return max(self.theta, 1e-6) - dist
@@ -635,6 +659,22 @@ class MonomerSourceCatalogIndex:
         tv, ti = self.rank_local(self.project_queries(xq), k)
         world = self._world()
         return (tv, ti) if world == 1 else _gather_merge(tv, ti, self.group, world)
+
+    def auc_per_query(self, xq: torch.Tensor, pos_idx: torch.Tensor):
+        """As ``SourceCatalogIndex.auc_per_query`` with the monomer distance (direct form on the CUDA cores);
+        ``pos_idx`` holds GLOBAL source rows."""
+        return _auc_per_query("monomer_source", self.project_queries(xq), self.a, self.gate, pos_idx, self.idx_base,
+                              self.n_total, self.group, self._world())
+
+    def within(self, xq: torch.Tensor, radius, max_results: int = nat.WITHIN_MAX_RESULTS):
+        """As ``SourceCatalogIndex.within`` with the monomer distance (direct form on the CUDA cores); the distances
+        are bit-identical to those ``rank`` reports."""
+        return _within("monomer_source", self.project_queries(xq), self.a, self.gate, radius, self.idx_base, self.group,
+                       self._world(), max_results)
+
+    def compatible(self, xq: torch.Tensor, max_results: int = nat.WITHIN_MAX_RESULTS):
+        """As ``SourceCatalogIndex.compatible``: ``within`` at the Thresholder radius max(theta, 1e-6)."""
+        return self.within(xq, compatible_radius(self.theta), max_results=max_results)
 
     def scores(self, dist: torch.Tensor) -> torch.Tensor:
         """Thresholder (blocks.py:21-22): max(theta, 1e-6) - dist."""

@@ -11,6 +11,11 @@
 // catalog shards (int64 all-reduce), which makes the AUC independent of the sharding.  The pcd
 // arithmetic is that of merge_rescore_kernel (score.cu), i.e. of the values cfl_score_topk reports;
 // the monomer arithmetic is that of score_monomer_kernel.
+//
+// The source modes swap the roles (queries = target items, catalog rows = source items): pcd_source takes e = the
+// query's e0 and p = the row's K prototypes (merge_rescore_src_kernel's values), monomer_source takes the query's
+// K prototypes and the row's a and gate w (mono_rescore_src_kernel's values).  The bodies below take the role as a
+// template argument; the kernels of the forward modes keep their names and code, the source modes have their own.
 #include "score.cuh"
 #include "direct.cuh"
 
@@ -19,13 +24,31 @@ namespace cfl {
 constexpr int RC_QT = 8;          // queries per CTA
 constexpr int RC_THREADS = 128;   // one thread per catalog row of a 128-row tile
 constexpr int RC_MAX_J = 32;
+constexpr size_t RC_SMEM_MAX = 200 * 1024;
+
+// Roles of the query and the catalog row.  Floats per catalog row staged in shared memory / per query:
+//   RC_PCD      row e0 [d],          query K prototypes [K*d]
+//   RC_MONO     row K prototypes,    query a [d] (gate Wq per query)
+//   RC_PCD_SRC  row K prototypes,    query e0 [d]
+//   RC_MONO_SRC row a [d] + gate [K] (Wq per row), query K prototypes
+constexpr int RC_PCD = 0, RC_MONO = 1, RC_PCD_SRC = 2, RC_MONO_SRC = 3;
+__host__ __device__ constexpr int rc_role(int mode) {
+  return mode == CFL_MONOMER ? RC_MONO : mode == CFL_PCD_SOURCE ? RC_PCD_SRC : mode == CFL_MONOMER_SOURCE ? RC_MONO_SRC
+                                                                                                          : RC_PCD;
+}
+__host__ __device__ constexpr int rc_row_floats(int role, int K, int d) {
+  return role == RC_PCD ? d : role == RC_MONO_SRC ? d + K : K * d;
+}
+__host__ __device__ constexpr int rc_query_floats(int role, int K, int d) {
+  return role == RC_MONO || role == RC_PCD_SRC ? d : K * d;
+}
 
 struct RcArgs {
   int mode, K, d, J;
   int64_t Q, N, ldq, lde;
-  const float* Pq;         // pcd: [Q, ldq] K prototypes per query; monomer: [Q, ldq] embedding a_q
-  const float* Wq;         // monomer: [Q, K]
-  const float* E;          // pcd: [N, lde] embeddings; monomer: [N, lde] K prototypes per row
+  const float* Pq;         // [Q, ldq] rc_query_floats per query (roles above)
+  const float* Wq;         // the monomer gate: [Q, K] (monomer), [N, K] (monomer_source)
+  const float* E;          // [N, lde] catalog rows (roles above; monomer_source: a, its gate in Wq)
   const float* thr;        // [Q, J] distances of the positives (NaN = no positive)
   const int64_t* pos_idx;  // [Q, J] gather kernel
   float* pos_dist;         // [Q, J] gather kernel output
@@ -97,6 +120,90 @@ __device__ __forceinline__ void pcd_direct4(const float* __restrict__ er, const 
   }
 }
 
+// The source roles: e = the query (four of them in q4), p = the row's K prototypes (er[k * d + j]) -- pcd_direct's
+// operation order with the swapped accessors.
+template <int K>
+__device__ __forceinline__ void pcd_src_direct4(const float* __restrict__ er, const float4* __restrict__ q4, int d,
+                                                float (&dist)[4]) {
+  float dk[4][K];
+  float mn[4] = {3.0e38f, 3.0e38f, 3.0e38f, 3.0e38f};
+#pragma unroll
+  for (int k = 0; k < K; ++k) {
+    float acc[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll 4
+    for (int j = 0; j < d; ++j) {
+      const float p = er[k * d + j];
+      const float4 e = q4[j * 2];
+      float df;
+      df = e.x - p; acc[0] = fmaf(df, df, acc[0]);
+      df = e.y - p; acc[1] = fmaf(df, df, acc[1]);
+      df = e.z - p; acc[2] = fmaf(df, df, acc[2]);
+      df = e.w - p; acc[3] = fmaf(df, df, acc[3]);
+    }
+#pragma unroll
+    for (int c = 0; c < 4; ++c) { dk[c][k] = acc[c]; mn[c] = fminf(mn[c], acc[c]); }
+  }
+  if (K == 1) {
+#pragma unroll
+    for (int c = 0; c < 4; ++c) dist[c] = dk[c][0];
+    return;
+  }
+  float inv[4];
+#pragma unroll
+  for (int c = 0; c < 4; ++c) {
+    float sum = 0.0f;
+#pragma unroll
+    for (int k = 0; k < K; ++k) { dk[c][k] = expf(mn[c] - dk[c][k]); sum += dk[c][k]; }
+    inv[c] = 1.0f / sum;
+    dist[c] = 0.0f;
+  }
+#pragma unroll 2
+  for (int j = 0; j < d; ++j) {
+    const float4 e = q4[j * 2];
+    float m[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+      const float p = er[k * d + j];
+      m[0] = fmaf(dk[0][k] * inv[0], p, m[0]);
+      m[1] = fmaf(dk[1][k] * inv[1], p, m[1]);
+      m[2] = fmaf(dk[2][k] * inv[2], p, m[2]);
+      m[3] = fmaf(dk[3][k] * inv[3], p, m[3]);
+    }
+    float r;
+    r = e.x - m[0]; dist[0] = fmaf(r, r, dist[0]);
+    r = e.y - m[1]; dist[1] = fmaf(r, r, dist[1]);
+    r = e.z - m[2]; dist[2] = fmaf(r, r, dist[2]);
+    r = e.w - m[3]; dist[3] = fmaf(r, r, dist[3]);
+  }
+}
+
+// monomer_source: the row is a (er[0, d)) and its gate (er[d, d + K)), the queries' K prototypes in q4 -- monomer_direct
+// with e = the query's prototypes, a / w = the row's.
+template <int K>
+__device__ __forceinline__ void monomer_src_direct4(const float* __restrict__ er, const float4* __restrict__ p4, int d,
+                                                    float (&dist)[4]) {
+  float acc[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll
+  for (int k = 0; k < K; ++k) {
+    float dk[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll 4
+    for (int j = 0; j < d; ++j) {
+      const float a = er[j];
+      const float4 p = p4[(k * d + j) * 2];
+      float df;
+      df = a + (-p.x); dk[0] = fmaf(df, df, dk[0]);
+      df = a + (-p.y); dk[1] = fmaf(df, df, dk[1]);
+      df = a + (-p.z); dk[2] = fmaf(df, df, dk[2]);
+      df = a + (-p.w); dk[3] = fmaf(df, df, dk[3]);
+    }
+    const float w = er[d + k];
+#pragma unroll
+    for (int c = 0; c < 4; ++c) acc[c] = fmaf(w, dk[c], acc[c]);
+  }
+#pragma unroll
+  for (int c = 0; c < 4; ++c) dist[c] = acc[c];
+}
+
 template <int K>
 __device__ __forceinline__ void monomer_direct4(const float* __restrict__ er, const float4* __restrict__ a4,
                                                 const float* __restrict__ w /* [4][K] */, int d, float (&dist)[4]) {
@@ -121,19 +228,21 @@ __device__ __forceinline__ void monomer_direct4(const float* __restrict__ er, co
   for (int c = 0; c < 4; ++c) dist[c] = acc[c];
 }
 
-// VW = floats per staging load (4 when the row length, the row stride and the base pointer allow 128-bit loads).
+// VW = floats per staging load (4 when the row length, the row stride and the base pointer allow 128-bit loads); VW = 0
+// (pcd_source when 128 rows of K*d floats do not fit shared memory): no staging, each thread reads its row in place
+// through L1, in the same order.
 // EMIT: instead of counting, the rows closer than the (single) threshold are appended to their query's segment -- one
 // ballot and one cursor atomic per (warp, query); with `only`, for the flagged queries alone.
-template <int K, bool MONO, int VW, bool EMIT>
+template <int K, int ROLE, int VW, bool EMIT>
 __device__ __forceinline__ void rank_count_body(const RcArgs& A, const RcEmit& X) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int d = A.d, J = A.J;
-  const int ew = MONO ? K * d : d;            // floats per catalog row
-  const int qw = MONO ? d : K * d;            // floats per query
+  const int ew = rc_row_floats(ROLE, K, d);   // floats per catalog row
+  const int qw = rc_query_floats(ROLE, K, d); // floats per query
   const int ldt = ew + 1;
   float4* q4 = (float4*)smem_raw;                             // [qw][2]: element i of queries 0-3 | 4-7 (zero padded)
-  float* et = (float*)(q4 + 2 * qw);                          // [128][ew+1]
-  float* ws = et + 128 * ldt;                                 // [QT][K] (monomer)
+  float* et = (float*)(q4 + 2 * qw);                          // [128][ew+1] (none when VW = 0)
+  float* ws = et + (VW == 0 ? 0 : 128 * ldt);                // [QT][K] (monomer)
   float* thr = ws + RC_QT * K;                                // [QT][J]
   int* cnt = (int*)(thr + RC_QT * J);                         // [4 warps][QT][J][2]
 
@@ -155,19 +264,19 @@ __device__ __forceinline__ void rank_count_body(const RcArgs& A, const RcEmit& X
     const int ql = i / qw, e = i % qw;
     ((float*)q4)[e * RC_QT + ql] = ql < nq ? A.Pq[(q0 + ql) * A.ldq + e] : 0.0f;
   }
-  if (MONO) for (int i = tid; i < RC_QT * K; i += RC_THREADS) ws[i] = i < nq * K ? A.Wq[q0 * K + i] : 0.0f;
+  if (ROLE == RC_MONO) for (int i = tid; i < RC_QT * K; i += RC_THREADS) ws[i] = i < nq * K ? A.Wq[q0 * K + i] : 0.0f;
   for (int i = tid; i < nq * J; i += RC_THREADS) thr[i] = A.thr[q0 * J + i];
   for (int i = tid; i < (RC_THREADS / 32) * RC_QT * J * 2; i += RC_THREADS) cnt[i] = 0;
   int* mycnt = cnt + wid * RC_QT * J * 2;
   const int64_t t0 = A.tiles * part / A.parts;
   const int64_t t1 = A.tiles * (part + 1) / A.parts;
-  const int dv = ew / VW;
+  const int dv = (ROLE == RC_MONO_SRC ? d : ew) / (VW > 0 ? VW : 1);   // staging loads per row from E
   const int sr0 = tid / dv, sj0 = tid % dv, sdr = RC_THREADS / dv, sdj = RC_THREADS % dv;
 
   for (int64_t tile = t0; tile < t1; ++tile) {
     const int64_t r0 = tile * 128;
     __syncthreads();
-    for (int i = tid, r = sr0, j = sj0; i < 128 * dv; i += RC_THREADS) {
+    for (int i = tid, r = sr0, j = sj0; VW > 0 && i < 128 * dv; i += RC_THREADS) {
       const int64_t row = r0 + r;
       const float* src = A.E + row * A.lde + VW * j;
       float* dst = et + r * ldt + VW * j;
@@ -180,13 +289,20 @@ __device__ __forceinline__ void rank_count_body(const RcArgs& A, const RcEmit& X
       r += sdr; j += sdj;
       if (j >= dv) { j -= dv; ++r; }
     }
+    if (ROLE == RC_MONO_SRC)                                   // the row's gate behind its a
+      for (int i = tid; i < 128 * K; i += RC_THREADS) {
+        const int64_t row = r0 + i / K;
+        et[(i / K) * ldt + d + i % K] = row < A.N ? A.Wq[row * K + i % K] : 0.0f;
+      }
     __syncthreads();
     const bool valid = r0 + tid < A.N;
-    const float* er = et + tid * ldt;
+    const float* er = VW > 0 ? et + tid * ldt : A.E + (valid ? r0 + tid : 0) * A.lde;
     for (int qh = 0; qh * 4 < nq; ++qh) {
       float dist[4];
-      if (MONO) monomer_direct4<K>(er, q4 + qh, ws + qh * 4 * K, d, dist);
-      else      pcd_direct4<K>(er, q4 + qh, d, dist);
+      if (ROLE == RC_MONO)          monomer_direct4<K>(er, q4 + qh, ws + qh * 4 * K, d, dist);
+      else if (ROLE == RC_PCD_SRC)  pcd_src_direct4<K>(er, q4 + qh, d, dist);
+      else if (ROLE == RC_MONO_SRC) monomer_src_direct4<K>(er, q4 + qh, d, dist);
+      else                          pcd_direct4<K>(er, q4 + qh, d, dist);
 #pragma unroll
       for (int c = 0; c < 4; ++c) {
         const int ql = qh * 4 + c;
@@ -233,18 +349,31 @@ __device__ __forceinline__ void rank_count_body(const RcArgs& A, const RcEmit& X
 template <int K, bool MONO, int VW>
 __global__ void __launch_bounds__(RC_THREADS)
 rank_count_kernel(RcArgs A) {
-  rank_count_body<K, MONO, VW, false>(A, RcEmit{});
+  rank_count_body<K, MONO ? RC_MONO : RC_PCD, VW, false>(A, RcEmit{});
 }
 
 template <int K, bool MONO, int VW>
 __global__ void __launch_bounds__(RC_THREADS)
 within_emit_kernel(RcArgs A, RcEmit X) {
-  rank_count_body<K, MONO, VW, true>(A, X);
+  rank_count_body<K, MONO ? RC_MONO : RC_PCD, VW, true>(A, X);
+}
+
+// the source modes (MONO: monomer_source, else pcd_source)
+template <int K, bool MONO, int VW>
+__global__ void __launch_bounds__(RC_THREADS)
+rank_count_src_kernel(RcArgs A) {
+  rank_count_body<K, MONO ? RC_MONO_SRC : RC_PCD_SRC, VW, false>(A, RcEmit{});
+}
+
+template <int K, bool MONO, int VW>
+__global__ void __launch_bounds__(RC_THREADS)
+within_emit_src_kernel(RcArgs A, RcEmit X) {
+  rank_count_body<K, MONO ? RC_MONO_SRC : RC_PCD_SRC, VW, true>(A, X);
 }
 
 // One thread per (query, positive): the same device functions on rows gathered from global memory.
-template <int K, bool MONO>
-__global__ void pair_dist_rows_kernel(RcArgs A) {
+template <int K, int ROLE>
+__device__ __forceinline__ void dist_rows_body(const RcArgs& A) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= A.Q * A.J) return;
   const int64_t q = i / A.J;
@@ -254,15 +383,31 @@ __global__ void pair_dist_rows_kernel(RcArgs A) {
     const float* er = A.E + row * A.lde;
     const float* qv = A.Pq + q * A.ldq;
     const int d = A.d;
-    if (MONO) {
+    if (ROLE == RC_MONO) {
       const float* wv = A.Wq + q * K;
       dist = monomer_direct<K>([&](int k, int j) { return er[k * d + j]; }, [&](int j) { return qv[j]; },
+                               [&](int k) { return wv[k]; }, d);
+    } else if (ROLE == RC_PCD_SRC) {
+      dist = pcd_direct<K>([&](int j) { return qv[j]; }, [&](int k, int j) { return er[k * d + j]; }, d);
+    } else if (ROLE == RC_MONO_SRC) {
+      const float* wv = A.Wq + row * K;
+      dist = monomer_direct<K>([&](int k, int j) { return qv[k * d + j]; }, [&](int j) { return er[j]; },
                                [&](int k) { return wv[k]; }, d);
     } else {
       dist = pcd_direct<K>([&](int j) { return er[j]; }, [&](int k, int j) { return qv[k * d + j]; }, d);
     }
   }
   A.pos_dist[i] = dist;
+}
+
+template <int K, bool MONO>
+__global__ void pair_dist_rows_kernel(RcArgs A) {
+  dist_rows_body<K, MONO ? RC_MONO : RC_PCD>(A);
+}
+
+template <int K, bool MONO>
+__global__ void source_dist_rows_kernel(RcArgs A) {
+  dist_rows_body<K, MONO ? RC_MONO_SRC : RC_PCD_SRC>(A);
 }
 
 // Counts over a DENSE distance matrix (the tensor-core route: cfl_score_topk's dist_out holds the Gram-form
@@ -304,23 +449,39 @@ dense_rank_count_kernel(const float* __restrict__ dense, int64_t N, int64_t ldn,
   if (t < 2 * J && sc[t]) atomicAdd(&counts[q * J * 2 + t], (unsigned long long)sc[t]);
 }
 
-static size_t rc_smem_bytes(int K, int d, int J, bool mono) {
-  const int ew = mono ? K * d : d, qw = mono ? d : K * d;
-  return (size_t)RC_QT * qw * 4 + (size_t)128 * (ew + 1) * 4 + (size_t)RC_QT * K * 4 + (size_t)RC_QT * J * 4 +
-         (size_t)(RC_THREADS / 32) * RC_QT * J * 2 * 4;
+static size_t rc_smem_bytes(int K, int d, int J, int role, bool staged = true) {
+  const int ew = rc_row_floats(role, K, d), qw = rc_query_floats(role, K, d);
+  return (size_t)RC_QT * qw * 4 + (staged ? (size_t)128 * (ew + 1) * 4 : 0) + (size_t)RC_QT * K * 4 +
+         (size_t)RC_QT * J * 4 + (size_t)(RC_THREADS / 32) * RC_QT * J * 2 * 4;
 }
 
-template <int K, bool MONO>
+template <int K, bool MONO, bool SRC>
 static int rc_launch(const RcArgs& a, bool gather, const RcEmit* emit, cudaStream_t cs) {
+  constexpr int role = SRC ? (MONO ? RC_MONO_SRC : RC_PCD_SRC) : (MONO ? RC_MONO : RC_PCD);
   if (gather) {
     const int64_t n = a.Q * a.J;
-    pair_dist_rows_kernel<K, MONO><<<(unsigned)((n + 127) / 128), 128, 0, cs>>>(a);
+    if (SRC) source_dist_rows_kernel<K, MONO><<<(unsigned)((n + 127) / 128), 128, 0, cs>>>(a);
+    else pair_dist_rows_kernel<K, MONO><<<(unsigned)((n + 127) / 128), 128, 0, cs>>>(a);
   } else {
-    const size_t smem = rc_smem_bytes(K, a.d, a.J, MONO);
-    const int ew = MONO ? K * a.d : a.d;
-    const bool v4 = ew % 4 == 0 && a.lde % 4 == 0 && ((uintptr_t)a.E & 15u) == 0;
-    auto kern = v4 ? rank_count_kernel<K, MONO, 4> : rank_count_kernel<K, MONO, 1>;
-    auto ekern = v4 ? within_emit_kernel<K, MONO, 4> : within_emit_kernel<K, MONO, 1>;
+    // pcd_source rows of K*d floats: staged while 128 of them fit, read in place beyond (VW = 0)
+    const bool staged = rc_smem_bytes(K, a.d, a.J, role) <= RC_SMEM_MAX;
+    const size_t smem = rc_smem_bytes(K, a.d, a.J, role, staged);
+    const int ea = role == RC_MONO_SRC ? a.d : rc_row_floats(role, K, a.d);
+    const bool v4 = ea % 4 == 0 && a.lde % 4 == 0 && ((uintptr_t)a.E & 15u) == 0;
+    void (*kern)(RcArgs);
+    void (*ekern)(RcArgs, RcEmit);
+    if constexpr (!SRC) {
+      kern = v4 ? rank_count_kernel<K, MONO, 4> : rank_count_kernel<K, MONO, 1>;
+      ekern = v4 ? within_emit_kernel<K, MONO, 4> : within_emit_kernel<K, MONO, 1>;
+    } else if constexpr (MONO) {                               // d + K floats per row: always staged
+      kern = v4 ? rank_count_src_kernel<K, true, 4> : rank_count_src_kernel<K, true, 1>;
+      ekern = v4 ? within_emit_src_kernel<K, true, 4> : within_emit_src_kernel<K, true, 1>;
+    } else {
+      kern = !staged ? rank_count_src_kernel<K, false, 0>
+                     : v4 ? rank_count_src_kernel<K, false, 4> : rank_count_src_kernel<K, false, 1>;
+      ekern = !staged ? within_emit_src_kernel<K, false, 0>
+                      : v4 ? within_emit_src_kernel<K, false, 4> : within_emit_src_kernel<K, false, 1>;
+    }
     // one wave: as many catalog parts as keep every CTA resident at once (only resident warps hide the
     // shared-memory latency; a partial second wave idles most SMs)
     int resident = 0;
@@ -349,9 +510,15 @@ static int rc_launch(const RcArgs& a, bool gather, const RcEmit* emit, cudaStrea
 }
 
 static int rc_dispatch(const RcArgs& a, bool gather, cudaStream_t cs, const RcEmit* emit = nullptr) {
-  const bool mono = a.mode == CFL_MONOMER;
-#define CFL_RC_CASE(KK) \
-  case KK: return mono ? rc_launch<KK, true>(a, gather, emit, cs) : rc_launch<KK, false>(a, gather, emit, cs);
+  const int role = rc_role(a.mode);
+#define CFL_RC_CASE(KK)                                                       \
+  case KK:                                                                    \
+    switch (role) {                                                           \
+      case RC_MONO: return rc_launch<KK, true, false>(a, gather, emit, cs);   \
+      case RC_PCD_SRC: return rc_launch<KK, false, true>(a, gather, emit, cs); \
+      case RC_MONO_SRC: return rc_launch<KK, true, true>(a, gather, emit, cs); \
+      default: return rc_launch<KK, false, false>(a, gather, emit, cs);       \
+    }
   switch (a.K) {
     CFL_RC_CASE(1) CFL_RC_CASE(2) CFL_RC_CASE(3) CFL_RC_CASE(4)
     CFL_RC_CASE(5) CFL_RC_CASE(6) CFL_RC_CASE(7) CFL_RC_CASE(8)
@@ -362,19 +529,19 @@ static int rc_dispatch(const RcArgs& a, bool gather, cudaStream_t cs, const RcEm
 
 static int rc_check(const char* what, int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* Wq,
                     const float* E, int64_t N, int64_t lde, int J) {
-  CFL_REQUIRE(mode == CFL_PCD || mode == CFL_SIAMESE || mode == CFL_MONOMER, CFL_ERR_INVALID, "%s: bad mode %d", what, mode);
+  CFL_REQUIRE(mode >= CFL_PCD && mode <= CFL_MONOMER_SOURCE, CFL_ERR_INVALID, "%s: bad mode %d", what, mode);
   CFL_REQUIRE(mode != CFL_SIAMESE || K == 1, CFL_ERR_INVALID, "%s: siamese needs K=1", what);
   CFL_REQUIRE(K >= 1 && K <= CFL_MAX_K, CFL_ERR_UNSUPPORTED, "%s: K=%d outside [1,%d]", what, K, CFL_MAX_K);
   CFL_REQUIRE(d >= 1 && d <= 128, CFL_ERR_UNSUPPORTED, "%s: d=%d outside [1,128]", what, d);
   CFL_REQUIRE(J >= 1 && J <= RC_MAX_J, CFL_ERR_UNSUPPORTED, "%s: J=%d outside [1,%d]", what, J, RC_MAX_J);
   CFL_REQUIRE(Q >= 0 && N >= 0, CFL_ERR_INVALID, "%s: bad Q/N", what);
-  const bool mono = mode == CFL_MONOMER;
-  CFL_REQUIRE(ldq >= (mono ? d : (int64_t)K * d) && lde >= (mono ? (int64_t)K * d : d), CFL_ERR_INVALID,
-              "%s: leading dimension too small", what);
-  CFL_REQUIRE(Q == 0 || (Pq && (!mono || Wq)), CFL_ERR_INVALID, "%s: NULL query argument", what);
-  CFL_REQUIRE(Q == 0 || N == 0 || E, CFL_ERR_INVALID, "%s: NULL catalog", what);
+  const int role = rc_role(mode);
+  const int64_t ldq_min = rc_query_floats(role, K, d), lde_min = role == RC_MONO_SRC ? d : rc_row_floats(role, K, d);
+  CFL_REQUIRE(ldq >= ldq_min && lde >= lde_min, CFL_ERR_INVALID, "%s: leading dimension too small", what);
+  CFL_REQUIRE(Q == 0 || (Pq && (role != RC_MONO || Wq)), CFL_ERR_INVALID, "%s: NULL query argument", what);
+  CFL_REQUIRE(Q == 0 || N == 0 || (E && (role != RC_MONO_SRC || Wq)), CFL_ERR_INVALID, "%s: NULL catalog", what);
   // the tile of a monomer catalog (K*d floats per row) must fit the shared memory of one CTA
-  CFL_REQUIRE(rc_smem_bytes(K, d, J, mono) <= 200 * 1024, CFL_ERR_UNSUPPORTED,
+  CFL_REQUIRE(role != RC_MONO || rc_smem_bytes(K, d, J, role) <= RC_SMEM_MAX, CFL_ERR_UNSUPPORTED,
               "%s: K*d = %d too large for the monomer rank-count tile", what, K * d);
   return CFL_OK;
 }

@@ -22,6 +22,14 @@
 // maximum of |D~ - direct| / m over all ambiguous records; rank_fix_kernel reports it in the call's statistics and
 // tests/test_rank_counts.py asserts the headroom).  A query whose records do not fit the list is recounted from
 // scratch by the CUDA-core kernel (rank_count_kernel, restricted by `only`).
+//
+// SRC (pcd_source: rank_count_src_umma_kernel / within_emit_src_umma_kernel, the fix kernels rank_fix_src_kernel /
+// within_fix_src_kernel): the pipeline of score_src_umma_kernel -- the catalog rows are SOURCE items with K prototype
+// planes (cfl_source_catalog_pack), the queries TARGET embeddings (one vector each, a query image packed with K = 1).
+// The row's soft-min block is broadcast to each query pair, |e_q - mu|^2 is per query, and the band takes
+// S = |e_q - mu|^2 + max_k |p_ck - mu|^2 (the row's first K block entries).  There is no skip test: the affine hull
+// belongs to the row, not to the query.  The records are checked with pcd_direct(e = query row, p = catalog row), the
+// values cfl_score_topk_source reports.
 #include "gram_pipe.cuh"
 #include <stdlib.h>
 #include "direct.cuh"
@@ -35,8 +43,10 @@ constexpr int RT_QT_MAX = 64;
 constexpr float RT_REL1_DEFAULT = 1.0f / 262144.0f;     // 2^-18: Gram-form (3xTF32) + direct-form rounding, relative to S
 constexpr float RT_REL2_DEFAULT = 1.0f / 2097152.0f;    // 2^-21: exponent error relative to S (sensitivity term)
 
-int rank_tc_qt(int K, int d) {
-  int qt = score_umma_qt(K, d);
+// query tile: <= RT_QT_MAX and, with the query groups of gram_gq(K), at most NGW groups per epilogue warp (rank_umma_body);
+// the source tile also keeps K*qt <= 256 TMEM columns per accumulator buffer (score_src_qt)
+int rank_tc_qt(int K, int d, bool src = false) {
+  int qt = src ? score_src_qt(K, d) : score_umma_qt(K, d);
   return qt > RT_QT_MAX ? RT_QT_MAX : qt;
 }
 
@@ -45,11 +55,11 @@ struct RtArgs {
   int64_t Q, N;
   int qt, nqt, parts, dpad;
   int64_t tiles;
-  const float* qpar;
-  const float* qplane;            // per query: affine-hull bound block (score.cuh)
+  const float* qpar;              // per query: soft-min block (SRC: |e_q - mu|^2)
+  const float* qplane;            // per query: affine-hull bound block (score.cuh); SRC: unused
   const void* qimg;
   const void* cimg;
-  const float* e2;
+  const float* e2;                // per row: |e - mu|^2; SRC: the rows' soft-min blocks (source_catalog_view().rowpar)
   const float* thr;               // [Q, J]
   unsigned long long* counts;     // [Q, J, 2]
   uint4* recs;                    // ambiguous (query, row) records
@@ -66,9 +76,10 @@ struct RtArgs {
 // Shared memory of the counting / emitting kernels: the Gram pipeline's regions and, behind the query blocks, the
 // epilogue's thresholds, max_k |p_k|^2, skip-test constants per query, per-threshold counts and records written.
 struct RtLayout { GramLayout g; uint32_t thr, qm, skp, cs, rcn; };
+template <bool SRC = false>
 __host__ __device__ inline RtLayout rt_layout(int K, int qt, int dpad) {
   RtLayout L;
-  L.g = gram_layout(K, qt, dpad, 0u);
+  L.g = gram_layout<SRC>(K, qt, dpad, 0u);
   uint32_t off = L.g.back;
   L.thr = off;     off += (uint32_t)qt * RT_JC * 4u;
   L.qm = off;      off += (uint32_t)qt * 4u;                           off = (off + 15u) & ~15u;
@@ -97,14 +108,18 @@ __device__ __forceinline__ float sqrt_approx(float x) {
 // thresholds) and the emitting kernel of cfl_score_within (EMIT = true, J = 1: a pair with D~ < t - m is appended to its
 // query's result segment at once, a pair inside the band goes to the record list exactly as for the counts).  Both
 // instantiations classify with the same arithmetic, so the emitted set and the count of the same radius agree pair for pair.
-template <int K, bool EMIT>
+template <int K, bool SRC, bool EMIT>
 __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
   extern __shared__ __align__(1024) unsigned char smem[];
-  constexpr int GQ = gram_gq(K);
-  constexpr int NGW = K <= 2 ? 1 : (K <= 4 ? 2 : 3);     // query groups per warp: ceil((qt / GQ) / GP_WPQ), qt <= 64 (48 at K = 5)
+  // SRC at K <= 2 (qt = 64): smaller query groups where 16 needs local memory (-Xptxas -v): 4 (count) / 16 (emit) at
+  // K = 1, 8 at K = 2
+  constexpr int GQ = SRC && K <= 2 ? (K == 1 ? (EMIT ? 16 : 4) : 8) : gram_gq(K);
+  // query groups per warp: ceil((qt / GQ) / GP_WPQ), qt <= 64 (48 at K = 5)
+  constexpr int NGW = SRC && K <= 2 ? 16 / GQ : K <= 2 ? 1 : (K <= 4 ? 2 : 3);
   constexpr int QPS = qpar_stride(K);
+  constexpr int NRP = source_rowpar_len(K);
   const int QT = A.qt;
-  const RtLayout L = rt_layout(K, QT, A.dpad);
+  const RtLayout L = rt_layout<SRC>(K, QT, A.dpad);
   const GramPipe P = gram_pipe(smem, L.g, K, QT, A.dpad);
   float* thr = (float*)(smem + L.thr);
   float* qm = (float*)(smem + L.qm);
@@ -121,7 +136,12 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
   const int ntiles = (int)(t1 - t0);
   const int jn = (A.J - A.j0 < RT_JC) ? (A.J - A.j0) : RT_JC;
 
-  gram_setup<K>(P, A.qpar, A.qplane, q0, nq, QT);
+  if constexpr (SRC) {
+    gram_init(P);
+    for (int i = tid; i < QT; i += GP_THREADS) P.qpar[i] = (i < nq) ? A.qpar[q0 + i] : 0.0f;     // |e_q - mu|^2
+  } else {
+    gram_setup<K>(P, A.qpar, A.qplane, q0, nq, QT);
+  }
   // thresholds: NaN (no positive in the slot), padding slots and padding queries become -inf = "count nothing"
   for (int i = tid; i < QT * RT_JC; i += GP_THREADS) {
     const int ql = i / RT_JC, j = i % RT_JC;
@@ -133,7 +153,7 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
     thr[i] = t;
     cs[i] = 0u;
   }
-  for (int ql = tid; ql < QT; ql += GP_THREADS) {
+  for (int ql = tid; ql < QT && !SRC; ql += GP_THREADS) {   // SRC: the prototypes belong to the row
     float pm = 0.0f;
     if (ql < nq)
       for (int k = 0; k < K; ++k) pm = fmaxf(pm, A.qpar[(q0 + ql) * QPS + k]);      // log2(e) |p_k|^2
@@ -143,7 +163,7 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
   //   D~ - m(D~) >= LB - S (rel1 + rel2 sqrt(LB Vq)) >= LB (1 - S k1) - S k0   (AM-GM with c = sqrt(Vq / tmax)),
   // k0 = rel1 + rel2 Vq / (2c), k1 = rel2 c / 2: when that exceeds the query's largest threshold the pair is farther than
   // every threshold and outside every band -- nothing to count, nothing to record.
-  for (int ql = tid; ql < QT; ql += GP_THREADS) {
+  for (int ql = tid; ql < QT && !SRC; ql += GP_THREADS) {
     float tmax = __int_as_float(0xff800000);
     float k0 = A.rel1, k1 = 0.0f;
     if (ql < nq) {
@@ -168,9 +188,9 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
   const uint32_t tmem_base = gram_start(P);
 
   if (warp == GP_NEPI) {
-    gram_mma(P, tmem_base, ntiles);
+    gram_mma<SRC ? K : 1>(P, tmem_base, ntiles);
   } else if (warp == GP_NEPI + 1) {
-    gram_tma(P, A.qimg, qtile, A.cimg, t0, 1, ntiles);
+    gram_tma<SRC ? K : 1>(P, A.qimg, qtile, A.cimg, t0, 1, ntiles);
   } else {
     // ======================================= epilogue ========================================
     const int lq = warp & 3, sub = warp >> 2;
@@ -212,12 +232,16 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
     int since_flush = 0;
     // the skip test pays when most groups are far from every threshold (labelled positives near the top of the ranking:
     // the usual evaluation); each warp measures its hit rate over the first 16 tiles and switches the test off otherwise
-    bool bound_on = true;
+    bool bound_on = !SRC;
     int grp_seen = 0, grp_skipped = 0;
     for (int t = 0; t < ntiles; ++t) {
       const int64_t row = (t0 + t) * 128 + lrow;
       const bool valid = row < A.N;
-      const float e2 = __ldg(A.e2 + row);                    // padded to whole tiles
+      float e2 = 0.0f;
+      // SRC: the row's soft-min block, read where it is used, per query pair (L1 hits after the first); held in registers
+      // across the TMEM loads and the group loop it pushed the counting kernel into local memory
+      const float* rp = A.e2 + (t0 + t) * 128 * NRP + lrow;
+      if constexpr (!SRC) e2 = __ldg(A.e2 + row);            // padded to whole tiles
       const uint32_t taddr = gram_acquire(P, tmem_base, t, lq);
 #pragma unroll
       for (int gi = 0; gi < NGW; ++gi) {
@@ -225,7 +249,7 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
         if (g * GQ >= nq) continue;                           // warp-uniform
         float gk[K][GQ];
         gram_load_group<K, GQ>(taddr, QT, g, gk);
-        if (bound_on) {
+        if (!SRC && bound_on) {
           constexpr int PBS = qplane_stride(K);
           const float e2s = e2 * (1.0f - CFL_PLANE_REL);
           const f2_t e2sp = pk2(e2s, e2s);
@@ -253,19 +277,36 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
         float dist[GQ], var[GQ];
 #pragma unroll
         for (int pi = 0; pi < GQ / 2; ++pi) {
-          f2_t qv[QPS];
-          load_pair_block<QPS>(qg + pi * QPS * 2, qv);
           float gA[K], gB[K];
 #pragma unroll
           for (int k = 0; k < K; ++k) { gA[k] = gk[k][2 * pi]; gB[k] = gk[k][2 * pi + 1]; }
-          softmin_pair_var<K>(gA, gB, e2, qv, dist[2 * pi], dist[2 * pi + 1], var[2 * pi], var[2 * pi + 1]);
+          if constexpr (SRC) {
+            const f2_t e2q = *(const f2_t*)(P.qpar + g * GQ + 2 * pi);
+            f2_t rq[NRP];                                     // the row's block broadcast to the query pair
+#pragma unroll
+            for (int j = 0; j < NRP; ++j) {
+              const float v = __ldg(rp + j * 128);
+              rq[j] = (j < K) ? pk2(-v, -v) : pk2(v, v);
+            }
+            softmin_pair_var<K>(gA, gB, e2q, rq, dist[2 * pi], dist[2 * pi + 1], var[2 * pi], var[2 * pi + 1]);
+          } else {
+            f2_t qv[QPS];
+            load_pair_block<QPS>(qg + pi * QPS * 2, qv);
+            softmin_pair_var<K>(gA, gB, pk2(e2, e2), qv, dist[2 * pi], dist[2 * pi + 1], var[2 * pi], var[2 * pi + 1]);
+          }
+        }
+        float pm = 0.0f;                                     // SRC: max_k |p_k|^2 of the row
+        if constexpr (SRC) {
+#pragma unroll
+          for (int k = 0; k < K; ++k) pm = fmaxf(pm, __ldg(rp + k * 128));      // log2(e) |p_k|^2
+          pm *= CFL_LN2;
         }
         uint32_t amb = 0u, sure = 0u;
 #pragma unroll
         for (int i = 0; i < GQ; ++i) {
           const int ql = g * GQ + i;
           // band m = S * (rel1 + rel2 * sqrt(D~ * V)); var[] keeps it for the record
-          const float S = e2 + qm[ql];
+          const float S = SRC ? P.qpar[ql] + pm : e2 + qm[ql];
           const float sens = K == 1 ? 0.0f : sqrt_approx(fmaxf(dist[i], 0.0f) * fmaxf(var[i], 0.0f));
           const float m = S * fmaf(A.rel2, sens, A.rel1);
           var[i] = m;
@@ -357,14 +398,27 @@ __device__ __forceinline__ void rank_umma_body(const RtArgs& A) {
 template <int K>
 __global__ void __launch_bounds__(GP_THREADS, 1)     // 18 warps = 5 on one sub-partition: 5 x 32 x 96 registers is its whole file
 rank_count_umma_kernel(RtArgs A) {
-  rank_umma_body<K, false>(A);
+  rank_umma_body<K, false, false>(A);
 }
 
 // cfl_score_within's emitting pass (J = 1: A.thr = the radii)
 template <int K>
 __global__ void __launch_bounds__(GP_THREADS, 1)
 within_emit_umma_kernel(RtArgs A) {
-  rank_umma_body<K, true>(A);
+  rank_umma_body<K, false, true>(A);
+}
+
+// the same two passes over a source catalog (pcd_source)
+template <int K>
+__global__ void __launch_bounds__(GP_THREADS, 1)
+rank_count_src_umma_kernel(RtArgs A) {
+  rank_umma_body<K, true, false>(A);
+}
+
+template <int K>
+__global__ void __launch_bounds__(GP_THREADS, 1)
+within_emit_src_umma_kernel(RtArgs A) {
+  rank_umma_body<K, true, true>(A);
 }
 
 // Exact verdicts of the ambiguous pairs: one thread per record, the direct-form device function of direct.cuh on the raw
@@ -374,8 +428,9 @@ within_emit_umma_kernel(RtArgs A) {
 constexpr int FX_THREADS = 128;
 constexpr int FX_BLOCKS = 4;                        // blocks per list slice
 // EMIT (cfl_score_within, J = 1): a record whose direct-form distance is below the radius is appended to its query's
-// segment instead of correcting a count.
-template <int K, bool EMIT>
+// segment instead of correcting a count.  SRC: the query tile holds one vector per query and each record's K*d-float
+// row is read in place (128 of them would not fit shared memory at K*d = 1024).
+template <int K, bool SRC, bool EMIT>
 __device__ __forceinline__ void
 rank_fix_body(const uint4* __restrict__ recs_all, const unsigned int* __restrict__ rec_n, unsigned int slice,
               const float* __restrict__ Pq, int64_t ldq, const float* __restrict__ E, int64_t lde, int64_t N, int64_t Q,
@@ -387,9 +442,9 @@ rank_fix_body(const uint4* __restrict__ recs_all, const unsigned int* __restrict
   if (n == 0 || (unsigned int)blockIdx.x * FX_THREADS >= n) return;
   const uint4* recs = recs_all + (size_t)blockIdx.y * slice;
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  const int KD = K * d, ldp = KD + 1, lder = d + 1;
-  float* pq = fx_smem;                                       // [qt][K*d + 1]: the slice's query tile
-  float* er = pq + (size_t)qt * ldp;                         // [FX_THREADS][d + 1]: one catalog row per thread
+  const int KD = SRC ? d : K * d, ldp = KD + 1, lder = d + 1;
+  float* pq = fx_smem;                                       // [qt][K*d + 1]: the slice's query tile (SRC: [qt][d + 1])
+  float* er = pq + (size_t)qt * ldp;                         // [FX_THREADS][d + 1]: one catalog row per thread (not SRC)
   const int64_t q0 = (int64_t)(blockIdx.y / parts) * qt;     // CTA (part, qtile) of the scoring kernel = qtile * parts + part
   const int nq = (int)((Q - q0 < qt) ? (Q - q0) : qt);
   for (int i = tid; i < nq * KD; i += FX_THREADS) {
@@ -405,6 +460,7 @@ rank_fix_body(const uint4* __restrict__ recs_all, const unsigned int* __restrict
     const int64_t q = r.x, row = r.y;
     const bool live = have && !only[q] && row < N;
     // the warp gathers its 32 rows with coalesced loads; every thread then walks its own row in shared memory
+    if constexpr (!SRC) {
     __syncwarp();
     for (int rr = 0; rr < 32; ++rr) {
       const int64_t rw = __shfl_sync(0xffffffffu, (unsigned int)r.y, rr);
@@ -414,10 +470,17 @@ rank_fix_body(const uint4* __restrict__ recs_all, const unsigned int* __restrict
       for (int j = lane; j < d; j += 32) dst[j] = E[rw * lde + j];
     }
     __syncwarp();
+    }
     if (!live) continue;
-    const float* ev = er + tid * lder;
     const float* qv = pq + (int)(q - q0) * ldp;
-    const float dist = pcd_direct<K>([&](int j) { return ev[j]; }, [&](int k, int j) { return qv[k * d + j]; }, d);
+    float dist;
+    if constexpr (SRC) {
+      const float* pr = E + row * lde;
+      dist = pcd_direct<K, 1>([&](int j) { return qv[j]; }, [&](int k, int j) { return __ldg(pr + k * d + j); }, d);
+    } else {
+      const float* ev = er + tid * lder;
+      dist = pcd_direct<K>([&](int j) { return ev[j]; }, [&](int k, int j) { return qv[k * d + j]; }, d);
+    }
     const float Dg = __uint_as_float(r.z), m = __uint_as_float(r.w);
     if constexpr (EMIT) {
       if (dist < thr[q]) {                                   // every record of a J = 1 pass lies inside its band
@@ -456,8 +519,19 @@ rank_fix_kernel(const uint4* __restrict__ recs_all, const unsigned int* __restri
                 const float* __restrict__ Pq, int64_t ldq, const float* __restrict__ E, int64_t lde, int64_t N, int64_t Q,
                 int d, int qt, int parts, const float* __restrict__ thr, int J, int j0, const int* __restrict__ only,
                 unsigned long long* __restrict__ counts, unsigned long long* __restrict__ stats) {
-  rank_fix_body<K, false>(recs_all, rec_n, slice, Pq, ldq, E, lde, N, Q, d, qt, parts, thr, J, j0, only, counts, stats,
-                          nullptr, nullptr, nullptr);
+  rank_fix_body<K, false, false>(recs_all, rec_n, slice, Pq, ldq, E, lde, N, Q, d, qt, parts, thr, J, j0, only, counts,
+                                 stats, nullptr, nullptr, nullptr);
+}
+
+template <int K>
+__global__ void __launch_bounds__(FX_THREADS)
+rank_fix_src_kernel(const uint4* __restrict__ recs_all, const unsigned int* __restrict__ rec_n, unsigned int slice,
+                    const float* __restrict__ Pq, int64_t ldq, const float* __restrict__ E, int64_t lde, int64_t N,
+                    int64_t Q, int d, int qt, int parts, const float* __restrict__ thr, int J, int j0,
+                    const int* __restrict__ only, unsigned long long* __restrict__ counts,
+                    unsigned long long* __restrict__ stats) {
+  rank_fix_body<K, true, false>(recs_all, rec_n, slice, Pq, ldq, E, lde, N, Q, d, qt, parts, thr, J, j0, only, counts,
+                                stats, nullptr, nullptr, nullptr);
 }
 
 template <int K>
@@ -467,8 +541,19 @@ within_fix_kernel(const uint4* __restrict__ recs_all, const unsigned int* __rest
                   int64_t Q, int d, int qt, int parts, const float* __restrict__ radius, const int* __restrict__ only,
                   unsigned long long* __restrict__ stats, const int64_t* __restrict__ offsets,
                   unsigned int* __restrict__ cursor, int64_t* __restrict__ out) {
-  rank_fix_body<K, true>(recs_all, rec_n, slice, Pq, ldq, E, lde, N, Q, d, qt, parts, radius, 1, 0, only, nullptr, stats,
-                         offsets, cursor, out);
+  rank_fix_body<K, false, true>(recs_all, rec_n, slice, Pq, ldq, E, lde, N, Q, d, qt, parts, radius, 1, 0, only, nullptr,
+                                stats, offsets, cursor, out);
+}
+
+template <int K>
+__global__ void __launch_bounds__(FX_THREADS)
+within_fix_src_kernel(const uint4* __restrict__ recs_all, const unsigned int* __restrict__ rec_n, unsigned int slice,
+                      const float* __restrict__ Pq, int64_t ldq, const float* __restrict__ E, int64_t lde, int64_t N,
+                      int64_t Q, int d, int qt, int parts, const float* __restrict__ radius, const int* __restrict__ only,
+                      unsigned long long* __restrict__ stats, const int64_t* __restrict__ offsets,
+                      unsigned int* __restrict__ cursor, int64_t* __restrict__ out) {
+  rank_fix_body<K, true, true>(recs_all, rec_n, slice, Pq, ldq, E, lde, N, Q, d, qt, parts, radius, 1, 0, only, nullptr,
+                               stats, offsets, cursor, out);
 }
 
 // queries whose records were dropped are recounted from scratch: clear what the fast path added
@@ -502,8 +587,10 @@ static unsigned int rank_tc_rec_cap(int64_t Q, int64_t N) {
   return (unsigned int)cap;
 }
 
+// SRC: the forward layout, so that cfl_rank_counts_packed_stats finds the statistics at the same offset; the source query
+// regions (centred query vectors, |e_q - mu|^2, the query image of one vector per query) reuse the forward ones.
 struct RtWs { size_t pc, qpar, qimg, recs, recn, only, stats, total; };
-static RtWs rank_tc_ws(int64_t Q, int K, int d, int64_t N) {
+static RtWs rank_tc_ws(int64_t Q, int K, int d, int64_t N, bool src = false) {
   RtWs w;
   const int qt = rank_tc_qt(K, d);
   const int nqt = qt > 0 ? (int)((Q + qt - 1) / qt) : 0;
@@ -516,21 +603,37 @@ static RtWs rank_tc_ws(int64_t Q, int K, int d, int64_t N) {
   w.recn = off;  off = align_up(off + 4096 * sizeof(unsigned int), 256);
   w.only = off;  off = align_up(off + (size_t)Q * sizeof(int), 256);
   w.stats = off; off = align_up(off + CFL_RANK_NSTATS * sizeof(unsigned long long), 256);
+  if (src) {     // Q*d centred vectors and Q norms always fit the forward pc / qpar regions; the query image of sqt
+                 // vectors per tile fits the forward one unless Q is small against the tile (then it goes behind stats)
+    const int sqt = rank_tc_qt(K, d, true);
+    const int snqt = sqt > 0 ? (int)((Q + sqt - 1) / sqt) : 0;
+    const size_t sbytes = (size_t)snqt * qimg_tile_bytes(dpad, sqt);
+    if (sbytes > (size_t)nqt * qimg_tile_bytes(dpad, K * qt)) {
+      off = align_up(off, 1024);
+      w.qimg = off;  off = align_up(off + sbytes, 256);
+    }
+  }
   w.total = off + 1024;
   return w;
 }
 
-template <int K>
+// The fix kernel stages the slice's query tile (K*d floats per query; SRC: d) and, forward, one d-float row per thread.
+__host__ inline size_t fix_smem_bytes(bool src, int K, int d, int qt) {
+  return ((size_t)qt * ((src ? 1 : K) * d + 1) + (src ? 0 : (size_t)FX_THREADS * (d + 1))) * sizeof(float);
+}
+
+template <int K, bool SRC>
 static int rank_tc_launch(const RtArgs& a, const float* Pq, int64_t ldq, const float* E, int64_t lde,
                           unsigned long long* stats, cudaStream_t cs) {
-  const size_t smem = rt_layout(K, a.qt, a.dpad).g.total + 1024;
-  CFL_SMEM_LIMIT(rank_count_umma_kernel<K>, smem);
-  dim3 grid((unsigned)a.parts, (unsigned)a.nqt);
-  rank_count_umma_kernel<K><<<grid, GP_THREADS, smem, cs>>>(a);
+  auto kern = SRC ? rank_count_src_umma_kernel<K> : rank_count_umma_kernel<K>;
+  auto fix = SRC ? rank_fix_src_kernel<K> : rank_fix_kernel<K>;
+  const size_t smem = rt_layout<SRC>(K, a.qt, a.dpad).g.total + 1024;
+  CFL_SMEM_LIMIT(kern, smem);
+  kern<<<dim3((unsigned)a.parts, (unsigned)a.nqt), GP_THREADS, smem, cs>>>(a);
   CFL_LAUNCH_CHECK();
-  const size_t fx_smem = ((size_t)a.qt * (K * a.d + 1) + (size_t)FX_THREADS * (a.d + 1)) * sizeof(float);
-  CFL_SMEM_LIMIT(rank_fix_kernel<K>, fx_smem);
-  rank_fix_kernel<K><<<dim3(FX_BLOCKS, (unsigned)(a.parts * a.nqt)), FX_THREADS, fx_smem, cs>>>(
+  const size_t fx_smem = fix_smem_bytes(SRC, K, a.d, a.qt);
+  CFL_SMEM_LIMIT(fix, fx_smem);
+  fix<<<dim3(FX_BLOCKS, (unsigned)(a.parts * a.nqt)), FX_THREADS, fx_smem, cs>>>(
       a.recs, a.rec_n, a.rec_slice, Pq, ldq, E, lde, a.N, a.Q, a.d, a.qt, a.parts, a.thr, a.J, a.j0, a.only, a.counts, stats);
   CFL_LAUNCH_CHECK();
   return CFL_OK;
@@ -538,19 +641,22 @@ static int rank_tc_launch(const RtArgs& a, const float* Pq, int64_t ldq, const f
 
 // Query prep shared by the counting and the emitting pass: centred prototypes, soft-min and plane-bound blocks, the
 // packed query image, the grid, the record list (cleared flags) and the band constants.
-static int rank_tc_prepare(const char* what, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const void* image,
-                           int64_t N, const float* mu, void* ws, const RtWs& w, RtArgs& a, cudaStream_t cs) {
-  const int qt = rank_tc_qt(K, d);
-  CFL_REQUIRE(qt > 0 && score_umma_supported(K, d), CFL_ERR_UNSUPPORTED, "%s: shape K=%d d=%d has no tcgen05 tiling",
-              what, K, d);
+// src (pcd_source): the source-catalog call's prep (centred query vectors, |e_q - mu|^2, a query image with K = 1).
+static int rank_tc_prepare(const char* what, bool src, const float* Pq, int64_t Q, int K, int d, int64_t ldq,
+                           const void* image, int64_t N, const float* mu, void* ws, const RtWs& w, RtArgs& a,
+                           cudaStream_t cs) {
+  const int qt = rank_tc_qt(K, d, src);
+  CFL_REQUIRE(qt > 0 && (src || score_umma_supported(K, d)), CFL_ERR_UNSUPPORTED,
+              "%s: shape K=%d d=%d has no tcgen05 tiling", what, K, d);
   char* base = (char*)ws;
   float* Pc = (float*)(base + w.pc);
   float* qpar = (float*)(base + w.qpar);
-  float* qplane = qpar + (size_t)Q * qpar_stride(K);
-  int st = score_prep_queries_launch(Pq, Q, K, d, ldq, mu, Pc, qpar, qplane, cs);
+  float* qplane = src ? nullptr : qpar + (size_t)Q * qpar_stride(K);
+  int st = src ? score_prep_source_queries_launch(Pq, Q, d, ldq, mu, Pc, qpar, cs)
+               : score_prep_queries_launch(Pq, Q, K, d, ldq, mu, Pc, qpar, qplane, cs);
   if (st != CFL_OK) return st;
   ScoreArgs sa = {};
-  sa.K = K; sa.d = d; sa.Q = Q; sa.Pc = Pc;
+  sa.K = K; sa.d = d; sa.Q = Q; sa.Pc = Pc; sa.src = src;
   sa.plan.qt = qt; sa.plan.nqt = (int)((Q + qt - 1) / qt); sa.plan.dpad = (d + 7) / 8 * 8;
   st = score_umma_pack_queries(sa, base + w.qimg, cs);
   if (st != CFL_OK) return st;
@@ -564,8 +670,13 @@ static int rank_tc_prepare(const char* what, const float* Pq, int64_t Q, int K, 
   if (parts < 1) parts = 1;
   if (parts > a.tiles) parts = a.tiles;
   a.parts = (int)parts;
-  a.qpar = qpar; a.qplane = qplane; a.qimg = base + w.qimg; a.cimg = image;
-  a.e2 = catalog_view(image, N, d).e2;
+  a.qpar = qpar; a.qplane = qplane; a.qimg = base + w.qimg;
+  if (src) {
+    const SourceCatalogView v = source_catalog_view(image, N, K, d);
+    a.cimg = v.blocks; a.e2 = v.rowpar;
+  } else {
+    a.cimg = image; a.e2 = catalog_view(image, N, d).e2;
+  }
   CFL_REQUIRE((int64_t)a.parts * a.nqt <= 4096, CFL_ERR_UNSUPPORTED, "%s: Q=%lld needs more than 4096 CTAs", what,
               (long long)Q);
   a.recs = (uint4*)(base + w.recs); a.rec_slice = rank_tc_rec_cap(Q, N) / (unsigned int)(a.parts * a.nqt);
@@ -584,38 +695,46 @@ __global__ void within_reset_flagged_kernel(const int* __restrict__ only, int64_
   atomicAdd(&stats[3], 1ull);
 }
 
-template <int K>
+template <int K, bool SRC>
 static int within_tc_launch(const RtArgs& a, const float* Pq, int64_t ldq, const float* E, int64_t lde,
                             unsigned long long* stats, cudaStream_t cs) {
-  const size_t smem = rt_layout(K, a.qt, a.dpad).g.total + 1024;
-  CFL_SMEM_LIMIT(within_emit_umma_kernel<K>, smem);
-  within_emit_umma_kernel<K><<<dim3((unsigned)a.parts, (unsigned)a.nqt), GP_THREADS, smem, cs>>>(a);
+  auto kern = SRC ? within_emit_src_umma_kernel<K> : within_emit_umma_kernel<K>;
+  auto fix = SRC ? within_fix_src_kernel<K> : within_fix_kernel<K>;
+  const size_t smem = rt_layout<SRC>(K, a.qt, a.dpad).g.total + 1024;
+  CFL_SMEM_LIMIT(kern, smem);
+  kern<<<dim3((unsigned)a.parts, (unsigned)a.nqt), GP_THREADS, smem, cs>>>(a);
   CFL_LAUNCH_CHECK();
-  const size_t fx_smem = ((size_t)a.qt * (K * a.d + 1) + (size_t)FX_THREADS * (a.d + 1)) * sizeof(float);
-  CFL_SMEM_LIMIT(within_fix_kernel<K>, fx_smem);
-  within_fix_kernel<K><<<dim3(FX_BLOCKS, (unsigned)(a.parts * a.nqt)), FX_THREADS, fx_smem, cs>>>(
+  const size_t fx_smem = fix_smem_bytes(SRC, K, a.d, a.qt);
+  CFL_SMEM_LIMIT(fix, fx_smem);
+  fix<<<dim3(FX_BLOCKS, (unsigned)(a.parts * a.nqt)), FX_THREADS, fx_smem, cs>>>(
       a.recs, a.rec_n, a.rec_slice, Pq, ldq, E, lde, a.N, a.Q, a.d, a.qt, a.parts, a.thr, a.only, stats, a.offsets,
       a.cursor, a.out);
   CFL_LAUNCH_CHECK();
   return CFL_OK;
 }
 
-size_t within_tc_workspace_bytes(int64_t Q, int K, int d, int64_t N) { return rank_tc_ws(Q, K, d, N).total; }
+size_t within_tc_workspace_bytes(int64_t Q, int K, int d, int64_t N, bool src) {
+  return rank_tc_ws(Q, K, d, N, src).total;
+}
 
-// Emitting pass of cfl_score_within on the tensor cores (pcd / siamese): sure rows straight from the scoring epilogue,
+// Emitting pass of cfl_score_within on the tensor cores (pcd / siamese / pcd_source): sure rows straight from the scoring epilogue,
 // band rows after the direct-form check, queries whose records overflowed the list re-emitted from scratch on the
 // CUDA cores.  cursor[Q] must be zero; stats as CFL_WITHIN_NSTATS.
 int within_tc_emit(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* E, const void* image,
                    int64_t N, int64_t lde, const float* mu, const float* radius, const int64_t* offsets,
                    unsigned int* cursor, int64_t* out, void* ws, unsigned long long* stats, cudaStream_t cs) {
-  const RtWs w = rank_tc_ws(Q, K, d, N);
+  const bool src = mode == CFL_PCD_SOURCE;
+  const RtWs w = rank_tc_ws(Q, K, d, N, src);
   RtArgs a = {};
-  int st = rank_tc_prepare("score_within", Pq, Q, K, d, ldq, image, N, mu, ws, w, a, cs);
+  int st = rank_tc_prepare("score_within", src, Pq, Q, K, d, ldq, image, N, mu, ws, w, a, cs);
   if (st != CFL_OK) return st;
   a.J = 1; a.j0 = 0; a.thr = radius;
   a.offsets = offsets; a.cursor = cursor; a.out = out;
   CFL_CUDA(cudaMemsetAsync(a.rec_n, 0, 4096 * sizeof(unsigned int), cs));
-  st = with_k(K, [&](auto KC) { return within_tc_launch<KC>(a, Pq, ldq, E, lde, stats, cs); });
+  st = with_k(K, [&](auto KC) {
+    return src ? within_tc_launch<KC, true>(a, Pq, ldq, E, lde, stats, cs)
+               : within_tc_launch<KC, false>(a, Pq, ldq, E, lde, stats, cs);
+  });
   if (st != CFL_OK) return st;
   within_reset_flagged_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, cs>>>(a.only, Q, cursor, stats);
   CFL_LAUNCH_CHECK();
@@ -633,32 +752,40 @@ size_t cfl_rank_counts_packed_workspace_bytes(int64_t Q, int K, int d, int64_t N
   return rank_tc_ws(Q, K, d, N).total;
 }
 
+size_t cfl_rank_counts_packed_source_workspace_bytes(int64_t Q, int K, int d, int64_t N) {
+  if (Q <= 0 || N <= 0 || K < 1 || K > CFL_MAX_K || d < 1 || d > 128) return 4096;
+  return rank_tc_ws(Q, K, d, N, true).total;
+}
+
 int cfl_rank_counts_packed(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* E,
                            const void* image, int64_t N, int64_t lde, const float* mu, const float* pos_dist, int J,
                            int64_t* counts, void* ws, size_t ws_bytes, void* stream) {
   int st = device_check();
   if (st != CFL_OK) return st;
-  CFL_REQUIRE(mode == CFL_PCD || mode == CFL_SIAMESE, CFL_ERR_UNSUPPORTED,
-              "rank_counts_packed: mode %d not supported (pcd, siamese)", mode);
+  CFL_REQUIRE(mode == CFL_PCD || mode == CFL_SIAMESE || mode == CFL_PCD_SOURCE, CFL_ERR_UNSUPPORTED,
+              "rank_counts_packed: mode %d not supported (pcd, siamese, pcd_source)", mode);
+  const bool src = mode == CFL_PCD_SOURCE;
   CFL_REQUIRE(mode != CFL_SIAMESE || K == 1, CFL_ERR_INVALID, "rank_counts_packed: siamese needs K=1");
   CFL_REQUIRE(K >= 1 && K <= CFL_MAX_K, CFL_ERR_UNSUPPORTED, "rank_counts_packed: K=%d outside [1,%d]", K, CFL_MAX_K);
   CFL_REQUIRE(d >= 1 && d <= 128, CFL_ERR_UNSUPPORTED, "rank_counts_packed: d=%d outside [1,128]", d);
   CFL_REQUIRE(J >= 1 && J <= CFL_MAX_RANK_J, CFL_ERR_UNSUPPORTED, "rank_counts_packed: J=%d outside [1,%d]", J, CFL_MAX_RANK_J);
   CFL_REQUIRE(Q >= 0 && N >= 0 && N < ((int64_t)1 << 32) && Q < ((int64_t)1 << 31), CFL_ERR_INVALID, "rank_counts_packed: bad Q/N");
-  CFL_REQUIRE(ldq >= (int64_t)K * d && lde >= d, CFL_ERR_INVALID, "rank_counts_packed: leading dimension too small");
+  CFL_REQUIRE(ldq >= (src ? d : (int64_t)K * d) && lde >= (src ? (int64_t)K * d : d), CFL_ERR_INVALID,
+              "rank_counts_packed: leading dimension too small");
   if (Q == 0) return CFL_OK;
   CFL_REQUIRE(Pq && pos_dist && counts, CFL_ERR_INVALID, "rank_counts_packed: NULL argument");
   cudaStream_t cs = (cudaStream_t)stream;
   CFL_CUDA(cudaMemsetAsync(counts, 0, (size_t)Q * J * 2 * sizeof(int64_t), cs));
   if (N == 0) return CFL_OK;
   CFL_REQUIRE(E && image, CFL_ERR_INVALID, "rank_counts_packed: NULL catalog / image");
-  CFL_REQUIRE(rank_tc_qt(K, d) > 0 && score_umma_supported(K, d), CFL_ERR_UNSUPPORTED,
+  CFL_REQUIRE(!src || ((uintptr_t)image & 1023u) == 0, CFL_ERR_INVALID, "rank_counts_packed: image must be 1024-byte aligned");
+  CFL_REQUIRE(rank_tc_qt(K, d, src) > 0 && (src || score_umma_supported(K, d)), CFL_ERR_UNSUPPORTED,
               "rank_counts_packed: shape K=%d d=%d has no tcgen05 tiling", K, d);
-  const RtWs w = rank_tc_ws(Q, K, d, N);
+  const RtWs w = rank_tc_ws(Q, K, d, N, src);
   CFL_REQUIRE(ws && ws_bytes >= w.total, CFL_ERR_WORKSPACE, "rank_counts_packed: workspace too small (%zu < %zu)",
               ws_bytes, w.total);
   RtArgs a = {};
-  st = rank_tc_prepare("rank_counts_packed", Pq, Q, K, d, ldq, image, N, mu, ws, w, a, cs);
+  st = rank_tc_prepare("rank_counts_packed", src, Pq, Q, K, d, ldq, image, N, mu, ws, w, a, cs);
   if (st != CFL_OK) return st;
   a.J = J;
   a.thr = pos_dist; a.counts = (unsigned long long*)counts;
@@ -668,7 +795,10 @@ int cfl_rank_counts_packed(int mode, const float* Pq, int64_t Q, int K, int d, i
   for (int j0 = 0; j0 < J; j0 += RT_JC) {
     a.j0 = j0;
     CFL_CUDA(cudaMemsetAsync(a.rec_n, 0, 4096 * sizeof(unsigned int), cs));
-    st = with_k(K, [&](auto KC) { return rank_tc_launch<KC>(a, Pq, ldq, E, lde, stats, cs); });
+    st = with_k(K, [&](auto KC) {
+      return src ? rank_tc_launch<KC, true>(a, Pq, ldq, E, lde, stats, cs)
+                 : rank_tc_launch<KC, false>(a, Pq, ldq, E, lde, stats, cs);
+    });
     if (st != CFL_OK) return st;
   }
   timer_record(1, cs);

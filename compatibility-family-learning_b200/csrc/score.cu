@@ -172,6 +172,13 @@ __global__ void prep_source_queries_kernel(const float* __restrict__ Eq, int64_t
   if (lane == 0) e2q[q] = acc;
 }
 
+int score_prep_source_queries_launch(const float* Eq, int64_t Q, int d, int64_t ldq, const float* mu, float* Ec,
+                                     float* e2q, cudaStream_t st) {
+  prep_source_queries_kernel<<<(unsigned)((Q + 3) / 4), 128, 0, st>>>(Eq, Q, d, ldq, mu, Ec, e2q);
+  CFL_LAUNCH_CHECK();
+  return CFL_OK;
+}
+
 // ---- CUDA-core scoring kernel ---------------------------------------------------------------
 template <int K>
 __global__ void __launch_bounds__(SIMT_THREADS)
@@ -1401,8 +1408,8 @@ static int score_topk_source_impl(const float* Eq, int64_t ldq, int64_t Q, int K
   if (N == 0) {
     CFL_CUDA(cudaMemsetAsync(a.counts, 0, (size_t)plan.parts * Q * sizeof(int), cs));
   } else {
-    prep_source_queries_kernel<<<(unsigned)((Q + 3) / 4), 128, 0, cs>>>(Eq, Q, d, ldq, mu, (float*)a.Pc, (float*)a.qpar);
-    CFL_LAUNCH_CHECK();
+    st = score_prep_source_queries_launch(Eq, Q, d, ldq, mu, (float*)a.Pc, (float*)a.qpar, cs);
+    if (st != CFL_OK) return st;
     const SourceCatalogView v = source_catalog_view(image, N, K, d);
     a.cimg = v.blocks; a.e2 = v.rowpar;
     st = score_umma_pack_queries(a, c.base + c.ws.qimg, cs);

@@ -143,6 +143,9 @@ int score_src_qt(int K, int d);
 // query prep shared with the rank-count path (rank_counts_tc.cu): centred prototypes, soft-min and plane-bound blocks
 int score_prep_queries_launch(const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* mu, float* Pc,
                               float* qpar, float* qplane, cudaStream_t st);
+// the same for the source-catalog direction: centred query vectors Ec [Q,d] and |e_q - mu|^2
+int score_prep_source_queries_launch(const float* Eq, int64_t Q, int d, int64_t ldq, const float* mu, float* Ec,
+                                     float* e2q, cudaStream_t st);
 // rank_counts.cu: the CUDA-core rank count restricted to the queries flagged in only[Q] (adds into counts)
 int rank_counts_only_launch(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* E, int64_t N,
                             int64_t lde, const float* pos_dist, int J, unsigned long long* counts, const int* only,
@@ -152,7 +155,7 @@ int rank_counts_only_launch(int mode, const float* Pq, int64_t Q, int K, int d, 
 int within_emit_launch(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* Wq, const float* E,
                        int64_t N, int64_t lde, const float* radius, const int64_t* offsets, unsigned int* cursor,
                        int64_t* out, const int* only, cudaStream_t st);
-size_t within_tc_workspace_bytes(int64_t Q, int K, int d, int64_t N);
+size_t within_tc_workspace_bytes(int64_t Q, int K, int d, int64_t N, bool src);
 int within_tc_emit(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* E, const void* image,
                    int64_t N, int64_t lde, const float* mu, const float* radius, const int64_t* offsets,
                    unsigned int* cursor, int64_t* out, void* ws, unsigned long long* stats, cudaStream_t st);
@@ -299,14 +302,14 @@ __device__ __forceinline__ void softmin_pair(const float (&gA)[K], const float (
   softmin_pair2<K>(gA, gB, pk2(e2, e2), qp2, dA, dB);
 }
 
-// softmin_pair that also returns V = sum_k s_k |p_k|^2 - |sum_k s_k p_k|^2, the spread of the prototypes under the
+// softmin_pair2 that also returns V = sum_k s_k |p_k|^2 - |sum_k s_k p_k|^2, the spread of the prototypes under the
 // soft-min weights: d dist / d(exponent k) = s_k * (-2 (e - m).(p_k - m)), so an error du on the exponents moves dist by
-// at most 2 sqrt(dist * V) |du| -- the sensitivity term of the rank-count rounding band (rank_counts_tc.cu).
+// at most 2 sqrt(dist * V) |du| -- the sensitivity term of the rank-count rounding band (rank_counts_tc.cu).  e2p as
+// softmin_pair2: pk2(e2, e2) for a catalog row of embeddings, the two queries' |e|^2 for a source catalog.
 template <int K>
-__device__ __forceinline__ void softmin_pair_var(const float (&gA)[K], const float (&gB)[K], float e2,
+__device__ __forceinline__ void softmin_pair_var(const float (&gA)[K], const float (&gB)[K], f2_t e2p,
                                                  const f2_t* __restrict__ qp2, float& dA, float& dB, float& vA, float& vB) {
   const f2_t C2 = pk2(2.0f * CFL_LOG2E, 2.0f * CFL_LOG2E);
-  const f2_t e2p = pk2(e2, e2);
   f2_t g[K], a[K];
 #pragma unroll
   for (int k = 0; k < K; ++k) { g[k] = pk2(gA[k], gB[k]); a[k] = fma2(C2, g[k], qp2[k]); }

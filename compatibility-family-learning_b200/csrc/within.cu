@@ -32,14 +32,17 @@ __device__ __forceinline__ int64_t seg_of(const int64_t* __restrict__ offsets, i
   return lo;
 }
 
-template <int K, bool MONO>
-__global__ void __launch_bounds__(WR_THREADS)
-within_rescore_kernel(const float* __restrict__ Pq, int64_t ldq, const float* __restrict__ Wq,
-                      const float* __restrict__ E, int64_t lde, int64_t N, int d, int64_t Q,
-                      const int64_t* __restrict__ offsets, const unsigned int* __restrict__ cursor,
-                      int64_t* __restrict__ out) {
+// SRC (pcd_source / monomer_source): the direct form with the roles swapped, the accessors of merge_rescore_src_kernel
+// (score.cu) and mono_rescore_src_kernel (score_monomer_tc.cu), so the bits are those cfl_score_topk_source /
+// _monomer_source report.  STAGED: the warp gathers its rows into shared memory (every forward call; pcd_source while
+// 128 rows of K*d floats fit); otherwise each thread reads its row in place (monomer_source: d + K floats).
+template <int K, bool MONO, bool SRC, bool STAGED>
+__device__ __forceinline__ void within_rescore_body(const float* __restrict__ Pq, int64_t ldq, const float* __restrict__ Wq,
+                                                    const float* __restrict__ E, int64_t lde, int64_t N, int d, int64_t Q,
+                                                    const int64_t* __restrict__ offsets,
+                                                    const unsigned int* __restrict__ cursor, int64_t* __restrict__ out) {
   extern __shared__ __align__(16) float wr_smem[];
-  const int ew = MONO ? K * d : d, lder = ew + 1;
+  const int ew = MONO || SRC ? K * d : d, lder = ew + 1;
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const int64_t begin = offsets[0], end = offsets[Q];
   for (int64_t c0 = begin + (int64_t)blockIdx.x * WR_THREADS; c0 < end; c0 += (int64_t)gridDim.x * WR_THREADS) {
@@ -54,6 +57,7 @@ within_rescore_kernel(const float* __restrict__ Pq, int64_t ldq, const float* __
         live = row >= 0 && row < N;
       }
     }
+    if constexpr (STAGED) {
     __syncwarp();
     for (int rr = 0; rr < 32; ++rr) {                      // the warp gathers its 32 rows with coalesced loads
       const int64_t rw = __shfl_sync(0xffffffffu, row, rr);
@@ -62,13 +66,20 @@ within_rescore_kernel(const float* __restrict__ Pq, int64_t ldq, const float* __
       for (int j = lane; j < ew; j += 32) dst[j] = E[rw * lde + j];
     }
     __syncwarp();
+    }
     if (i >= end) continue;
     unsigned long long key = CFL_KEY_INF;
     if (live) {
-      const float* ev = wr_smem + tid * lder;
+      const float* ev = STAGED ? wr_smem + tid * lder : E + row * lde;
       const float* qv = Pq + q * ldq;
       float dist;
-      if (MONO) {
+      if (SRC && MONO) {                                   // e = the query's prototypes, a / w = the row's
+        const float* wv = Wq + row * K;
+        dist = monomer_direct<K>([&](int k, int j) { return qv[k * d + j]; }, [&](int j) { return ev[j]; },
+                                 [&](int k) { return wv[k]; }, d);
+      } else if (SRC) {                                    // e = the query row, p = the row's prototypes (shared when STAGED)
+        dist = pcd_direct<K, 1>([&](int j) { return qv[j]; }, [&](int k, int j) { return ev[k * d + j]; }, d);
+      } else if (MONO) {
         const float* wv = Wq + q * K;
         dist = monomer_direct<K>([&](int k, int j) { return ev[k * d + j]; }, [&](int j) { return qv[j]; },
                                  [&](int k) { return wv[k]; }, d);
@@ -79,6 +90,24 @@ within_rescore_kernel(const float* __restrict__ Pq, int64_t ldq, const float* __
     }
     out[i] = (int64_t)key;
   }
+}
+
+template <int K, bool MONO>
+__global__ void __launch_bounds__(WR_THREADS)
+within_rescore_kernel(const float* __restrict__ Pq, int64_t ldq, const float* __restrict__ Wq,
+                      const float* __restrict__ E, int64_t lde, int64_t N, int d, int64_t Q,
+                      const int64_t* __restrict__ offsets, const unsigned int* __restrict__ cursor,
+                      int64_t* __restrict__ out) {
+  within_rescore_body<K, MONO, false, true>(Pq, ldq, Wq, E, lde, N, d, Q, offsets, cursor, out);
+}
+
+template <int K, bool MONO, bool STAGED>
+__global__ void __launch_bounds__(WR_THREADS)
+within_rescore_src_kernel(const float* __restrict__ Pq, int64_t ldq, const float* __restrict__ Wq,
+                          const float* __restrict__ E, int64_t lde, int64_t N, int d, int64_t Q,
+                          const int64_t* __restrict__ offsets, const unsigned int* __restrict__ cursor,
+                          int64_t* __restrict__ out) {
+  within_rescore_body<K, MONO, true, STAGED>(Pq, ldq, Wq, E, lde, N, d, Q, offsets, cursor, out);
 }
 
 // Ascending sort of s[0, n) by NT threads; positions n .. P-1 (P = next power of two) act as +inf keys that are never
@@ -189,21 +218,35 @@ static WsLayout within_ws(int mode, int64_t Q, int K, int d, int64_t N) {
   w.stats = off;  off = align_up(off + CFL_WITHIN_NSTATS * sizeof(unsigned long long), 256);
   w.cursor = off; off = align_up(off + (size_t)(Q > 0 ? Q : 0) * sizeof(unsigned int), 1024);
   w.tc = off;
-  if (mode != CFL_MONOMER && Q > 0 && N > 0 && score_umma_supported(K, d)) off += within_tc_workspace_bytes(Q, K, d, N);
+  if (mode == CFL_PCD_SOURCE && Q > 0 && N > 0) off += within_tc_workspace_bytes(Q, K, d, N, true);
+  else if ((mode == CFL_PCD || mode == CFL_SIAMESE) && Q > 0 && N > 0 && score_umma_supported(K, d))
+    off += within_tc_workspace_bytes(Q, K, d, N, false);
   w.total = off;
   return w;
 }
 
-template <int K, bool MONO>
+template <int K, bool MONO, bool SRC>
 static int within_rescore_launch(const float* Pq, int64_t ldq, const float* Wq, const float* E, int64_t lde, int64_t N,
                                  int d, int64_t Q, const int64_t* offsets, const unsigned int* cursor, int64_t* out,
                                  cudaStream_t cs) {
-  const size_t smem = (size_t)WR_THREADS * ((MONO ? K * d : d) + 1) * sizeof(float);
-  CFL_SMEM_LIMIT((within_rescore_kernel<K, MONO>), smem);
   int sms = sm_count();
   if (sms <= 0) sms = 148;
-  within_rescore_kernel<K, MONO><<<(unsigned)(sms * 8), WR_THREADS, smem, cs>>>(Pq, ldq, Wq, E, lde, N, d, Q, offsets,
-                                                                             cursor, out);
+  if constexpr (SRC) {
+    const size_t smem = (size_t)WR_THREADS * (K * d + 1) * sizeof(float);
+    if (!MONO && smem <= 200 * 1024) {
+      CFL_SMEM_LIMIT((within_rescore_src_kernel<K, false, true>), smem);
+      within_rescore_src_kernel<K, false, true><<<(unsigned)(sms * 8), WR_THREADS, smem, cs>>>(Pq, ldq, Wq, E, lde, N, d,
+                                                                                             Q, offsets, cursor, out);
+    } else {
+      within_rescore_src_kernel<K, MONO, false><<<(unsigned)(sms * 8), WR_THREADS, 0, cs>>>(Pq, ldq, Wq, E, lde, N, d, Q,
+                                                                                          offsets, cursor, out);
+    }
+  } else {
+    const size_t smem = (size_t)WR_THREADS * ((MONO ? K * d : d) + 1) * sizeof(float);
+    CFL_SMEM_LIMIT((within_rescore_kernel<K, MONO>), smem);
+    within_rescore_kernel<K, MONO><<<(unsigned)(sms * 8), WR_THREADS, smem, cs>>>(Pq, ldq, Wq, E, lde, N, d, Q, offsets,
+                                                                               cursor, out);
+  }
   CFL_LAUNCH_CHECK();
   return CFL_OK;
 }
@@ -225,21 +268,26 @@ int cfl_score_within(int mode, const float* Pq, int64_t Q, int K, int d, int64_t
                      size_t ws_bytes, void* stream) {
   int st = device_check();
   if (st != CFL_OK) return st;
-  CFL_REQUIRE(mode == CFL_PCD || mode == CFL_SIAMESE || mode == CFL_MONOMER, CFL_ERR_INVALID, "score_within: bad mode %d",
-              mode);
+  CFL_REQUIRE(mode >= CFL_PCD && mode <= CFL_MONOMER_SOURCE, CFL_ERR_INVALID, "score_within: bad mode %d", mode);
   CFL_REQUIRE(mode != CFL_SIAMESE || K == 1, CFL_ERR_INVALID, "score_within: siamese needs K=1");
   CFL_REQUIRE(K >= 1 && K <= CFL_MAX_K, CFL_ERR_UNSUPPORTED, "score_within: K=%d outside [1,%d]", K, CFL_MAX_K);
   CFL_REQUIRE(d >= 1 && d <= 128, CFL_ERR_UNSUPPORTED, "score_within: d=%d outside [1,128]", d);
   CFL_REQUIRE(Q >= 0 && N >= 0 && N < ((int64_t)1 << 32) && Q < ((int64_t)1 << 31), CFL_ERR_INVALID,
               "score_within: bad Q/N");
-  const bool mono = mode == CFL_MONOMER;
-  CFL_REQUIRE(ldq >= (mono ? d : (int64_t)K * d) && lde >= (mono ? (int64_t)K * d : d), CFL_ERR_INVALID,
+  const bool mono = mode == CFL_MONOMER, msrc = mode == CFL_MONOMER_SOURCE, src = mode == CFL_PCD_SOURCE || msrc;
+  // per query: K*d floats (pcd, monomer_source) or d (monomer, pcd_source); per row: the other one
+  const bool qd = mono || mode == CFL_PCD_SOURCE;
+  CFL_REQUIRE(ldq >= (qd ? d : (int64_t)K * d) && lde >= (qd ? (int64_t)K * d : d), CFL_ERR_INVALID,
               "score_within: leading dimension too small");
-  CFL_REQUIRE(!mono || image == nullptr, CFL_ERR_UNSUPPORTED, "score_within: monomer runs on the CUDA cores (image NULL)");
+  CFL_REQUIRE(!(mono || msrc) || image == nullptr, CFL_ERR_UNSUPPORTED,
+              "score_within: monomer runs on the CUDA cores (image NULL)");
   CFL_REQUIRE(!mono || (size_t)(128 * (K * d + 1) + 9 * d + 8 * K + 72) * 4 <= 200 * 1024, CFL_ERR_UNSUPPORTED,
               "score_within: K*d = %d too large for the monomer tile", K * d);
+  CFL_REQUIRE(mode != CFL_PCD_SOURCE || ((uintptr_t)image & 1023u) == 0, CFL_ERR_INVALID,
+              "score_within: image must be 1024-byte aligned");
   if (Q == 0) return CFL_OK;
-  CFL_REQUIRE(Pq && radius && offsets && (!mono || Wq) && (N == 0 || E), CFL_ERR_INVALID, "score_within: NULL argument");
+  CFL_REQUIRE(Pq && radius && offsets && (!(mono || msrc) || Wq) && (N == 0 || E), CFL_ERR_INVALID,
+              "score_within: NULL argument");
   const WsLayout w = within_ws(mode, Q, K, d, N);
   CFL_REQUIRE(ws && ws_bytes >= w.total, CFL_ERR_WORKSPACE, "score_within: workspace too small (%zu < %zu)", ws_bytes,
               w.total);
@@ -260,8 +308,10 @@ int cfl_score_within(int mode, const float* Pq, int64_t Q, int K, int d, int64_t
     if (st != CFL_OK) return st;
 #define CFL_WR_CASE(KK)                                                                                              \
   case KK:                                                                                                           \
-    st = mono ? within_rescore_launch<KK, true>(Pq, ldq, Wq, E, lde, N, d, Q, offsets, cursor, out_idx, cs)          \
-              : within_rescore_launch<KK, false>(Pq, ldq, Wq, E, lde, N, d, Q, offsets, cursor, out_idx, cs);         \
+    st = src ? (msrc ? within_rescore_launch<KK, true, true>(Pq, ldq, Wq, E, lde, N, d, Q, offsets, cursor, out_idx, cs) \
+                     : within_rescore_launch<KK, false, true>(Pq, ldq, Wq, E, lde, N, d, Q, offsets, cursor, out_idx, cs)) \
+             : mono ? within_rescore_launch<KK, true, false>(Pq, ldq, Wq, E, lde, N, d, Q, offsets, cursor, out_idx, cs)  \
+                    : within_rescore_launch<KK, false, false>(Pq, ldq, Wq, E, lde, N, d, Q, offsets, cursor, out_idx, cs); \
     break;
     switch (K) {
       CFL_WR_CASE(1) CFL_WR_CASE(2) CFL_WR_CASE(3) CFL_WR_CASE(4)

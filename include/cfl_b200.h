@@ -37,8 +37,11 @@ typedef enum {
   CFL_ERR_DEVICE = -5       /* no sm_100 device                               */
 } cfl_status;
 
-/* dist_type -- cfl/models/base.py:109 (monomer), :119 (siamese), :125 (pcd*) */
-typedef enum { CFL_PCD = 0, CFL_MONOMER = 1, CFL_SIAMESE = 2 } cfl_mode;
+/* dist_type -- cfl/models/base.py:109 (monomer), :119 (siamese), :125 (pcd*).  CFL_PCD_SOURCE and CFL_MONOMER_SOURCE
+ * are the same distances with the roles swapped (queries = TARGET items, catalog = SOURCE items); only the
+ * rank-count and range-query entry points take them (cfl_pair_dist_rows, cfl_rank_counts, cfl_rank_counts_packed,
+ * cfl_score_within).  The paired-loss and top-k entry points reject every mode above CFL_SIAMESE. */
+typedef enum { CFL_PCD = 0, CFL_MONOMER = 1, CFL_SIAMESE = 2, CFL_PCD_SOURCE = 3, CFL_MONOMER_SOURCE = 4 } cfl_mode;
 /* act_type -- cfl/models/cfl.py:579-586 (+ lrelu, cfl/ops.py:10, for hidden layers) */
 typedef enum { CFL_ACT_LINEAR = 0, CFL_ACT_TANH = 1, CFL_ACT_SIGMOID = 2, CFL_ACT_RELU = 3,
                CFL_ACT_LRELU = 4 } cfl_act;
@@ -284,6 +287,14 @@ int cfl_auc(const float* pos_scores, int64_t n_pos, const float* neg_scores, int
  *   monomer:       Pq[Q,d] query embeddings (ldq >= d), Wq[Q,K] gate softmax, E[N,K,d] candidate
  *                  prototypes (lde >= K*d); the 128-row tile of K*d floats per row must fit one CTA's shared
  *                  memory: K*d <= ~380, else CFL_ERR_UNSUPPORTED.
+ *   pcd_source:    (CFL_PCD_SOURCE) Pq[Q,d] = the TARGET items' e0 (ldq >= d), Wq NULL, E[N,K,d] = the SOURCE items'
+ *                  prototypes (lde >= K*d); dist(q,c) = the pcd direct form with e = Pq[q], p = E[c] (the values
+ *                  cfl_score_topk_source reports).  Every K <= 8, d <= 128.
+ *   monomer_source: (CFL_MONOMER_SOURCE) Pq[Q,K,d] = the TARGET items' prototypes (ldq >= K*d), E[N,d] = the SOURCE
+ *                  items' a (lde >= d), Wq[N,K] = the SOURCE items' gate softmax: the gate argument belongs to
+ *                  whichever side is the monomer source.  dist(q,c) = sum_k Wq[c,k] |E[c] - Pq[q,k]|^2 in the
+ *                  operation order of cfl_score_topk_monomer_source.
+ * The integers, sets, bits and tie rules are the same for every mode.
  * cfl_pair_dist_rows: pos_dist[q,j] = dist(q, row pos_idx[q,j]) for the J labelled positives of each
  *   query; pos_idx is LOCAL to this shard, entries outside [0,N) (e.g. -1: positive lives on another
  *   shard, or padding) give NaN.
@@ -294,10 +305,10 @@ int cfl_auc(const float* pos_scores, int64_t n_pos, const float* neg_scores, int
  * candidates in total and the positives' own contributions removed, AUC_q = 2U_q / (2 J (n - J)).
  * ------------------------------------------------------------------------------------- */
 #define CFL_MAX_RANK_J 32
-int cfl_pair_dist_rows(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* Wq,
+int cfl_pair_dist_rows(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* Wgate,
                        const float* E, int64_t N, int64_t lde, const int64_t* pos_idx, int J,
                        float* pos_dist, void* stream);
-int cfl_rank_counts(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* Wq,
+int cfl_rank_counts(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* Wgate,
                     const float* E, int64_t N, int64_t lde, const float* pos_dist, int J,
                     int64_t* counts, void* stream);
 
@@ -312,13 +323,17 @@ int cfl_dense_rank_counts(const float* dense, int64_t Q, int64_t N, int64_t ldn,
 /* The same counts on the tensor cores, taken inside the fused scoring kernel's epilogue (no Q x N matrix anywhere):
  * image = cfl_catalog_pack of the same E / mu.  Every (row, query) Gram-form distance is classified against the
  * thresholds with a rounding band; pairs inside a band (exact ties included) are re-evaluated in the direct form of
- * cfl_pair_dist_rows, so counts == cfl_rank_counts(...) for pos_dist produced by cfl_pair_dist_rows.  pcd / siamese.
+ * cfl_pair_dist_rows, so counts == cfl_rank_counts(...) for pos_dist produced by cfl_pair_dist_rows.  pcd / siamese,
+ * and CFL_PCD_SOURCE with the operands of cfl_rank_counts and image = cfl_source_catalog_pack of the same E / mu (its
+ * workspace: cfl_rank_counts_packed_source_workspace_bytes; the forward layout, its query regions reused, so
+ * cfl_rank_counts_packed_stats reads both with the same Q, K, d, N).
  * Replaces roc_auc_score over all candidates (cfl/utils.py:267-268); see csrc/rank_counts_tc.cu.  One call takes up
  * to 4096 scoring CTAs' worth of queries (>= 131072 queries; CFL_ERR_UNSUPPORTED beyond: split the query batch).
  * cfl_rank_counts_packed_stats (synchronises the stream): out[CFL_RANK_NSTATS] = {ambiguous records, largest
  * |Gram - direct| / band in units of 2^-20, records beyond half the band, queries recounted on the CUDA cores}. */
 #define CFL_RANK_NSTATS 4
 size_t cfl_rank_counts_packed_workspace_bytes(int64_t Q, int K, int d, int64_t N);
+size_t cfl_rank_counts_packed_source_workspace_bytes(int64_t Q, int K, int d, int64_t N);
 int cfl_rank_counts_packed(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* E,
                            const void* image, int64_t N, int64_t lde, const float* mu, const float* pos_dist, int J,
                            int64_t* counts, void* ws, size_t ws_bytes, void* stream);
@@ -338,9 +353,10 @@ int cfl_rank_counts_packed_stats(int64_t Q, int K, int d, int64_t N, const void*
  * pos_dist = r (J = 1), whose verdicts are the same arithmetic -- and lays out offsets[Q + 1] (device,
  * an exclusive scan of the counts; offsets[0] may be non-zero, out_idx / out_dist are indexed by them) and
  * the outputs; cfl_score_within then fills the segments.
- *   image != NULL (pcd / siamese, cfl_catalog_pack of E / mu): rows emitted from the tensor-core scoring
- *   epilogue (3xTF32 Gram form, rounding band, direct-form check of the pairs inside it); image == NULL: the
- *   CUDA-core direct form (monomer; pcd shapes without a tcgen05 tiling).  N < 2^32; one call takes up to
+ *   image != NULL (pcd / siamese, cfl_catalog_pack of E / mu; pcd_source, cfl_source_catalog_pack of E / mu): rows
+ *   emitted from the tensor-core scoring epilogue (3xTF32 Gram form, rounding band, direct-form check of the pairs
+ *   inside it); image == NULL: the CUDA-core direct form (monomer and monomer_source, where image must be NULL; pcd
+ *   shapes without a tcgen05 tiling; pcd_source without an image).  Both routes return the same lists.  N < 2^32; one call takes up to
  *   4096 scoring CTAs' worth of queries (split larger batches).  Segments beyond 16384 rows are sorted in
  *   global memory by one CTA (correct, slower).
  * cfl_score_within_stats (synchronises the stream): out[CFL_WITHIN_NSTATS] of the last call on `ws` = {band
@@ -351,7 +367,7 @@ int cfl_rank_counts_packed_stats(int64_t Q, int K, int d, int64_t N, const void*
  * scan of the per-query sums.  The merged lists are ordered by (distance, index), independent of R. */
 #define CFL_WITHIN_NSTATS 5
 size_t cfl_score_within_workspace_bytes(int mode, int64_t Q, int K, int d, int64_t N);
-int cfl_score_within(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* Wq, const float* E,
+int cfl_score_within(int mode, const float* Pq, int64_t Q, int K, int d, int64_t ldq, const float* Wgate, const float* E,
                      const void* image, int64_t N, int64_t lde, const float* mu, const float* radius,
                      const int64_t* offsets, int64_t idx_base, int64_t* out_idx, float* out_dist, void* ws,
                      size_t ws_bytes, void* stream);
